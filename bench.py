@@ -16,6 +16,8 @@ independent, so N GPUs run N disjoint batches with no collective on the data pat
   cfg2 / e2e_model / steady_200_replays / nms_sat.cpu_baseline / box_iou   side records (single GPU only)
 
 `--impl reference` times that CPU port alone with all host threads (rank 0 only): one step = one whole frame.
+`--dump-outputs DIR` saves the fused BEV maps of the last timed step of rank 0 as DIR/fused_g<group>.npy (float32), so that
+two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -86,6 +88,32 @@ def measured_tensor_peak():
             p = json.load(f)
         return float(p.get("bf16_tflops_sustained", p.get("bf16_tflops", 1390.0))), "measured (MEASURED_PEAKS.json, sustained)"
     return 1390.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BUDGET_BYTES = 60 * 2 ** 20   # all dumped arrays together, under 64 MB with the .npy headers
+
+
+def dump_outputs(dirname, named, budget=DUMP_BUDGET_BYTES, seed=0):
+    """Writes every (name, tensor) as dirname/<name>.npy in float32.  The budget is split evenly between the tensors; one
+    with more elements than its share is saved as a 1-D sample of that many elements, taken at the sorted flat indices
+    `sample_indices(numel, share, seed)`, the same positions on every run with the same shapes."""
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    share = budget // 4 // max(1, len(named))
+    for name, t in named:
+        t = t.detach()
+        if t.numel() > share:
+            idx = torch.from_numpy(sample_indices(t.numel(), share, seed)).to(t.device)
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(dirname, f"{name}.npy"), t.float().cpu().numpy())
+
+
+def sample_indices(numel, n, seed=0):
+    """n distinct flat indices out of numel, increasing: [0, numel) is cut into n equal strata and each gives one index at
+    an offset drawn from a generator seeded with `seed` (O(n) time and memory, the whole map covered evenly)."""
+    edges = np.arange(n + 1, dtype=np.int64) * numel // n
+    offsets = (np.random.default_rng(seed).random(n) * (edges[1:] - edges[:-1])).astype(np.int64)
+    return edges[:-1] + offsets
 
 
 class ClockSampler:
@@ -350,7 +378,7 @@ def run_gpu(args):
         torch.cuda.synchronize()
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            pipe.step()
+            graph_outs = pipe.step()      # every replay rewrites these tensors
         for _ in range(3):
             graph.replay()
     run_step = graph.replay if graph is not None else pipe.step
@@ -363,11 +391,14 @@ def run_gpu(args):
     c_lo = sampler.mark()
     e0.record()
     for _ in range(args.steps):
-        run_step()
+        last_outs = run_step()
     e1.record()
     barrier()
     c_hi = sampler.mark()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        last_outs = graph_outs if graph is not None else last_outs
+        dump_outputs(args.dump_outputs, [(f"fused_g{sc['group']}", o) for sc, o in zip(wl["scales"], last_outs)])
     launches = launches_per_step * args.steps
     clocks = sampler.stop(c_lo, c_hi) if rank == 0 else None
     # the same step over a longer region (the contract's K steps are ~20 ms: one hiccup would move them)
@@ -822,7 +853,16 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the side records (cfg2 sub-record, model end to end)")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of a CUDA-graph replay")
     ap.add_argument("--bucket-size", type=float, default=None, help="K-1 bucket pitch in metres (default: config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save the fused BEV maps of the last one (rank 0) as DIR/fused_g<group>.npy, "
+                         "float32, 60 MiB in all: a map larger than its share is saved as a seeded sample (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs is not None:
+        if args.workload == "train" or args.impl == "reference":
+            ap.error("--dump-outputs saves the fused maps of the GPU fusion path; "
+                     "it cannot be used with --workload train or --impl reference")
+        if args.steps < 1:
+            ap.error("--dump-outputs needs at least one timed step (--steps >= 1)")
     if args.workload == "train":
         run_train(args)
     elif args.impl == "reference":

@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference through
-oracle/ref_shims.py) on seeded inputs.  Run in the build container only:
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from $CF_REFERENCE_DIR through
+oracle/ref_shims.py) on seeded inputs:
 
-    python oracle/gen_golden.py
+    CF_REFERENCE_DIR=<checkout of the original project> python oracle/gen_golden.py
 
 Each fixture stores the inputs and the reference's outputs; tests compare the CPU oracle (CPU suite) and
 the CUDA path (GPU suite) against them.  numpy 2.3.5 / torch 2.11 / scipy 1.18.1 (SURVEY 8c: the reference's

@@ -1,8 +1,9 @@
-"""Import the UNMODIFIED reference from /root/reference inside the build container.
+"""Import the UNMODIFIED reference from the directory named by the environment variable CF_REFERENCE_DIR
+(a checkout of the original project; it is not part of this repository).
 
-TEST INFRASTRUCTURE ONLY.  /root/reference does not exist on the GPU box, so nothing that runs
-there (``-m gpu`` tests, smoke(), bench.py) imports this module; it is used by
-oracle/gen_golden.py (fixture generation) and by CPU tests that skip when the tree is absent.
+TEST INFRASTRUCTURE ONLY.  Nothing on the product path (``-m gpu`` tests, smoke(), bench.py) imports
+this module; it is used by oracle/gen_golden.py (fixture generation) and by two CPU tests that skip
+when the reference is not available.  The fixtures it produced are stored under tests/golden/.
 
 Shims (harness-side only, the reference files are never edited or copied):
   * empty stand-ins for matplotlib / h5py / numpy-quaternion, which the container lacks and which
@@ -18,11 +19,11 @@ import os
 import sys
 import types
 
-REFERENCE_DIR = os.environ.get("CF_REFERENCE_DIR", "/root/reference")
+REFERENCE_DIR = os.environ.get("CF_REFERENCE_DIR", "")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_DIR, "separation_axis_theorem.py"))
+    return bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "separation_axis_theorem.py"))
 
 
 _loaded = {}
@@ -33,7 +34,7 @@ def load():
     if _loaded:
         return types.SimpleNamespace(**_loaded)
     if not available():
-        raise RuntimeError("reference tree not present")
+        raise RuntimeError("reference tree not present: set CF_REFERENCE_DIR to a checkout of the original project")
     for name in ("matplotlib", "matplotlib.pyplot", "h5py", "quaternion"):
         if name not in sys.modules:
             sys.modules[name] = types.ModuleType(name)

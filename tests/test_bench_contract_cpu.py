@@ -43,3 +43,39 @@ def test_reference_arm_is_silent_on_other_ranks():
 def test_train_workload_has_no_reference():
     lines = _run("--workload", "train", "--impl", "reference")
     assert len(lines) == 1 and lines[0]["impl"] == "reference" and "unavailable" in lines[0]
+
+
+def test_dump_outputs_keeps_small_maps_whole_and_samples_large_ones(tmp_path):
+    """--dump-outputs: float32 files within the budget; a tensor over its share of the budget is saved at the same seeded
+    positions on every run, so that two builds are compared value for value."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    small = torch.arange(12, dtype=torch.float64).reshape(3, 4)
+    big = torch.randn(2, 500, generator=torch.Generator().manual_seed(1))
+    budget = 2 * 100 * 4                                                   # 100 float32 values per tensor
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), [("small", small), ("big", big)], budget=budget)
+    a_small, a_big = np.load(tmp_path / "a" / "small.npy"), np.load(tmp_path / "a" / "big.npy")
+    assert a_small.dtype == a_big.dtype == np.float32
+    assert np.array_equal(a_small, small.float().numpy())
+    idx = bench.sample_indices(1000, 100)
+    assert idx.shape == (100,) and np.unique(idx).size == 100 and (np.diff(idx) > 0).all() and idx[-1] < 1000
+    assert np.array_equal(a_big, big.numpy().reshape(-1)[idx])
+    assert a_small.nbytes + a_big.nbytes <= budget
+    assert np.array_equal(np.load(tmp_path / "b" / "big.npy"), a_big)
+    # the full-size workload: five maps of up to 287 MB fit the 64 MB the option promises, .npy headers included
+    assert bench.DUMP_BUDGET_BYTES + 5 * 128 <= 64e6
+    idx = bench.sample_indices(71_680_000, 3_145_728)                      # scale 1 of configs[1]
+    assert (np.diff(idx) > 0).all() and idx[0] >= 0 and idx[-1] < 71_680_000 and idx[-1] > 71_000_000
+
+
+def test_dump_outputs_is_refused_where_it_cannot_be_honoured(tmp_path):
+    """The reference arm and the train workload compute no fused maps, and zero timed steps have no last step: asking for
+    a dump there is an error, not a run that silently writes nothing."""
+    for args in (["--impl", "reference", "--workload", "tiny"], ["--workload", "train"], ["--steps", "0"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(tmp_path / "d")],
+                           capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and "--dump-outputs" in r.stderr, (args, r.stderr[-500:])
+        assert not (tmp_path / "d").exists()

@@ -1,10 +1,10 @@
 """CPU: host-side logic -- geometry, synthetic generator, the drop-in nn.Module tree, reference parity of the
 untouched LiDAR-only path, and post-process plumbing."""
-import os
-
 import numpy as np
 import pytest
 import torch
+
+from oracle import ref_shims
 
 
 def test_scale_geometry_follows_voxel_mapping(dcf):
@@ -64,10 +64,9 @@ def test_dropin_module_tree_and_lidar_only_path(dcf):
     assert torch.allclose(cls[:, 0] + cls[:, 1], torch.ones_like(cls[:, 0]), atol=1e-5)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not ref_shims.available(), reason="needs the original project: set CF_REFERENCE_DIR to its checkout")
 def test_lidar_only_path_equals_reference_model(dcf):
     """Same weights -> same output as the reference's LidarBackboneNetwork, and its checkpoints load."""
-    from oracle import ref_shims
     ref = ref_shims.load()
     torch.manual_seed(0)
     ref_net = ref.model.LidarBackboneNetwork().eval()
