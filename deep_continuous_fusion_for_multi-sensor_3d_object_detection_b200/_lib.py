@@ -11,6 +11,7 @@ SO_PATH = os.path.join(_PKG, "libcf_b200.so")
 CSRC = os.path.join(_PKG, "csrc")
 
 MODE_FP32, MODE_BF16, MODE_SIMT, MODE_BF16_TABLES = 0, 1, 2, 3
+BWD_DETERMINISTIC = 0x100   # CF_BWD_DETERMINISTIC: OR-ed into the mode of cf_fusion_bwd
 # "bf16t" = CF_MODE_BF16_TABLES: bf16 operands AND bf16 layer-1 tables (inference only)
 MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "simt": MODE_SIMT, "bf16t": MODE_BF16_TABLES}
 MAX_K = 16
@@ -47,6 +48,10 @@ SIGNATURES = {
                                 _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp]),
     "cf_point_gather_bwd": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp,
                                       C.POINTER(C.c_float), _vp, _i32, _f32, _f32, _vp]),
+    "cf_fusion_bwd_det_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32, _i32, _i32]),
+    "cf_point_gather_bwd_det_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32]),
+    "cf_point_gather_bwd_det": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp,
+                                          C.POINTER(C.c_float), _vp, _i32, _f32, _f32, _vp, _vp]),
     "cf_voxelize_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32]),
     "cf_voxelize_project": (C.c_int, [_vp, _vp, _i32, _i32, C.POINTER(C.c_float), C.POINTER(C.c_float), _i32, _i32, _i32,
                                       C.POINTER(C.c_float), _f32, _f32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -17,6 +17,8 @@
 // stay in device memory, and every later kernel is launched for the dense upper bound and clamps itself to the count
 // (no host synchronisation; blocks beyond the count exit at once).  All arithmetic is fp32 on CUDA cores; reductions
 // over rows use split accumulation + atomics, so gradients are reproducible to rounding, not bit for bit.
+// With CF_BWD_DETERMINISTIC in `mode` the same kernels run with ordered list positions, per-split partials instead of
+// atomics (summed in split order by cf_bwd_det.cu) and a gather for dT: gradients are then bit-identical run to run.
 #include "cf_common.cuh"
 
 namespace cf {
@@ -33,7 +35,15 @@ int bwd_tc_gemm_nn(const float *X, int64_t ldx, int64_t R, const int32_t *d_R, i
                    float *Out, int64_t ldo, int epi, const float *aux, int64_t ldaux, cudaStream_t st);
 int bwd_tc_gemm_tn(const float *X, int64_t ldx, int32_t M, const float *Y, int64_t ldy, int32_t N, const float *Y2,
                    int64_t rs2, int64_t cs2, int32_t n2, const float *wcol, int64_t R, const int32_t *d_R, float *dW,
-                   int64_t ldw, float *db, cudaStream_t st);
+                   int64_t ldw, float *db, cudaStream_t st, float *part = nullptr);
+// cf_bwd_det.cu: the pieces of the deterministic mode
+size_t det_cell_blocks(int64_t ncell);
+int det_compact_bases(const int32_t *knn, int64_t ncell, int32_t K, int32_t *blk, int32_t *counters, cudaStream_t st);
+int det_reduce(const float *part, int32_t M, int32_t n_w, int32_t n_out, int32_t nsplit, int64_t R, const int32_t *d_R,
+               int64_t unit, int64_t per_fixed, float *dW, int64_t ldw, int64_t cs, float *db, cudaStream_t st);
+size_t det_dT_words(int64_t pts, int64_t rows);
+int det_dT(const float *dA, int32_t C, const int32_t *row_pt, const int32_t *n_rows, int64_t rows, int64_t pts, float *dT,
+           void *ws, cudaStream_t st);
 
 namespace {
 
@@ -97,11 +107,13 @@ __global__ void __launch_bounds__(256) k_sgemm_nn(const float *__restrict__ A, i
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// C[M x N] += scale * A[R x M]^T * B[R x N]   (reduction over the long dimension R, split across blockIdx.z, atomics)
+// C[M x N] += scale * A[R x M]^T * B[R x N]   (reduction over the long dimension R, split across blockIdx.z, atomics;
+// part != nullptr: each split stores its tile to part[z][M][N] instead, for a fixed-order sum)
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_sgemm_tn(const float *__restrict__ A, int64_t lda, const float *__restrict__ Bm,
                                                   int64_t ldb, float *__restrict__ Cm, int64_t ldc, int64_t R, int32_t M,
-                                                  int32_t N, int64_t rows_per_split, const int32_t *__restrict__ d_R)
+                                                  int32_t N, int64_t rows_per_split, const int32_t *__restrict__ d_R,
+                                                  float *__restrict__ part)
 {
     __shared__ float As[16][64 + 4];
     __shared__ float Bs[16][64 + 4];
@@ -138,22 +150,26 @@ __global__ void __launch_bounds__(256) k_sgemm_tn(const float *__restrict__ A, i
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int32_t m = m0 + ty * 4 + i, n = n0 + tx * 4 + j;
-            if (m < M && n < N && acc[i][j] != 0.0f) atomicAdd(Cm + (int64_t)m * ldc + n, acc[i][j]);
+            if (m >= M || n >= N) continue;
+            if (part) part[((int64_t)blockIdx.z * M + m) * N + n] = acc[i][j];
+            else if (acc[i][j] != 0.0f) atomicAdd(Cm + (int64_t)m * ldc + n, acc[i][j]);
         }
 }
 
 // out[n] += scale * sum_r w[r] * X[r, n]   (w == nullptr: plain column sum).
-// grid (row slabs of 1024, column chunks of 32); a warp owns every 8th row of the slab, lane = column: 128-byte row
-// segments, 4 independent partial sums per lane, then an 8-warp reduction in shared memory and one atomicAdd per column.
+// grid (row slabs of `slab` rows, column chunks of 32); a warp owns every 8th row of the slab, lane = column: 128-byte row
+// segments, 4 independent partial sums per lane, then an 8-warp reduction in shared memory and one atomicAdd per column
+// (slab_out != nullptr: the slab's sums are stored to slab_out[slab][N] instead, for a fixed-order sum).
 __global__ void __launch_bounds__(256) k_colsum(const float *__restrict__ X, int64_t ldx, int64_t R, int32_t N,
                                                 const float *__restrict__ w, float scale, float *__restrict__ out,
-                                                int64_t out_stride, const int32_t *__restrict__ d_R)
+                                                int64_t out_stride, const int32_t *__restrict__ d_R, int64_t slab,
+                                                float *__restrict__ slab_out)
 {
     __shared__ float part[8][32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int32_t n = blockIdx.y * 32 + lane;
     if (d_R) R = min(R, (int64_t)__ldg(d_R));
-    const int64_t r_begin = (int64_t)blockIdx.x * 1024, r_end = min(R, r_begin + 1024);
+    const int64_t r_begin = (int64_t)blockIdx.x * slab, r_end = min(R, r_begin + slab);
     if (r_begin >= R) return;
     float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
     if (n < N) {
@@ -174,7 +190,8 @@ __global__ void __launch_bounds__(256) k_colsum(const float *__restrict__ X, int
         float s = 0.f;
 #pragma unroll
         for (int i = 0; i < 8; ++i) s += part[i][lane];
-        if (s != 0.0f) atomicAdd(out + (int64_t)n * out_stride, s * scale);
+        if (slab_out) slab_out[(int64_t)blockIdx.x * N + n] = s * scale;
+        else if (s != 0.0f) atomicAdd(out + (int64_t)n * out_stride, s * scale);
     }
 }
 
@@ -184,6 +201,8 @@ __global__ void __launch_bounds__(256) k_colsum(const float *__restrict__ X, int
 //   row_pt[r] = b * N + point            row_cell[r] = ci              row_cx / row_cy[r] = the cell's centre
 //   row_off[j * row_cap + r], j = 0..2 = (px - cx, py - cy, pz): the three offset inputs of layer 1 for that row
 // counters[0] = live cells, counters[1] = live rows (zeroed by the caller of the kernel).
+// block_base != nullptr: the block's first cell / row slot is block_base[2 * block + 0 / 1] (an exclusive scan of the
+// block totals, counters already hold the totals): the lists are then in grid order.
 __global__ void __launch_bounds__(256) k_bwd_compact(const int32_t *__restrict__ knn, int64_t ncell, int64_t cells, int32_t W,
                                                      int32_t K, int32_t N, float x0, float y0, float dx, float dy,
                                                      int32_t *__restrict__ counters, int32_t *__restrict__ cell_list,
@@ -191,7 +210,7 @@ __global__ void __launch_bounds__(256) k_bwd_compact(const int32_t *__restrict__
                                                      int32_t *__restrict__ row_pt, int32_t *__restrict__ row_cell,
                                                      float *__restrict__ row_cx, float *__restrict__ row_cy,
                                                      const float *__restrict__ points, float *__restrict__ row_off,
-                                                     int64_t row_cap)
+                                                     int64_t row_cap, const int32_t *__restrict__ block_base)
 {
     __shared__ int32_t warp_cells[8], warp_rows[8], base[2];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -220,8 +239,13 @@ __global__ void __launch_bounds__(256) k_bwd_compact(const int32_t *__restrict__
             c += tc;
             r += tr;
         }
-        base[0] = c ? atomicAdd(counters, c) : 0;
-        base[1] = r ? atomicAdd(counters + 1, r) : 0;
+        if (block_base) {
+            base[0] = block_base[2 * blockIdx.x];
+            base[1] = block_base[2 * blockIdx.x + 1];
+        } else {
+            base[0] = c ? atomicAdd(counters, c) : 0;
+            base[1] = r ? atomicAdd(counters + 1, r) : 0;
+        }
     }
     __syncthreads();
     if (nv == 0) return;
@@ -412,11 +436,14 @@ struct BwdWs {
     float *H1, *H2, *pooled, *G, *dPooled, *row_cx, *row_cy, *row_off, *cell_nv, *T, *dT, *W2t;
     int32_t *cell_list, *cell_row0, *row_pt, *row_cell, *counters;
     void *pW2, *pW2t, *pW3t, *pW1t;  // bf16 hi | lo operand images of the weights (tensor-core path)
+    int32_t *blk;                    // deterministic mode: scanned (cells, rows) totals of the compaction blocks
+    float *part;                     // deterministic mode: per-split partials of one row reduction at a time
+    void *csr;                       // deterministic mode: rows of each point (det_dT)
     size_t bytes;
 };
 
-// sized for the dense upper bound (every slot of every cell holds a neighbour)
-static BwdWs carve(void *base, int32_t B, int32_t N, int32_t C, int32_t Ci, int64_t cells, int32_t K)
+// sized for the dense upper bound (every slot of every cell holds a neighbour); the deterministic mode appends its buffers
+static BwdWs carve(void *base, int32_t B, int32_t N, int32_t C, int32_t Ci, int64_t cells, int32_t K, bool det)
 {
     BwdWs w;
     size_t off = 0;
@@ -447,6 +474,16 @@ static BwdWs carve(void *base, int32_t B, int32_t N, int32_t C, int32_t Ci, int6
     w.pW2t = take(bwd_tc_packed_bytes(C, C) / 4);
     w.pW3t = take(bwd_tc_packed_bytes(C, C) / 4);
     w.pW1t = take(bwd_tc_packed_bytes(Ci, C) / 4);
+    w.blk = nullptr;
+    w.part = nullptr;
+    w.csr = nullptr;
+    if (det) {
+        // partials: at most kDetSplits splits of an (M <= C) x (n_out <= max(C, Ci) + 16) tile (the tcgen05 TN GEMM
+        // halves the splits when M = C spans two 128-row tiles)
+        w.blk = (int32_t *)take(2 * det_cell_blocks(ncell));
+        w.part = (float *)take((size_t)kDetSplits * C * (std::max(C, Ci) + 16));
+        w.csr = take(det_dT_words((int64_t)B * N, (int64_t)rows));
+    }
     w.bytes = off;
     return w;
 }
@@ -474,13 +511,20 @@ int point_mlp1_simt(const float *d_feat, const float *d_points, const int64_t *d
 extern "C" size_t cf_fusion_bwd_workspace_bytes(int32_t B, int32_t N, int32_t C, int32_t Ci, int32_t H, int32_t W, int32_t K)
 {
     if (B <= 0 || N <= 0 || C <= 0 || Ci <= 0 || H <= 0 || W <= 0 || K <= 0) return 0;
-    return cf::carve(nullptr, B, N, C, Ci, (int64_t)H * W, K).bytes;
+    return cf::carve(nullptr, B, N, C, Ci, (int64_t)H * W, K, false).bytes;
+}
+
+extern "C" size_t cf_fusion_bwd_det_workspace_bytes(int32_t B, int32_t N, int32_t C, int32_t Ci, int32_t H, int32_t W, int32_t K)
+{
+    if (B <= 0 || N <= 0 || C <= 0 || Ci <= 0 || H <= 0 || W <= 0 || K <= 0) return 0;
+    return cf::carve(nullptr, B, N, C, Ci, (int64_t)H * W, K, true).bytes;
 }
 
 // Gradients are ACCUMULATED into d_gW1 (C,Ci+3), d_gb1, d_gW2 (C,C), d_gb2, d_gW3, d_gb3 and d_gfeat (B,N,Ci): the
 // caller zero-initialises them (or passes buffers that already hold other scales' contributions).  d bev = d_gout.
 // d_T: the table the forward computed with cf_point_mlp1 (nullptr: it is recomputed here).
 // mode: CF_MODE_FP32_SIMT = every GEMM on CUDA cores (cross-check); otherwise the GEMMs whose operands fit run on tcgen05.
+// mode | CF_BWD_DETERMINISTIC: bit-reproducible gradients (workspace: cf_fusion_bwd_det_workspace_bytes).
 extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const float *d_points,
                              const int64_t *d_num_points, const int32_t *d_knn_idx, int32_t B, int32_t N, int32_t C,
                              int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy,
@@ -490,6 +534,8 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
 {
     using namespace cf;
     CF_TRY(require_sm100());
+    const bool det = (mode & CF_BWD_DETERMINISTIC) != 0;
+    mode &= ~CF_BWD_DETERMINISTIC;
     CF_REQUIRE(d_gout && d_feat && d_points && d_num_points && d_knn_idx && d_W1 && d_b1 && d_W2 && d_b2 && d_W3 &&
                    d_gW1 && d_gb1 && d_gW2 && d_gb2 && d_gW3 && d_gb3 && d_gfeat && d_workspace,
                CF_ERR_ARG, "cf_fusion_bwd: null pointer");
@@ -503,7 +549,7 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     const int64_t cells = (int64_t)H * W, ncell = cells * B, rows = cells * K * B;
     CF_REQUIRE(rows < (int64_t)1 << 31 && (int64_t)B * N < (int64_t)1 << 31, CF_ERR_ARG,
                "cf_fusion_bwd: B*H*W*K and B*N must stay below 2^31");
-    BwdWs w = carve(d_workspace, B, N, C, Ci, cells, K);
+    BwdWs w = carve(d_workspace, B, N, C, Ci, cells, K, det);
     const int32_t ldw1 = Ci + 3;
     const int32_t *n_cells = w.counters, *n_rows = w.counters + 1;
     const unsigned cchunks = (unsigned)((C + 31) / 32), ctiles = (unsigned)((C + 63) / 64);
@@ -518,12 +564,31 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     const bool tc_pt_tn = tc && bwd_tc_tn_fits(C, Ci);    // dW1 | db1 = dT^T [F | P | 1]
     const bool col2 = tc_row_tn && C + 1 <= 256;          // db2 / db3 ride in the GEMM as an extra column
     int launches = 0;
+    float *part = det ? w.part : nullptr;
+    // the two FFMA row reductions; deterministic mode: a fixed number of splits (shapes only), partials, ordered sum
+    auto sgemm_tn = [&](const float *A, const float *Bm, int64_t ldb, float *Cm, int64_t ldc, int64_t R, int32_t M, int32_t N,
+                        int64_t split, const int32_t *d_R) -> int {
+        if (det) split = std::max<int64_t>(256, ceil_div64(R, kDetSplits));
+        const unsigned z = (unsigned)ceil_div64(R, split);
+        k_sgemm_tn<<<dim3((unsigned)((M + 63) / 64), (unsigned)((N + 63) / 64), z), 256, 0, st>>>(A, C, Bm, ldb, Cm, ldc, R, M, N,
+                                                                                                 split, d_R, part);
+        ++launches;
+        return det ? det_reduce(part, M, N, N, (int32_t)z, R, d_R, 1, split, Cm, ldc, 1, nullptr, st) : CF_OK;
+    };
+    auto colsum = [&](const float *X, int64_t R, const float *wv, float *out, int64_t out_stride, const int32_t *d_R) -> int {
+        const int64_t slab = det ? std::max<int64_t>(1024, ceil_div64(R, kDetSplits)) : 1024;
+        const unsigned gx = (unsigned)ceil_div64(R, slab);
+        k_colsum<<<dim3(gx, cchunks), 256, 0, st>>>(X, C, R, C, wv, 1.0f, out, out_stride, d_R, slab, part);
+        ++launches;
+        return det ? det_reduce(part, 1, C, C, (int32_t)gx, R, d_R, 1, slab, out, 0, out_stride, nullptr, st) : CF_OK;
+    };
 
     // ---- live cells / rows, then the forward intermediates on them ----------------------------------------------------
     CF_TRY(cuda_status(cudaMemsetAsync(w.counters, 0, 2 * sizeof(int32_t), st), "cf_fusion_bwd memset"));
+    if (det) CF_TRY(det_compact_bases(d_knn_idx, ncell, K, w.blk, w.counters, st));
     k_bwd_compact<<<(unsigned)ceil_div64(ncell, 256), 256, 0, st>>>(d_knn_idx, ncell, cells, W, K, N, x0, y0, dx, dy, w.counters,
                                                                    w.cell_list, w.cell_row0, w.cell_nv, w.row_pt, w.row_cell,
-                                                                   w.row_cx, w.row_cy, d_points, w.row_off, rows);
+                                                                   w.row_cx, w.row_cy, d_points, w.row_off, rows, w.blk);
     const float *T = d_T;
     if (!T) {
         CF_TRY(point_mlp1_simt(d_feat, d_points, d_num_points, B, N, Ci, C, d_W1, d_b1, w.T, st));
@@ -585,18 +650,11 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     launches += 2;
     if (tc_row_tn) {
         CF_TRY(bwd_tc_gemm_tn(w.G, C, C, w.pooled, C, C, nullptr, 0, 0, 0, w.cell_nv, ncell, n_cells, d_gW3, C,
-                              col2 ? d_gb3 : nullptr, st));
+                              col2 ? d_gb3 : nullptr, st, part));
     } else {
-        const int64_t split3 = std::max<int64_t>(256, ceil_div64(ncell, 1184));
-        k_sgemm_tn<<<dim3(ctiles, ctiles, (unsigned)ceil_div64(ncell, split3)), 256, 0, st>>>(w.G, C, w.pooled, C, d_gW3, C, ncell,
-                                                                                             C, C, split3, n_cells);
-        ++launches;
+        CF_TRY(sgemm_tn(w.G, w.pooled, C, d_gW3, C, ncell, C, C, std::max<int64_t>(256, ceil_div64(ncell, 1184)), n_cells));
     }
-    if (!(tc_row_tn && col2)) {
-        k_colsum<<<dim3((unsigned)ceil_div64(ncell, 1024), cchunks), 256, 0, st>>>(w.G, C, ncell, C, w.cell_nv, 1.0f, d_gb3, 1,
-                                                                                  n_cells);
-        ++launches;
-    }
+    if (!(tc_row_tn && col2)) CF_TRY(colsum(w.G, ncell, w.cell_nv, d_gb3, 1, n_cells));
     // dPooled = G W3   (W3 is (out, in) row-major: exactly the [K=out x N=in] operand)
     if (tc_row_nn) {
         CF_TRY(row_nn(w.G, ncell, n_cells, w.pW3t, w.dPooled, EPI_STORE, nullptr, 0));
@@ -613,18 +671,11 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     ++launches;
     if (tc_row_tn) {
         CF_TRY(bwd_tc_gemm_tn(w.H2, C, C, w.H1, C, C, nullptr, 0, 0, 0, nullptr, rows, n_rows, d_gW2, C,
-                              col2 ? d_gb2 : nullptr, st));
+                              col2 ? d_gb2 : nullptr, st, part));
     } else {
-        const int64_t split2 = std::max<int64_t>(256, ceil_div64(rows, 1184));
-        k_sgemm_tn<<<dim3(ctiles, ctiles, (unsigned)ceil_div64(rows, split2)), 256, 0, st>>>(w.H2, C, w.H1, C, d_gW2, C, rows, C,
-                                                                                            C, split2, n_rows);
-        ++launches;
+        CF_TRY(sgemm_tn(w.H2, w.H1, C, d_gW2, C, rows, C, C, std::max<int64_t>(256, ceil_div64(rows, 1184)), n_rows));
     }
-    if (!(tc_row_tn && col2)) {
-        k_colsum<<<dim3((unsigned)ceil_div64(rows, 1024), cchunks), 256, 0, st>>>(w.H2, C, rows, C, nullptr, 1.0f, d_gb2, 1,
-                                                                                 n_rows);
-        ++launches;
-    }
+    if (!(tc_row_tn && col2)) CF_TRY(colsum(w.H2, rows, nullptr, d_gb2, 1, n_rows));
     // dA = (dZ2 W2) * [H1 > 0]   written over H1 (the mask is read before the overwrite, element by element)
     if (tc_row_nn) {
         CF_TRY(row_nn(w.H2, rows, n_rows, w.pW2t, w.H1, EPI_MASK, w.H1, C));
@@ -639,27 +690,25 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     // forward (small numbers), not as the difference of two large point-side and cell-side sums
     if (tc_row_tn) {
         CF_TRY(bwd_tc_gemm_tn(w.H1, C, C, nullptr, 0, 0, w.row_off, 1, rows, 3, nullptr, rows, n_rows, d_gW1 + Ci, ldw1, nullptr,
-                              st));
+                              st, part));
     } else {
-        for (int j = 0; j < 3; ++j)
-            k_colsum<<<dim3((unsigned)ceil_div64(rows, 1024), cchunks), 256, 0, st>>>(w.H1, C, rows, C, w.row_off + j * rows, 1.0f,
-                                                                                     d_gW1 + Ci + j, ldw1, n_rows);
-        launches += 3;
+        for (int j = 0; j < 3; ++j) CF_TRY(colsum(w.H1, rows, w.row_off + j * rows, d_gW1 + Ci + j, ldw1, n_rows));
     }
-    CF_TRY(cuda_status(cudaMemsetAsync(w.dT, 0, (size_t)B * N * C * sizeof(float), st), "cf_fusion_bwd memset"));
-    k_bwd_scatter<<<blocks_for(rows, 8), 256, 0, st>>>(w.H1, w.row_pt, w.counters, C, w.dT);
-    ++launches;
     const int64_t pts = (int64_t)B * N;
+    if (det) {
+        // dT as a gather over each point's rows in ascending row order (one writer per row of dT)
+        CF_TRY(det_dT(w.H1, C, w.row_pt, n_rows, rows, pts, w.dT, w.csr, st));
+    } else {
+        CF_TRY(cuda_status(cudaMemsetAsync(w.dT, 0, (size_t)B * N * C * sizeof(float), st), "cf_fusion_bwd memset"));
+        k_bwd_scatter<<<blocks_for(rows, 8), 256, 0, st>>>(w.H1, w.row_pt, w.counters, C, w.dT);
+        ++launches;
+    }
     // feat rows beyond num_points are zero and never referenced by knn, so their dT rows are zero as well
     if (tc_pt_tn) {
-        CF_TRY(bwd_tc_gemm_tn(w.dT, C, C, d_feat, Ci, Ci, nullptr, 0, 0, 0, nullptr, pts, nullptr, d_gW1, ldw1, d_gb1, st));
+        CF_TRY(bwd_tc_gemm_tn(w.dT, C, C, d_feat, Ci, Ci, nullptr, 0, 0, 0, nullptr, pts, nullptr, d_gW1, ldw1, d_gb1, st, part));
     } else {
-        const int64_t splitp = std::max<int64_t>(512, ceil_div64(pts, 148));
-        k_sgemm_tn<<<dim3(ctiles, (unsigned)((Ci + 63) / 64), (unsigned)ceil_div64(pts, splitp)), 256, 0, st>>>(
-            w.dT, C, d_feat, Ci, d_gW1, ldw1, pts, C, Ci, splitp, nullptr);
-        k_colsum<<<dim3((unsigned)ceil_div64(pts, 1024), cchunks), 256, 0, st>>>(w.dT, C, pts, C, nullptr, 1.0f, d_gb1, 1,
-                                                                                nullptr);
-        launches += 2;
+        CF_TRY(sgemm_tn(w.dT, d_feat, Ci, d_gW1, ldw1, pts, C, Ci, std::max<int64_t>(512, ceil_div64(pts, 148)), nullptr));
+        CF_TRY(colsum(w.dT, pts, nullptr, d_gb1, 1, nullptr));
     }
     // dF += dT W1[:, :Ci]
     if (tc_pt_nn) {

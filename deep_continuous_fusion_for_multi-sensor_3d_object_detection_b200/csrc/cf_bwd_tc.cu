@@ -252,6 +252,7 @@ struct TnParams {
     float *dW;
     int64_t ldw;
     float *db;
+    float *part;        // deterministic mode: this CTA's tile goes to part[split][M][n_out] instead of the atomics
 };
 
 __global__ void __launch_bounds__(kNT) k_bwd_gemm_tn_tc(const TnParams p)
@@ -388,13 +389,19 @@ __global__ void __launch_bounds__(kNT) k_bwd_gemm_tn_tc(const TnParams p)
     __syncthreads();
     const int n_w = N + p.n2;  // columns [0, n_w) go to dW, column n_w to db
     const int n_out = n_w + (p.db ? 1 : 0);
-    for (int m = warp; m < Mv; m += kNT / 32) {
-        float *dw = p.dW + (int64_t)(m0 + m) * p.ldw;
-        for (int n = lane; n < n_out; n += 32) {
-            const float v = sD[m * ldd + n];
-            if (v == 0.0f) continue;
-            if (n < n_w) atomicAdd(dw + n, v);
-            else atomicAdd(p.db + m0 + m, v);
+    if (p.part) {
+        float *dst = p.part + ((int64_t)blockIdx.x * p.M + m0) * n_out;
+        for (int m = warp; m < Mv; m += kNT / 32)
+            for (int n = lane; n < n_out; n += 32) dst[(int64_t)m * n_out + n] = sD[m * ldd + n];
+    } else {
+        for (int m = warp; m < Mv; m += kNT / 32) {
+            float *dw = p.dW + (int64_t)(m0 + m) * p.ldw;
+            for (int n = lane; n < n_out; n += 32) {
+                const float v = sD[m * ldd + n];
+                if (v == 0.0f) continue;
+                if (n < n_w) atomicAdd(dw + n, v);
+                else atomicAdd(p.db + m0 + m, v);
+            }
         }
     }
     tc::fence_before_sync();
@@ -462,9 +469,13 @@ int bwd_tc_gemm_nn(const float *X, int64_t ldx, int64_t R, const int32_t *d_R, i
     return launch_status("cf_fusion_bwd (nn)");
 }
 
+int det_reduce(const float *part, int32_t M, int32_t n_w, int32_t n_out, int32_t nsplit, int64_t R, const int32_t *d_R,
+               int64_t unit, int64_t per_fixed, float *dW, int64_t ldw, int64_t cs, float *db, cudaStream_t st);
+
+// part != nullptr (deterministic mode): kDetSplits / mtiles row splits whatever the GPU, partials summed in split order
 int bwd_tc_gemm_tn(const float *X, int64_t ldx, int32_t M, const float *Y, int64_t ldy, int32_t N, const float *Y2,
                    int64_t rs2, int64_t cs2, int32_t n2, const float *wcol, int64_t R, const int32_t *d_R, float *dW,
-                   int64_t ldw, float *db, cudaStream_t st)
+                   int64_t ldw, float *db, cudaStream_t st, float *part)
 {
     static int attr_done = 0;
     const int32_t Nt = (N + n2 + (db ? 1 : 0) + 15) / 16 * 16;
@@ -472,7 +483,7 @@ int bwd_tc_gemm_tn(const float *X, int64_t ldx, int32_t M, const float *Y, int64
         set_error("cf_fusion_bwd (tn): %d columns exceed one MMA", Nt);
         return CF_ERR_ARG;
     }
-    TnParams p{X, ldx, M, Y, ldy, N, Y2, rs2, cs2, n2, wcol, Nt, R, d_R, dW, ldw, db};
+    TnParams p{X, ldx, M, Y, ldy, N, Y2, rs2, cs2, n2, wcol, Nt, R, d_R, dW, ldw, db, part};
     const int smem = 2 * (2 * kRows * kTnKC * 2 + 2 * Nt * kTnKC * 2);
     if (!attr_done) {
         CF_TRY(cuda_status(cudaFuncSetAttribute(k_bwd_gemm_tn_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024),
@@ -483,10 +494,16 @@ int bwd_tc_gemm_tn(const float *X, int64_t ldx, int32_t M, const float *Y, int64
     const int per_sm = std::max(1, std::min({(220 * 1024) / (smem + 1024), 512 / tmem_cols(Nt), 2048 / kNT}));
     const int64_t chunks = ceil_div64(R, kTnKC);
     // at least 4 stages of rows per CTA, at most one wave of CTAs
-    const int64_t splits = std::max<int64_t>(1, std::min<int64_t>(ceil_div64(chunks, 4), (int64_t)sm_count() * per_sm / mtiles));
+    const int64_t ctas = part ? kDetSplits : (int64_t)sm_count() * per_sm;
+    const int64_t splits = std::max<int64_t>(1, std::min<int64_t>(ceil_div64(chunks, 4), ctas / mtiles));
     k_bwd_gemm_tn_tc<<<dim3((unsigned)splits, (unsigned)mtiles), kNT, smem, st>>>(p);
     count_launches(1);
-    return launch_status("cf_fusion_bwd (tn)");
+    CF_TRY(launch_status("cf_fusion_bwd (tn)"));
+    if (part) {
+        const int32_t n_w = N + n2;
+        return det_reduce(part, M, n_w, n_w + (db ? 1 : 0), (int32_t)splits, R, d_R, kTnKC, 0, dW, ldw, 1, db, st);
+    }
+    return CF_OK;
 }
 
 }  // namespace cf
@@ -519,5 +536,6 @@ extern "C" int cf_debug_bwd_gemm_tn(const float *d_X, int32_t M, const float *d_
     CF_REQUIRE(d_X && d_dW && R > 0 && (N == 0 || d_Y) && (n2 == 0 || d_Y2) && n2 >= 0 && n2 <= 15, CF_ERR_ARG,
                "cf_debug_bwd_gemm_tn: bad arguments");
     CF_REQUIRE(bwd_tc_tn_fits(M, N), CF_ERR_ARG, "cf_debug_bwd_gemm_tn: M=%d N=%d has no tensor-core instantiation", M, N);
-    return bwd_tc_gemm_tn(d_X, M, M, d_Y, N, N, d_Y2, n2, 1, n2, d_wcol, R, d_R, d_dW, N + n2, d_db, (cudaStream_t)stream);
+    return bwd_tc_gemm_tn(d_X, M, M, d_Y, N, N, d_Y2, n2, 1, n2, d_wcol, R, d_R, d_dW, N + n2, d_db, (cudaStream_t)stream,
+                          nullptr);
 }

@@ -37,6 +37,10 @@ void count_launches(int n);
 
 static inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+// Row splits of the fixed-order reductions of the deterministic backward (cf_bwd_det.cu): a constant, so the summation
+// order depends on shapes and live counts only, not on the SM count of the GPU.
+constexpr int kDetSplits = 128;
+
 __host__ __device__ static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 // number of valid points of frame b, clamped to [0, N]

@@ -265,7 +265,8 @@ class _GatherFunction(torch.autograd.Function):
     def backward(ctx, grad_feat):
         points, num_points, uv = ctx.saved_tensors
         gimg = ops.point_gather_bwd(grad_feat, ctx.img_like, points, num_points, calib=None if ctx.has_uv else ctx.calib,
-                                    uv=uv if ctx.has_uv else None, img_size=ctx.img_size)
+                                    uv=uv if ctx.has_uv else None, img_size=ctx.img_size,
+                                    deterministic=torch.are_deterministic_algorithms_enabled())
         return gimg, None, None, None, None, None
 
 
@@ -289,7 +290,8 @@ class _FusionFunction(torch.autograd.Function):
     def backward(ctx, grad_out):
         feat, points, num_points, knn_idx, w1, b1, w2, b2, w3, b3, table = ctx.saved_tensors
         gw1, gb1, gw2, gb2, gw3, gb3, gfeat = ops.fusion_bwd(grad_out, feat, points, num_points, knn_idx, ctx.geom, w1, b1,
-                                                             w2, b2, w3, table=table, mode=ctx.mode)
+                                                             w2, b2, w3, table=table, mode=ctx.mode,
+                                                             deterministic=torch.are_deterministic_algorithms_enabled())
         # d out / d bev is the identity
         return grad_out, gfeat, None, None, None, None, None, gw1, gb1, gw2, gb2, gw3, gb3, None, None, None
 

@@ -17,6 +17,7 @@ here only so that the module tree and parameter names match.
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -28,6 +29,65 @@ from .fusion import ContinuousFusion, FrameContext
 
 def _conv(cin, cout, k, stride=1):
     return nn.Conv2d(cin, cout, kernel_size=(k, k), stride=(stride, stride), padding=(k // 2, k // 2), bias=False)
+
+
+_INTERP_MATS = {}   # (n_in, n_out, align_corners, device, dtype) -> (n_out, n_in) interpolation matrix
+
+
+def _interp_matrix(n_in, n_out, align_corners, device, dtype):
+    """The (n_out, n_in) matrix of 1-D linear interpolation along one axis of F.interpolate(mode="bilinear"), built once
+    per shape and device (a CUDA-graph capture of the step finds it cached from the eager warm-up)."""
+    key = (int(n_in), int(n_out), bool(align_corners), device, dtype)
+    m = _INTERP_MATS.get(key)
+    if m is None:
+        # the weights in fp32, as PyTorch's kernels compute them (scale, source coordinate, fraction)
+        f = np.float32
+        dst = np.arange(n_out, dtype=f)
+        if align_corners:
+            src = dst * (f(n_in - 1) / f(n_out - 1) if n_out > 1 else f(0))
+        else:
+            src = np.maximum((dst + f(0.5)) * (f(n_in) / f(n_out)) - f(0.5), f(0))
+        i0 = np.minimum(src.astype(np.int64), n_in - 1)
+        i1 = np.minimum(i0 + 1, n_in - 1)
+        l1 = (src - i0.astype(f)).astype(f)
+        a = np.zeros((n_out, n_in), np.float64)
+        np.add.at(a, (np.arange(n_out), i0), f(1) - l1)
+        np.add.at(a, (np.arange(n_out), i1), l1)
+        m = _INTERP_MATS[key] = torch.from_numpy(a).to(device=device, dtype=dtype)
+    return m
+
+
+class _BilinearDeterministic(torch.autograd.Function):
+    """F.interpolate(mode="bilinear") whose backward is the separable adjoint  Ry^T g Rx  (two matmuls) instead of
+    PyTorch's atomic scatter, which torch.use_deterministic_algorithms(True) rejects.  The forward is the same call."""
+
+    @staticmethod
+    def forward(ctx, x, size, scale_factor, align_corners):
+        ctx.hw_in, ctx.align_corners = tuple(x.shape[-2:]), align_corners
+        return F.interpolate(x, size, scale_factor, "bilinear", align_corners)
+
+    @staticmethod
+    def backward(ctx, g):
+        (hi, wi), (ho, wo) = ctx.hw_in, g.shape[-2:]
+        ry = _interp_matrix(hi, ho, ctx.align_corners, g.device, g.dtype)
+        rx = _interp_matrix(wi, wo, ctx.align_corners, g.device, g.dtype)
+        return ry.t() @ (g @ rx), None, None, None
+
+
+def bilinear(x, size=None, scale_factor=None, align_corners=False):
+    """F.interpolate(x, size, scale_factor, mode="bilinear", align_corners).  Under torch.use_deterministic_algorithms(True)
+    the backward is a fixed-order pair of matmuls (on CUDA these need CUBLAS_WORKSPACE_CONFIG=:4096:8, as PyTorch itself
+    requires for cuBLAS in that mode); otherwise it is exactly the PyTorch call."""
+    if torch.are_deterministic_algorithms_enabled():
+        return _BilinearDeterministic.apply(x, size, scale_factor, align_corners)
+    return F.interpolate(x, size, scale_factor, "bilinear", align_corners)
+
+
+def _upsample(module: nn.UpsamplingBilinear2d, x):
+    """`module(x)`, routed through `bilinear` in deterministic mode (same forward, fixed-order backward)."""
+    if torch.are_deterministic_algorithms_enabled():
+        return _BilinearDeterministic.apply(x, module.size, module.scale_factor, module.align_corners)
+    return module(x)
 
 
 class ResidualBlock(nn.Module):
@@ -155,8 +215,8 @@ class LidarBackboneNetwork(nn.Module):
 
     def forward(self, x, fuse=None):
         x4, x3, x2 = self.backbone(x, fuse)
-        x3 = self.latconv1(x3) + self.upscale1(self.downconv1(x4))
-        x2 = self.latconv2(x2) + self.upscale2(x3)
+        x3 = self.latconv1(x3) + _upsample(self.upscale1, self.downconv1(x4))
+        x2 = self.latconv2(x2) + _upsample(self.upscale2, x3)
         x_pred = self.conv3(x2)
         x_cls = self.classconv(x_pred)
         x_cls = torch.cat((self.softmax1(x_cls[:, :2]), self.softmax2(x_cls[:, 2:4])), dim=1)
@@ -187,8 +247,8 @@ class ImageBackbone(nn.Module):
         f1 = self.stage1(self.stem(x))
         f2 = self.stage2(f1)
         f3 = self.stage3(f2)
-        t = self.lat2(f2) + F.interpolate(self.lat3(f3), size=f2.shape[-2:], mode="bilinear", align_corners=False)
-        t = self.lat1(f1) + F.interpolate(t, size=f1.shape[-2:], mode="bilinear", align_corners=False)
+        t = self.lat2(f2) + bilinear(self.lat3(f3), size=f2.shape[-2:], align_corners=False)
+        t = self.lat1(f1) + bilinear(t, size=f1.shape[-2:], align_corners=False)
         return self.out(t).contiguous(memory_format=torch.channels_last)
 
 

@@ -31,6 +31,18 @@ def _contig(t: torch.Tensor, name: str, dtype, ndim=None):
     return t if t.is_contiguous() else t.contiguous()
 
 
+def _scratch(nbytes: int, device) -> torch.Tensor:
+    """Workspace that the kernels write before they read it.  torch.use_deterministic_algorithms(True) makes torch.empty fill
+    new memory (hundreds of MB per backward call here); scratch needs no fill, so it is allocated without one."""
+    import torch.utils.deterministic as det
+    prev = det.fill_uninitialized_memory
+    det.fill_uninitialized_memory = False
+    try:
+        return torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=device)
+    finally:
+        det.fill_uninitialized_memory = prev
+
+
 def as_counts(num_points, B: int, device) -> torch.Tensor:
     """sample["num_points_raw"] after collation is a (B,) int64 CPU tensor (data_import_carla.py:262)."""
     if not isinstance(num_points, torch.Tensor):
@@ -352,10 +364,11 @@ def fusion_fwd(bev, T, knn_idx, geom, W1, W2, b2, W3, b3, mode="fp32", out=None,
 
 
 def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2, W3, grad_feat=None, table=None,
-               mode="fp32"):
+               mode="fp32", deterministic=False):
     """K-4b.  Returns (gW1, gb1, gW2, gb2, gW3, gb3, gfeat); d bev is grad_out itself.
     `table`: the forward's point_mlp1 output (B,N,C) if it was kept (else it is recomputed); `mode` "simt" keeps every
-    GEMM on CUDA cores, any other mode runs them on tcgen05 with fp32-accurate split operands."""
+    GEMM on CUDA cores, any other mode runs them on tcgen05 with fp32-accurate split operands.
+    `deterministic`: fixed summation order everywhere (CF_BWD_DETERMINISTIC): identical inputs give bit-identical gradients."""
     lib = load()
     grad_out = _contig(grad_out, "grad_out", torch.float32, 4)
     feat = _contig(feat, "feat", torch.float32, 3)
@@ -374,16 +387,22 @@ def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2
         table = _contig(table, "table", torch.float32, 3)
         if tuple(table.shape) != (B, N, Cc):
             raise ValueError("fusion_bwd: table must be (B, N, C)")
-    ws = torch.empty((max(lib.cf_fusion_bwd_workspace_bytes(B, N, Cc, Ci, H, W, K), 16),), dtype=torch.uint8, device=dev)
+    ws_bytes = (lib.cf_fusion_bwd_det_workspace_bytes if deterministic else lib.cf_fusion_bwd_workspace_bytes)(B, N, Cc, Ci, H, W, K)
+    ws = _scratch(ws_bytes, dev)
+    m = _lib.MODES[mode] if isinstance(mode, str) else int(mode)
+    if deterministic:
+        m |= _lib.BWD_DETERMINISTIC
     x0, y0, dx, dy = [float(g) for g in geom]
     check(lib.cf_fusion_bwd(ptr(grad_out), ptr(feat), ptr(points), ptr(num_points), ptr(knn_idx), B, N, Cc, H, W, K, x0, y0,
                             dx, dy, ptr(W1), ptr(b1), Ci, ptr(W2), ptr(b2), ptr(W3), ptr(table), ptr(gW1), ptr(gb1), ptr(gW2),
-                            ptr(gb2), ptr(gW3), ptr(gb3), ptr(gfeat), (_lib.MODES[mode] if isinstance(mode, str) else int(mode)), ptr(ws), stream_ptr()), "cf_fusion_bwd")
+                            ptr(gb2), ptr(gW3), ptr(gb3), ptr(gfeat), m, ptr(ws), stream_ptr()), "cf_fusion_bwd")
     return gW1, gb1, gW2, gb2, gW3, gb3, gfeat
 
 
-def point_gather_bwd(grad_feat, img_like, points, num_points, calib=None, uv=None, img_size=(640.0, 480.0)):
-    """Adjoint of point_gather: gradient w.r.t. the camera feature map (same shape / memory format as img_like)."""
+def point_gather_bwd(grad_feat, img_like, points, num_points, calib=None, uv=None, img_size=(640.0, 480.0),
+                     deterministic=False):
+    """Adjoint of point_gather: gradient w.r.t. the camera feature map (same shape / memory format as img_like).
+    `deterministic`: each pixel sums its (point, tap) contributions in a fixed order (cf_point_gather_bwd_det)."""
     lib = load()
     grad_feat = _contig(grad_feat, "grad_feat", torch.float32, 3)
     points = _contig(points, "points", torch.float32, 3)
@@ -395,8 +414,15 @@ def point_gather_bwd(grad_feat, img_like, points, num_points, calib=None, uv=Non
         calib_arr = _calib_host(calib)
     else:
         uv = _contig(uv, "uv", torch.float32, 3)
+    N = points.shape[1]
+    if deterministic:
+        ws = _scratch(lib.cf_point_gather_bwd_det_workspace_bytes(B, N, Hf, Wf), gimg.device)
+        check(lib.cf_point_gather_bwd_det(ptr(grad_feat), ptr(gimg), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv),
+                                          calib_arr, ptr(num_points), N, float(img_size[0]), float(img_size[1]), ptr(ws),
+                                          stream_ptr()), "cf_point_gather_bwd_det")
+        return gimg
     check(lib.cf_point_gather_bwd(ptr(grad_feat), ptr(gimg), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv), calib_arr,
-                                  ptr(num_points), points.shape[1], float(img_size[0]), float(img_size[1]), stream_ptr()),
+                                  ptr(num_points), N, float(img_size[0]), float(img_size[1]), stream_ptr()),
           "cf_point_gather_bwd")
     return gimg
 

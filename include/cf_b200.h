@@ -157,12 +157,27 @@ CF_API int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t *d_
  * (cf_fusion_bwd_workspace_bytes), for the (cell, k) slots that hold a neighbour only.
  * mode CF_MODE_FP32 / CF_MODE_BF16: the GEMMs run on tcgen05 (fp32 operands split into bf16 hi + lo, three MMAs,
  * fp32 accumulate -- gradients are fp32-accurate in both modes); CF_MODE_FP32_SIMT, or shapes without a
- * tensor-core instantiation: FFMA kernels.  Reductions over rows use atomics (reproducible to rounding).
+ * tensor-core instantiation: FFMA kernels.
+ * Two summation paths:
+ *   default            the live-cell / live-row lists are placed with atomics and the reductions over rows (dW, db,
+ *                      dT, d img) use float atomics: reproducible to rounding, not bit for bit.
+ *   deterministic      mode | CF_BWD_DETERMINISTIC, workspace cf_fusion_bwd_det_workspace_bytes: the lists come from
+ *                      device-wide scans (grid order), every row reduction writes per-split partials that are summed in
+ *                      a fixed order (the splits depend on shapes and on the device-side live counts only, not on the
+ *                      GPU's SM count), dT is a gather over each point's rows in ascending row order.  Identical inputs
+ *                      give bit-identical gradients on sm_100, in every mode and at every width; still no host
+ *                      synchronisation (capturable in a CUDA graph).
  * cf_point_gather_bwd is the adjoint of cf_point_gather: d_gimg (+)= bilinear scatter of d_gfeat; d_gimg has the
- * camera map's logical shape and the given element strides.
+ * camera map's logical shape and the given element strides.  cf_point_gather_bwd_det computes the same with a fixed
+ * order: the (point, tap) contributions are listed per pixel (counting sort, each list in ascending (point, tap)) and
+ * one thread per (pixel, channel) sums its list and adds the sum into d_gimg; workspace
+ * cf_point_gather_bwd_det_workspace_bytes(B, N, Hf, Wf).
  * ------------------------------------------------------------------------------------------- */
+#define CF_BWD_DETERMINISTIC 0x100 /* OR-ed into `mode` of cf_fusion_bwd */
 CF_API size_t cf_fusion_bwd_workspace_bytes(int32_t B, int32_t N, int32_t C, int32_t Ci, int32_t H, int32_t W,
                                             int32_t K);
+CF_API size_t cf_fusion_bwd_det_workspace_bytes(int32_t B, int32_t N, int32_t C, int32_t Ci, int32_t H, int32_t W,
+                                                int32_t K);
 CF_API int cf_fusion_bwd(const float *d_gout, const float *d_feat, const float *d_points,
                   const int64_t *d_num_points, const int32_t *d_knn_idx, int32_t B, int32_t N, int32_t C,
                   int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy,
@@ -173,6 +188,11 @@ CF_API int cf_point_gather_bwd(const float *d_gfeat, float *d_gimg, int64_t sb, 
                         int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
                         const float *d_uv, const float *h_calib, const int64_t *d_num_points, int32_t N,
                         float img_w, float img_h, void *stream);
+CF_API size_t cf_point_gather_bwd_det_workspace_bytes(int32_t B, int32_t N, int32_t Hf, int32_t Wf);
+CF_API int cf_point_gather_bwd_det(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sc, int64_t sh, int64_t sw,
+                            int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
+                            const float *d_uv, const float *h_calib, const int64_t *d_num_points, int32_t N,
+                            float img_w, float img_h, void *d_workspace, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Dataset side on the device (SURVEY 8f-2): CarlaDataset.Voxelization_Projection + .Projection,

@@ -43,7 +43,13 @@ def main(argv=None):
     ap.add_argument("--mse", action="store_true", help="close the step with an MSE instead of LossTotal")
     ap.add_argument("--graph", action="store_true", help="capture forward + backward + Adam as ONE CUDA graph and replay it "
                     "(single process only): the step time without the host's launch overhead")
+    ap.add_argument("--deterministic", action="store_true", help="torch.use_deterministic_algorithms(True): bit-reproducible "
+                    "gradients (the fusion layer's fixed-order backward, the trunk's matmul adjoint of the bilinear resizes)")
     a = ap.parse_args(argv)
+    if a.deterministic:
+        # before CUDA initialises: cuBLAS reads its workspace setting when the first handle is created
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")
+        torch.use_deterministic_algorithms(True)
     rank, world, local = dcf.dist_util.env_rank_world()
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -117,7 +123,7 @@ def main(argv=None):
     ms = dcf.dist_util.max_over_ranks([e0.elapsed_time(e1) / a.steps], device=dev)[0]
     res = {"what": "train step (fwd + bwd + Adam), ObjectDetection_DCF, YAML grid 384x256",
            "fusion": not a.no_fusion, "loss": "mse" if a.mse else "LossTotal (device target assignment)",
-           "launch": "cuda_graph_replay" if a.graph else "eager",
+           "launch": "cuda_graph_replay" if a.graph else "eager", "deterministic": a.deterministic,
            "batch_per_gpu": a.batch, "n_gpus": world, "steps": a.steps, "ms_per_step": round(ms, 3),
            "host_enqueue_ms_per_step": round(host_ms, 3),
            "frames_per_sec": round(a.batch * world / ms * 1e3, 1), "loss_value": float(loss)}
