@@ -12,6 +12,7 @@ CSRC = os.path.join(_PKG, "csrc")
 
 MODE_FP32, MODE_BF16, MODE_SIMT, MODE_BF16_TABLES = 0, 1, 2, 3
 BWD_DETERMINISTIC = 0x100   # CF_BWD_DETERMINISTIC: OR-ed into the mode of cf_fusion_bwd
+IO_BF16 = 0x200             # CF_IO_BF16: OR-ed into the mode of cf_fusion_fwd / cf_fusion_bwd for bf16 BEV maps
 # "bf16t" = CF_MODE_BF16_TABLES: bf16 operands AND bf16 layer-1 tables (inference only)
 MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "simt": MODE_SIMT, "bf16t": MODE_BF16_TABLES}
 MAX_K = 16
@@ -33,6 +34,8 @@ SIGNATURES = {
     "cf_gather_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i64]),
     "cf_point_gather": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp, C.POINTER(C.c_float),
                                   _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
+    "cf_point_gather_bf16": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp, C.POINTER(C.c_float),
+                                       _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
     "cf_point_mlp1_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "cf_point_mlp1": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "cf_point_mlp1_pack_weights": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),

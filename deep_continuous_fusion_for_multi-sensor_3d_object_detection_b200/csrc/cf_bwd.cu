@@ -274,8 +274,10 @@ __global__ void __launch_bounds__(256) k_bwd_compact(const int32_t *__restrict__
 }
 
 // G[ci, c] = gout[b, c, cell] for the live cells (32 cells x 32 channels per block through a shared-memory transpose;
-// list neighbours are mostly grid neighbours, so the reads of a warp still fall into few lines)
-__global__ void __launch_bounds__(256) k_bwd_gather_g(const float *__restrict__ gout, int32_t C, int64_t cells,
+// list neighbours are mostly grid neighbours, so the reads of a warp still fall into few lines).  The only reader of gout:
+// a bf16 gout (CF_IO_BF16) is widened exactly here, and everything downstream is the fp32 path.
+template <typename MT>
+__global__ void __launch_bounds__(256) k_bwd_gather_g(const MT *__restrict__ gout, int32_t C, int64_t cells,
                                                       const int32_t *__restrict__ cell_list,
                                                       const int32_t *__restrict__ counters, float *__restrict__ G)
 {
@@ -293,7 +295,7 @@ __global__ void __launch_bounds__(256) k_bwd_gather_g(const float *__restrict__ 
     }
     for (int r = ty; r < 32; r += 8) {
         const int32_t c = c0 + r;
-        tile[r][tx] = (src >= 0 && c < C) ? __ldg(gout + src + (int64_t)c * cells) : 0.0f;
+        tile[r][tx] = (src >= 0 && c < C) ? map_ldg(gout + src + (int64_t)c * cells) : 0.0f;
     }
     __syncthreads();
     for (int r = ty; r < 32; r += 8) {
@@ -535,7 +537,8 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     using namespace cf;
     CF_TRY(require_sm100());
     const bool det = (mode & CF_BWD_DETERMINISTIC) != 0;
-    mode &= ~CF_BWD_DETERMINISTIC;
+    const bool io16 = (mode & CF_IO_BF16) != 0;   // d_gout is a bf16 map
+    mode = mode_base(mode);
     CF_REQUIRE(d_gout && d_feat && d_points && d_num_points && d_knn_idx && d_W1 && d_b1 && d_W2 && d_b2 && d_W3 &&
                    d_gW1 && d_gb1 && d_gW2 && d_gb2 && d_gW3 && d_gb3 && d_gfeat && d_workspace,
                CF_ERR_ARG, "cf_fusion_bwd: null pointer");
@@ -645,8 +648,11 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
                                                               tc_row_nn ? 1 : 0);
 
     // ---- layer 3 ------------------------------------------------------------------------------------------------------
-    k_bwd_gather_g<<<dim3((unsigned)ceil_div64(ncell, 32), cchunks), 256, 0, st>>>(d_gout, C, cells, w.cell_list, w.counters,
-                                                                                  w.G);
+    const dim3 g_grid((unsigned)ceil_div64(ncell, 32), cchunks);
+    if (io16)
+        k_bwd_gather_g<<<g_grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16 *>(d_gout), C, cells, w.cell_list, w.counters, w.G);
+    else
+        k_bwd_gather_g<<<g_grid, 256, 0, st>>>(d_gout, C, cells, w.cell_list, w.counters, w.G);
     launches += 2;
     if (tc_row_tn) {
         CF_TRY(bwd_tc_gemm_tn(w.G, C, C, w.pooled, C, C, nullptr, 0, 0, 0, w.cell_nv, ncell, n_cells, d_gW3, C,

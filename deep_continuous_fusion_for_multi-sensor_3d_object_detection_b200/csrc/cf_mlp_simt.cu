@@ -103,13 +103,14 @@ __global__ void __launch_bounds__(256) k_transpose_sq(const float *__restrict__ 
     Wt[(size_t)i * C + o] = W[idx];
 }
 
-__global__ void __launch_bounds__(256) k_fusion_simt(const float *__restrict__ bev, const float *__restrict__ T,
+template <typename MT>   // map element: float, or __nv_bfloat16 (CF_IO_BF16: widened on load, rounded once on store)
+__global__ void __launch_bounds__(256) k_fusion_simt(const MT *__restrict__ bev, const float *__restrict__ T,
                                                      const int32_t *__restrict__ knn, int32_t N, int32_t C, int32_t H,
                                                      int32_t W, int32_t K, float x0, float y0, float dx, float dy,
                                                      const float *__restrict__ W1, int32_t Ci,
                                                      const float *__restrict__ Wt2, const float *__restrict__ b2,
                                                      const float *__restrict__ Wt3, const float *__restrict__ b3,
-                                                     float *__restrict__ out)
+                                                     MT *__restrict__ out)
 {
     extern __shared__ float smem[];
     const int32_t ldp = C + 1;
@@ -186,7 +187,7 @@ __global__ void __launch_bounds__(256) k_fusion_simt(const float *__restrict__ b
 #pragma unroll 8
             for (int kk = 0; kk < C; ++kk) s = fmaf(pr[kk], __ldg(Wt3 + (size_t)kk * C + c), s);
             const size_t o = ((size_t)b * C + c) * cells + cell;
-            out[o] = __ldg(bev + o) + s;
+            map_st(out + o, map_ldg(bev + o) + s);
         }
     }
 }
@@ -205,7 +206,7 @@ size_t fusion_simt_workspace_bytes(int32_t C) { return (size_t)2 * C * C * sizeo
 int fusion_simt(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_t B, int32_t N, int32_t C,
                 int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy, const float *d_W1,
                 int32_t Ci, const float *d_W2, const float *d_b2, const float *d_W3, const float *d_b3,
-                float *d_out, void *d_workspace, cudaStream_t st)
+                float *d_out, bool io16, void *d_workspace, cudaStream_t st)
 {
     float *Wt2 = (float *)d_workspace, *Wt3 = Wt2 + (size_t)C * C;
     const int tb = (C * C + 255) / 256;
@@ -215,14 +216,20 @@ int fusion_simt(const float *d_bev, const float *d_T, const int32_t *d_knn, int3
                         (size_t)(32 * CF_MAX_K + 32) * sizeof(int32_t);
     static bool attr_set = false;
     if (!attr_set) {
-        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_simt, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024),
+        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_simt<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024),
+                           "k_fusion_simt smem attribute"));
+        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_simt<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024),
                            "k_fusion_simt smem attribute"));
         attr_set = true;
     }
     const int64_t tiles = ceil_div64((int64_t)H * W, 32);
     const int gx = (int)std::min<int64_t>(tiles, (int64_t)sm_count() * 8);
-    k_fusion_simt<<<dim3(gx, B), 256, smem, st>>>(d_bev, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2,
-                                                  d_b2, Wt3, d_b3, d_out);
+    if (io16)
+        k_fusion_simt<<<dim3(gx, B), 256, smem, st>>>(reinterpret_cast<const __nv_bfloat16 *>(d_bev), d_T, d_knn, N, C, H, W, K, x0,
+                                                      y0, dx, dy, d_W1, Ci, Wt2, d_b2, Wt3, d_b3, reinterpret_cast<__nv_bfloat16 *>(d_out));
+    else
+        k_fusion_simt<<<dim3(gx, B), 256, smem, st>>>(d_bev, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2,
+                                                      d_b2, Wt3, d_b3, d_out);
     count_launches(3);
     return launch_status("cf_fusion_fwd (simt)");
 }
@@ -245,6 +252,7 @@ extern "C" int cf_point_mlp1_pack_weights(const float *d_W1, int32_t Ci, int32_t
 {
     using namespace cf;
     CF_TRY(require_sm100());
+    mode = mode_base(mode);
     CF_REQUIRE(d_W1 && d_packed && aligned16(d_packed), CF_ERR_ARG, "cf_point_mlp1_pack_weights: bad pointer");
     CF_REQUIRE(mode == CF_MODE_FP32 || mode == CF_MODE_BF16 || mode == CF_MODE_BF16_TABLES, CF_ERR_ARG,
                "cf_point_mlp1_pack_weights: mode %d has no packed form", mode);
@@ -253,6 +261,7 @@ extern "C" int cf_point_mlp1_pack_weights(const float *d_W1, int32_t Ci, int32_t
 
 extern "C" size_t cf_point_mlp1_workspace_bytes(int32_t Ci, int32_t C, int32_t mode)
 {
+    mode = cf::mode_base(mode);
     if (mode == CF_MODE_FP32_SIMT || Ci <= 0 || C <= 0) return 0;
     return cf::point_mlp1_tc_workspace_bytes(Ci, C, mode);
 }
@@ -263,6 +272,7 @@ extern "C" int cf_point_mlp1(const float *d_feat, const float *d_points, const i
 {
     using namespace cf;
     CF_TRY(require_sm100());
+    mode = mode_base(mode);
     CF_REQUIRE(d_feat && d_points && d_num_points && d_W1 && d_b1 && d_T, CF_ERR_ARG, "cf_point_mlp1: null pointer");
     CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && C > 0, CF_ERR_ARG, "cf_point_mlp1: bad extents");
     CF_REQUIRE(Ci % 4 == 0, CF_ERR_ARG, "cf_point_mlp1: Ci=%d must be a multiple of 4", Ci);
@@ -299,6 +309,7 @@ extern "C" int cf_point_mlp1_multi(const float *d_feat, const float *d_points, c
 {
     using namespace cf;
     CF_TRY(require_sm100());
+    mode = mode_base(mode);
     CF_REQUIRE(d_feat && d_points && d_num_points && h_C && h_W1 && h_b1 && h_T && h_packed, CF_ERR_ARG,
                "cf_point_mlp1_multi: null pointer");
     CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && n_scales > 0, CF_ERR_ARG, "cf_point_mlp1_multi: bad extents");

@@ -70,7 +70,7 @@ constexpr int kTile = 128;  // cells per tile == UMMA M
 constexpr int kThreads = 128;
 
 struct TcParams {
-    const float *bev;
+    const float *bev;      // bev / out: elements of the kernel's map type MT (float, or bf16 with CF_IO_BF16)
     const float *T;
     const int32_t *knn;
     float *out;
@@ -280,7 +280,7 @@ struct TcShape {
     static constexpr int kMinBlocks = C <= 32 ? CF_MB32 : C <= 64 ? CF_MB64 : 1;
 };
 
-template <int C, int NS, bool TH = false>
+template <int C, int NS, bool TH = false, typename MT = float>
 __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks) k_fusion_tc(const TcParams p)
 {
     using TT = typename TableT<TH>::type;   // fp32 tables, or bf16 tables in CF_MODE_BF16_TABLES (NS == 1)
@@ -529,7 +529,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             const uint32_t idx0 = sidx_addr + (uint32_t)((par * K * kTile + rg0 * 8 + r8) * 4);
             const uint32_t ctr0 = sctr_addr + (uint32_t)((par * kTile + rg0 * 8 + r8) * 16);
             const uint32_t dst0 = sA_addr + tc::unit_offset(r8, ku, kc_units) + (uint32_t)(rg0 * kc_units * 128);
-            const float *src_bev = p.bev + (size_t)b * C * cells + cell;
+            const MT *src_bev = reinterpret_cast<const MT *>(p.bev) + (size_t)b * C * cells + cell;
             // Pipelined shapes (both layers resident, 4 items per warp and round): tv holds the gathered neighbour rows
             // of the NEXT round while this round's MMA and epilogue run; in the last round the same 32 registers take the
             // bev values of this thread's first two output chunks instead.
@@ -543,7 +543,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                     for (int j = 0; j < 2; ++j) {
                         if (grp + j * G < kChunksE) {
 #pragma unroll
-                            for (int i = 0; i < EW; ++i) tv[j * EW + i] = __ldcs(src_bev + (size_t)((grp + j * G) * EW + i) * cells);
+                            for (int i = 0; i < EW; ++i) tv[j * EW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * EW + i) * cells);
                         }
                     }
                 }
@@ -736,7 +736,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // ---- final epilogue: out = bev + acc (thread = cell: a warp touches 128 contiguous bytes per channel) ---------
             __syncwarp();
             if (R > 0 || p.out != p.bev) {
-                float *dst_out = p.out + (size_t)b * C * cells + cell;
+                MT *dst_out = reinterpret_cast<MT *>(p.out) + (size_t)b * C * cells + cell;
 #pragma unroll
                 for (int j = 0; j < (kChunksE + G - 1) / G; ++j) {
                     const int cc = grp + j * G;
@@ -747,16 +747,16 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                             if (j < kPre) {
 #pragma unroll
                                 for (int i = 0; i < EW; ++i)
-                                    __stcs(dst_out + (size_t)(cc * EW + i) * cells, R > 0 ? tv[(j & 1) * EW + i] + z[i] : tv[(j & 1) * EW + i]);
+                                    map_stcs(dst_out + (size_t)(cc * EW + i) * cells, R > 0 ? tv[(j & 1) * EW + i] + z[i] : tv[(j & 1) * EW + i]);
                             } else {
 #pragma unroll
                                 for (int h = 0; h < EW; h += 8) {   // 8 loads in flight, then 8 stores
                                     float bv[8];
 #pragma unroll
-                                    for (int i = 0; i < 8; ++i) bv[i] = __ldcs(src_bev + (size_t)(cc * EW + h + i) * cells);
+                                    for (int i = 0; i < 8; ++i) bv[i] = map_ldcs(src_bev + (size_t)(cc * EW + h + i) * cells);
 #pragma unroll
                                     for (int i = 0; i < 8; ++i)
-                                        __stcs(dst_out + (size_t)(cc * EW + h + i) * cells, R > 0 ? bv[i] + z[h + i] : bv[i]);
+                                        map_stcs(dst_out + (size_t)(cc * EW + h + i) * cells, R > 0 ? bv[i] + z[h + i] : bv[i]);
                                 }
                             }
                         }
@@ -779,11 +779,12 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             if (uframe[u] >= 0 && ucell[u] >= 0) {   // uframe is uniform; ucell < 0: a row past the end of the list
                 constexpr int CG = C / G;
                 const size_t o = ((size_t)uframe[u] * C + grp * CG) * cells + ucell[u];
-                const float *src = p.bev + o;
-                float *dst = p.out + o;
+                using RB = typename MapBits<MT>::type;   // a bf16 map is copied as raw 16-bit elements
+                const RB *src = reinterpret_cast<const RB *>(p.bev) + o;
+                RB *dst = reinterpret_cast<RB *>(p.out) + o;
 #pragma unroll 1
                 for (int c = 0; c < CG; c += kCopyBatch) {   // kCopyBatch loads in flight per thread, then the stores
-                    float v[kCopyBatch];
+                    RB v[kCopyBatch];
 #pragma unroll
                     for (int i = 0; i < kCopyBatch; ++i) {
                         v[i] = __ldcs(src);
@@ -836,7 +837,7 @@ struct SkLayout {
     static constexpr int kTmemCols = tmem_cols_for(3 * C);          // two accumulators + the pooled sum
 };
 
-template <int C, int NS, bool TH = false>
+template <int C, int NS, bool TH = false, typename MT = float>
 __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks) k_fusion_sk(const TcParams p)
 {
     using TT = typename TableT<TH>::type;
@@ -1013,7 +1014,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             const uint32_t idx0 = sidx_addr + (uint32_t)((par * K * kTile + rg0 * 8 + r8) * 4);
             const uint32_t ctr0 = sctr_addr + (uint32_t)((par * kTile + rg0 * 8 + r8) * 8);
             const uint32_t dst0 = sA_addr + tc::unit_offset(r8, ku, kc_units) + (uint32_t)(rg0 * kc_units * 128);
-            const float *src_bev = p.bev + (size_t)b * C * cells + cell;
+            const MT *src_bev = reinterpret_cast<const MT *>(p.bev) + (size_t)b * C * cells + cell;
             float tv[32];   // neighbour rows of the next round to build; in the last round: bev values of the final epilogue
             auto gather_round = [&](int k) {
 #pragma unroll
@@ -1028,7 +1029,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                     for (int j = 0; j < 2; ++j) {
                         if (grp + j * G < kChunksE) {
 #pragma unroll
-                            for (int i = 0; i < EW; ++i) tv[j * EW + i] = __ldcs(src_bev + (size_t)((grp + j * G) * EW + i) * cells);
+                            for (int i = 0; i < EW; ++i) tv[j * EW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * EW + i) * cells);
                         }
                     }
                 }
@@ -1162,7 +1163,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             __syncwarp();
             if (R > 0 || p.out != p.bev) {
                 const uint32_t acc_l = tmem_base + (uint32_t)(((R - 1) & 1) * C) + lane_off;
-                float *dst_out = p.out + (size_t)b * C * cells + cell;
+                MT *dst_out = reinterpret_cast<MT *>(p.out) + (size_t)b * C * cells + cell;
 #pragma unroll
                 for (int j = 0; j < (kChunksE + G - 1) / G; ++j) {
                     const int cc = grp + j * G;
@@ -1173,16 +1174,16 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                             if (j < 2) {
 #pragma unroll
                                 for (int i = 0; i < EW; ++i)
-                                    __stcs(dst_out + (size_t)(cc * EW + i) * cells, R > 0 ? tv[(j & 1) * EW + i] + z[i] : tv[(j & 1) * EW + i]);
+                                    map_stcs(dst_out + (size_t)(cc * EW + i) * cells, R > 0 ? tv[(j & 1) * EW + i] + z[i] : tv[(j & 1) * EW + i]);
                             } else {
 #pragma unroll
                                 for (int h = 0; h < EW; h += 8) {
                                     float bv[8];
 #pragma unroll
-                                    for (int i = 0; i < 8; ++i) bv[i] = __ldcs(src_bev + (size_t)(cc * EW + h + i) * cells);
+                                    for (int i = 0; i < 8; ++i) bv[i] = map_ldcs(src_bev + (size_t)(cc * EW + h + i) * cells);
 #pragma unroll
                                     for (int i = 0; i < 8; ++i)
-                                        __stcs(dst_out + (size_t)(cc * EW + h + i) * cells, R > 0 ? bv[i] + z[h + i] : bv[i]);
+                                        map_stcs(dst_out + (size_t)(cc * EW + h + i) * cells, R > 0 ? bv[i] + z[h + i] : bv[i]);
                                 }
                             }
                         }
@@ -1201,11 +1202,12 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             if (uframe[u] >= 0 && ucell[u] >= 0) {
                 constexpr int CG = C / G;
                 const size_t o = ((size_t)uframe[u] * C + grp * CG) * cells + ucell[u];
-                const float *src = p.bev + o;
-                float *dst = p.out + o;
+                using RB = typename MapBits<MT>::type;
+                const RB *src = reinterpret_cast<const RB *>(p.bev) + o;
+                RB *dst = reinterpret_cast<RB *>(p.out) + o;
 #pragma unroll 1
                 for (int c = 0; c < CG; c += kCopyBatch) {
-                    float v[kCopyBatch];
+                    RB v[kCopyBatch];
 #pragma unroll
                     for (int i = 0; i < kCopyBatch; ++i) {
                         v[i] = __ldcs(src);
@@ -1799,7 +1801,7 @@ int resident_ctas(Kern kern, int threads, int smem, int tmem_cols, int *regs_cac
     return CF_OK;
 }
 
-template <int C, int NS, bool TH = false>
+template <int C, int NS, bool TH = false, typename MT = float>
 int launch_tc(const TcParams &p, cudaStream_t st)
 {
     using L = TcLayout<C, NS>;
@@ -1807,23 +1809,23 @@ int launch_tc(const TcParams &p, cudaStream_t st)
     const int smem = L::smem_bytes(p.K);
     static int attr_bytes = 0, regs = 0;
     if (smem > attr_bytes) {
-        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_tc<C, NS, TH>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_tc<C, NS, TH, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
                            "k_fusion_tc smem attribute"));
         attr_bytes = smem;
     }
     int per_sm = 1;
-    CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH>, NT, smem, L::kTmemCols, &regs, &per_sm));
+    CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH, MT>, NT, smem, L::kTmemCols, &regs, &per_sm));
     per_sm = std::max(1, per_sm);
     if (tuning().max_ctas > 0) per_sm = std::max(1, std::min(per_sm, tuning().max_ctas));
     const int64_t grid = std::min<int64_t>(p.tiles_total, (int64_t)sm_count() * per_sm);
     if (tuning().debug_launch) fprintf(stderr, "k_fusion_tc<%d,%d>: %d CTAs/SM grid %lld smem %d\n", C, NS, per_sm, (long long)grid, smem);
-    k_fusion_tc<C, NS, TH><<<(unsigned)grid, NT, smem, st>>>(p);
+    k_fusion_tc<C, NS, TH, MT><<<(unsigned)grid, NT, smem, st>>>(p);
     return CF_OK;
 }
 
 // The double-buffered kernel (k_fusion_sk) is used when its shared memory fits and it keeps the residency of k_fusion_tc;
 // returns CF_ERR_UNSUPPORTED (nothing launched) otherwise.  CF_NO_SKEW=1 forces k_fusion_tc (A/B measurements).
-template <int C, int NS, bool TH = false>
+template <int C, int NS, bool TH = false, typename MT = float>
 int launch_sk(const TcParams &p, cudaStream_t st)
 {
     using L = SkLayout<C, NS>;
@@ -1833,18 +1835,18 @@ int launch_sk(const TcParams &p, cudaStream_t st)
     if (smem > 227 * 1024 || tuning().no_skew) return CF_ERR_UNSUPPORTED;
     static int attr_bytes = 0, regs = 0, regs0 = 0;
     int per_sm = 0, per_sm0 = 0;
-    CF_TRY(resident_ctas(k_fusion_sk<C, NS, TH>, NT, smem, L::kTmemCols, &regs, &per_sm));
-    CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH>, NT, L0::smem_bytes(p.K), L0::kTmemCols, &regs0, &per_sm0));
+    CF_TRY(resident_ctas(k_fusion_sk<C, NS, TH, MT>, NT, smem, L::kTmemCols, &regs, &per_sm));
+    CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH, MT>, NT, L0::smem_bytes(p.K), L0::kTmemCols, &regs0, &per_sm0));
     if (per_sm < 1 || per_sm < per_sm0) return CF_ERR_UNSUPPORTED;
     if (smem > attr_bytes) {
-        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_sk<C, NS, TH>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
+        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_sk<C, NS, TH, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
                            "k_fusion_sk smem attribute"));
         attr_bytes = smem;
     }
     if (tuning().max_ctas > 0) per_sm = std::max(1, std::min(per_sm, tuning().max_ctas));
     const int64_t grid = std::min<int64_t>(p.tiles_total, (int64_t)sm_count() * per_sm);
     if (tuning().debug_launch) fprintf(stderr, "k_fusion_sk<%d,%d>: %d CTAs/SM grid %lld smem %d\n", C, NS, per_sm, (long long)grid, smem);
-    k_fusion_sk<C, NS, TH><<<(unsigned)grid, NT, smem, st>>>(p);
+    k_fusion_sk<C, NS, TH, MT><<<(unsigned)grid, NT, smem, st>>>(p);
     return CF_OK;
 }
 
@@ -1856,12 +1858,12 @@ int fusion_seg(const float *d_bev, const float *d_T, const int32_t *d_knn, int32
 
 static size_t tc_weight_bytes(int32_t C, int NS) { return ((size_t)2 * NS * C * C * 2 + 255) / 256 * 256; }
 
-size_t fusion_tc_packed_bytes(int32_t C, int32_t mode) { return tc_weight_bytes(C, mode == CF_MODE_FP32 ? 2 : 1); }
+size_t fusion_tc_packed_bytes(int32_t C, int32_t mode) { return tc_weight_bytes(C, mode_base(mode) == CF_MODE_FP32 ? 2 : 1); }
 
 int fusion_tc_pack(const float *d_W2, const float *d_W3, int32_t C, int32_t mode, void *d_packed, cudaStream_t st)
 {
     CF_REQUIRE(C % 32 == 0 && C >= 32 && C <= 256, CF_ERR_UNSUPPORTED, "cf_fusion_pack_weights: C=%d", C);
-    const int NS = mode == CF_MODE_FP32 ? 2 : 1;
+    const int NS = mode_base(mode) == CF_MODE_FP32 ? 2 : 1;
     const int KC = kc_for(C, NS);
     const int pack_blocks = (C * (C / 8) + 255) / 256;
     k_pack_weights<<<pack_blocks, 256, 0, st>>>(d_W2, C, C, C, KC, NS, (uint8_t *)d_packed);
@@ -1872,7 +1874,7 @@ int fusion_tc_pack(const float *d_W2, const float *d_W3, int32_t C, int32_t mode
 
 size_t fusion_tc_workspace_bytes(int32_t C, int32_t mode, int32_t B, int32_t H, int32_t W)
 {
-    const int NS = mode == CF_MODE_FP32 ? 2 : 1;
+    const int NS = mode_base(mode) == CF_MODE_FP32 ? 2 : 1;
     // packed W2/W3 images | per-frame counts (with / without a neighbour) | per-frame cell lists
     return tc_weight_bytes(C, NS) + 512 + (size_t)B * H * W * sizeof(int32_t);
 }
@@ -1883,6 +1885,8 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
               const void *d_packed, void *d_workspace, cudaStream_t st)
 {
     CF_REQUIRE(C % 32 == 0, CF_ERR_UNSUPPORTED, "cf_fusion_fwd: tensor-core path needs C %% 32 == 0 (C=%d)", C);
+    const bool io16 = (mode & CF_IO_BF16) != 0;   // d_bev / d_out hold bf16 maps
+    mode = mode_base(mode);
     const int NS = mode == CF_MODE_FP32 ? 2 : 1;
     const int KC = kc_for(C, NS);
     // packed W2 | W3 operand images: the caller's cached copy (cf_fusion_pack_weights) or packed here
@@ -1906,7 +1910,7 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     const bool compact = ceil_div64(n_cells, kTile) * B >= min_tiles;
     // fine scales (many more tiles than SMs): segment tiles, all neighbour slots in one MMA batch (cf_fusion_seg.cu); its
     // lists live where the cell lists of the kernels below would
-    if (compact && tuning().seg && mode != CF_MODE_BF16_TABLES) {
+    if (compact && tuning().seg && mode != CF_MODE_BF16_TABLES && !io16) {
         const int rc = fusion_seg(d_bev, d_T, d_knn, B, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, d_b2, d_b3, d_out, mode, img2,
                                   img3, cell_count, st);
         if (rc != CF_ERR_UNSUPPORTED) return rc;
@@ -1928,15 +1932,17 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     p.copy_dead = compact && d_out != d_bev;
     int rc = CF_ERR_UNSUPPORTED;
     const bool th = mode == CF_MODE_BF16_TABLES;   // d_T holds bf16 rows
+#define CF_TC_LAUNCH(fn, c, MT) \
+    (NS == 2 ? fn<c, 2, false, MT>(p, st) : th ? fn<c, 1, true, MT>(p, st) : fn<c, 1, false, MT>(p, st))
 #define CF_TC_CASE(c)                                                                                          \
     case c:                                                                                                    \
-        rc = NS == 2 ? launch_tc<c, 2>(p, st) : th ? launch_tc<c, 1, true>(p, st) : launch_tc<c, 1>(p, st);    \
+        rc = io16 ? CF_TC_LAUNCH(launch_tc, c, __nv_bfloat16) : CF_TC_LAUNCH(launch_tc, c, float);             \
         break;
 #define CF_SK_CASE(c)                                                                                          \
     case c:                                                                                                    \
-        rc = NS == 2 ? launch_sk<c, 2>(p, st) : th ? launch_sk<c, 1, true>(p, st) : launch_sk<c, 1>(p, st);    \
+        rc = io16 ? CF_TC_LAUNCH(launch_sk, c, __nv_bfloat16) : CF_TC_LAUNCH(launch_sk, c, float);             \
         if (rc == CF_ERR_UNSUPPORTED)                                                                          \
-            rc = NS == 2 ? launch_tc<c, 2>(p, st) : th ? launch_tc<c, 1, true>(p, st) : launch_tc<c, 1>(p, st); \
+            rc = io16 ? CF_TC_LAUNCH(launch_tc, c, __nv_bfloat16) : CF_TC_LAUNCH(launch_tc, c, float);         \
         break;
     switch (C) {
         // measured on B200 (profiles/README.md): the double-buffered kernel wins where the MMAs of a round are long
@@ -1948,6 +1954,7 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     }
 #undef CF_TC_CASE
 #undef CF_SK_CASE
+#undef CF_TC_LAUNCH
     CF_TRY(rc);
     count_launches(1);
     return launch_status("cf_fusion_fwd (tcgen05)");

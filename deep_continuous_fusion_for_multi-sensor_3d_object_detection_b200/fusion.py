@@ -197,16 +197,19 @@ class FusionRunner:
     A serving loop copies a batch into `.points (B,N,3)`, `.num_points (B,) int64`, `.img_feat (B,Ci,Hf,Wf)` and
     `.bevs[s] (B,C_s,H_s,W_s)` (e.g. straight from pinned host memory), calls the runner, and reads `.outs[s]`
     (the same tensors as `.bevs` when `inplace=True`).  Replaying the graph costs one launch on the host instead of the
-    ~20 launches and several stream hand-offs of the eager path, which matters when the host is the slow side."""
+    ~20 launches and several stream hand-offs of the eager path, which matters when the host is the slow side.
+    `dtype=torch.bfloat16`: `.img_feat`, `.bevs` and `.outs` are bf16 maps (half the bytes to copy in and out)."""
 
     def __init__(self, layers, grid, batch, max_points, img_shape, bev_shapes, calib=None, img_size=(640.0, 480.0),
-                 inplace=True, device=None):
+                 inplace=True, device=None, dtype=torch.float32):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.layers, self.grid, self.calib, self.img_size, self.inplace = list(layers), grid, calib, tuple(img_size), inplace
         self.points = torch.zeros((batch, max_points, 3), dtype=torch.float32, device=dev)
         self.num_points = torch.zeros((batch,), dtype=torch.int64, device=dev)
-        self.img_feat = torch.zeros((batch,) + tuple(img_shape), dtype=torch.float32, device=dev)
-        self.bevs = [torch.zeros((batch,) + tuple(sh), dtype=torch.float32, device=dev) for sh in bev_shapes]
+        if dtype not in ops.MAP_DTYPES:
+            raise TypeError(f"FusionRunner: dtype must be torch.float32 or torch.bfloat16, got {dtype}")
+        self.img_feat = torch.zeros((batch,) + tuple(img_shape), dtype=dtype, device=dev)
+        self.bevs = [torch.zeros((batch,) + tuple(sh), dtype=dtype, device=dev) for sh in bev_shapes]
         self.outs = None
         self.graph = None
         side = torch.cuda.Stream(dev)
@@ -330,6 +333,8 @@ class ContinuousFusion(nn.Module):
 
     def forward(self, bev, img_feat=None, points=None, num_points=None, calib=None, uv=None, frames: FrameContext = None,
                 geom=None, return_knn: bool = False, out=None):
+        """Returns a map of bev's dtype: fp32, or bf16 (under torch.autocast the maps arrive in bf16; autocast does not cast
+        the inputs of this layer, which widens bf16 maps exactly and computes in fp32 with fp32 weights)."""
         geom = tuple(float(g) for g in geom) if geom is not None else self.geom
         if geom is None:
             raise ValueError("ContinuousFusion: BEV geometry (x0,y0,dx,dy) not set")

@@ -31,6 +31,16 @@ def _contig(t: torch.Tensor, name: str, dtype, ndim=None):
     return t if t.is_contiguous() else t.contiguous()
 
 
+MAP_DTYPES = (torch.float32, torch.bfloat16)   # feature maps (BEV, camera, their gradients): fp32, or bf16 under autocast
+
+
+def _map(t: torch.Tensor, name: str, ndim=4):
+    """A feature map: fp32, or bf16 (widened exactly to fp32 by the kernels, results rounded once when stored)."""
+    if isinstance(t, torch.Tensor) and t.is_cuda and t.dtype not in MAP_DTYPES:
+        raise TypeError(f"{name}: expected dtype torch.float32 or torch.bfloat16 (the supported half type), got {t.dtype}")
+    return _req(t, name, t.dtype if isinstance(t, torch.Tensor) else torch.float32, ndim)
+
+
 def _scratch(nbytes: int, device) -> torch.Tensor:
     """Workspace that the kernels write before they read it.  torch.use_deterministic_algorithms(True) makes torch.empty fill
     new memory (hundreds of MB per backward call here); scratch needs no fill, so it is allocated without one."""
@@ -168,10 +178,11 @@ def knn_subsample(knn_fine, step, Hc, Wc):
 
 
 def point_gather(img_feat, points, num_points, calib=None, uv=None, img_size=(640.0, 480.0), out=None, workspace=None):
-    """K-3.  img_feat logical (B,Ci,Hf,Wf) (any strides; channels_last avoids the re-layout pass),
-    points (B,N,3), exactly one of calib ((4,3) array, host) / uv ((B,N,2) device) -> feat (B,N,Ci)."""
+    """K-3.  img_feat logical (B,Ci,Hf,Wf) fp32 or bf16 (any strides; channels_last avoids the re-layout pass),
+    points (B,N,3), exactly one of calib ((4,3) array, host) / uv ((B,N,2) device) -> feat (B,N,Ci) fp32.
+    A bf16 map gives exactly the features of the same map widened to fp32."""
     lib = load()
-    _req(img_feat, "img_feat", torch.float32, 4)
+    _map(img_feat, "img_feat")
     points = _contig(points, "points", torch.float32, 3)
     B, Ci, Hf, Wf = img_feat.shape
     N = points.shape[1]
@@ -190,9 +201,9 @@ def point_gather(img_feat, points, num_points, calib=None, uv=None, img_size=(64
     need = lib.cf_gather_workspace_bytes(B, Ci, Hf, Wf, sc)
     if need and (workspace is None or workspace.numel() < need):
         workspace = torch.empty((need,), dtype=torch.uint8, device=points.device)
-    check(lib.cf_point_gather(ptr(img_feat), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv), calib_arr,
-                              ptr(num_points), N, float(img_size[0]), float(img_size[1]), ptr(out), ptr(workspace),
-                              stream_ptr()), "cf_point_gather")
+    fn = lib.cf_point_gather_bf16 if img_feat.dtype == torch.bfloat16 else lib.cf_point_gather
+    check(fn(ptr(img_feat), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv), calib_arr, ptr(num_points), N,
+             float(img_size[0]), float(img_size[1]), ptr(out), ptr(workspace), stream_ptr()), "cf_point_gather")
     return out, workspace
 
 
@@ -326,17 +337,21 @@ def point_mlp1_multi(feat, points, num_points, W1s, b1s, packeds, mode="fp32", o
 
 
 def fusion_fwd(bev, T, knn_idx, geom, W1, W2, b2, W3, b3, mode="fp32", out=None, workspace=None, packed=None):
-    """K-4.  out = bev + W3 sum_k relu(W2 relu(T[idx_k] - e_cell) + b2) + n_valid b3."""
+    """K-4.  out = bev + W3 sum_k relu(W2 relu(T[idx_k] - e_cell) + b2) + n_valid b3.
+    `bev` (and `out`, which must have bev's dtype) fp32 or bf16: a bf16 map is widened exactly, the layer computes in fp32 as
+    for an fp32 map and `out` is rounded once to bf16 -- equal to the fp32 result on bev.float(), rounded."""
     lib = load()
-    _req(bev, "bev", torch.float32, 4)
+    _map(bev, "bev")
     if out is not None:
-        _req(out, "out", torch.float32, 4)
+        _map(out, "out")
+        if out.dtype != bev.dtype:
+            raise ValueError(f"fusion_fwd: out must have bev's dtype {bev.dtype}, got {out.dtype}")
         if out.shape != bev.shape or out.device != bev.device or not out.is_contiguous():
             raise ValueError(f"fusion_fwd: out must be a contiguous (dense NCHW) tensor of bev's shape {tuple(bev.shape)} on "
                              f"{bev.device}, got shape {tuple(out.shape)}, strides {out.stride()}, device {out.device}")
         if out.data_ptr() == bev.data_ptr() and not bev.is_contiguous():
             raise ValueError("fusion_fwd: in-place operation (out is bev) needs a contiguous (dense NCHW) map")
-    bev = _contig(bev, "bev", torch.float32, 4)
+    bev = _contig(bev, "bev", bev.dtype, 4)
     T = _contig(T, "T", table_dtype(mode), 3)
     knn_idx = _contig(knn_idx, "knn_idx", torch.int32, 4)
     B, Cc, H, W = bev.shape
@@ -357,6 +372,8 @@ def fusion_fwd(bev, T, knn_idx, geom, W1, W2, b2, W3, b3, mode="fp32", out=None,
     if out is None:
         out = torch.empty_like(bev)
     x0, y0, dx, dy = [float(g) for g in geom]
+    if bev.dtype == torch.bfloat16:
+        m |= _lib.IO_BF16
     check(lib.cf_fusion_fwd(ptr(bev), ptr(T), ptr(knn_idx), B, N, Cc, H, W, K, x0, y0, dx, dy, ptr(W1), Ci, ptr(W2),
                             ptr(b2), ptr(W3), ptr(b3), ptr(out), m, ptr(packed), ptr(workspace), stream_ptr()),
           "cf_fusion_fwd")
@@ -368,9 +385,11 @@ def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2
     """K-4b.  Returns (gW1, gb1, gW2, gb2, gW3, gb3, gfeat); d bev is grad_out itself.
     `table`: the forward's point_mlp1 output (B,N,C) if it was kept (else it is recomputed); `mode` "simt" keeps every
     GEMM on CUDA cores, any other mode runs them on tcgen05 with fp32-accurate split operands.
-    `deterministic`: fixed summation order everywhere (CF_BWD_DETERMINISTIC): identical inputs give bit-identical gradients."""
+    `deterministic`: fixed summation order everywhere (CF_BWD_DETERMINISTIC): identical inputs give bit-identical gradients.
+    `grad_out` fp32 or bf16 (widened exactly; every gradient is fp32)."""
     lib = load()
-    grad_out = _contig(grad_out, "grad_out", torch.float32, 4)
+    _map(grad_out, "grad_out")
+    grad_out = _contig(grad_out, "grad_out", grad_out.dtype, 4)
     feat = _contig(feat, "feat", torch.float32, 3)
     points = _contig(points, "points", torch.float32, 3)
     knn_idx = _contig(knn_idx, "knn_idx", torch.int32, 4)
@@ -392,6 +411,8 @@ def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2
     m = _lib.MODES[mode] if isinstance(mode, str) else int(mode)
     if deterministic:
         m |= _lib.BWD_DETERMINISTIC
+    if grad_out.dtype == torch.bfloat16:
+        m |= _lib.IO_BF16
     x0, y0, dx, dy = [float(g) for g in geom]
     check(lib.cf_fusion_bwd(ptr(grad_out), ptr(feat), ptr(points), ptr(num_points), ptr(knn_idx), B, N, Cc, H, W, K, x0, y0,
                             dx, dy, ptr(W1), ptr(b1), Ci, ptr(W2), ptr(b2), ptr(W3), ptr(table), ptr(gW1), ptr(gb1), ptr(gW2),
@@ -401,12 +422,14 @@ def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2
 
 def point_gather_bwd(grad_feat, img_like, points, num_points, calib=None, uv=None, img_size=(640.0, 480.0),
                      deterministic=False):
-    """Adjoint of point_gather: gradient w.r.t. the camera feature map (same shape / memory format as img_like).
-    `deterministic`: each pixel sums its (point, tap) contributions in a fixed order (cf_point_gather_bwd_det)."""
+    """Adjoint of point_gather: gradient w.r.t. the camera feature map (same shape, dtype and memory format as img_like).
+    `deterministic`: each pixel sums its (point, tap) contributions in a fixed order (cf_point_gather_bwd_det).
+    A bf16 img_like: the taps are summed into an fp32 map, which is rounded to bf16 once at the end."""
     lib = load()
+    _map(img_like, "img_like")
     grad_feat = _contig(grad_feat, "grad_feat", torch.float32, 3)
     points = _contig(points, "points", torch.float32, 3)
-    gimg = torch.zeros_like(img_like)
+    gimg = torch.zeros_like(img_like, dtype=torch.float32)
     B, Ci, Hf, Wf = gimg.shape
     sb, sc, sh, sw = gimg.stride()
     calib_arr = None
@@ -420,11 +443,11 @@ def point_gather_bwd(grad_feat, img_like, points, num_points, calib=None, uv=Non
         check(lib.cf_point_gather_bwd_det(ptr(grad_feat), ptr(gimg), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv),
                                           calib_arr, ptr(num_points), N, float(img_size[0]), float(img_size[1]), ptr(ws),
                                           stream_ptr()), "cf_point_gather_bwd_det")
-        return gimg
-    check(lib.cf_point_gather_bwd(ptr(grad_feat), ptr(gimg), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv), calib_arr,
-                                  ptr(num_points), N, float(img_size[0]), float(img_size[1]), stream_ptr()),
-          "cf_point_gather_bwd")
-    return gimg
+    else:
+        check(lib.cf_point_gather_bwd(ptr(grad_feat), ptr(gimg), sb, sc, sh, sw, B, Ci, Hf, Wf, ptr(points), ptr(uv), calib_arr,
+                                      ptr(num_points), N, float(img_size[0]), float(img_size[1]), stream_ptr()),
+              "cf_point_gather_bwd")
+    return gimg.to(img_like.dtype)   # a no-op for fp32; bf16 keeps the memory format (preserve_format)
 
 
 # ------------------------------------------------------------------------------------------ post-process

@@ -97,12 +97,19 @@ CF_API int cf_knn_subsample(const int32_t *d_fine, int32_t B, int32_t Hf, int32_
  *               or h_calib, 12 HOST floats = CRT_tensor (4,3), data_import_carla.py:31-34,199-200
  *   d_feat      (B,N,Ci) fp32 out; rows >= num_points[b] are zero filled
  *   d_workspace cf_gather_workspace_bytes(...) bytes (pixel-major copy of the map when sc != 1)
+ * cf_point_gather_bf16: the same with a bf16 camera map (any element strides; channels_last: every pixel 8-byte
+ *   aligned; same workspace, an upper bound for its bf16 pixel-major copy).  Each tap is widened exactly to fp32 and the
+ *   blend is the fp32 sequence of cf_point_gather, so the result equals cf_point_gather on the widened map; d_feat is fp32.
  * ------------------------------------------------------------------------------------------- */
 CF_API size_t cf_gather_workspace_bytes(int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc);
 CF_API int cf_point_gather(const float *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B,
                     int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_uv,
                     const float *h_calib, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
                     float *d_feat, void *d_workspace, void *stream);
+CF_API int cf_point_gather_bf16(const void *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B,
+                         int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_uv,
+                         const float *h_calib, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
+                         float *d_feat, void *d_workspace, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K-4a per-point half of MLP layer 1 (exact factorisation of Appendix A8/A9):
@@ -140,7 +147,14 @@ CF_API int cf_fusion_pack_weights(const float *d_W2, const float *d_W3, int32_t 
  *   d_bev/d_out (B,C,H,W) fp32 NCHW contiguous (may alias: in place); C % 16 == 0, 16 <= C <= 256; d_T 32-byte aligned.
  *   mode: CF_MODE_*.   d_workspace: cf_fusion_workspace_bytes(C, mode, B, H, W) bytes (packed weights and the
  *   compacted list of cells that have a neighbour).  B <= 64 frames per call.
+ *   mode | CF_IO_BF16: d_bev and d_out are bf16 (B,C,H,W) NCHW maps (may alias, as for fp32).  bev is widened exactly to
+ *   fp32, everything else is computed as without the flag and out is rounded once to bf16 (nearest even) when stored:
+ *   the result equals the fp32 call on the widened map, rounded.  T, weights and the workspace size are unchanged.
+ *   The opt-in segment-tile kernel (CF_SEG=1) is fp32-only and is skipped with this flag.
+ * Every function that takes a `mode` ignores the flag bits (CF_IO_BF16, CF_BWD_DETERMINISTIC) when it picks the
+ * arithmetic, the operand layout or a workspace size.
  * ------------------------------------------------------------------------------------------- */
+#define CF_IO_BF16 0x200 /* OR-ed into `mode` of cf_fusion_fwd (bf16 bev / out) and cf_fusion_bwd (bf16 d_gout) */
 CF_API size_t cf_fusion_workspace_bytes(int32_t C, int32_t mode, int32_t B, int32_t H, int32_t W);
 CF_API int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t *d_knn_idx, int32_t B, int32_t N,
                   int32_t C, int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy,
@@ -150,7 +164,8 @@ CF_API int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t *d_
 
 /* ---------------------------------------------------------------------------------------------
  * K-4b backward of cf_point_mlp1 + cf_fusion_fwd for one scale (training only).  d_gout = dL/d out (B,C,H,W);
- * dL/d bev is d_gout itself.  Gradients are ACCUMULATED into d_gW1 (C,Ci+3), d_gb1 (C), d_gW2 (C,C), d_gb2,
+ * dL/d bev is d_gout itself.  mode | CF_IO_BF16: d_gout is bf16 (widened exactly on load; combines with
+ * CF_BWD_DETERMINISTIC, and with it the gradients equal those of the fp32 call on the widened d_gout).  Gradients are ACCUMULATED into d_gW1 (C,Ci+3), d_gb1 (C), d_gW2 (C,C), d_gb2,
  * d_gW3, d_gb3 and d_gfeat (B,N,Ci) -- zero them first (d_gfeat collects every scale's contribution).
  * The forward saves only indices, inputs and weights (and, optionally, its table: d_T = the output of
  * cf_point_mlp1, NULL = recompute it); H1/H2/pooled are recomputed into the workspace
@@ -171,7 +186,8 @@ CF_API int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t *d_
  * camera map's logical shape and the given element strides.  cf_point_gather_bwd_det computes the same with a fixed
  * order: the (point, tap) contributions are listed per pixel (counting sort, each list in ascending (point, tap)) and
  * one thread per (pixel, channel) sums its list and adds the sum into d_gimg; workspace
- * cf_point_gather_bwd_det_workspace_bytes(B, N, Hf, Wf).
+ * cf_point_gather_bwd_det_workspace_bytes(B, N, Hf, Wf).  d_gimg is fp32; for a bf16 camera map accumulate into an fp32
+ * buffer and round it once (summing the taps in bf16 would lose precision and the fixed order's guarantee).
  * ------------------------------------------------------------------------------------------- */
 #define CF_BWD_DETERMINISTIC 0x100 /* OR-ed into `mode` of cf_fusion_bwd */
 CF_API size_t cf_fusion_bwd_workspace_bytes(int32_t B, int32_t N, int32_t C, int32_t Ci, int32_t H, int32_t W,

@@ -45,6 +45,8 @@ def main(argv=None):
                     "(single process only): the step time without the host's launch overhead")
     ap.add_argument("--deterministic", action="store_true", help="torch.use_deterministic_algorithms(True): bit-reproducible "
                     "gradients (the fusion layer's fixed-order backward, the trunk's matmul adjoint of the bilinear resizes)")
+    ap.add_argument("--amp", action="store_true", help="forward and loss under torch.autocast('cuda', dtype=torch.bfloat16): "
+                    "bf16 convolutions, bf16 BEV / camera maps through the fusion layer (fp32 weights and gradients)")
     a = ap.parse_args(argv)
     if a.deterministic:
         # before CUDA initialises: cuBLAS reads its workspace setting when the first handle is created
@@ -78,10 +80,14 @@ def main(argv=None):
     extra = {} if a.no_fusion else dict(pointcloud_raw=to(wl["points"]), num_points_raw=to(wl["num_points"]),
                                         projected_loc_uv=to(wl["uv"]))
 
+    # the autocast weight cache would hold casts made during a graph capture outside the graph's pool: off under --graph
+    amp = lambda: torch.autocast("cuda", dtype=torch.bfloat16, enabled=a.amp, cache_enabled=not a.graph)
+
     def step():
         opt.zero_grad(set_to_none=True)
-        pred = model(x_lidar, x_image, **extra)
-        loss = closing_loss(pred)
+        with amp():
+            pred = model(x_lidar, x_image, **extra)
+            loss = closing_loss(pred)
         loss.backward()
         opt.step()
         return loss
@@ -99,8 +105,9 @@ def main(argv=None):
         graph = torch.cuda.CUDAGraph()
         opt.zero_grad(set_to_none=True)
         with torch.cuda.graph(graph):
-            pred = model(x_lidar, x_image, **extra)
-            static_loss = closing_loss(pred)
+            with amp():
+                pred = model(x_lidar, x_image, **extra)
+                static_loss = closing_loss(pred)
             static_loss.backward()
             opt.step()
 
@@ -124,6 +131,7 @@ def main(argv=None):
     res = {"what": "train step (fwd + bwd + Adam), ObjectDetection_DCF, YAML grid 384x256",
            "fusion": not a.no_fusion, "loss": "mse" if a.mse else "LossTotal (device target assignment)",
            "launch": "cuda_graph_replay" if a.graph else "eager", "deterministic": a.deterministic,
+           "amp": "bf16" if a.amp else None,
            "batch_per_gpu": a.batch, "n_gpus": world, "steps": a.steps, "ms_per_step": round(ms, 3),
            "host_enqueue_ms_per_step": round(host_ms, 3),
            "frames_per_sec": round(a.batch * world / ms * 1e3, 1), "loss_value": float(loss)}
