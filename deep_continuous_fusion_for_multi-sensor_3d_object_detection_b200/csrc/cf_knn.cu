@@ -8,8 +8,6 @@
 // strictly below a conservative lower bound of everything not yet visited, or when the bounding
 // square of the radius disc is exhausted.  Distances use __fsub_rn/__fmul_rn/__fadd_rn so no FMA
 // contraction can make d2 differ from the CPU oracle (Appendix A2).
-#include <stdlib.h>
-
 #include "cf_common.cuh"
 
 namespace cf {
@@ -307,20 +305,13 @@ __global__ void __launch_bounds__(128) k_knn_patch(const int32_t *__restrict__ b
     }
 }
 
-// CF_KNN_NO_PATCH (A/B measurements only): read from the environment once
-static bool knn_no_patch()
-{
-    static const bool v = getenv("CF_KNN_NO_PATCH") != nullptr;
-    return v;
-}
-
 template <int K>
 static void launch_knn(const int32_t *bs, const float4 *sp, int32_t B, int32_t N, const BucketGrid &g,
                        const KnnGeom &q, int32_t *out, cudaStream_t st)
 {
     // fine scales (patch of 4 x 8 cells small against the radius): warp-per-patch kernel; coarse scales: thread per cell
     const float hx = 0.5f * (kPatchI - 1) * fabsf(q.dx), hy = 0.5f * (kPatchJ - 1) * fabsf(q.dy);
-    const bool use_patch = sqrtf(hx * hx + hy * hy) <= 0.75f * q.radius && !knn_no_patch();
+    const bool use_patch = sqrtf(hx * hx + hy * hy) <= 0.75f * q.radius;
     if (use_patch) {
         const int64_t patches = (int64_t)((q.H + kPatchI - 1) / kPatchI) * ((q.W + kPatchJ - 1) / kPatchJ);
         dim3 grid((unsigned)ceil_div64(patches, 4), (unsigned)B);

@@ -40,25 +40,19 @@
 
 namespace cf {
 
-// tuning aids (A/B measurements only), read from the environment ONCE, when the library first launches a fused kernel
+// debugging aids, read from the environment ONCE, when the library first launches a fused kernel.  Neither selects a
+// kernel for speed: CF_DEBUG_LAUNCH only prints, and CF_NO_TMA_STORE reaches the direct-store fallback (the path taken
+// when the tensor maps cannot be encoded) so that tests can compare it with the TMA-store path.
 struct Tuning {
-    int max_ctas = 0;             // CF_MAX_CTAS: cap on resident CTAs per SM of the persistent fused kernels
     bool debug_launch = false;    // CF_DEBUG_LAUNCH: print the launch shape
-    bool no_skew = false;         // CF_NO_SKEW: never use the double-buffered kernel
-    bool seg = false;             // CF_SEG: route the fine scales through the segment-tile kernel (cf_fusion_seg.cu)
     bool no_tma_store = false;    // CF_NO_TMA_STORE: the layer-1 kernel stores every tile directly (the path taken without tensor maps)
-    long long compact_min_tiles = -1;   // CF_COMPACT_MIN_TILES
 };
 static const Tuning &tuning()
 {
     static const Tuning t = [] {
         Tuning v;
-        if (const char *e = getenv("CF_MAX_CTAS")) v.max_ctas = atoi(e);
         v.debug_launch = getenv("CF_DEBUG_LAUNCH") != nullptr;
-        v.no_skew = getenv("CF_NO_SKEW") != nullptr;
-        v.seg = getenv("CF_SEG") != nullptr;
         v.no_tma_store = getenv("CF_NO_TMA_STORE") != nullptr;
-        if (const char *e = getenv("CF_COMPACT_MIN_TILES")) v.compact_min_tiles = atoll(e);
         return v;
     }();
     return t;
@@ -94,34 +88,13 @@ __host__ __device__ constexpr int kc_for(int C, int NS)
     return C <= 128 ? C : 64;
 }
 
-// launch shape of the two small-C instantiations (measured on B200, BASELINE configs[1]: several small CTAs per SM --
-// more independent tiles in flight -- beat fewer barrier rounds per tile; see profiles/README.md)
-#ifndef CF_PIPE
-#define CF_PIPE 1
-#endif
-#ifndef CF_FETCH_UNITS_MINC
-#define CF_FETCH_UNITS_MINC 32
-#endif
-#ifndef CF_PIPE_MAXC
-#define CF_PIPE_MAXC 128
-#endif
-#ifndef CF_G32
-#define CF_G32 1
-#define CF_G64 2
-#define CF_MB32 4
-#define CF_MB64 2
-#endif
-
 __host__ __device__ constexpr int tmem_cols_for(int cols)
 {
     return cols <= 32 ? 32 : cols <= 64 ? 64 : cols <= 128 ? 128 : cols <= 256 ? 256 : 512;
 }
 
 constexpr int kEW = 16;  // TMEM columns per epilogue step
-#ifndef CF_COPY_BATCH
-#define CF_COPY_BATCH 16
-#endif
-constexpr int kCopyBatch = CF_COPY_BATCH;  // channels per copy unit and thread loaded before the first store
+constexpr int kCopyBatch = 16;  // channels per copy unit and thread loaded before the first store
 
 // the "row" a cell without a k-th neighbour gathers: relu(-1e30 - e) = 0, so the operand build needs no select
 #define CF_NEG8 -1e30f, -1e30f, -1e30f, -1e30f, -1e30f, -1e30f, -1e30f, -1e30f
@@ -274,10 +247,12 @@ __global__ void __launch_bounds__(256) k_cell_compact(const int32_t *__restrict_
 // Thread layout: G groups of 128 threads.  Thread (row = tid % 128, grp = tid / 128) owns BEV cell `row` of the
 // tile; the G threads of a row split the 16-byte operand units of the A tile and the 16-column chunks of the
 // epilogues between them (warp w may only touch TMEM lanes 32*(w%4)..+31, which is exactly its rows).
+// Launch shape of the two small-C instantiations (measured on B200, BASELINE configs[1]: several small CTAs per SM --
+// more independent tiles in flight -- beat fewer barrier rounds per tile; see profiles/README.md).
 template <int C>
 struct TcShape {
-    static constexpr int G = C <= 32 ? CF_G32 : C <= 64 ? CF_G64 : C == 96 || C == 192 ? 3 : 4;
-    static constexpr int kMinBlocks = C <= 32 ? CF_MB32 : C <= 64 ? CF_MB64 : 1;
+    static constexpr int G = C <= 32 ? 1 : C <= 64 ? 2 : C == 96 || C == 192 ? 3 : 4;
+    static constexpr int kMinBlocks = C <= 32 ? 4 : C <= 64 ? 2 : 1;
 };
 
 template <int C, int NS, bool TH = false, typename MT = float>
@@ -500,7 +475,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // list entries of the copy units that follow this tile: in flight during the whole tile (at C = 32 this used to push
             // the mbarrier phase into local memory, 264 -> 283 us; with the gathers moved in front of the barrier it fits:
             // 260 -> 256 us)
-            if (C >= CF_FETCH_UNITS_MINC) fetch_units();
+            fetch_units();
             int32_t nb = cb, nq = cq;
             advance(nb, nq, (int32_t)gridDim.x);
             seek_live(nb, nq);
@@ -533,7 +508,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // Pipelined shapes (both layers resident, 4 items per warp and round): tv holds the gathered neighbour rows
             // of the NEXT round while this round's MMA and epilogue run; in the last round the same 32 registers take the
             // bev values of this thread's first two output chunks instead.
-            constexpr bool kPipe = CF_PIPE && C <= CF_PIPE_MAXC && kEven && L::kChunks == 1 && kItems == 4;
+            constexpr bool kPipe = C <= 128 && kEven && L::kChunks == 1 && kItems == 4;
             constexpr int kPre = kPipe ? 2 : 0;   // output chunks whose bev values are prefetched
             constexpr bool kGatherEarly = kPipe && C <= 32;
             float tv[32];
@@ -556,7 +531,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // Chunked shapes (C > 128: a round is kChunks chunk steps of KC input channels): the neighbour rows of the NEXT
             // chunk step are gathered into registers right after this step's MMAs are issued and are built after its wait --
             // the L2 round trip of the gather (~1 us of a ~3 us chunk step) leaves the tile's chain.
-            constexpr bool kPipe2 = CF_PIPE && !kPipe && L::kChunks > 1;
+            constexpr bool kPipe2 = !kPipe && L::kChunks > 1;
             constexpr int kMaxItems = (16 + kStep - 1) / kStep;
             float pv[kPipe2 ? kMaxItems * 8 : 1];
             auto gather_chunk = [&](int k, int ch) {
@@ -1816,7 +1791,6 @@ int launch_tc(const TcParams &p, cudaStream_t st)
     int per_sm = 1;
     CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH, MT>, NT, smem, L::kTmemCols, &regs, &per_sm));
     per_sm = std::max(1, per_sm);
-    if (tuning().max_ctas > 0) per_sm = std::max(1, std::min(per_sm, tuning().max_ctas));
     const int64_t grid = std::min<int64_t>(p.tiles_total, (int64_t)sm_count() * per_sm);
     if (tuning().debug_launch) fprintf(stderr, "k_fusion_tc<%d,%d>: %d CTAs/SM grid %lld smem %d\n", C, NS, per_sm, (long long)grid, smem);
     k_fusion_tc<C, NS, TH, MT><<<(unsigned)grid, NT, smem, st>>>(p);
@@ -1824,7 +1798,7 @@ int launch_tc(const TcParams &p, cudaStream_t st)
 }
 
 // The double-buffered kernel (k_fusion_sk) is used when its shared memory fits and it keeps the residency of k_fusion_tc;
-// returns CF_ERR_UNSUPPORTED (nothing launched) otherwise.  CF_NO_SKEW=1 forces k_fusion_tc (A/B measurements).
+// returns CF_ERR_UNSUPPORTED (nothing launched) otherwise.
 template <int C, int NS, bool TH = false, typename MT = float>
 int launch_sk(const TcParams &p, cudaStream_t st)
 {
@@ -1832,7 +1806,7 @@ int launch_sk(const TcParams &p, cudaStream_t st)
     using L0 = TcLayout<C, NS>;
     constexpr int NT = kTile * TcShape<C>::G;
     const int smem = L::smem_bytes(p.K);
-    if (smem > 227 * 1024 || tuning().no_skew) return CF_ERR_UNSUPPORTED;
+    if (smem > 227 * 1024) return CF_ERR_UNSUPPORTED;
     static int attr_bytes = 0, regs = 0, regs0 = 0;
     int per_sm = 0, per_sm0 = 0;
     CF_TRY(resident_ctas(k_fusion_sk<C, NS, TH, MT>, NT, smem, L::kTmemCols, &regs, &per_sm));
@@ -1843,7 +1817,6 @@ int launch_sk(const TcParams &p, cudaStream_t st)
                            "k_fusion_sk smem attribute"));
         attr_bytes = smem;
     }
-    if (tuning().max_ctas > 0) per_sm = std::max(1, std::min(per_sm, tuning().max_ctas));
     const int64_t grid = std::min<int64_t>(p.tiles_total, (int64_t)sm_count() * per_sm);
     if (tuning().debug_launch) fprintf(stderr, "k_fusion_sk<%d,%d>: %d CTAs/SM grid %lld smem %d\n", C, NS, per_sm, (long long)grid, smem);
     k_fusion_sk<C, NS, TH, MT><<<(unsigned)grid, NT, smem, st>>>(p);
@@ -1851,10 +1824,6 @@ int launch_sk(const TcParams &p, cudaStream_t st)
 }
 
 }  // namespace
-
-int fusion_seg(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_t B, int32_t N, int32_t C, int32_t H, int32_t W,
-               int32_t K, float x0, float y0, float dx, float dy, const float *d_W1, int32_t Ci, const float *d_b2, const float *d_b3,
-               float *d_out, int32_t mode, const uint8_t *img2, const uint8_t *img3, void *d_ws, cudaStream_t st);
 
 static size_t tc_weight_bytes(int32_t C, int NS) { return ((size_t)2 * NS * C * C * 2 + 255) / 256 * 256; }
 
@@ -1898,9 +1867,8 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     const int64_t n_cells = (int64_t)H * W;
     // Compaction pays when there are many more tiles than SMs.  On the small coarse scales the cells with a neighbour are
     // one contiguous blob, so the tiles are already either full or empty (empty tiles just copy bev -> out) and
-    // compaction only adds a launch (measured: 123 -> 148 us at 88x100x192).  CF_COMPACT_MIN_TILES overrides (tuning aid).
-    int64_t min_tiles = 4 * (int64_t)sm_count();
-    if (tuning().compact_min_tiles >= 0) min_tiles = tuning().compact_min_tiles;
+    // compaction only adds a launch (measured: 123 -> 148 us at 88x100x192).
+    const int64_t min_tiles = 4 * (int64_t)sm_count();
     if (!d_packed) {
         const int pack_blocks = (C * (C / 8) + 255) / 256;
         k_pack_weights<<<pack_blocks, 256, 0, st>>>(d_W2, C, C, C, KC, NS, (uint8_t *)d_workspace);
@@ -1908,13 +1876,6 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
         count_launches(2);
     }
     const bool compact = ceil_div64(n_cells, kTile) * B >= min_tiles;
-    // fine scales (many more tiles than SMs): segment tiles, all neighbour slots in one MMA batch (cf_fusion_seg.cu); its
-    // lists live where the cell lists of the kernels below would
-    if (compact && tuning().seg && mode != CF_MODE_BF16_TABLES && !io16) {
-        const int rc = fusion_seg(d_bev, d_T, d_knn, B, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, d_b2, d_b3, d_out, mode, img2,
-                                  img3, cell_count, st);
-        if (rc != CF_ERR_UNSUPPORTED) return rc;
-    }
     if (compact) {
         CF_TRY(cuda_status(cudaMemsetAsync(cell_count, 0, 512, st), "cf_fusion_fwd memset"));
         k_cell_compact<<<dim3((unsigned)ceil_div64(n_cells, 256), (unsigned)B), 256, 0, st>>>(d_knn, K, n_cells, cell_list,

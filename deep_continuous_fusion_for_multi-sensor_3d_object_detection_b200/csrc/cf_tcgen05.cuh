@@ -55,7 +55,7 @@ __device__ __forceinline__ void mma_bf16(uint32_t tmem_d, uint64_t desc_a, uint6
 // One lane of a CONVERGED warp (all 32 lanes must execute this).  Guarding the tcgen05.mma / commit sequence with
 // `warp == w && elect_one()` instead of `tid == 0` lets ptxas keep descriptors in uniform registers and emit the UTCHMMAs
 // back to back; under a plain thread-index test it wraps every UTCHMMA in an ELECT / BRA.U.ANY loop (~70 cycles per MMA,
-// measured: 15 % of the segment kernel's tile time went into issuing 35 small MMAs).
+// measured: 15 % of the tile time of a since-removed segment-tile variant of K-4 went into issuing 35 small MMAs).
 __device__ __forceinline__ bool elect_one()
 {
     uint32_t pred;
@@ -104,25 +104,10 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity)
     } while (!done);
 }
 
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// named barrier among `nthreads` threads of the CTA (id 1..15; id 0 is __syncthreads)
-__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads)
-{
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-
-
-// ---- TMA (cp.async.bulk.tensor) through a 2-D tensor map, completion on an mbarrier / bulk groups ---------------------------
+// ---- TMA (cp.async.bulk, cp.async.bulk.tensor), completion on an mbarrier / bulk groups ---------------------------------------
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar_addr, uint32_t bytes)
 {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_addr), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_a(uint32_t bar_addr)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar_addr) : "memory");
 }
 __device__ __forceinline__ bool mbar_test(uint32_t bar_addr, uint32_t parity)
 {
@@ -138,36 +123,10 @@ __device__ __forceinline__ bool mbar_test(uint32_t bar_addr, uint32_t parity)
         : "memory");
     return done != 0;
 }
-// non-blocking probe (mbarrier.test_wait returns at once; try_wait may suspend the thread for a system-dependent time)
-__device__ __forceinline__ bool mbar_poll(uint32_t bar_addr, uint32_t parity)
-{
-    uint32_t done;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}\n"
-        : "=r"(done)
-        : "r"(bar_addr), "r"(parity)
-        : "memory");
-    return done != 0;
-}
 __device__ __forceinline__ void mbar_wait_a(uint32_t bar_addr, uint32_t parity)
 {
     while (!mbar_test(bar_addr, parity)) {
     }
-}
-// box (x = fastest coordinate, y) of the tensor behind `tmap` -> shared memory; complete_tx on the mbarrier
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const void *tmap, int32_t x, int32_t y, uint32_t bar_addr)
-{
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-                 "l"(tmap), "r"(x), "r"(y), "r"(bar_addr)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_store_2d(const void *tmap, int32_t x, int32_t y, uint32_t src)
-{
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];" ::"l"(tmap), "r"(x), "r"(y), "r"(src) : "memory");
 }
 __device__ __forceinline__ void tma_store_3d(const void *tmap, int32_t x, int32_t y, int32_t z, uint32_t src)
 {
@@ -187,7 +146,6 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void *src, uint32_t bytes
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
@@ -332,15 +290,6 @@ __device__ __forceinline__ void ldg_row8(const __nv_bfloat16 *p, float *v)
         v[2 * i] = __uint_as_float(r[i] << 16);
         v[2 * i + 1] = __uint_as_float(r[i] & 0xffff0000u);
     }
-}
-
-// the same load pinned in program order (volatile asm): keeps a software-pipelined gather where it was written instead of
-// letting the scheduler hoist every load of a tile to its top (register pressure)
-__device__ __forceinline__ void ldg_nc_f32x8_pinned(const float *p, float *v)
-{
-    asm volatile("ld.global.nc.v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]), "=f"(v[4]), "=f"(v[5]), "=f"(v[6]), "=f"(v[7])
-                 : "l"(p));
 }
 
 // 256-bit global store (sm_100: STG.E.256): a full 32-byte sector per lane, 32-byte aligned

@@ -150,7 +150,6 @@ CF_API int cf_fusion_pack_weights(const float *d_W2, const float *d_W3, int32_t 
  *   mode | CF_IO_BF16: d_bev and d_out are bf16 (B,C,H,W) NCHW maps (may alias, as for fp32).  bev is widened exactly to
  *   fp32, everything else is computed as without the flag and out is rounded once to bf16 (nearest even) when stored:
  *   the result equals the fp32 call on the widened map, rounded.  T, weights and the workspace size are unchanged.
- *   The opt-in segment-tile kernel (CF_SEG=1) is fp32-only and is skipped with this flag.
  * Every function that takes a `mode` ignores the flag bits (CF_IO_BF16, CF_BWD_DETERMINISTIC) when it picks the
  * arithmetic, the operand layout or a workspace size.
  * ------------------------------------------------------------------------------------------- */

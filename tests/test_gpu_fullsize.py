@@ -68,15 +68,3 @@ def test_cfg2_full_frame_bf16(dcf, oracle):
     for sc, x, y in zip(wl["scales"], outs_t, outs_ti):
         assert np.array_equal(x, y), f"group {sc['group']}: bf16 tables, in place != out of place"
 
-
-def test_segment_kernel_opt_in_matches_oracle():
-    """The opt-in segment-tile kernel (csrc/cf_fusion_seg.cu, CF_SEG=1: operand ring, TMA boxes for every BEV byte, polled TMA
-    copies of the empty segments) passes the same full-size configs[1] check.  The switch is read once per process, so the
-    check runs in a child process; CF_DEBUG_LAUNCH shows that the kernel really ran."""
-    import subprocess
-    import sys
-    env = dict(os.environ, CF_SEG="1", CF_DEBUG_LAUNCH="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", f"{os.path.abspath(__file__)}::test_cfg1_full_frames_fp32", "-x", "-q", "-s", "-m", "gpu"],
-                       env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "k_fusion_seg<32,2,5>" in r.stdout + r.stderr
