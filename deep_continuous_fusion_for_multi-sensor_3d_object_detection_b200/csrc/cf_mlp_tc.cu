@@ -255,6 +255,227 @@ struct TcShape {
     static constexpr int kMinBlocks = C <= 32 ? 4 : C <= 64 ? 2 : 1;
 };
 
+// ---------------------------------------------------------------------------------------------------------------
+// Pieces shared by the two fused kernels, k_fusion_tc and k_fusion_sk, which must give bit-identical results.  What
+// differs between the kernels (A-buffer address, K-chunk, bias-operand size) is an argument.
+// ---------------------------------------------------------------------------------------------------------------
+
+// One-time setup of the negated offset weights and the bias operands (contains a CTA barrier).  The kernel's bias A
+// operands (ab_bytes from sAb) are followed by the bias B operands of layer 2 and layer 3 (C rows x 16 bf16 each).
+template <int C, int NT>
+__device__ __forceinline__ void setup_offsets_and_bias(const TcParams &p, int tid, float *swn, uint8_t *sAb, int ab_bytes)
+{
+    // negated offset weights, per block of 8 channels: -w1x[8] | -w1y[8]  (what one lane of the operand build needs)
+    for (int c = tid; c < C; c += NT) {
+        swn[(c >> 3) * 16 + (c & 7)] = -__ldg(p.W1 + (size_t)c * (p.Ci + 3) + p.Ci);
+        swn[(c >> 3) * 16 + 8 + (c & 7)] = -__ldg(p.W1 + (size_t)c * (p.Ci + 3) + p.Ci + 1);
+    }
+    // bias operands.  A side (rewritten per round): row r, k-columns 0 and 1 = the row's flag, the other 14 stay 0.
+    // B side: row n = (hi(b[n]), lo(b[n]), 0 ...), so flag * (hi + lo) lands in the accumulator with one K=16 step.
+    for (int o = tid * 16; o < ab_bytes + 2 * C * 32; o += NT * 16) *reinterpret_cast<uint4 *>(sAb + o) = make_uint4(0, 0, 0, 0);
+    __syncthreads();
+    uint8_t *sWb = sAb + ab_bytes;
+    for (int n = tid; n < 2 * C; n += NT) {
+        const int layer = n / C, c = n - layer * C;
+        const float bv = __ldg((layer ? p.b3 : p.b2) + c);
+        const __nv_bfloat16 h = __float2bfloat16_rn(bv);
+        const __nv_bfloat16 l = __float2bfloat16_rn(bv - __bfloat162float(h));
+        const uint32_t packed = (uint32_t)__bfloat16_as_ushort(h) | ((uint32_t)__bfloat16_as_ushort(l) << 16);
+        *reinterpret_cast<uint32_t *>(sWb + layer * C * 32 + tc::unit_offset(c, 0, 2)) = packed;
+    }
+}
+
+// the bev values of this thread's first kPre output chunks -> tv (they ride in the registers of the gathered rows)
+template <int C, int G, int kPre, typename MT>
+__device__ __forceinline__ void prefetch_bev(float *tv, const MT *src_bev, int64_t cells, int grp)
+{
+#pragma unroll
+    for (int j = 0; j < kPre; ++j) {
+        if (grp + j * G < C / kEW) {
+#pragma unroll
+            for (int i = 0; i < kEW; ++i) tv[j * kEW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * kEW + i) * cells);
+        }
+    }
+}
+
+// ---- layer 3 operand: KC channels of pooled (TMEM, this warp's lanes) -> the A buffer at a_addr; with bias_col, the
+// row's bias column = n_valid (acc = n_valid * b3 + pooled * W3^T) ------------------------------------------------
+template <int NS, int KC, int G>
+__device__ __forceinline__ void pooled_to_operand(uint32_t pool, uint32_t a_addr, int row, int grp, bool bias_col, uint32_t ab_row,
+                                                  int n_valid)
+{
+    constexpr int EW = kEW;
+    __syncwarp();
+#pragma unroll 1
+    for (int cc = grp; cc < KC / EW; cc += G) {
+        float s[EW];
+        tc::tmem_ld<EW>(pool + cc * EW, s);
+#pragma unroll
+        for (int q = 0; q < EW / 8; ++q) {
+            float2 v[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) v[i] = make_float2(s[q * 8 + 2 * i], s[q * 8 + 2 * i + 1]);
+            uint4 hi, lo;
+            tc::relu_split_bf16x8(v, hi, lo, NS == 2);   // pooled >= 0: the ReLU is the identity here
+            const uint32_t off = a_addr + tc::unit_offset(row, cc * (EW / 8) + q, KC / 8);
+            tc::sts_u32x4(off, hi);
+            if (NS == 2) tc::sts_u32x4(off + kTile * KC * 2, lo);
+        }
+    }
+    if (bias_col && grp == 0) {
+        const uint32_t nv16 = __float_as_uint((float)n_valid) >> 16;   // small integers are exact in bf16
+        tc::sts_u32(ab_row, nv16 | (nv16 << 16));
+    }
+}
+
+__device__ __forceinline__ void store_ctr(float4 *s, float cx, float cy) { *s = make_float4(cx, cx, cy, cy); }   // k_fusion_tc
+__device__ __forceinline__ void store_ctr(float2 *s, float cx, float cy) { *s = make_float2(cx, cy); }           // k_fusion_sk
+
+// ---- tile sequencing (uniform across the CTA) ------------------------------------------------------------------
+// Tile t covers entries [e0, e0 + 128) of frame b's lists: of the cells WITH a neighbour (an MLP tile) and, from the
+// other end, of the cells WITHOUT one (a copy unit).  The CTA walks both sequences with two cursors and interleaves
+// them, so the memory-bound copies overlap the MLP tiles of the CTAs that share the SM.
+// Positions in the tile sequence are (frame b, tile q within the frame); this CTA visits every gridDim.x-th tile.
+// The cursors stay in the kernel; Ctr is the kernel's format of a cell centre in the tile header.
+template <typename Ctr>
+struct TileWalk {
+    const TcParams &p;
+    const int64_t cells;
+    const int32_t tpf;        // tiles per frame
+    const int row;            // this thread's row of a tile
+    const int K;
+    const uint32_t sidx_addr; // tile header, double-buffered by tile parity: int32 [2][K][128] neighbour indices (slot-major),
+    Ctr *const sctr;          // [2][128] cell centres
+    int32_t *const scell;     // and [2][128] cells (-1: the list ends before the row)
+    int32_t *const swmax;     // [2][4] per warp of group 0: its largest neighbour count
+
+    __device__ __forceinline__ int32_t n_live_of(int b) const { return p.cell_list ? __ldg(p.cell_count + b) : (int32_t)cells; }
+    __device__ __forceinline__ void advance(int32_t &b, int32_t &q, int32_t step) const
+    {
+        q += step;
+        while (q >= tpf) {
+            q -= tpf;
+            ++b;
+        }
+    }
+    // forward (inclusive) to the next tile that has rows; b == B: none
+    __device__ __forceinline__ void seek_live(int32_t &b, int32_t &q) const
+    {
+        while (b < p.B && q * kTile >= n_live_of(b)) advance(b, q, (int32_t)gridDim.x);
+    }
+    // this CTA's first MLP tile (cb, cq) and copy unit (db, dq); fill: this thread prefetches its row of the first header
+    __device__ __forceinline__ void start(int32_t &cb, int32_t &cq, int32_t &db, int32_t &dq, bool fill) const
+    {
+        advance(cb, cq, (int32_t)blockIdx.x);
+        seek_live(cb, cq);
+        if (p.copy_dead) advance(db, dq, (int32_t)blockIdx.x); else db = p.B;
+        if (cb < p.B && fill) header_fill(cb, header_cell(cb, cq), 0);
+    }
+    // Tile header, prefetched one tile ahead by the 128 threads of group 0 (thread = row).
+    //   stage 1: the row's cell (-1: the list ends before this row)
+    //   stage 2: its K neighbour indices straight into shared memory (cp.async, slot-major), centre and cell
+    __device__ __forceinline__ int32_t header_cell(int32_t b, int32_t q) const
+    {
+        const int32_t e = q * kTile + row;
+        if (e >= n_live_of(b)) return -1;
+        return p.cell_list ? __ldg(p.cell_list + (size_t)b * cells + e) : e;
+    }
+    __device__ __forceinline__ void header_fill(int32_t b, int32_t cell, int par) const
+    {
+        const uint32_t dst = sidx_addr + (uint32_t)((par * K * kTile + row) * 4);
+        float cx = 0.f, cy = 0.f;
+        if (cell >= 0) {
+            const int32_t *kr = p.knn + ((size_t)b * cells + cell) * K;
+            for (int k = 0; k < K; ++k) tc::cp_async4(dst + k * kTile * 4, kr + k);
+            const int32_t i = (int32_t)((uint32_t)cell / (uint32_t)p.W), j = cell - i * p.W;
+            cx = __fadd_rn(p.x0, __fmul_rn((float)i, p.dx));
+            cy = __fadd_rn(p.y0, __fmul_rn((float)j, p.dy));
+        } else {
+            for (int k = 0; k < K; ++k) tc::sts_u32(dst + k * kTile * 4, 0xFFFFFFFFu);
+        }
+        tc::cp_async_commit();
+        store_ctr(sctr + par * kTile + row, cx, cy);
+        scell[par * kTile + row] = cell;
+    }
+    // The prefetched header of the tile with parity par (contains a CTA barrier): returns the tile's round count, the
+    // neighbour count of its best-connected cell; n_valid (group 0, grp0) = this row's neighbour count.
+    __device__ __forceinline__ int read_header(int par, bool grp0, int lane, int warp, int &n_valid) const
+    {
+        if (grp0) {
+            tc::cp_async_wait_all();
+            for (int k = 0; k < K; ++k) n_valid += (int32_t)tc::lds_u32(sidx_addr + (uint32_t)(((par * K + k) * kTile + row) * 4)) >= 0;
+            const int wm = __reduce_max_sync(0xffffffffu, n_valid);
+            if (lane == 0) swmax[par * 4 + warp] = wm;
+        }
+        __syncthreads();
+        const int4 wm = *reinterpret_cast<const int4 *>(swmax + par * 4);
+        return max(max(wm.x, wm.y), max(wm.z, wm.w));
+    }
+    // the list entries of the next two copy units from cursor (db, dq): frame (uniform, -1: none left) and this thread's
+    // cell (-1: past the end of the list)
+    __device__ __forceinline__ void fetch_units(int32_t &db, int32_t &dq, int32_t (&uframe)[2], int32_t (&ucell)[2]) const
+    {
+#pragma unroll
+        for (int u = 0; u < 2; ++u) {
+            uframe[u] = -1;
+            ucell[u] = -1;
+            int32_t n_dead = 0;
+            while (db < p.B) {
+                n_dead = (int32_t)cells - n_live_of(db);
+                if (dq * kTile < n_dead) break;
+                advance(db, dq, (int32_t)gridDim.x);
+            }
+            if (db < p.B) {
+                uframe[u] = db;
+                const int32_t j = dq * kTile + row;
+                if (j < n_dead) ucell[u] = __ldg(p.cell_list + (size_t)db * cells + (cells - 1 - j));
+                advance(db, dq, (int32_t)gridDim.x);
+            }
+        }
+    }
+};
+
+// ---- copy units: cells without a neighbour (back of the list): out = bev ----------------------------------------
+// (thread = cell, the G thread groups split the channels; two units are interleaved after every MLP tile; their list
+// entries were fetched at the start of the tile, so a unit costs one DRAM round trip per channel batch)
+template <int C, int G, typename MT>
+__device__ __forceinline__ void copy_units(const TcParams &p, const int32_t (&uframe)[2], const int32_t (&ucell)[2], int grp, int64_t cells)
+{
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+        if (uframe[u] >= 0 && ucell[u] >= 0) {   // uframe is uniform; ucell < 0: a row past the end of the list
+            constexpr int CG = C / G;
+            const size_t o = ((size_t)uframe[u] * C + grp * CG) * cells + ucell[u];
+            using RB = typename MapBits<MT>::type;   // a bf16 map is copied as raw 16-bit elements
+            const RB *src = reinterpret_cast<const RB *>(p.bev) + o;
+            RB *dst = reinterpret_cast<RB *>(p.out) + o;
+#pragma unroll 1
+            for (int c = 0; c < CG; c += kCopyBatch) {   // kCopyBatch loads in flight per thread, then the stores
+                RB v[kCopyBatch];
+#pragma unroll
+                for (int i = 0; i < kCopyBatch; ++i) {
+                    v[i] = __ldcs(src);
+                    src += cells;
+                }
+#pragma unroll
+                for (int i = 0; i < kCopyBatch; ++i) {
+                    __stcs(dst, v[i]);
+                    dst += cells;
+                }
+            }
+        }
+    }
+}
+
+// wait for the last copies, then free the tensor memory
+__device__ __forceinline__ void teardown(uint32_t tmem_base, int tmem_cols, int warp)
+{
+    tc::cp_async_wait_all();
+    tc::fence_before_sync();
+    __syncthreads();
+    if (warp == 0) tc::tmem_free(tmem_base, tmem_cols);
+}
+
 template <int C, int NS, bool TH = false, typename MT = float>
 __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks) k_fusion_tc(const TcParams p)
 {
@@ -296,23 +517,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
     }
     __syncwarp();
     if (warp == 0) tc::tmem_alloc(tmem_slot, L::kTmemCols);
-    // negated offset weights, per block of 8 channels: -w1x[8] | -w1y[8]  (what one lane of the operand build needs)
-    for (int c = tid; c < C; c += NT) {
-        swn[(c >> 3) * 16 + (c & 7)] = -__ldg(p.W1 + (size_t)c * (p.Ci + 3) + p.Ci);
-        swn[(c >> 3) * 16 + 8 + (c & 7)] = -__ldg(p.W1 + (size_t)c * (p.Ci + 3) + p.Ci + 1);
-    }
-    // bias operands.  A side (rewritten per round): row r, k-columns 0 and 1 = the row's flag, the other 14 stay 0.
-    // B side: row n = (hi(b[n]), lo(b[n]), 0 ...), so flag * (hi + lo) lands in the accumulator with one K=16 step.
-    for (int o = tid * 16; o < L::kAbBytes + 2 * L::kWbBytes; o += NT * 16) *reinterpret_cast<uint4 *>(sAb + o) = make_uint4(0, 0, 0, 0);
-    __syncthreads();
-    for (int n = tid; n < 2 * C; n += NT) {
-        const int layer = n / C, c = n - layer * C;
-        const float bv = __ldg((layer ? p.b3 : p.b2) + c);
-        const __nv_bfloat16 h = __float2bfloat16_rn(bv);
-        const __nv_bfloat16 l = __float2bfloat16_rn(bv - __bfloat162float(h));
-        const uint32_t packed = (uint32_t)__bfloat16_as_ushort(h) | ((uint32_t)__bfloat16_as_ushort(l) << 16);
-        *reinterpret_cast<uint32_t *>(sWb + layer * L::kWbBytes + tc::unit_offset(c, 0, 2)) = packed;
-    }
+    setup_offsets_and_bias<C, NT>(p, tid, swn, sAb, L::kAbBytes);
     // Streamed weights (C > 128): chunks of KC input channels travel L2 -> shared memory as ONE bulk copy each (TMA engine,
     // cp.async.bulk; the packed chunk is contiguous) into two buffers, always one chunk ahead of the MMAs; only the thread that
     // issues the MMAs waits for a chunk (mbarrier complete_tx).  `wn` counts the chunks consumed so far: chunk wn lives in
@@ -359,8 +564,6 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
     constexpr int kQuads = kc_units / 4;
     static_assert(NW % kQuads == 0, "warps per CTA must be a multiple of the unit quads per row");
     constexpr int kStep = NW / kQuads;   // row groups between two items of a warp
-    constexpr bool kEven = 16 % kStep == 0;
-    constexpr int kItems = kEven ? 16 / kStep : 1;
     const int ku = (warp % kQuads) * 4 + (lane >> 3);
     const int r8 = lane & 7;
     const int rg0 = warp / kQuads;
@@ -375,47 +578,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
         ny[0] = make_float2(y0.x, y0.y); ny[1] = make_float2(y0.z, y0.w); ny[2] = make_float2(y1.x, y1.y); ny[3] = make_float2(y1.z, y1.w);
     };
 
-    // ---- tile sequencing (uniform across the CTA) ------------------------------------------------------------------
-    // Tile t covers entries [e0, e0 + 128) of frame b's lists: of the cells WITH a neighbour (an MLP tile) and, from the
-    // other end, of the cells WITHOUT one (a copy unit).  The CTA walks both sequences with two cursors and interleaves
-    // them, so the memory-bound copies overlap the MLP tiles of the CTAs that share the SM.
-    // Positions in the tile sequence are (frame b, tile q within the frame); this CTA visits every gridDim.x-th tile.
-    const int32_t tpf = (int32_t)p.tiles_per_frame;
-    auto n_live_of = [&](int b) -> int32_t { return p.cell_list ? __ldg(p.cell_count + b) : (int32_t)cells; };
-    auto advance = [&](int32_t &b, int32_t &q, int32_t step) {
-        q += step;
-        while (q >= tpf) {
-            q -= tpf;
-            ++b;
-        }
-    };
-    auto seek_live = [&](int32_t &b, int32_t &q) {   // forward (inclusive) to the next tile that has rows; b == B: none
-        while (b < p.B && q * kTile >= n_live_of(b)) advance(b, q, (int32_t)gridDim.x);
-    };
-    // Tile header, prefetched one tile ahead by the 128 threads of group 0 (thread = row).
-    //   stage 1: the row's cell (-1: the list ends before this row)
-    //   stage 2: its K neighbour indices straight into shared memory (cp.async, slot-major), centre and cell
-    auto header_cell = [&](int32_t b, int32_t q) -> int32_t {
-        const int32_t e = q * kTile + row;
-        if (e >= n_live_of(b)) return -1;
-        return p.cell_list ? __ldg(p.cell_list + (size_t)b * cells + e) : e;
-    };
-    auto header_fill = [&](int32_t b, int32_t cell, int par) {
-        const uint32_t dst = sidx_addr + (uint32_t)((par * K * kTile + row) * 4);
-        float cx = 0.f, cy = 0.f;
-        if (cell >= 0) {
-            const int32_t *kr = p.knn + ((size_t)b * cells + cell) * K;
-            for (int k = 0; k < K; ++k) tc::cp_async4(dst + k * kTile * 4, kr + k);
-            const int32_t i = (int32_t)((uint32_t)cell / (uint32_t)p.W), j = cell - i * p.W;
-            cx = __fadd_rn(p.x0, __fmul_rn((float)i, p.dx));
-            cy = __fadd_rn(p.y0, __fmul_rn((float)j, p.dy));
-        } else {
-            for (int k = 0; k < K; ++k) tc::sts_u32(dst + k * kTile * 4, 0xFFFFFFFFu);
-        }
-        tc::cp_async_commit();
-        sctr[par * kTile + row] = make_float4(cx, cx, cy, cy);
-        scell[par * kTile + row] = cell;
-    };
+    const TileWalk<float4> walk{p, cells, (int32_t)p.tiles_per_frame, row, K, sidx_addr, sctr, scell, swmax};
 
     // ---- operand build ---------------------------------------------------------------------------------------------
     // one item = 8 rows x 32 channels per warp: lane (r8, u) turns 8 channels of one neighbour row into two 16-byte
@@ -438,34 +601,10 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
     };
 
     int32_t cb = 0, cq = 0, db = 0, dq = 0;   // cursors: MLP tiles (cb, cq), copy units (db, dq)
-    advance(cb, cq, (int32_t)blockIdx.x);
-    seek_live(cb, cq);
-    if (p.copy_dead) advance(db, dq, (int32_t)blockIdx.x); else db = p.B;
-    if (cb < p.B && grp == 0) header_fill(cb, header_cell(cb, cq), 0);
+    walk.start(cb, cq, db, dq, grp == 0);
 
-    // the next two copy units of this CTA: frame (uniform, -1: none left) and this thread's cell (-1: past the end)
-    int32_t uframe[2] = {-1, -1}, ucell[2] = {-1, -1};
+    int32_t uframe[2] = {-1, -1}, ucell[2] = {-1, -1};   // the next two copy units (TileWalk::fetch_units)
     bool units_ready = false;
-    auto fetch_units = [&]() {
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            uframe[u] = -1;
-            ucell[u] = -1;
-            int32_t n_dead = 0;
-            while (db < p.B) {
-                n_dead = (int32_t)cells - n_live_of(db);
-                if (dq * kTile < n_dead) break;
-                advance(db, dq, (int32_t)gridDim.x);
-            }
-            if (db < p.B) {
-                uframe[u] = db;
-                const int32_t j = dq * kTile + row;
-                if (j < n_dead) ucell[u] = __ldg(p.cell_list + (size_t)db * cells + (cells - 1 - j));
-                advance(db, dq, (int32_t)gridDim.x);
-            }
-        }
-        units_ready = true;
-    };
 
     while (cb < p.B || db < p.B) {
         if (cb < p.B) {
@@ -475,30 +614,20 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // list entries of the copy units that follow this tile: in flight during the whole tile (at C = 32 this used to push
             // the mbarrier phase into local memory, 264 -> 283 us; with the gathers moved in front of the barrier it fits:
             // 260 -> 256 us)
-            fetch_units();
+            walk.fetch_units(db, dq, uframe, ucell);
+            units_ready = true;
             int32_t nb = cb, nq = cq;
-            advance(nb, nq, (int32_t)gridDim.x);
-            seek_live(nb, nq);
+            walk.advance(nb, nq, (int32_t)gridDim.x);
+            walk.seek_live(nb, nq);
             const bool has_next = nb < p.B;
             // ---- header of this tile (prefetched): rounds = neighbour count of its best-connected cell -----------------
             int n_valid = 0;
-            if (grp == 0) {
-                tc::cp_async_wait_all();
-                for (int k = 0; k < K; ++k) n_valid += (int32_t)tc::lds_u32(sidx_addr + (uint32_t)(((par * K + k) * kTile + row) * 4)) >= 0;
-                const int wm = __reduce_max_sync(0xffffffffu, n_valid);
-                if (lane == 0) swmax[par * 4 + warp] = wm;
-            }
-            __syncthreads();
-            int R;
-            {
-                const int4 wm = *reinterpret_cast<const int4 *>(swmax + par * 4);
-                R = max(max(wm.x, wm.y), max(wm.z, wm.w));
-            }
+            const int R = walk.read_header(par, grp == 0, lane, warp, n_valid);
             const int32_t cell = scell[par * kTile + row];
             const bool in_range = cell >= 0;
             int32_t ncell = -1;   // stage 1 of the next tile's header: in flight during round 0
-            if (grp == 0 && has_next) ncell = header_cell(nb, nq);
-            if (R == 0 && grp == 0 && has_next) header_fill(nb, ncell, par ^ 1);
+            if (grp == 0 && has_next) ncell = walk.header_cell(nb, nq);
+            if (R == 0 && grp == 0 && has_next) walk.header_fill(nb, ncell, par ^ 1);
 
             const TT *Tb = reinterpret_cast<const TT *>(p.T) + (size_t)b * p.N * C;
             const uint32_t idx0 = sidx_addr + (uint32_t)((par * K * kTile + rg0 * 8 + r8) * 4);
@@ -508,20 +637,12 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // Pipelined shapes (both layers resident, 4 items per warp and round): tv holds the gathered neighbour rows
             // of the NEXT round while this round's MMA and epilogue run; in the last round the same 32 registers take the
             // bev values of this thread's first two output chunks instead.
-            constexpr bool kPipe = C <= 128 && kEven && L::kChunks == 1 && kItems == 4;
+            constexpr bool kPipe = L::kChunks == 1 && kStep == 4;
             constexpr int kPre = kPipe ? 2 : 0;   // output chunks whose bev values are prefetched
             constexpr bool kGatherEarly = kPipe && C <= 32;
             float tv[32];
-            auto prefetch_bev = [&]() {
-                if (kPipe && in_range) {
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) {
-                        if (grp + j * G < kChunksE) {
-#pragma unroll
-                            for (int i = 0; i < EW; ++i) tv[j * EW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * EW + i) * cells);
-                        }
-                    }
-                }
+            auto prefetch_tv = [&]() {
+                if (in_range) prefetch_bev<C, G, kPre>(tv, src_bev, cells, grp);
             };
             if (kPipe && R > 0) {
                 const TT *Tc = Tb + ku * 8, *neg = g_neg + ku * 8;
@@ -532,6 +653,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // chunk step are gathered into registers right after this step's MMAs are issued and are built after its wait --
             // the L2 round trip of the gather (~1 us of a ~3 us chunk step) leaves the tile's chain.
             constexpr bool kPipe2 = !kPipe && L::kChunks > 1;
+            static_assert(kPipe || kPipe2, "every shape builds its operands in one of the two pipelined forms");
             constexpr int kMaxItems = (16 + kStep - 1) / kStep;
             float pv[kPipe2 ? kMaxItems * 8 : 1];
             auto gather_chunk = [&](int k, int ch) {
@@ -541,7 +663,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                     if (rg0 + m * kStep < 16) gather(Tc, neg, idx0 + (uint32_t)(k * kTile * 4 + m * kStep * 32), pv + 8 * m);
             };
             if (kPipe2 && R > 0) gather_chunk(0, 0);
-            if (R == 0) prefetch_bev();
+            if (R == 0) prefetch_tv();
 
             for (int k = 0; k < R; ++k) {
                 const uint32_t idxk = idx0 + (uint32_t)(k * kTile * 4);
@@ -559,7 +681,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                             build(tv + 8 * i, ctr, dst0 + i * kStep * kc_units * 128);
                             ctr = ctr_next;
                         }
-                    } else if (kPipe2) {
+                    } else {
                         load_offset_weights(ch);
 #pragma unroll
                         for (int m = 0; m < kMaxItems; ++m) {
@@ -567,20 +689,6 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                                 const float4 cm = tc::lds_f32x4(ctr0 + m * kStep * 128);
                                 build(pv + 8 * m, cm, dst0 + m * kStep * kc_units * 128);
                             }
-                        }
-                    } else {
-                        load_offset_weights(ch);
-                        const TT *Tc = Tb + ch * KC + ku * 8, *neg = g_neg + ch * KC + ku * 8;
-#pragma unroll 1
-                        for (int rg = rg0; rg < 16; rg += 2 * kStep) {   // pairs of items: both gathers in flight
-                            float ta[8], tb[8];
-                            const bool two = rg + kStep < 16;
-                            gather(Tc, neg, idxk + (rg - rg0) * 32, ta);
-                            if (two) gather(Tc, neg, idxk + (rg - rg0 + kStep) * 32, tb);
-                            const float4 ca = tc::lds_f32x4(ctr0 + (rg - rg0) * 128);
-                            const float4 cb = tc::lds_f32x4(ctr0 + (two ? rg - rg0 + kStep : rg - rg0) * 128);
-                            build(ta, ca, dst0 + (rg - rg0) * kc_units * 128);
-                            if (two) build(tb, cb, dst0 + (rg - rg0 + kStep) * kc_units * 128);
                         }
                     }
                     if (ch == 0 && grp == 0)   // bias flag of the row: bf16 (1, 1) or (0, 0)
@@ -594,7 +702,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
 #pragma unroll
                             for (int i = 0; i < 4; ++i) gather(Tc, neg, idxk + kTile * 4 + i * kStep * 32, tv + 8 * i);
                         } else {
-                            prefetch_bev();
+                            prefetch_tv();
                         }
                     }
                     tc::fence_proxy_async();
@@ -624,7 +732,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                     if (ch == L::kChunks - 1) {
                         // work that overlaps this round's MMA and epilogue: the next tile's header, then the next round's
                         // gathers (or, in the last round, the bev values of the final epilogue)
-                        if (k == 0 && grp == 0 && has_next) header_fill(nb, ncell, par ^ 1);
+                        if (k == 0 && grp == 0 && has_next) walk.header_fill(nb, ncell, par ^ 1);
                         if (k + 1 < R) {
                             if (kPipe && !kGatherEarly) {
                                 const TT *Tc = Tb + ku * 8, *neg = g_neg + ku * 8;
@@ -632,7 +740,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                                 for (int i = 0; i < 4; ++i) gather(Tc, neg, idxk + kTile * 4 + i * kStep * 32, tv + 8 * i);
                             }
                         } else if (!kGatherEarly) {
-                            prefetch_bev();
+                            prefetch_tv();
                         }
                     }
                     tc::mbar_wait(bar, phase);
@@ -665,27 +773,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             if (R > 0) {
                 // ---- layer 3: acc = n_valid * b3 + pooled * W3^T -----------------------------------------------------------
                 for (int ch = 0; ch < L::kChunks; ++ch) {
-                    __syncwarp();
-#pragma unroll 1
-                    for (int cc = grp; cc < KC / EW; cc += G) {
-                        float s[EW];
-                        tc::tmem_ld<EW>(tmem_pool + lane_off + ch * KC + cc * EW, s);
-#pragma unroll
-                        for (int q = 0; q < EW / 8; ++q) {
-                            float2 v[4];
-#pragma unroll
-                            for (int i = 0; i < 4; ++i) v[i] = make_float2(s[q * 8 + 2 * i], s[q * 8 + 2 * i + 1]);
-                            uint4 hi, lo;
-                            tc::relu_split_bf16x8(v, hi, lo, NS == 2);   // pooled >= 0: the ReLU is the identity here
-                            const uint32_t off = sA_addr + tc::unit_offset(row, cc * (EW / 8) + q, kc_units);
-                            tc::sts_u32x4(off, hi);
-                            if (NS == 2) tc::sts_u32x4(off + kTile * KC * 2, lo);
-                        }
-                    }
-                    if (ch == 0 && grp == 0) {
-                        const uint32_t nv16 = __float_as_uint((float)n_valid) >> 16;   // small integers are exact in bf16
-                        tc::sts_u32(ab_row, nv16 | (nv16 << 16));
-                    }
+                    pooled_to_operand<NS, KC, G>(tmem_pool + lane_off + ch * KC, sA_addr, row, grp, ch == 0, ab_row, n_valid);
                     tc::fence_proxy_async();
                     tc::fence_before_sync();
                     __syncthreads();
@@ -744,42 +832,13 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             cb = nb;
             cq = nq;
         }
-        // ---- copy units: cells without a neighbour (back of the list): out = bev ----------------------------------------
-        // (thread = cell, the G thread groups split the channels; two units are interleaved after every MLP tile; their
-        // list entries were fetched at the start of the tile, so a unit costs one DRAM round trip per channel batch)
-        if (!units_ready) fetch_units();
+        if (!units_ready) walk.fetch_units(db, dq, uframe, ucell);
         units_ready = false;
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            if (uframe[u] >= 0 && ucell[u] >= 0) {   // uframe is uniform; ucell < 0: a row past the end of the list
-                constexpr int CG = C / G;
-                const size_t o = ((size_t)uframe[u] * C + grp * CG) * cells + ucell[u];
-                using RB = typename MapBits<MT>::type;   // a bf16 map is copied as raw 16-bit elements
-                const RB *src = reinterpret_cast<const RB *>(p.bev) + o;
-                RB *dst = reinterpret_cast<RB *>(p.out) + o;
-#pragma unroll 1
-                for (int c = 0; c < CG; c += kCopyBatch) {   // kCopyBatch loads in flight per thread, then the stores
-                    RB v[kCopyBatch];
-#pragma unroll
-                    for (int i = 0; i < kCopyBatch; ++i) {
-                        v[i] = __ldcs(src);
-                        src += cells;
-                    }
-#pragma unroll
-                    for (int i = 0; i < kCopyBatch; ++i) {
-                        __stcs(dst, v[i]);
-                        dst += cells;
-                    }
-                }
-            }
-        }
+        copy_units<C, G, MT>(p, uframe, ucell, grp, cells);
     }
 
-    tc::cp_async_wait_all();
     if (!L::kResident && tid == 0) tc::mbar_wait_a(wbar + (wn & 1) * 8, (wn >> 1) & 1u);   // the weight chunk prefetched for a tile that never came
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tc::tmem_free(tmem_base, L::kTmemCols);
+    teardown(tmem_base, L::kTmemCols, warp);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -849,20 +908,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
     }
     __syncwarp();
     if (warp == 0) tc::tmem_alloc(tmem_slot, L::kTmemCols);
-    for (int c = tid; c < C; c += NT) {
-        swn[(c >> 3) * 16 + (c & 7)] = -__ldg(p.W1 + (size_t)c * (p.Ci + 3) + p.Ci);
-        swn[(c >> 3) * 16 + 8 + (c & 7)] = -__ldg(p.W1 + (size_t)c * (p.Ci + 3) + p.Ci + 1);
-    }
-    for (int o = tid * 16; o < 2 * L::kAbBytes + 2 * L::kWbBytes; o += NT * 16) *reinterpret_cast<uint4 *>(sAb + o) = make_uint4(0, 0, 0, 0);
-    __syncthreads();
-    for (int n = tid; n < 2 * C; n += NT) {
-        const int layer = n / C, c = n - layer * C;
-        const float bv = __ldg((layer ? p.b3 : p.b2) + c);
-        const __nv_bfloat16 h = __float2bfloat16_rn(bv);
-        const __nv_bfloat16 l = __float2bfloat16_rn(bv - __bfloat162float(h));
-        const uint32_t packed = (uint32_t)__bfloat16_as_ushort(h) | ((uint32_t)__bfloat16_as_ushort(l) << 16);
-        *reinterpret_cast<uint32_t *>(sWb + layer * L::kWbBytes + tc::unit_offset(c, 0, 2)) = packed;
-    }
+    setup_offsets_and_bias<C, NT>(p, tid, swn, sAb, 2 * L::kAbBytes);
     copy_chunk<NT>(sW, p.wimg2, L::kWBytes);
     tc::fence_proxy_async();
     tc::fence_before_sync();
@@ -889,39 +935,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
         ny[0] = make_float2(y0.x, y0.y); ny[1] = make_float2(y0.z, y0.w); ny[2] = make_float2(y1.x, y1.y); ny[3] = make_float2(y1.z, y1.w);
     };
 
-    const int32_t tpf = (int32_t)p.tiles_per_frame;
-    auto n_live_of = [&](int b) -> int32_t { return p.cell_list ? __ldg(p.cell_count + b) : (int32_t)cells; };
-    auto advance = [&](int32_t &b, int32_t &q, int32_t step) {
-        q += step;
-        while (q >= tpf) {
-            q -= tpf;
-            ++b;
-        }
-    };
-    auto seek_live = [&](int32_t &b, int32_t &q) {
-        while (b < p.B && q * kTile >= n_live_of(b)) advance(b, q, (int32_t)gridDim.x);
-    };
-    auto header_cell = [&](int32_t b, int32_t q) -> int32_t {
-        const int32_t e = q * kTile + row;
-        if (e >= n_live_of(b)) return -1;
-        return p.cell_list ? __ldg(p.cell_list + (size_t)b * cells + e) : e;
-    };
-    auto header_fill = [&](int32_t b, int32_t cell, int par) {
-        const uint32_t dst = sidx_addr + (uint32_t)((par * K * kTile + row) * 4);
-        float cx = 0.f, cy = 0.f;
-        if (cell >= 0) {
-            const int32_t *kr = p.knn + ((size_t)b * cells + cell) * K;
-            for (int k = 0; k < K; ++k) tc::cp_async4(dst + k * kTile * 4, kr + k);
-            const int32_t i = (int32_t)((uint32_t)cell / (uint32_t)p.W), j = cell - i * p.W;
-            cx = __fadd_rn(p.x0, __fmul_rn((float)i, p.dx));
-            cy = __fadd_rn(p.y0, __fmul_rn((float)j, p.dy));
-        } else {
-            for (int k = 0; k < K; ++k) tc::sts_u32(dst + k * kTile * 4, 0xFFFFFFFFu);
-        }
-        tc::cp_async_commit();
-        sctr[par * kTile + row] = make_float2(cx, cy);
-        scell[par * kTile + row] = cell;
-    };
+    const TileWalk<float2> walk{p, cells, (int32_t)p.tiles_per_frame, row, K, sidx_addr, sctr, scell, swmax};
     auto wait_bar = [&](uint32_t a) {
         tc::mbar_wait(&bar[a], (ph >> a) & 1u);
         ph ^= 1u << a;
@@ -929,61 +943,28 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
     };
 
     int32_t cb = 0, cq = 0, db = 0, dq = 0;   // cursors: MLP tiles (cb, cq), copy units (db, dq)
-    advance(cb, cq, (int32_t)blockIdx.x);
-    seek_live(cb, cq);
-    if (p.copy_dead) advance(db, dq, (int32_t)blockIdx.x); else db = p.B;
-    if (cb < p.B && grp == 0) header_fill(cb, header_cell(cb, cq), 0);
+    walk.start(cb, cq, db, dq, grp == 0);
 
-    int32_t uframe[2] = {-1, -1}, ucell[2] = {-1, -1};   // the next two copy units: frame (uniform) and this thread's cell
+    int32_t uframe[2] = {-1, -1}, ucell[2] = {-1, -1};   // the next two copy units (TileWalk::fetch_units)
     bool units_ready = false;
-    auto fetch_units = [&]() {
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            uframe[u] = -1;
-            ucell[u] = -1;
-            int32_t n_dead = 0;
-            while (db < p.B) {
-                n_dead = (int32_t)cells - n_live_of(db);
-                if (dq * kTile < n_dead) break;
-                advance(db, dq, (int32_t)gridDim.x);
-            }
-            if (db < p.B) {
-                uframe[u] = db;
-                const int32_t j = dq * kTile + row;
-                if (j < n_dead) ucell[u] = __ldg(p.cell_list + (size_t)db * cells + (cells - 1 - j));
-                advance(db, dq, (int32_t)gridDim.x);
-            }
-        }
-        units_ready = true;
-    };
 
     while (cb < p.B || db < p.B) {
         if (cb < p.B) {
             const int par = iter & 1;
             ++iter;
             const int b = cb;
-            fetch_units();   // list entries of the copy units that follow this tile: in flight during the whole tile
+            walk.fetch_units(db, dq, uframe, ucell);   // list entries of the copy units that follow this tile: in flight during the whole tile
+            units_ready = true;
             int32_t nb = cb, nq = cq;
-            advance(nb, nq, (int32_t)gridDim.x);
-            seek_live(nb, nq);
+            walk.advance(nb, nq, (int32_t)gridDim.x);
+            walk.seek_live(nb, nq);
             const bool has_next = nb < p.B;
             int n_valid = 0;
-            if (grp == 0) {
-                tc::cp_async_wait_all();
-                for (int k = 0; k < K; ++k) n_valid += (int32_t)tc::lds_u32(sidx_addr + (uint32_t)(((par * K + k) * kTile + row) * 4)) >= 0;
-                const int wm = __reduce_max_sync(0xffffffffu, n_valid);
-                if (lane == 0) swmax[par * 4 + warp] = wm;
-            }
-            __syncthreads();
-            int R;
-            {
-                const int4 wm = *reinterpret_cast<const int4 *>(swmax + par * 4);
-                R = max(max(wm.x, wm.y), max(wm.z, wm.w));
-            }
+            const int R = walk.read_header(par, grp == 0, lane, warp, n_valid);
             const int32_t cell = scell[par * kTile + row];
             const bool in_range = cell >= 0;
             int32_t ncell = -1;
-            if (grp == 0 && has_next) ncell = header_cell(nb, nq);
+            if (grp == 0 && has_next) ncell = walk.header_cell(nb, nq);
 
             const TT *Tc = reinterpret_cast<const TT *>(p.T) + (size_t)b * p.N * C + ku * 8, *neg = g_neg + ku * 8;
             const uint32_t idx0 = sidx_addr + (uint32_t)((par * K * kTile + rg0 * 8 + r8) * 4);
@@ -998,16 +979,8 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                     tc::ldg_row8(pr >= 0 ? Tc + (size_t)pr * C : neg, tv + 8 * i);
                 }
             };
-            auto prefetch_bev = [&]() {
-                if (in_range) {
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) {
-                        if (grp + j * G < kChunksE) {
-#pragma unroll
-                            for (int i = 0; i < EW; ++i) tv[j * EW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * EW + i) * cells);
-                        }
-                    }
-                }
+            auto prefetch_tv = [&]() {
+                if (in_range) prefetch_bev<C, G, 2>(tv, src_bev, cells, grp);
             };
             // A[buf] = relu(T[idx_k] - e) for the rows gathered in tv; bias flag of round k -> Ab[buf]
             auto build_round = [&](int k, uint32_t buf) {
@@ -1073,8 +1046,8 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             };
 
             if (R == 0) {
-                if (grp == 0 && has_next) header_fill(nb, ncell, par ^ 1);
-                prefetch_bev();
+                if (grp == 0 && has_next) walk.header_fill(nb, ncell, par ^ 1);
+                prefetch_tv();
             } else {
                 // ---- prologue: round 0 -------------------------------------------------------------------------------------
                 gather_round(0);
@@ -1083,12 +1056,12 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                 tc::fence_before_sync();
                 __syncthreads();
                 issue_round(0, 0, sW_addr, sWb_addr);
-                if (grp == 0 && has_next) header_fill(nb, ncell, par ^ 1);
+                if (grp == 0 && has_next) walk.header_fill(nb, ncell, par ^ 1);
                 if (R > 1) {
                     gather_round(1);
                 } else {
                     stream_w3(1);
-                    prefetch_bev();
+                    prefetch_tv();
                 }
                 for (int k = 0; k < R; ++k) {
                     const uint32_t a = k & 1;
@@ -1098,7 +1071,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                         tc::fence_before_sync();
                         __syncthreads();
                         issue_round(a ^ 1, a ^ 1, sW_addr, sWb_addr);
-                        if (k + 2 < R) gather_round(k + 2); else prefetch_bev();
+                        if (k + 2 < R) gather_round(k + 2); else prefetch_tv();
                     }
                     wait_bar(a);
                     if (k == R - 2) stream_w3(a);   // A[a] is free now; the last round uses A[a ^ 1]
@@ -1106,27 +1079,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                 }
                 // ---- layer 3: acc = n_valid * b3 + pooled * W3^T  (pooled -> A[l]; W3 sits in A[l ^ 1]) --------------------
                 const uint32_t l = (R - 1) & 1;
-                __syncwarp();
-#pragma unroll 1
-                for (int cc = grp; cc < C / EW; cc += G) {
-                    float s[EW];
-                    tc::tmem_ld<EW>(tmem_pool + lane_off + cc * EW, s);
-#pragma unroll
-                    for (int q = 0; q < EW / 8; ++q) {
-                        float2 v[4];
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) v[i] = make_float2(s[q * 8 + 2 * i], s[q * 8 + 2 * i + 1]);
-                        uint4 hi, lo;
-                        tc::relu_split_bf16x8(v, hi, lo, NS == 2);   // pooled >= 0: the ReLU is the identity here
-                        const uint32_t off = sA_addr + l * L::kABytes + tc::unit_offset(row, cc * (EW / 8) + q, kc_units);
-                        tc::sts_u32x4(off, hi);
-                        if (NS == 2) tc::sts_u32x4(off + kTile * C * 2, lo);
-                    }
-                }
-                if (grp == 0) {
-                    const uint32_t nv16 = __float_as_uint((float)n_valid) >> 16;   // small integers are exact in bf16
-                    tc::sts_u32(ab_row + l * L::kAbBytes, nv16 | (nv16 << 16));
-                }
+                pooled_to_operand<NS, C, G>(tmem_pool + lane_off, sA_addr + l * L::kABytes, row, grp, true, ab_row + l * L::kAbBytes, n_valid);
                 tc::cp_async_wait_all();   // this thread's part of W3 has landed
                 tc::fence_proxy_async();
                 tc::fence_before_sync();
@@ -1169,39 +1122,12 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             cb = nb;
             cq = nq;
         }
-        // ---- copy units: cells without a neighbour (back of the list): out = bev (list entries fetched at tile start) ----
-        if (!units_ready) fetch_units();
+        if (!units_ready) walk.fetch_units(db, dq, uframe, ucell);
         units_ready = false;
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            if (uframe[u] >= 0 && ucell[u] >= 0) {
-                constexpr int CG = C / G;
-                const size_t o = ((size_t)uframe[u] * C + grp * CG) * cells + ucell[u];
-                using RB = typename MapBits<MT>::type;
-                const RB *src = reinterpret_cast<const RB *>(p.bev) + o;
-                RB *dst = reinterpret_cast<RB *>(p.out) + o;
-#pragma unroll 1
-                for (int c = 0; c < CG; c += kCopyBatch) {
-                    RB v[kCopyBatch];
-#pragma unroll
-                    for (int i = 0; i < kCopyBatch; ++i) {
-                        v[i] = __ldcs(src);
-                        src += cells;
-                    }
-#pragma unroll
-                    for (int i = 0; i < kCopyBatch; ++i) {
-                        __stcs(dst, v[i]);
-                        dst += cells;
-                    }
-                }
-            }
-        }
+        copy_units<C, G, MT>(p, uframe, ucell, grp, cells);
     }
 
-    tc::cp_async_wait_all();
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tc::tmem_free(tmem_base, L::kTmemCols);
+    teardown(tmem_base, L::kTmemCols, warp);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1776,51 +1702,56 @@ int resident_ctas(Kern kern, int threads, int smem, int tmem_cols, int *regs_cac
     return CF_OK;
 }
 
-template <int C, int NS, bool TH = false, typename MT = float>
-int launch_tc(const TcParams &p, cudaStream_t st)
+template <bool SK, int C, int NS, bool TH, typename MT>
+int launch_kernel(const TcParams &p, cudaStream_t st)
 {
-    using L = TcLayout<C, NS>;
+    using L = std::conditional_t<SK, SkLayout<C, NS>, TcLayout<C, NS>>;
+    void (*kern)(TcParams);
+    if constexpr (SK) kern = k_fusion_sk<C, NS, TH, MT>; else kern = k_fusion_tc<C, NS, TH, MT>;
+    const char *name = SK ? "k_fusion_sk" : "k_fusion_tc";
     constexpr int NT = kTile * TcShape<C>::G;
     const int smem = L::smem_bytes(p.K);
     static int attr_bytes = 0, regs = 0;
     if (smem > attr_bytes) {
-        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_tc<C, NS, TH, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
-                           "k_fusion_tc smem attribute"));
+        CF_TRY(cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem), "fused kernel smem attribute"));
         attr_bytes = smem;
     }
     int per_sm = 1;
-    CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH, MT>, NT, smem, L::kTmemCols, &regs, &per_sm));
+    CF_TRY(resident_ctas(kern, NT, smem, L::kTmemCols, &regs, &per_sm));
     per_sm = std::max(1, per_sm);
     const int64_t grid = std::min<int64_t>(p.tiles_total, (int64_t)sm_count() * per_sm);
-    if (tuning().debug_launch) fprintf(stderr, "k_fusion_tc<%d,%d>: %d CTAs/SM grid %lld smem %d\n", C, NS, per_sm, (long long)grid, smem);
-    k_fusion_tc<C, NS, TH, MT><<<(unsigned)grid, NT, smem, st>>>(p);
+    if (tuning().debug_launch) fprintf(stderr, "%s<%d,%d>: %d CTAs/SM grid %lld smem %d\n", name, C, NS, per_sm, (long long)grid, smem);
+    kern<<<(unsigned)grid, NT, smem, st>>>(p);
     return CF_OK;
 }
 
-// The double-buffered kernel (k_fusion_sk) is used when its shared memory fits and it keeps the residency of k_fusion_tc;
-// returns CF_ERR_UNSUPPORTED (nothing launched) otherwise.
-template <int C, int NS, bool TH = false, typename MT = float>
-int launch_sk(const TcParams &p, cudaStream_t st)
+// Kernel choice.  Measured on B200 (profiles/README.md): the double-buffered k_fusion_sk wins where the MMAs of a round are
+// long (C = 128: 165 -> 148 us), is a wash at C = 64 and loses at C = 32, where the round is all operand build.  At C = 96
+// and 128 it keeps the residency of k_fusion_tc (1 CTA per SM: registers, and its 3C TMEM columns), so it runs wherever its
+// shared memory fits: always, except at C = 128 in fp32 mode (NS = 2) from K = 15 on.
+template <int C, int NS, bool TH, typename MT>
+int launch_fused(const TcParams &p, cudaStream_t st)
 {
-    using L = SkLayout<C, NS>;
-    using L0 = TcLayout<C, NS>;
-    constexpr int NT = kTile * TcShape<C>::G;
-    const int smem = L::smem_bytes(p.K);
-    if (smem > 227 * 1024) return CF_ERR_UNSUPPORTED;
-    static int attr_bytes = 0, regs = 0, regs0 = 0;
-    int per_sm = 0, per_sm0 = 0;
-    CF_TRY(resident_ctas(k_fusion_sk<C, NS, TH, MT>, NT, smem, L::kTmemCols, &regs, &per_sm));
-    CF_TRY(resident_ctas(k_fusion_tc<C, NS, TH, MT>, NT, L0::smem_bytes(p.K), L0::kTmemCols, &regs0, &per_sm0));
-    if (per_sm < 1 || per_sm < per_sm0) return CF_ERR_UNSUPPORTED;
-    if (smem > attr_bytes) {
-        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_sk<C, NS, TH, MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
-                           "k_fusion_sk smem attribute"));
-        attr_bytes = smem;
+    if constexpr (C == 96 || (C == 128 && NS == 1)) {
+        static_assert(SkLayout<C, NS>::smem_bytes(CF_MAX_K) <= 227 * 1024, "k_fusion_sk fits every K at this width");
+        return launch_kernel<true, C, NS, TH, MT>(p, st);
+    } else if constexpr (C == 128) {
+        if (SkLayout<C, NS>::smem_bytes(p.K) <= 227 * 1024) return launch_kernel<true, C, NS, TH, MT>(p, st);
+        return launch_kernel<false, C, NS, TH, MT>(p, st);
+    } else {
+        return launch_kernel<false, C, NS, TH, MT>(p, st);
     }
-    const int64_t grid = std::min<int64_t>(p.tiles_total, (int64_t)sm_count() * per_sm);
-    if (tuning().debug_launch) fprintf(stderr, "k_fusion_sk<%d,%d>: %d CTAs/SM grid %lld smem %d\n", C, NS, per_sm, (long long)grid, smem);
-    k_fusion_sk<C, NS, TH, MT><<<(unsigned)grid, NT, smem, st>>>(p);
-    return CF_OK;
+}
+
+// the fused launch of one width for the mode (NS, bf16 tables th) and the map type (io16: bf16 maps)
+template <int C>
+int launch_fused_width(const TcParams &p, int NS, bool th, bool io16, cudaStream_t st)
+{
+    if (io16)
+        return NS == 2 ? launch_fused<C, 2, false, __nv_bfloat16>(p, st)
+               : th    ? launch_fused<C, 1, true, __nv_bfloat16>(p, st)
+                       : launch_fused<C, 1, false, __nv_bfloat16>(p, st);
+    return NS == 2 ? launch_fused<C, 2, false, float>(p, st) : th ? launch_fused<C, 1, true, float>(p, st) : launch_fused<C, 1, false, float>(p, st);
 }
 
 }  // namespace
@@ -1857,7 +1788,6 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     const bool io16 = (mode & CF_IO_BF16) != 0;   // d_bev / d_out hold bf16 maps
     mode = mode_base(mode);
     const int NS = mode == CF_MODE_FP32 ? 2 : 1;
-    const int KC = kc_for(C, NS);
     // packed W2 | W3 operand images: the caller's cached copy (cf_fusion_pack_weights) or packed here
     const uint8_t *img2 = d_packed ? (const uint8_t *)d_packed : (const uint8_t *)d_workspace;
     const uint8_t *img3 = img2 + (size_t)NS * C * C * 2;
@@ -1869,12 +1799,7 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     // one contiguous blob, so the tiles are already either full or empty (empty tiles just copy bev -> out) and
     // compaction only adds a launch (measured: 123 -> 148 us at 88x100x192).
     const int64_t min_tiles = 4 * (int64_t)sm_count();
-    if (!d_packed) {
-        const int pack_blocks = (C * (C / 8) + 255) / 256;
-        k_pack_weights<<<pack_blocks, 256, 0, st>>>(d_W2, C, C, C, KC, NS, (uint8_t *)d_workspace);
-        k_pack_weights<<<pack_blocks, 256, 0, st>>>(d_W3, C, C, C, KC, NS, (uint8_t *)d_workspace + (size_t)NS * C * C * 2);
-        count_launches(2);
-    }
+    if (!d_packed) CF_TRY(fusion_tc_pack(d_W2, d_W3, C, mode, d_workspace, st));
     const bool compact = ceil_div64(n_cells, kTile) * B >= min_tiles;
     if (compact) {
         CF_TRY(cuda_status(cudaMemsetAsync(cell_count, 0, 512, st), "cf_fusion_fwd memset"));
@@ -1893,29 +1818,17 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     p.copy_dead = compact && d_out != d_bev;
     int rc = CF_ERR_UNSUPPORTED;
     const bool th = mode == CF_MODE_BF16_TABLES;   // d_T holds bf16 rows
-#define CF_TC_LAUNCH(fn, c, MT) \
-    (NS == 2 ? fn<c, 2, false, MT>(p, st) : th ? fn<c, 1, true, MT>(p, st) : fn<c, 1, false, MT>(p, st))
-#define CF_TC_CASE(c)                                                                                          \
-    case c:                                                                                                    \
-        rc = io16 ? CF_TC_LAUNCH(launch_tc, c, __nv_bfloat16) : CF_TC_LAUNCH(launch_tc, c, float);             \
-        break;
-#define CF_SK_CASE(c)                                                                                          \
-    case c:                                                                                                    \
-        rc = io16 ? CF_TC_LAUNCH(launch_sk, c, __nv_bfloat16) : CF_TC_LAUNCH(launch_sk, c, float);             \
-        if (rc == CF_ERR_UNSUPPORTED)                                                                          \
-            rc = io16 ? CF_TC_LAUNCH(launch_tc, c, __nv_bfloat16) : CF_TC_LAUNCH(launch_tc, c, float);         \
-        break;
     switch (C) {
-        // measured on B200 (profiles/README.md): the double-buffered kernel wins where the MMAs of a round are long
-        // (C = 128: 165 -> 148 us), is a wash at C = 64 and loses at C = 32, where the round is all operand build
-        CF_TC_CASE(32) CF_TC_CASE(64) CF_SK_CASE(96) CF_SK_CASE(128) CF_TC_CASE(192) CF_TC_CASE(256)
+        case 32: rc = launch_fused_width<32>(p, NS, th, io16, st); break;
+        case 64: rc = launch_fused_width<64>(p, NS, th, io16, st); break;
+        case 96: rc = launch_fused_width<96>(p, NS, th, io16, st); break;
+        case 128: rc = launch_fused_width<128>(p, NS, th, io16, st); break;
+        case 192: rc = launch_fused_width<192>(p, NS, th, io16, st); break;
+        case 256: rc = launch_fused_width<256>(p, NS, th, io16, st); break;
         default:
             set_error("cf_fusion_fwd: unsupported C=%d on the tensor-core path", C);
             return CF_ERR_UNSUPPORTED;
     }
-#undef CF_TC_CASE
-#undef CF_SK_CASE
-#undef CF_TC_LAUNCH
     CF_TRY(rc);
     count_launches(1);
     return launch_status("cf_fusion_fwd (tcgen05)");
@@ -1946,10 +1859,7 @@ int point_mlp1_tc(const float *d_feat, const float *d_points, const int64_t *d_n
     if (Ci % 16 != 0 || Ci > 256 || C % 32 != 0) return CF_ERR_UNSUPPORTED;
     if ((size_t)NS * (C + kTile) * Ci * 2 + 4 * C * 4 > 220 * 1024) return CF_ERR_UNSUPPORTED;
     const uint8_t *img = d_packed ? (const uint8_t *)d_packed : (const uint8_t *)d_workspace;
-    if (!d_packed) {
-        k_pack_weights<<<(C * (Ci / 8) + 255) / 256, 256, 0, st>>>(d_W1, C, Ci, Ci + 3, Ci, NS, (uint8_t *)d_workspace);
-        count_launches(1);
-    }
+    if (!d_packed) CF_TRY(point_mlp1_tc_pack(d_W1, Ci, C, mode, d_workspace, st));
     Mlp1Params p;
     p.feat = d_feat; p.points = d_points; p.num_points = d_num_points; p.wimg = img; p.W1 = d_W1; p.b1 = d_b1; p.T = d_T;
     p.B = B; p.N = N; p.Ci = Ci; p.tiles_per_frame = (N + kTile - 1) / kTile;
