@@ -16,6 +16,7 @@ IO_BF16 = 0x200             # CF_IO_BF16: OR-ed into the mode of cf_fusion_fwd /
 # "bf16t" = CF_MODE_BF16_TABLES: bf16 operands AND bf16 layer-1 tables (inference only)
 MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "simt": MODE_SIMT, "bf16t": MODE_BF16_TABLES}
 MAX_K = 16
+MAX_CAMERAS = 8             # CF_MAX_CAMERAS: cameras of a rig (cf_point_gather_multi)
 ABI_VERSION = 2
 
 _vp, _i32, _i64, _f32, _sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -36,6 +37,16 @@ SIGNATURES = {
                                   _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
     "cf_point_gather_bf16": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _vp, _vp, C.POINTER(C.c_float),
                                        _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
+    "cf_gather_multi_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32, _i64]),
+    "cf_point_gather_multi": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i32,
+                                        _f32, _f32, _vp, _vp, _vp]),
+    "cf_point_gather_multi_bf16": (C.c_int, [_vp, _i64, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _vp,
+                                             _i32, _f32, _f32, _vp, _vp, _vp]),
+    "cf_point_gather_multi_bwd": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _vp,
+                                            _vp, _i32, _f32, _f32, _vp]),
+    "cf_point_gather_multi_bwd_det_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32]),
+    "cf_point_gather_multi_bwd_det": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _i32, _vp,
+                                                _vp, _vp, _i32, _f32, _f32, _vp, _vp]),
     "cf_point_mlp1_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "cf_point_mlp1": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "cf_point_mlp1_pack_weights": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),

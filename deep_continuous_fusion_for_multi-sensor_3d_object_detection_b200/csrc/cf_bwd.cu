@@ -432,6 +432,52 @@ __global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restric
     }
 }
 
+// Camera rig: d img[b, m, c, y, x] += (w_mt / n_vis) * dF[b, p, c] for the 4 taps of every camera m that sees point p
+// (adjoint of k_point_gather_multi; with n_vis == 1 the products of k_point_gather_bwd).  Lane m < M projects into camera m.
+__global__ void __launch_bounds__(256) k_point_gather_multi_bwd(const float *__restrict__ dF, int64_t sb, int64_t sm, int64_t sc,
+                                                                int64_t sh, int64_t sw, int32_t M, int32_t Ci, int32_t Hf,
+                                                                int32_t Wf, const float *__restrict__ points,
+                                                                const float *__restrict__ calib,
+                                                                const int64_t *__restrict__ num_points, int32_t N, float sx,
+                                                                float sy, float *__restrict__ dimg)
+{
+    const int b = blockIdx.y;
+    const int32_t n = valid_points(num_points, b, N);
+    const int lane = threadIdx.x & 31;
+    const int32_t warps = gridDim.x * (blockDim.x >> 5);
+    const float *crt = calib + ((size_t)b * M + (lane < M ? lane : 0)) * 12;
+    for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < n; p += warps) {
+        const float *q = points + ((size_t)b * N + p) * 3;
+        float uf = 0.0f, vf = 0.0f;
+        const bool mine = lane < M && rig_project(crt, __ldg(q), __ldg(q + 1), __ldg(q + 2), sx, sy, Hf, Wf, uf, vf);
+        const unsigned vis = __ballot_sync(0xffffffffu, mine);
+        if (vis == 0) continue;
+        const float nv = (float)__popc(vis);
+        const float fx = floorf(uf), fy = floorf(vf);
+        const int32_t lix = (int32_t)fx, liy = (int32_t)fy;
+        const float wx1 = __fsub_rn(uf, fx), wy1 = __fsub_rn(vf, fy), wx0 = __fsub_rn(1.0f, wx1), wy0 = __fsub_rn(1.0f, wy1);
+        const float l0 = __fdiv_rn(__fmul_rn(wx0, wy0), nv), l1 = __fdiv_rn(__fmul_rn(wx1, wy0), nv);
+        const float l2 = __fdiv_rn(__fmul_rn(wx0, wy1), nv), l3 = __fdiv_rn(__fmul_rn(wx1, wy1), nv);
+        const float *src = dF + ((size_t)b * N + p) * Ci;
+        for (unsigned mk = vis; mk; mk &= mk - 1) {
+            const int m = __ffs(mk) - 1;
+            const int32_t ix = __shfl_sync(0xffffffffu, lix, m), iy = __shfl_sync(0xffffffffu, liy, m);
+            const float wt[4] = {__shfl_sync(0xffffffffu, l0, m), __shfl_sync(0xffffffffu, l1, m),
+                                 __shfl_sync(0xffffffffu, l2, m), __shfl_sync(0xffffffffu, l3, m)};
+            const int32_t tx[4] = {ix, ix + 1, ix, ix + 1}, ty[4] = {iy, iy, iy + 1, iy + 1};
+            float *dst = dimg + b * sb + m * sm;
+            for (int32_t c = lane; c < Ci; c += 32) {
+                const float gval = __ldg(src + c);
+                if (gval == 0.0f) continue;
+#pragma unroll
+                for (int t = 0; t < 4; ++t)
+                    if (tx[t] >= 0 && tx[t] < Wf && ty[t] >= 0 && ty[t] < Hf)
+                        atomicAdd(dst + c * sc + ty[t] * sh + tx[t] * sw, __fmul_rn(wt[t], gval));
+            }
+        }
+    }
+}
+
 static size_t up256(size_t v) { return (v + 255) / 256 * 256; }
 
 struct BwdWs {
@@ -749,4 +795,26 @@ extern "C" int cf_point_gather_bwd(const float *d_gfeat, float *d_gimg, int64_t 
                                                                           (float)Wf / img_w, (float)Hf / img_h, d_gimg);
     count_launches(1);
     return launch_status("cf_point_gather_bwd");
+}
+
+// adjoint of cf_point_gather_multi: d_gimg (the rig's logical (B,M,Ci,Hf,Wf) shape / strides) += scatter of d_gfeat (B,N,Ci)
+extern "C" int cf_point_gather_multi_bwd(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc, int64_t sh,
+                                         int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                         const float *d_points, const float *d_calib, const int64_t *d_num_points, int32_t N,
+                                         float img_w, float img_h, void *stream)
+{
+    using namespace cf;
+    CF_TRY(require_sm100());
+    CF_REQUIRE(d_gfeat && d_gimg && d_points && d_calib && d_num_points, CF_ERR_ARG, "cf_point_gather_multi_bwd: null pointer");
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "cf_point_gather_multi_bwd: M=%d cameras, expected 1..%d", M,
+               CF_MAX_CAMERAS);
+    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
+               "cf_point_gather_multi_bwd: bad extents");
+    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_multi_bwd: d_calib must be 4-byte aligned");
+    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
+    k_point_gather_multi_bwd<<<dim3(blocks, B), 256, 0, (cudaStream_t)stream>>>(d_gfeat, sb, sm, sc, sh, sw, M, Ci, Hf, Wf,
+                                                                                d_points, d_calib, d_num_points, N,
+                                                                                (float)Wf / img_w, (float)Hf / img_h, d_gimg);
+    count_launches(1);
+    return launch_status("cf_point_gather_multi_bwd");
 }

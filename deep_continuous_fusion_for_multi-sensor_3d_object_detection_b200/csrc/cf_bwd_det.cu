@@ -299,6 +299,82 @@ __global__ void __launch_bounds__(256) k_gdet_sum(const float *__restrict__ dF, 
     }
 }
 
+// Camera rig: every (b, m) map is one "frame" of the lists above (map index bm = b * M + m).  fill == 0: cnt[pixel] += 1 per
+// tap inside its camera's map;  fill == 1: place (key = 4 p + t, weight w_mt / n_vis) into the pixel's segment.  Thread =
+// point of frame blockIdx.y; cameras in ascending order.
+__global__ void __launch_bounds__(256) k_gdet_multi_taps(const float *__restrict__ points, const float *__restrict__ calib,
+                                                         const int64_t *__restrict__ num_points, int32_t M, int32_t N,
+                                                         int32_t Hf, int32_t Wf, float sx, float sy, int fill,
+                                                         int32_t *__restrict__ cnt, const int32_t *__restrict__ off,
+                                                         int32_t *__restrict__ key, float *__restrict__ wgt)
+{
+    const int b = blockIdx.y;
+    const int32_t n = valid_points(num_points, b, N);
+    const int64_t plane = (int64_t)Hf * Wf;
+    for (int32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
+        const float *q = points + ((size_t)b * N + p) * 3;
+        const float x = __ldg(q), y = __ldg(q + 1), z = __ldg(q + 2);
+        float uf[CF_MAX_CAMERAS], vf[CF_MAX_CAMERAS];
+        unsigned vis = 0;
+#pragma unroll
+        for (int m = 0; m < CF_MAX_CAMERAS; ++m)
+            if (m < M && rig_project(calib + ((size_t)b * M + m) * 12, x, y, z, sx, sy, Hf, Wf, uf[m], vf[m])) vis |= 1u << m;
+        const float nv = (float)__popc(vis);
+#pragma unroll
+        for (int m = 0; m < CF_MAX_CAMERAS; ++m) {
+            if (!(vis >> m & 1u)) continue;
+            const float fx = floorf(uf[m]), fy = floorf(vf[m]);
+            const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
+            const float wx1 = __fsub_rn(uf[m], fx), wy1 = __fsub_rn(vf[m], fy), wx0 = __fsub_rn(1.0f, wx1),
+                        wy0 = __fsub_rn(1.0f, wy1);
+            const float wt[4] = {__fmul_rn(wx0, wy0), __fmul_rn(wx1, wy0), __fmul_rn(wx0, wy1), __fmul_rn(wx1, wy1)};
+            const int32_t tx[4] = {ix, ix + 1, ix, ix + 1}, ty[4] = {iy, iy, iy + 1, iy + 1};
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                if (!(tx[t] >= 0 && tx[t] < Wf && ty[t] >= 0 && ty[t] < Hf)) continue;
+                const int64_t px = ((int64_t)b * M + m) * plane + (int64_t)ty[t] * Wf + tx[t];
+                if (!fill) {
+                    atomicAdd(cnt + px, 1);
+                } else {
+                    const int32_t pos = __ldg(off + px) + atomicSub(cnt + px, 1) - 1;
+                    key[pos] = p * 4 + t;
+                    wgt[pos] = __fdiv_rn(wt[t], nv);
+                }
+            }
+        }
+    }
+}
+
+// d img[b, m, c, y, x] += sum over the pixel's taps in ascending (point, tap) of w * dF[b, p, c]  (one warp per pixel of the
+// B*M maps; the sibling of k_gdet_sum with the frame of map bm = b * M + m)
+__global__ void __launch_bounds__(256) k_gdet_multi_sum(const float *__restrict__ dF, int32_t M, int32_t Ci, int32_t N,
+                                                        int32_t Hf, int32_t Wf, int64_t npx, const int32_t *__restrict__ off,
+                                                        const int32_t *__restrict__ key, const float *__restrict__ wgt,
+                                                        int32_t *__restrict__ key_s, float *__restrict__ wgt_s, int64_t sb,
+                                                        int64_t sm, int64_t sc, int64_t sh, int64_t sw,
+                                                        float *__restrict__ dimg)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t plane = (int64_t)Hf * Wf;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t px = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); px < npx; px += warps) {
+        const int32_t s0 = __ldg(off + px), L = __ldg(off + px + 1) - s0;
+        if (L == 0) continue;
+        warp_rank_sort(key, wgt, s0, L, key_s, wgt_s);
+        const int64_t bm = px / plane, yx = px - bm * plane, y = yx / Wf, x = yx - y * Wf;
+        const int64_t b = bm / M, m = bm - b * M;
+        const float *src = dF + (size_t)b * N * Ci;
+        float *dst = dimg + b * sb + m * sm + y * sh + x * sw;
+        for (int32_t c = lane; c < Ci; c += 32) {
+            float s = 0.0f;
+            for (int32_t j = 0; j < L; ++j)
+                s = __fadd_rn(s, __fmul_rn(wgt_s[s0 + j], __ldg(src + (size_t)(key_s[s0 + j] >> 2) * Ci + c)));
+            dst[c * sc] += s;
+        }
+        __syncwarp();
+    }
+}
+
 size_t up256(size_t v) { return (v + 255) / 256 * 256; }
 
 // off[0, n] = exclusive prefix of cnt[0, n), off[n] = total: three launches
@@ -445,4 +521,45 @@ extern "C" int cf_point_gather_bwd_det(const float *d_gfeat, float *d_gimg, int6
         d_gfeat, Ci, N, Hf, Wf, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s, sb, sc, sh, sw, d_gimg);
     count_launches(2);
     return launch_status("cf_point_gather_bwd_det");
+}
+
+extern "C" size_t cf_point_gather_multi_bwd_det_workspace_bytes(int32_t B, int32_t M, int32_t N, int32_t Hf, int32_t Wf)
+{
+    if (B <= 0 || M <= 0 || N <= 0 || Hf <= 0 || Wf <= 0) return 0;
+    return gdet_carve(nullptr, B * M, N, Hf, Wf).bytes;   // B*M maps, up to 4 taps per point in each
+}
+
+// cf_point_gather_multi_bwd with a fixed summation order: the lists of cf_point_gather_bwd_det over the B*M maps
+extern "C" int cf_point_gather_multi_bwd_det(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc,
+                                             int64_t sh, int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                             const float *d_points, const float *d_calib, const int64_t *d_num_points,
+                                             int32_t N, float img_w, float img_h, void *d_workspace, void *stream)
+{
+    using namespace cf;
+    CF_TRY(require_sm100());
+    CF_REQUIRE(d_gfeat && d_gimg && d_points && d_calib && d_num_points && d_workspace, CF_ERR_ARG,
+               "cf_point_gather_multi_bwd_det: null pointer");
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "cf_point_gather_multi_bwd_det: M=%d cameras, expected 1..%d", M,
+               CF_MAX_CAMERAS);
+    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
+               "cf_point_gather_multi_bwd_det: bad extents");
+    CF_REQUIRE((int64_t)4 * B * M * N < ((int64_t)1 << 31) && (int64_t)B * M * Hf * Wf < ((int64_t)1 << 31), CF_ERR_ARG,
+               "cf_point_gather_multi_bwd_det: 4*B*M*N and B*M*Hf*Wf must stay below 2^31");
+    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN,
+               "cf_point_gather_multi_bwd_det: d_calib must be 4-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    GdetWs w = gdet_carve(d_workspace, B * M, N, Hf, Wf);
+    const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
+    const int64_t npx = (int64_t)B * M * Hf * Wf;
+    CF_TRY(cuda_status(cudaMemsetAsync(w.cnt, 0, (size_t)npx * sizeof(int32_t), st), "cf_point_gather_multi_bwd_det memset"));
+    const dim3 tg((unsigned)std::min<int64_t>(ceil_div64(N, 256), 148 * 4), (unsigned)B);
+    k_gdet_multi_taps<<<tg, 256, 0, st>>>(d_points, d_calib, d_num_points, M, N, Hf, Wf, sx, sy, 0, w.cnt, nullptr, nullptr,
+                                          nullptr);
+    count_launches(1);
+    CF_TRY(scan_counts(w.cnt, npx, w.off, w.tiles, st));
+    k_gdet_multi_taps<<<tg, 256, 0, st>>>(d_points, d_calib, d_num_points, M, N, Hf, Wf, sx, sy, 1, w.cnt, w.off, w.key, w.wgt);
+    k_gdet_multi_sum<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div64(npx, 8), 148 * 16)), 256, 0, st>>>(
+        d_gfeat, M, Ci, N, Hf, Wf, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s, sb, sm, sc, sh, sw, d_gimg);
+    count_launches(2);
+    return launch_status("cf_point_gather_multi_bwd_det");
 }

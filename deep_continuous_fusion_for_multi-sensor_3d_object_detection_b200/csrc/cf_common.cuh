@@ -74,6 +74,24 @@ __device__ __forceinline__ int32_t valid_points(const int64_t *num_points, int b
     return (int32_t)n;
 }
 
+// Camera of a rig (cf_point_gather_multi*): projects (x,y,z) with the row-vector CRT at `crt` (12 floats, w > 0 in front)
+// into map coordinates, with the fp32 sequence of k_point_gather.  True when the camera sees the point: w > 0 and at least
+// one of the four bilinear taps lies inside the (Hf, Wf) map.
+__device__ __forceinline__ bool rig_project(const float *__restrict__ crt, float x, float y, float z, float sx, float sy,
+                                            int32_t Hf, int32_t Wf, float &uf, float &vf)
+{
+    float r[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+        r[c] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(x, __ldg(crt + c)), __fmul_rn(y, __ldg(crt + 3 + c))),
+                                   __fmul_rn(z, __ldg(crt + 6 + c))),
+                         __ldg(crt + 9 + c));
+    if (!(r[2] > 0.0f)) return false;
+    uf = __fsub_rn(__fmul_rn(__fadd_rn(__fdiv_rn(r[0], r[2]), 0.5f), sx), 0.5f);
+    vf = __fsub_rn(__fmul_rn(__fadd_rn(__fdiv_rn(r[1], r[2]), 0.5f), sy), 0.5f);
+    return uf > -1.0f && uf < (float)Wf && vf > -1.0f && vf < (float)Hf;
+}
+
 // uniform bucket grid over the BEV plane (K-1/K-2)
 struct BucketGrid {
     float gx0, gy0, cell, inv_cell;

@@ -9,6 +9,8 @@
 // shared-memory tile transpose (coalesced on both sides).  A channels_last map (sc == 1) is used in place.
 // A bf16 map (cf_point_gather_bf16) stays bf16 in its pixel-major copy; every tap is widened exactly to fp32 and blended
 // with the same fp32 sequence, so the features equal those of the widened fp32 map.
+// A camera rig (cf_point_gather_multi*) projects with device-side (B,M,4,3) calibrations (w > 0 in front) and averages the
+// blends of the cameras that see a point (semantics: include/cf_b200.h).
 #include "cf_common.cuh"
 
 namespace cf {
@@ -170,6 +172,144 @@ int point_gather(const MT *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64
     return launch_status("cf_point_gather");
 }
 
+// Camera rig: one warp per point.  Lane m < M projects the point into camera m (its CRT is read from the device, the same
+// 12 floats for every point of the frame); a ballot gives the visible set.  Each visible camera's taps and weights are
+// shuffled to the warp in ascending camera order, the warp blends its Ci channels (float4 per lane, the sequence of
+// k_point_gather) and sums the blends in registers; one division by n_vis, one store.
+template <typename MT>
+__global__ void __launch_bounds__(256) k_point_gather_multi(const MT *__restrict__ pix,  // (B, M, Hf*Wf, Ci) pixel-major
+                                                            int64_t pb, int64_t pm, int64_t ph, int64_t pw,  // pc == 1
+                                                            int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                                            const float *__restrict__ points, const float *__restrict__ calib,
+                                                            const int64_t *__restrict__ num_points, int32_t N, float sx,
+                                                            float sy, float *__restrict__ feat)
+{
+    const int b = blockIdx.y;
+    const int32_t n = valid_points(num_points, b, N);
+    const int lane = threadIdx.x & 31;
+    const int32_t warps_per_grid = gridDim.x * (blockDim.x >> 5);
+    const int32_t c4n = Ci >> 2;
+    const float *crt = calib + ((size_t)b * M + (lane < M ? lane : 0)) * 12;
+    for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < N; p += warps_per_grid) {
+        float4 *o = reinterpret_cast<float4 *>(feat + ((size_t)b * N + p) * Ci);
+        unsigned vis = 0;
+        float uf = 0.0f, vf = 0.0f;
+        if (p < n) {
+            const float *q = points + ((size_t)b * N + p) * 3;
+            const bool mine = lane < M && rig_project(crt, __ldg(q), __ldg(q + 1), __ldg(q + 2), sx, sy, Hf, Wf, uf, vf);
+            vis = __ballot_sync(0xffffffffu, mine);
+        }
+        if (vis == 0) {  // padding row, or no camera sees the point
+            for (int32_t c4 = lane; c4 < c4n; c4 += 32) o[c4] = make_float4(0.f, 0.f, 0.f, 0.f);
+            continue;
+        }
+        // this lane's camera: taps and weights exactly as k_point_gather (meaningful on the visible lanes only)
+        const float fx = floorf(uf), fy = floorf(vf);
+        const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
+        const float wx1 = __fsub_rn(uf, fx), wy1 = __fsub_rn(vf, fy);
+        const float wx0 = __fsub_rn(1.0f, wx1), wy0 = __fsub_rn(1.0f, wy1);
+        const bool okx0 = ix >= 0 && ix < Wf, okx1 = ix + 1 >= 0 && ix + 1 < Wf;
+        const bool oky0 = iy >= 0 && iy < Hf, oky1 = iy + 1 >= 0 && iy + 1 < Hf;
+        const float l00 = (okx0 && oky0) ? __fmul_rn(wx0, wy0) : 0.0f;
+        const float l01 = (okx1 && oky0) ? __fmul_rn(wx1, wy0) : 0.0f;
+        const float l10 = (okx0 && oky1) ? __fmul_rn(wx0, wy1) : 0.0f;
+        const float l11 = (okx1 && oky1) ? __fmul_rn(wx1, wy1) : 0.0f;
+        const int32_t lx0 = okx0 ? ix : 0, lx1 = okx1 ? ix + 1 : 0, ly0 = oky0 ? iy : 0, ly1 = oky1 ? iy + 1 : 0;
+        const int nv = __popc(vis);
+        for (int32_t cb = 0; cb < c4n; cb += 32) {  // warp-uniform trip count: every lane takes part in the shuffles
+            const int32_t c4 = cb + lane;
+            float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+            bool first = true;
+            for (unsigned mk = vis; mk; mk &= mk - 1) {
+                const int m = __ffs(mk) - 1;
+                const float w00 = __shfl_sync(0xffffffffu, l00, m), w01 = __shfl_sync(0xffffffffu, l01, m);
+                const float w10 = __shfl_sync(0xffffffffu, l10, m), w11 = __shfl_sync(0xffffffffu, l11, m);
+                const int32_t x0c = __shfl_sync(0xffffffffu, lx0, m), x1c = __shfl_sync(0xffffffffu, lx1, m);
+                const int32_t y0c = __shfl_sync(0xffffffffu, ly0, m), y1c = __shfl_sync(0xffffffffu, ly1, m);
+                if (c4 < c4n) {
+                    const MT *base = pix + b * pb + m * pm;
+                    const float4 a = ld_px4(base + y0c * ph + x0c * pw, c4), bq = ld_px4(base + y0c * ph + x1c * pw, c4);
+                    const float4 c = ld_px4(base + y1c * ph + x0c * pw, c4), d = ld_px4(base + y1c * ph + x1c * pw, c4);
+                    float4 r;
+                    r.x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.x), __fmul_rn(w01, bq.x)), __fmul_rn(w10, c.x)), __fmul_rn(w11, d.x));
+                    r.y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.y), __fmul_rn(w01, bq.y)), __fmul_rn(w10, c.y)), __fmul_rn(w11, d.y));
+                    r.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.z), __fmul_rn(w01, bq.z)), __fmul_rn(w10, c.z)), __fmul_rn(w11, d.z));
+                    r.w = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.w), __fmul_rn(w01, bq.w)), __fmul_rn(w10, c.w)), __fmul_rn(w11, d.w));
+                    if (first) {
+                        acc = r;  // not 0 + r: a -0.0 blend keeps its sign, so one camera gives the bits of k_point_gather
+                    } else {
+                        acc.x = __fadd_rn(acc.x, r.x);
+                        acc.y = __fadd_rn(acc.y, r.y);
+                        acc.z = __fadd_rn(acc.z, r.z);
+                        acc.w = __fadd_rn(acc.w, r.w);
+                    }
+                }
+                first = false;
+            }
+            if (c4 < c4n) {
+                if (nv > 1) {
+                    const float fn = (float)nv;
+                    acc = make_float4(__fdiv_rn(acc.x, fn), __fdiv_rn(acc.y, fn), __fdiv_rn(acc.z, fn), __fdiv_rn(acc.w, fn));
+                }
+                o[c4] = acc;
+            }
+        }
+    }
+}
+
+template <typename MT>
+int point_gather_multi(const MT *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw, int32_t B, int32_t M,
+                       int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_calib,
+                       const int64_t *d_num_points, int32_t N, float img_w, float img_h, float *d_feat, void *d_workspace,
+                       void *stream)
+{
+    CF_TRY(require_sm100());
+    CF_REQUIRE(d_img_feat && d_points && d_calib && d_num_points && d_feat, CF_ERR_ARG, "cf_point_gather_multi: null pointer");
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "cf_point_gather_multi: M=%d cameras, expected 1..%d", M,
+               CF_MAX_CAMERAS);
+    CF_REQUIRE(B > 0 && (int64_t)B * M <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0, CF_ERR_ARG,
+               "cf_point_gather_multi: bad extents");
+    CF_REQUIRE(Ci % 4 == 0, CF_ERR_ARG, "cf_point_gather_multi: Ci=%d must be a multiple of 4", Ci);
+    CF_REQUIRE(img_w > 0.0f && img_h > 0.0f, CF_ERR_ARG, "cf_point_gather_multi: bad image size");
+    CF_REQUIRE(aligned16(d_feat), CF_ERR_ALIGN, "cf_point_gather_multi: d_feat must be 16-byte aligned");
+    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_multi: d_calib must be 4-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    const MT *pix = d_img_feat;
+    int64_t pb = sb, pm = sm, ph = sh, pw = sw;
+    if (sc != 1) {
+        CF_REQUIRE(d_workspace != nullptr, CF_ERR_ARG, "cf_point_gather_multi: workspace required for channel-major maps");
+        CF_REQUIRE(aligned16(d_workspace), CF_ERR_ALIGN, "cf_point_gather_multi: workspace must be 16-byte aligned");
+        const int32_t HW = Hf * Wf;
+        MT *dst = (MT *)d_workspace;
+        const unsigned gx = (unsigned)((HW + 31) / 32), gy = (unsigned)((Ci + 31) / 32);
+        if (sb == (int64_t)M * sm) {  // the B*M maps are one run of stride sm: one launch re-lays them all
+            k_to_pixel_major<<<dim3(gx, gy, (unsigned)(B * M)), 256, 0, st>>>(d_img_feat, sm, sc, sh, sw, Ci, Hf, Wf, dst);
+            count_launches(1);
+        } else {
+            for (int32_t b = 0; b < B; ++b)
+                k_to_pixel_major<<<dim3(gx, gy, (unsigned)M), 256, 0, st>>>(d_img_feat + b * sb, sm, sc, sh, sw, Ci, Hf, Wf,
+                                                                          dst + (size_t)b * M * HW * Ci);
+            count_launches(B);
+        }
+        pix = dst;
+        pm = (int64_t)HW * Ci;
+        pb = (int64_t)M * pm;
+        ph = (int64_t)Wf * Ci;
+        pw = Ci;
+    } else {
+        CF_REQUIRE((reinterpret_cast<uintptr_t>(d_img_feat) & (4 * sizeof(MT) - 1)) == 0 && sb % 4 == 0 && sm % 4 == 0 &&
+                       sh % 4 == 0 && sw % 4 == 0,
+                   CF_ERR_ALIGN, "cf_point_gather_multi: channels_last maps must be %d-byte aligned per pixel",
+                   (int)(4 * sizeof(MT)));
+    }
+    const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
+    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
+    k_point_gather_multi<<<dim3(blocks, B), 256, 0, st>>>(pix, pb, pm, ph, pw, M, Ci, Hf, Wf, d_points, d_calib, d_num_points,
+                                                          N, sx, sy, d_feat);
+    count_launches(1);
+    return launch_status("cf_point_gather_multi");
+}
+
 }  // namespace cf
 
 extern "C" size_t cf_gather_workspace_bytes(int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc)
@@ -194,4 +334,28 @@ extern "C" int cf_point_gather_bf16(const void *d_img_feat, int64_t sb, int64_t 
 {
     return cf::point_gather(static_cast<const __nv_bfloat16 *>(d_img_feat), sb, sc, sh, sw, B, Ci, Hf, Wf, d_points, d_uv,
                             h_calib, d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
+}
+
+extern "C" size_t cf_gather_multi_workspace_bytes(int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc)
+{
+    if (sc == 1) return 0;
+    return (size_t)B * (size_t)M * (size_t)Ci * (size_t)Hf * (size_t)Wf * sizeof(float);
+}
+
+extern "C" int cf_point_gather_multi(const float *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
+                                     int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
+                                     const float *d_calib, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
+                                     float *d_feat, void *d_workspace, void *stream)
+{
+    return cf::point_gather_multi(d_img_feat, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, d_points, d_calib, d_num_points, N, img_w,
+                                  img_h, d_feat, d_workspace, stream);
+}
+
+extern "C" int cf_point_gather_multi_bf16(const void *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
+                                          int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
+                                          const float *d_calib, const int64_t *d_num_points, int32_t N, float img_w,
+                                          float img_h, float *d_feat, void *d_workspace, void *stream)
+{
+    return cf::point_gather_multi(static_cast<const __nv_bfloat16 *>(d_img_feat), sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, d_points,
+                                  d_calib, d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
 }

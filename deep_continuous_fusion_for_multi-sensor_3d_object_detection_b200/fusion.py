@@ -52,6 +52,20 @@ class FrameContext:
             t.record_stream(main)
 
     def gather(self, img_feat, calib=None, uv=None, img_size=(640.0, 480.0)):
+        """K-3.  A (B,Ci,Hf,Wf) map: one camera, `calib` the reference's (4,3) CRT_tensor or `uv` the projected points.
+        A (B,M,Ci,Hf,Wf) map: a rig of M cameras, `calib` a (B,M,4,3) or (M,4,3) CUDA tensor with w > 0 in front
+        (geometry.camera_rig), read on the device; each point gets the mean feature of the cameras that see it."""
+        if isinstance(img_feat, torch.Tensor) and img_feat.dim() == 5:
+            if uv is not None:
+                raise ValueError("gather: precomputed uv cannot be used with a camera rig (5-D map); pass the rig's calib")
+            if calib is None:
+                raise ValueError("gather: a camera rig (5-D map) needs calib (B,M,4,3) or (M,4,3)")
+            if torch.is_grad_enabled() and img_feat.requires_grad:
+                self.feat = _GatherMultiFunction.apply(img_feat, self.points, self.num_points, calib, tuple(img_size))
+            else:
+                self.feat, self._gather_ws = ops.point_gather_multi(img_feat, self.points, self.num_points, calib,
+                                                                    img_size=img_size, workspace=self._gather_ws)
+            return self.feat
         if torch.is_grad_enabled() and img_feat.requires_grad:
             self.feat = _GatherFunction.apply(img_feat, self.points, self.num_points, calib, uv, tuple(img_size))
         else:
@@ -198,16 +212,27 @@ class FusionRunner:
     `.bevs[s] (B,C_s,H_s,W_s)` (e.g. straight from pinned host memory), calls the runner, and reads `.outs[s]`
     (the same tensors as `.bevs` when `inplace=True`).  Replaying the graph costs one launch on the host instead of the
     ~20 launches and several stream hand-offs of the eager path, which matters when the host is the slow side.
-    `dtype=torch.bfloat16`: `.img_feat`, `.bevs` and `.outs` are bf16 maps (half the bytes to copy in and out)."""
+    `dtype=torch.bfloat16`: `.img_feat`, `.bevs` and `.outs` are bf16 maps (half the bytes to copy in and out).
+    `cameras=M`: a camera rig.  `.img_feat` is (B,M,Ci,Hf,Wf) and `.calib` a static (B,M,4,3) float32 device buffer
+    (initialised from `calib`, an (M,4,3) or (B,M,4,3) rig such as geometry.camera_rig, if given): calibrations written into
+    it between replays take effect without a new capture."""
 
     def __init__(self, layers, grid, batch, max_points, img_shape, bev_shapes, calib=None, img_size=(640.0, 480.0),
-                 inplace=True, device=None, dtype=torch.float32):
+                 inplace=True, device=None, dtype=torch.float32, cameras=None):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.layers, self.grid, self.calib, self.img_size, self.inplace = list(layers), grid, calib, tuple(img_size), inplace
         self.points = torch.zeros((batch, max_points, 3), dtype=torch.float32, device=dev)
         self.num_points = torch.zeros((batch,), dtype=torch.int64, device=dev)
         if dtype not in ops.MAP_DTYPES:
             raise TypeError(f"FusionRunner: dtype must be torch.float32 or torch.bfloat16, got {dtype}")
+        if cameras is not None:
+            cameras = int(cameras)
+            if not 1 <= cameras <= G.MAX_CAMERAS:
+                raise ValueError(f"FusionRunner: cameras={cameras}, expected 1..{G.MAX_CAMERAS}")
+            self.calib = torch.zeros((batch, cameras, 4, 3), dtype=torch.float32, device=dev)
+            if calib is not None:
+                self.calib.copy_(torch.as_tensor(calib, dtype=torch.float32, device=dev).expand(batch, cameras, 4, 3))
+            img_shape = (cameras,) + tuple(img_shape)
         self.img_feat = torch.zeros((batch,) + tuple(img_shape), dtype=dtype, device=dev)
         self.bevs = [torch.zeros((batch,) + tuple(sh), dtype=dtype, device=dev) for sh in bev_shapes]
         self.outs = None
@@ -271,6 +296,25 @@ class _GatherFunction(torch.autograd.Function):
                                     uv=uv if ctx.has_uv else None, img_size=ctx.img_size,
                                     deterministic=torch.are_deterministic_algorithms_enabled())
         return gimg, None, None, None, None, None
+
+
+class _GatherMultiFunction(torch.autograd.Function):
+    """K-3 of a camera rig with its adjoint; the deterministic kernel under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, img_feats, points, num_points, calib, img_size):
+        feat, _ = ops.point_gather_multi(img_feats, points, num_points, calib, img_size=img_size)
+        ctx.save_for_backward(points, num_points, calib)
+        ctx.img_size, ctx.img_like = img_size, img_feats
+        return feat
+
+    @staticmethod
+    def backward(ctx, grad_feat):
+        points, num_points, calib = ctx.saved_tensors
+        det = torch.are_deterministic_algorithms_enabled()
+        gimg = ops.point_gather_multi_bwd(grad_feat, ctx.img_like, points, num_points, calib, img_size=ctx.img_size,
+                                          deterministic=det)
+        return gimg, None, None, None, None
 
 
 class _FusionFunction(torch.autograd.Function):

@@ -37,6 +37,7 @@ FUSION_DEFAULTS = {
     "fusion_image_stride": 4,      # camera map is (image_height/stride, image_width/stride)
     "fusion_mlp_mode": "fp32",     # "fp32" | "bf16" | "bf16t" (bf16 + bf16 tables, inference only) | "simt" (A12)
     "fusion_bucket_size": 0.5,     # metres, K-1 grid pitch
+    "fusion_camera_yaws": None,    # degrees, one per camera of a rig (geometry.camera_rig); None = the single camera
 }
 
 
@@ -99,11 +100,12 @@ def bucket_grid(config: dict, cell: float | None = None):
     return np.float32(gx0), np.float32(gy0), np.float32(cell), nbx, nby
 
 
-def calibration_crt() -> np.ndarray:
-    """CRT_tensor of data_import_carla.py:31-34 as a (4,3) float32 array: [x y z 1] @ CRT = (u*w, v*w, w).
+def _projection64(yaw: float = 0.0) -> np.ndarray:
+    """(3,4) float64 projection Cm [R | 0] of the reference camera turned by `yaw` radians about the LiDAR z axis.
 
     The reference builds R with numpy-quaternion's from_euler_angles(v_cam - v_lidar) (:180-188), i.e. the
-    Z-Y-Z Euler convention R = Rz(alpha) Ry(beta) Rz(gamma); translation 0; intrinsics from :190-194.
+    Z-Y-Z Euler convention R = Rz(alpha) Ry(beta) Rz(gamma); translation 0; intrinsics from :190-194.  A camera turned by
+    yaw sees the point p where the reference camera sees Rz(-yaw) p, so its rotation is R Rz(-yaw) (yaw 0 leaves R as it is).
     """
     a, b, g = (np.array([-3.13498819, 1.59196951, 1.56942932]) - np.array([-1.57079633, 3.12042851, -1.57079633]))
 
@@ -114,6 +116,29 @@ def calibration_crt() -> np.ndarray:
         return np.array([[math.cos(t), 0.0, math.sin(t)], [0.0, 1.0, 0.0], [-math.sin(t), 0.0, math.cos(t)]])
 
     R = rz(a) @ ry(b) @ rz(g)
+    if yaw != 0.0:
+        R = R @ rz(-yaw)
     RT = np.concatenate([R, np.zeros((3, 1))], axis=1)
     Cm = np.array([[268.51188197672957, 0.0, 320.0], [0.0, 268.51188197672957, 240.0], [0.0, 0.0, 1.0]])
-    return np.ascontiguousarray((Cm @ RT).T.astype(np.float32))
+    return Cm @ RT
+
+
+def calibration_crt() -> np.ndarray:
+    """CRT_tensor of data_import_carla.py:31-34 as a (4,3) float32 array: [x y z 1] @ CRT = (u*w, v*w, w), w < 0 for points
+    in front of the camera (the reference's orientation)."""
+    return np.ascontiguousarray(_projection64().T.astype(np.float32))
+
+
+MAX_CAMERAS = 8   # CF_MAX_CAMERAS of include/cf_b200.h
+
+
+def camera_rig(yaws_deg) -> np.ndarray:
+    """(M,4,3) float32 calibrations of a rig of M reference cameras, camera m turned by yaws_deg[m] degrees about the LiDAR
+    z axis (positive toward +y, i.e. to the left), for cf_point_gather_multi: [x y z 1] @ CRT_m = (u*w, v*w, w) with w > 0 in
+    front of the camera.  Computed in float64, rounded once to float32 and negated (exact), so yaw 0 is exactly
+    -calibration_crt() and every camera's (u, v) is the reference camera's (u, v) of the point turned by -yaw."""
+    yaws = [float(y) for y in np.asarray(yaws_deg, dtype=np.float64).reshape(-1)]
+    if not 1 <= len(yaws) <= MAX_CAMERAS:
+        raise ValueError(f"camera_rig: {len(yaws)} cameras, expected 1..{MAX_CAMERAS}")
+    crt = np.stack([_projection64(math.radians(y)).T.astype(np.float32) for y in yaws])
+    return np.ascontiguousarray(-crt)

@@ -273,17 +273,38 @@ class ObjectDetection_DCF(nn.Module):
                                                         mode=str(G.fusion_option(config, "fusion_mlp_mode")))
         self._grid = ops.BucketGrid(*G.bucket_grid(config))
         self.register_buffer("calib", torch.from_numpy(G.calibration_crt()), persistent=False)
+        # optional camera rig (additive key): M reference cameras turned about the LiDAR z axis, one shared camera stream
+        yaws = G.fusion_option(config, "fusion_camera_yaws")
+        self.cameras = None if yaws is None else len(yaws)
+        if yaws is not None:
+            self.register_buffer("rig_calib", torch.from_numpy(G.camera_rig(yaws)), persistent=False)
 
-    def forward(self, x_lidar, x_image, pointcloud_raw=None, num_points_raw=None, projected_loc_uv=None):
+    def forward(self, x_lidar, x_image, pointcloud_raw=None, num_points_raw=None, projected_loc_uv=None, camera_calib=None):
+        """With `fusion_camera_yaws` in the config, x_image is (B,M,3,H,W) (one image per camera) and `camera_calib`
+        (B,M,4,3) float32, w > 0 in front (geometry.camera_rig), optionally replaces the rig built from the yaws."""
         fuse = None
+        if self.cameras is None and camera_calib is not None:
+            raise ValueError("camera_calib needs a camera rig (config key fusion_camera_yaws)")
+        if self.cameras is not None and pointcloud_raw is not None:
+            if projected_loc_uv is not None:
+                raise ValueError("projected_loc_uv cannot be used with a camera rig (fusion_camera_yaws): the rig projects "
+                                 "every point on the device")
+            if x_image.dim() != 5 or x_image.shape[1] != self.cameras:
+                raise ValueError(f"x_image: expected (B,{self.cameras},3,H,W) for the {self.cameras}-camera rig, got "
+                                 f"{tuple(x_image.shape)}")
         if pointcloud_raw is not None:
             if num_points_raw is None:
                 raise ValueError("num_points_raw is required with pointcloud_raw")
             # K-1 (point bucketing) is launched first, on its side stream: it runs under the camera trunk
             frames = FrameContext(pointcloud_raw.to(x_lidar.device), num_points_raw, self._grid)
-            img_feat = self.image_backbone(x_image)
+            if self.cameras is None:
+                img_feat = self.image_backbone(x_image)
+            else:   # the one camera stream runs on all B*M images; its channels_last output is viewed as (B,M,Ci,Hf,Wf)
+                img_feat = self.image_backbone(x_image.flatten(0, 1)).unflatten(0, tuple(x_image.shape[:2]))
             size = (float(self.config["image_width"]), float(self.config["image_height"]))
-            if projected_loc_uv is not None:
+            if self.cameras is not None:
+                frames.gather(img_feat, calib=self.rig_calib if camera_calib is None else camera_calib, img_size=size)
+            elif projected_loc_uv is not None:
                 frames.gather(img_feat, uv=projected_loc_uv.to(x_lidar.device), img_size=size)
             else:
                 frames.gather(img_feat, calib=self.calib, img_size=size)

@@ -207,6 +207,56 @@ def point_gather(img_feat, points, num_points, calib=None, uv=None, img_size=(64
     return out, workspace
 
 
+def _rig_args(img_feats, points, calib, name):
+    """Checks of a camera-rig call, made before anything is launched -> (B, M, Ci, Hf, Wf, N, calib (B,M,4,3))."""
+    for t, what in ((img_feats, "img_feats"), (points, "points"), (calib, "calib")):
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: {what} must be a torch.Tensor, got {type(t).__name__}")
+    if img_feats.dim() != 5:
+        raise ValueError(f"{name}: img_feats must be (B,M,Ci,Hf,Wf), got shape {tuple(img_feats.shape)}")
+    B, M, Ci, Hf, Wf = img_feats.shape
+    if not 1 <= M <= _lib.MAX_CAMERAS:
+        raise ValueError(f"{name}: {M} cameras, expected 1..{_lib.MAX_CAMERAS}")
+    if Ci % 4:
+        raise ValueError(f"{name}: Ci={Ci} must be a multiple of 4")
+    if points.dim() != 3 or points.shape[0] != B or points.shape[2] != 3:
+        raise ValueError(f"{name}: points must be ({B},N,3), got {tuple(points.shape)}")
+    if tuple(calib.shape) not in ((B, M, 4, 3), (M, 4, 3)):
+        raise ValueError(f"{name}: calib must be ({B},{M},4,3) or ({M},4,3), got {tuple(calib.shape)}")
+    if calib.dtype != torch.float32:
+        raise TypeError(f"{name}: calib must be torch.float32, got {calib.dtype}")
+    if img_feats.dtype not in MAP_DTYPES:
+        raise TypeError(f"{name}: img_feats: expected dtype torch.float32 or torch.bfloat16, got {img_feats.dtype}")
+    _req(calib, "calib", torch.float32)
+    if calib.device != points.device:
+        raise ValueError(f"{name}: calib is on {calib.device}, points on {points.device}")
+    # (M,4,3): one rig for every frame, broadcast on the device (a copy kernel, no host round trip)
+    calib = calib.expand(B, M, 4, 3).contiguous() if calib.dim() == 3 else calib.contiguous()
+    return B, M, Ci, Hf, Wf, points.shape[1], calib
+
+
+def point_gather_multi(img_feats, points, num_points, calib, img_size=(640.0, 480.0), out=None, workspace=None):
+    """K-3 for a camera rig (cf_point_gather_multi).  img_feats logical (B,M,Ci,Hf,Wf) fp32 or bf16, any strides (channels_last
+    per camera, as the model emits, needs no re-layout pass); points (B,N,3); calib (B,M,4,3) or (M,4,3) float32 CUDA tensor
+    with w > 0 in front of the camera (geometry.camera_rig), read on the device -> feat (B,N,Ci) fp32: the mean over the
+    cameras that see each point of their bilinear features (zero where none does)."""
+    lib = load()
+    B, M, Ci, Hf, Wf, N, calib = _rig_args(img_feats, points, calib, "point_gather_multi")
+    _req(num_points, "num_points", torch.int64, 1)
+    _map(img_feats, "img_feats", 5)
+    points = _contig(points, "points", torch.float32, 3)
+    sb, sm, sc, sh, sw = img_feats.stride()
+    if out is None:
+        out = torch.empty((B, N, Ci), dtype=torch.float32, device=points.device)
+    need = lib.cf_gather_multi_workspace_bytes(B, M, Ci, Hf, Wf, sc)
+    if need and (workspace is None or workspace.numel() < need):
+        workspace = torch.empty((need,), dtype=torch.uint8, device=points.device)
+    fn = lib.cf_point_gather_multi_bf16 if img_feats.dtype == torch.bfloat16 else lib.cf_point_gather_multi
+    check(fn(ptr(img_feats), sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, ptr(points), ptr(calib), ptr(num_points), N,
+             float(img_size[0]), float(img_size[1]), ptr(out), ptr(workspace), stream_ptr()), "cf_point_gather_multi")
+    return out, workspace
+
+
 class PackedWeights:
     """Cache of the UMMA operand images of one layer's weights.  Re-packs only when a weight tensor was modified
     in place (optimizer step -> Tensor._version changes) or replaced; in inference the weights are packed once."""
@@ -448,6 +498,30 @@ def point_gather_bwd(grad_feat, img_like, points, num_points, calib=None, uv=Non
                                       ptr(num_points), N, float(img_size[0]), float(img_size[1]), stream_ptr()),
               "cf_point_gather_bwd")
     return gimg.to(img_like.dtype)   # a no-op for fp32; bf16 keeps the memory format (preserve_format)
+
+
+def point_gather_multi_bwd(grad_feat, img_like, points, num_points, calib, img_size=(640.0, 480.0), deterministic=False):
+    """Adjoint of point_gather_multi: gradient w.r.t. the rig's camera maps (shape, dtype and strides of img_like (B,M,Ci,Hf,Wf)).
+    `deterministic`: each pixel sums its (point, tap) contributions in a fixed order (cf_point_gather_multi_bwd_det).
+    A bf16 img_like: the taps are summed into an fp32 map, which is rounded to bf16 once at the end."""
+    lib = load()
+    B, M, Ci, Hf, Wf, N, calib = _rig_args(img_like, points, calib, "point_gather_multi_bwd")
+    _req(num_points, "num_points", torch.int64, 1)
+    _map(img_like, "img_like", 5)
+    grad_feat = _contig(grad_feat, "grad_feat", torch.float32, 3)
+    if tuple(grad_feat.shape) != (B, N, Ci):
+        raise ValueError(f"point_gather_multi_bwd: grad_feat must be {(B, N, Ci)}, got {tuple(grad_feat.shape)}")
+    points = _contig(points, "points", torch.float32, 3)
+    gimg = torch.zeros_like(img_like, dtype=torch.float32)
+    sb, sm, sc, sh, sw = gimg.stride()
+    args = (ptr(grad_feat), ptr(gimg), sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, ptr(points), ptr(calib), ptr(num_points), N,
+            float(img_size[0]), float(img_size[1]))
+    if deterministic:
+        ws = _scratch(lib.cf_point_gather_multi_bwd_det_workspace_bytes(B, M, N, Hf, Wf), gimg.device)
+        check(lib.cf_point_gather_multi_bwd_det(*args, ptr(ws), stream_ptr()), "cf_point_gather_multi_bwd_det")
+    else:
+        check(lib.cf_point_gather_multi_bwd(*args, stream_ptr()), "cf_point_gather_multi_bwd")
+    return gimg.to(img_like.dtype)
 
 
 # ------------------------------------------------------------------------------------------ post-process

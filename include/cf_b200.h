@@ -112,6 +112,56 @@ CF_API int cf_point_gather_bf16(const void *d_img_feat, int64_t sb, int64_t sc, 
                          float *d_feat, void *d_workspace, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * K-3 for a camera rig: M cameras (1 <= M <= CF_MAX_CAMERAS) with one shared map shape and image size.
+ *   d_img_feat  camera maps, logical (B,M,Ci,Hf,Wf) fp32 (bf16: cf_point_gather_multi_bf16) with ELEMENT strides
+ *               sb,sm,sc,sh,sw (sc == 1, channels_last, is read in place: every pixel 16-byte (bf16: 8-byte) aligned;
+ *               otherwise the B*M maps are re-laid pixel-major into d_workspace, cf_gather_multi_workspace_bytes bytes)
+ *   d_calib     (B,M,4,3) fp32 DEVICE calibrations, one row-vector CRT per frame and camera, read by the kernel (so a
+ *               captured CUDA graph sees new values written into the same buffer):
+ *                 [x y z 1] @ CRT_m = (u*w, v*w, w),  w > 0 in FRONT of the camera.  The reference's CRT_tensor has
+ *                 w < 0 ahead; its negation (all 12 entries) gives the same u, v bit for bit.
+ *   visibility  camera m sees point p iff w_m > 0 and at least one bilinear tap lies inside the map (the in-range test of
+ *               cf_point_gather: uf > -1 && uf < Wf && vf > -1 && vf < Hf, uf/vf computed as there).
+ *   d_feat      (B,N,Ci) fp32 out.  With n_vis = number of cameras that see p:
+ *                 acc = blend_m0;  acc = acc + blend_m  (fp32, ascending camera order over the visible cameras);
+ *                 feat[p] = n_vis > 1 ? acc / n_vis : acc  (__fdiv_rn),
+ *               blend_m = the fp32 bilinear sequence of cf_point_gather in camera m's map.  n_vis == 0 and rows
+ *               >= num_points[b] are zero.  So M = 1 with CRT = -CRT_tensor gives the bits of cf_point_gather for every
+ *               point with w > 0.  bf16 maps: taps widened exactly, blend in fp32, as cf_point_gather_bf16.
+ *   B*M <= 65535.
+ * cf_point_gather_multi_bwd, the adjoint: tap t of every camera m that sees p receives
+ *     d_gimg[b,m,:,y_t,x_t] += (w_mt / n_vis) * d_gfeat[b,p,:]      (q = __fdiv_rn(w_mt, n_vis); __fmul_rn(q, g))
+ *   with w_mt the unmasked tap weight of cf_point_gather_bwd; taps outside the map are dropped.  For n_vis == 1 the
+ *   products are those of cf_point_gather_bwd.  Float atomics: reproducible to rounding.  d_gimg fp32, logical
+ *   (B,M,Ci,Hf,Wf) with the given element strides (for a bf16 map accumulate in fp32 and round once).
+ * cf_point_gather_multi_bwd_det: the same sums in a fixed order.  Each (b,m) map is one frame of cf_point_gather_bwd_det:
+ *   the (point, tap) contributions are listed per pixel of their own camera's map, each list in ascending (point, tap),
+ *   and one thread per (pixel, channel) computes s = 0; s = s + q_j * g_j over its list and adds s into d_gimg.
+ *   n_vis == 1 everywhere gives the bits of cf_point_gather_bwd_det.  The order depends on the inputs only (not on the SM
+ *   count).  Workspace cf_point_gather_multi_bwd_det_workspace_bytes(B, M, N, Hf, Wf); 4*B*M*N, B*M*Hf*Wf < 2^31.
+ * None of these synchronises with the host: all are capturable in a CUDA graph.
+ * ------------------------------------------------------------------------------------------- */
+#define CF_MAX_CAMERAS 8
+CF_API size_t cf_gather_multi_workspace_bytes(int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc);
+CF_API int cf_point_gather_multi(const float *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
+                                 int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
+                                 const float *d_calib, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
+                                 float *d_feat, void *d_workspace, void *stream);
+CF_API int cf_point_gather_multi_bf16(const void *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
+                                      int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
+                                      const float *d_calib, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
+                                      float *d_feat, void *d_workspace, void *stream);
+CF_API int cf_point_gather_multi_bwd(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc, int64_t sh,
+                                     int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                     const float *d_points, const float *d_calib, const int64_t *d_num_points, int32_t N,
+                                     float img_w, float img_h, void *stream);
+CF_API size_t cf_point_gather_multi_bwd_det_workspace_bytes(int32_t B, int32_t M, int32_t N, int32_t Hf, int32_t Wf);
+CF_API int cf_point_gather_multi_bwd_det(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc, int64_t sh,
+                                         int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                         const float *d_points, const float *d_calib, const int64_t *d_num_points,
+                                         int32_t N, float img_w, float img_h, void *d_workspace, void *stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K-4a per-point half of MLP layer 1 (exact factorisation of Appendix A8/A9):
  *   T[b,p,:] = W1[:, :Ci] f_p + W1[:, Ci:Ci+3] (px,py,pz) + b1        so that for BEV cell centre c
  *   relu(W1 [f_p, p - (cx,cy,0)] + b1) = relu(T[b,p,:] - W1[:,Ci]*cx - W1[:,Ci+1]*cy)
