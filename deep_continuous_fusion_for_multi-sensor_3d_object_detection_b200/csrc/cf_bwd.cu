@@ -382,14 +382,11 @@ __global__ void __launch_bounds__(256) k_bwd_scatter(const float *__restrict__ d
     }
 }
 
-// d img[b, c, y, x] += w_tap * dF[b, p, c] for the 4 bilinear taps of point p (adjoint of k_point_gather)
-struct CalibB {
-    float m[12];
-};
-__global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restrict__ dF, int64_t sb, int64_t sc, int64_t sh,
-                                                          int64_t sw, int32_t Ci, int32_t Hf, int32_t Wf,
-                                                          const float *__restrict__ points, const float *__restrict__ uv,
-                                                          CalibB cal, int use_calib, const int64_t *__restrict__ num_points,
+// d img[b, m, c, y, x] += (w_mt / n_vis) * dF[b, p, c] for the taps inside the map of every camera m that sees point p
+// (adjoint of k_point_gather; with n_vis == 1 the quotient is w_mt itself).  Lane m < M resolves camera m.
+__global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restrict__ dF, int64_t sb, int64_t sm, int64_t sc,
+                                                          int64_t sh, int64_t sw, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                                          const CamSource src, const int64_t *__restrict__ num_points,
                                                           int32_t N, float sx, float sy, float *__restrict__ dimg)
 {
     const int b = blockIdx.y;
@@ -397,85 +394,51 @@ __global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restric
     const int lane = threadIdx.x & 31;
     const int32_t warps = gridDim.x * (blockDim.x >> 5);
     for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < n; p += warps) {
-        float u, v;
-        if (use_calib) {
-            const float *q = points + ((size_t)b * N + p) * 3;
-            const float x = __ldg(q), y = __ldg(q + 1), z = __ldg(q + 2);
-            float r[3];
-#pragma unroll
-            for (int c = 0; c < 3; ++c)
-                r[c] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(x, cal.m[c]), __fmul_rn(y, cal.m[3 + c])),
-                                           __fmul_rn(z, cal.m[6 + c])), cal.m[9 + c]);
-            u = __fdiv_rn(r[0], r[2]);
-            v = __fdiv_rn(r[1], r[2]);
-        } else {
-            u = __ldg(uv + ((size_t)b * N + p) * 2);
-            v = __ldg(uv + ((size_t)b * N + p) * 2 + 1);
-        }
-        const float uf = __fsub_rn(__fmul_rn(__fadd_rn(u, 0.5f), sx), 0.5f);
-        const float vf = __fsub_rn(__fmul_rn(__fadd_rn(v, 0.5f), sy), 0.5f);
-        if (!(uf > -1.0f && uf < (float)Wf && vf > -1.0f && vf < (float)Hf)) continue;
-        const float fx = floorf(uf), fy = floorf(vf);
-        const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
-        const float wx1 = uf - fx, wy1 = vf - fy, wx0 = 1.0f - wx1, wy0 = 1.0f - wy1;
-        const float wt[4] = {wx0 * wy0, wx1 * wy0, wx0 * wy1, wx1 * wy1};
-        const int32_t tx[4] = {ix, ix + 1, ix, ix + 1}, ty[4] = {iy, iy, iy + 1, iy + 1};
-        const float *src = dF + ((size_t)b * N + p) * Ci;
-        for (int32_t c = lane; c < Ci; c += 32) {
-            const float gval = __ldg(src + c);
-            if (gval == 0.0f) continue;
-#pragma unroll
-            for (int t = 0; t < 4; ++t)
-                if (tx[t] >= 0 && tx[t] < Wf && ty[t] >= 0 && ty[t] < Hf)
-                    atomicAdd(dimg + b * sb + c * sc + ty[t] * sh + tx[t] * sw, wt[t] * gval);
-        }
-    }
-}
-
-// Camera rig: d img[b, m, c, y, x] += (w_mt / n_vis) * dF[b, p, c] for the 4 taps of every camera m that sees point p
-// (adjoint of k_point_gather_multi; with n_vis == 1 the products of k_point_gather_bwd).  Lane m < M projects into camera m.
-__global__ void __launch_bounds__(256) k_point_gather_multi_bwd(const float *__restrict__ dF, int64_t sb, int64_t sm, int64_t sc,
-                                                                int64_t sh, int64_t sw, int32_t M, int32_t Ci, int32_t Hf,
-                                                                int32_t Wf, const float *__restrict__ points,
-                                                                const float *__restrict__ calib,
-                                                                const int64_t *__restrict__ num_points, int32_t N, float sx,
-                                                                float sy, float *__restrict__ dimg)
-{
-    const int b = blockIdx.y;
-    const int32_t n = valid_points(num_points, b, N);
-    const int lane = threadIdx.x & 31;
-    const int32_t warps = gridDim.x * (blockDim.x >> 5);
-    const float *crt = calib + ((size_t)b * M + (lane < M ? lane : 0)) * 12;
-    for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < n; p += warps) {
-        const float *q = points + ((size_t)b * N + p) * 3;
         float uf = 0.0f, vf = 0.0f;
-        const bool mine = lane < M && rig_project(crt, __ldg(q), __ldg(q + 1), __ldg(q + 2), sx, sy, Hf, Wf, uf, vf);
-        const unsigned vis = __ballot_sync(0xffffffffu, mine);
+        const unsigned vis = __ballot_sync(0xffffffffu, lane < M && cam_project(src, b, N, p, lane, M, sx, sy, Hf, Wf, uf, vf));
         if (vis == 0) continue;
         const float nv = (float)__popc(vis);
-        const float fx = floorf(uf), fy = floorf(vf);
-        const int32_t lix = (int32_t)fx, liy = (int32_t)fy;
-        const float wx1 = __fsub_rn(uf, fx), wy1 = __fsub_rn(vf, fy), wx0 = __fsub_rn(1.0f, wx1), wy0 = __fsub_rn(1.0f, wy1);
-        const float l0 = __fdiv_rn(__fmul_rn(wx0, wy0), nv), l1 = __fdiv_rn(__fmul_rn(wx1, wy0), nv);
-        const float l2 = __fdiv_rn(__fmul_rn(wx0, wy1), nv), l3 = __fdiv_rn(__fmul_rn(wx1, wy1), nv);
-        const float *src = dF + ((size_t)b * N + p) * Ci;
+        const Taps tp = bilinear_taps(uf, vf, Hf, Wf);
+        const float l0 = __fdiv_rn(tp.w[0], nv), l1 = __fdiv_rn(tp.w[1], nv);
+        const float l2 = __fdiv_rn(tp.w[2], nv), l3 = __fdiv_rn(tp.w[3], nv);
+        const int lin = tp.in(0) | tp.in(1) << 1 | tp.in(2) << 2 | tp.in(3) << 3;
+        const float *g = dF + ((size_t)b * N + p) * Ci;
         for (unsigned mk = vis; mk; mk &= mk - 1) {
             const int m = __ffs(mk) - 1;
-            const int32_t ix = __shfl_sync(0xffffffffu, lix, m), iy = __shfl_sync(0xffffffffu, liy, m);
+            const int32_t ix = __shfl_sync(0xffffffffu, tp.x, m), iy = __shfl_sync(0xffffffffu, tp.y, m);
+            const int in = __shfl_sync(0xffffffffu, lin, m);
             const float wt[4] = {__shfl_sync(0xffffffffu, l0, m), __shfl_sync(0xffffffffu, l1, m),
                                  __shfl_sync(0xffffffffu, l2, m), __shfl_sync(0xffffffffu, l3, m)};
             const int32_t tx[4] = {ix, ix + 1, ix, ix + 1}, ty[4] = {iy, iy, iy + 1, iy + 1};
             float *dst = dimg + b * sb + m * sm;
             for (int32_t c = lane; c < Ci; c += 32) {
-                const float gval = __ldg(src + c);
+                const float gval = __ldg(g + c);
                 if (gval == 0.0f) continue;
 #pragma unroll
                 for (int t = 0; t < 4; ++t)
-                    if (tx[t] >= 0 && tx[t] < Wf && ty[t] >= 0 && ty[t] < Hf)
-                        atomicAdd(dst + c * sc + ty[t] * sh + tx[t] * sw, __fmul_rn(wt[t], gval));
+                    if (in >> t & 1) atomicAdd(dst + c * sc + ty[t] * sh + tx[t] * sw, __fmul_rn(wt[t], gval));
             }
         }
     }
+}
+
+// K-3's atomic adjoint for M cameras of one source; `fn` names the entry point in the error texts
+static int point_gather_bwd(const char *fn, const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc, int64_t sh,
+                            int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const CamSource &src,
+                            const int64_t *d_num_points, int32_t N, float img_w, float img_h, void *stream)
+{
+    CF_TRY(require_sm100());
+    CF_REQUIRE(d_gfeat && d_gimg && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points, CF_ERR_ARG,
+               "%s: null pointer", fn);
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
+    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
+               "%s: bad extents", fn);
+    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
+    k_point_gather_bwd<<<dim3(blocks, B), 256, 0, (cudaStream_t)stream>>>(d_gfeat, sb, sm, sc, sh, sw, M, Ci, Hf, Wf, src,
+                                                                          d_num_points, N, (float)Wf / img_w,
+                                                                          (float)Hf / img_h, d_gimg);
+    count_launches(1);
+    return launch_status(fn);
 }
 
 static size_t up256(size_t v) { return (v + 255) / 256 * 256; }
@@ -781,20 +744,9 @@ extern "C" int cf_point_gather_bwd(const float *d_gfeat, float *d_gimg, int64_t 
                                    float img_w, float img_h, void *stream)
 {
     using namespace cf;
-    CF_TRY(require_sm100());
-    CF_REQUIRE(d_gfeat && d_gimg && d_points && d_num_points, CF_ERR_ARG, "cf_point_gather_bwd: null pointer");
     CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG, "cf_point_gather_bwd: pass exactly one of d_uv / h_calib");
-    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
-               "cf_point_gather_bwd: bad extents");
-    CalibB cal{};
-    if (h_calib)
-        for (int i = 0; i < 12; ++i) cal.m[i] = h_calib[i];
-    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
-    k_point_gather_bwd<<<dim3(blocks, B), 256, 0, (cudaStream_t)stream>>>(d_gfeat, sb, sc, sh, sw, Ci, Hf, Wf, d_points, d_uv,
-                                                                          cal, h_calib != nullptr, d_num_points, N,
-                                                                          (float)Wf / img_w, (float)Hf / img_h, d_gimg);
-    count_launches(1);
-    return launch_status("cf_point_gather_bwd");
+    return point_gather_bwd("cf_point_gather_bwd", d_gfeat, d_gimg, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
+                            camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, stream);
 }
 
 // adjoint of cf_point_gather_multi: d_gimg (the rig's logical (B,M,Ci,Hf,Wf) shape / strides) += scatter of d_gfeat (B,N,Ci)
@@ -804,17 +756,7 @@ extern "C" int cf_point_gather_multi_bwd(const float *d_gfeat, float *d_gimg, in
                                          float img_w, float img_h, void *stream)
 {
     using namespace cf;
-    CF_TRY(require_sm100());
-    CF_REQUIRE(d_gfeat && d_gimg && d_points && d_calib && d_num_points, CF_ERR_ARG, "cf_point_gather_multi_bwd: null pointer");
-    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "cf_point_gather_multi_bwd: M=%d cameras, expected 1..%d", M,
-               CF_MAX_CAMERAS);
-    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
-               "cf_point_gather_multi_bwd: bad extents");
     CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_multi_bwd: d_calib must be 4-byte aligned");
-    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
-    k_point_gather_multi_bwd<<<dim3(blocks, B), 256, 0, (cudaStream_t)stream>>>(d_gfeat, sb, sm, sc, sh, sw, M, Ci, Hf, Wf,
-                                                                                d_points, d_calib, d_num_points, N,
-                                                                                (float)Wf / img_w, (float)Hf / img_h, d_gimg);
-    count_launches(1);
-    return launch_status("cf_point_gather_multi_bwd");
+    return point_gather_bwd("cf_point_gather_multi_bwd", d_gfeat, d_gimg, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf,
+                            rig_source(d_points, d_calib), d_num_points, N, img_w, img_h, stream);
 }

@@ -10,6 +10,8 @@
 //     (kDetSplits is a constant, not the SM count), so a result reproduces on any B200;
 //   - dT and d img are gathers over CSR lists (counting sort by point / pixel, each segment then ordered by its key), one
 //     writer per output row.
+#include <cstdio>
+
 #include "cf_common.cuh"
 
 namespace cf {
@@ -198,147 +200,38 @@ __global__ void __launch_bounds__(256) k_det_dT(const float *__restrict__ dA, in
 }
 
 // ---- camera-map gradient ---------------------------------------------------------------------------------------------
-struct CalibD {
-    float m[12];
-};
-
-// the four bilinear taps of point p of frame b, exactly as k_point_gather / k_point_gather_bwd compute them;
-// false when the point falls outside the map
-__device__ __forceinline__ bool point_taps(const float *__restrict__ points, const float *__restrict__ uv, const CalibD &cal,
-                                           int use_calib, int b, int32_t N, int32_t p, int32_t Hf, int32_t Wf, float sx,
-                                           float sy, int32_t tx[4], int32_t ty[4], float wt[4])
-{
-    float u, v;
-    if (use_calib) {
-        const float *q = points + ((size_t)b * N + p) * 3;
-        const float x = __ldg(q), y = __ldg(q + 1), z = __ldg(q + 2);
-        float r[3];
-#pragma unroll
-        for (int c = 0; c < 3; ++c)
-            r[c] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(x, cal.m[c]), __fmul_rn(y, cal.m[3 + c])), __fmul_rn(z, cal.m[6 + c])),
-                             cal.m[9 + c]);
-        u = __fdiv_rn(r[0], r[2]);
-        v = __fdiv_rn(r[1], r[2]);
-    } else {
-        u = __ldg(uv + ((size_t)b * N + p) * 2);
-        v = __ldg(uv + ((size_t)b * N + p) * 2 + 1);
-    }
-    const float uf = __fsub_rn(__fmul_rn(__fadd_rn(u, 0.5f), sx), 0.5f);
-    const float vf = __fsub_rn(__fmul_rn(__fadd_rn(v, 0.5f), sy), 0.5f);
-    if (!(uf > -1.0f && uf < (float)Wf && vf > -1.0f && vf < (float)Hf)) return false;
-    const float fx = floorf(uf), fy = floorf(vf);
-    const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
-    const float wx1 = __fsub_rn(uf, fx), wy1 = __fsub_rn(vf, fy), wx0 = __fsub_rn(1.0f, wx1), wy0 = __fsub_rn(1.0f, wy1);
-    wt[0] = __fmul_rn(wx0, wy0); wt[1] = __fmul_rn(wx1, wy0); wt[2] = __fmul_rn(wx0, wy1); wt[3] = __fmul_rn(wx1, wy1);
-    tx[0] = ix; tx[1] = ix + 1; tx[2] = ix; tx[3] = ix + 1;
-    ty[0] = iy; ty[1] = iy; ty[2] = iy + 1; ty[3] = iy + 1;
-    return true;
-}
-
-struct GatherArgs {
-    const float *points, *uv;
-    CalibD cal;
-    int use_calib;
-    const int64_t *num_points;
-    int32_t N, Hf, Wf;
-    float sx, sy;
-};
-
-// fill == 0: cnt[pixel] += 1 per tap inside the map;  fill == 1: place (key = 4 p + t, weight) into the pixel's segment
-// (thread = point of frame blockIdx.y)
-__global__ void __launch_bounds__(256) k_gdet_taps(const GatherArgs a, int fill, int32_t *__restrict__ cnt,
-                                                   const int32_t *__restrict__ off, int32_t *__restrict__ key,
-                                                   float *__restrict__ wgt)
-{
-    const int b = blockIdx.y;
-    const int32_t n = valid_points(a.num_points, b, a.N);
-    const int64_t plane = (int64_t)a.Hf * a.Wf;
-    for (int32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
-        int32_t tx[4], ty[4];
-        float wt[4];
-        if (!point_taps(a.points, a.uv, a.cal, a.use_calib, b, a.N, p, a.Hf, a.Wf, a.sx, a.sy, tx, ty, wt)) continue;
-#pragma unroll
-        for (int t = 0; t < 4; ++t) {
-            if (!(tx[t] >= 0 && tx[t] < a.Wf && ty[t] >= 0 && ty[t] < a.Hf)) continue;
-            const int64_t px = b * plane + (int64_t)ty[t] * a.Wf + tx[t];
-            if (!fill) {
-                atomicAdd(cnt + px, 1);
-            } else {
-                const int32_t pos = __ldg(off + px) + atomicSub(cnt + px, 1) - 1;
-                key[pos] = p * 4 + t;
-                wgt[pos] = wt[t];
-            }
-        }
-    }
-}
-
-// d img[b, c, y, x] += sum over the pixel's taps in ascending (point, tap) of w * dF[b, p, c]  (one warp per pixel)
-__global__ void __launch_bounds__(256) k_gdet_sum(const float *__restrict__ dF, int32_t Ci, int32_t N, int32_t Hf, int32_t Wf,
-                                                  int64_t npx, const int32_t *__restrict__ off, const int32_t *__restrict__ key,
-                                                  const float *__restrict__ wgt, int32_t *__restrict__ key_s,
-                                                  float *__restrict__ wgt_s, int64_t sb, int64_t sc, int64_t sh, int64_t sw,
-                                                  float *__restrict__ dimg)
-{
-    const int lane = threadIdx.x & 31;
-    const int64_t plane = (int64_t)Hf * Wf;
-    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
-    for (int64_t px = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); px < npx; px += warps) {
-        const int32_t s0 = __ldg(off + px), L = __ldg(off + px + 1) - s0;
-        if (L == 0) continue;
-        warp_rank_sort(key, wgt, s0, L, key_s, wgt_s);
-        const int64_t b = px / plane, yx = px - b * plane, y = yx / Wf, x = yx - y * Wf;
-        const float *src = dF + (size_t)b * N * Ci;
-        float *dst = dimg + b * sb + y * sh + x * sw;
-        for (int32_t c = lane; c < Ci; c += 32) {
-            float s = 0.0f;
-            for (int32_t j = 0; j < L; ++j)
-                s = __fadd_rn(s, __fmul_rn(wgt_s[s0 + j], __ldg(src + (size_t)(key_s[s0 + j] >> 2) * Ci + c)));
-            dst[c * sc] += s;
-        }
-        __syncwarp();
-    }
-}
-
-// Camera rig: every (b, m) map is one "frame" of the lists above (map index bm = b * M + m).  fill == 0: cnt[pixel] += 1 per
-// tap inside its camera's map;  fill == 1: place (key = 4 p + t, weight w_mt / n_vis) into the pixel's segment.  Thread =
+// Every (b, m) camera map is one "frame" of the lists (map index bm = b * M + m).  fill == 0: cnt[pixel] += 1 per tap
+// inside its camera's map;  fill == 1: place (key = 4 p + t, weight w_mt / n_vis) into the pixel's segment.  Thread =
 // point of frame blockIdx.y; cameras in ascending order.
-__global__ void __launch_bounds__(256) k_gdet_multi_taps(const float *__restrict__ points, const float *__restrict__ calib,
-                                                         const int64_t *__restrict__ num_points, int32_t M, int32_t N,
-                                                         int32_t Hf, int32_t Wf, float sx, float sy, int fill,
-                                                         int32_t *__restrict__ cnt, const int32_t *__restrict__ off,
-                                                         int32_t *__restrict__ key, float *__restrict__ wgt)
+__global__ void __launch_bounds__(256) k_gdet_taps(const CamSource src, const int64_t *__restrict__ num_points, int32_t M,
+                                                   int32_t N, int32_t Hf, int32_t Wf, float sx, float sy, int fill,
+                                                   int32_t *__restrict__ cnt, const int32_t *__restrict__ off,
+                                                   int32_t *__restrict__ key, float *__restrict__ wgt)
 {
     const int b = blockIdx.y;
     const int32_t n = valid_points(num_points, b, N);
     const int64_t plane = (int64_t)Hf * Wf;
     for (int32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
-        const float *q = points + ((size_t)b * N + p) * 3;
-        const float x = __ldg(q), y = __ldg(q + 1), z = __ldg(q + 2);
-        float uf[CF_MAX_CAMERAS], vf[CF_MAX_CAMERAS];
+        // the visible set first (n_vis divides every weight), then the taps of each visible camera, projected again
         unsigned vis = 0;
-#pragma unroll
-        for (int m = 0; m < CF_MAX_CAMERAS; ++m)
-            if (m < M && rig_project(calib + ((size_t)b * M + m) * 12, x, y, z, sx, sy, Hf, Wf, uf[m], vf[m])) vis |= 1u << m;
+        float uf, vf;
+        for (int m = 0; m < M; ++m)
+            if (cam_project(src, b, N, p, m, M, sx, sy, Hf, Wf, uf, vf)) vis |= 1u << m;
         const float nv = (float)__popc(vis);
-#pragma unroll
-        for (int m = 0; m < CF_MAX_CAMERAS; ++m) {
+        for (int m = 0; m < M; ++m) {
             if (!(vis >> m & 1u)) continue;
-            const float fx = floorf(uf[m]), fy = floorf(vf[m]);
-            const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
-            const float wx1 = __fsub_rn(uf[m], fx), wy1 = __fsub_rn(vf[m], fy), wx0 = __fsub_rn(1.0f, wx1),
-                        wy0 = __fsub_rn(1.0f, wy1);
-            const float wt[4] = {__fmul_rn(wx0, wy0), __fmul_rn(wx1, wy0), __fmul_rn(wx0, wy1), __fmul_rn(wx1, wy1)};
-            const int32_t tx[4] = {ix, ix + 1, ix, ix + 1}, ty[4] = {iy, iy, iy + 1, iy + 1};
+            cam_project(src, b, N, p, m, M, sx, sy, Hf, Wf, uf, vf);
+            const Taps tp = bilinear_taps(uf, vf, Hf, Wf);
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
-                if (!(tx[t] >= 0 && tx[t] < Wf && ty[t] >= 0 && ty[t] < Hf)) continue;
-                const int64_t px = ((int64_t)b * M + m) * plane + (int64_t)ty[t] * Wf + tx[t];
+                if (!tp.in(t)) continue;
+                const int64_t px = ((int64_t)b * M + m) * plane + (int64_t)(tp.y + (t >> 1)) * Wf + tp.x + (t & 1);
                 if (!fill) {
                     atomicAdd(cnt + px, 1);
                 } else {
                     const int32_t pos = __ldg(off + px) + atomicSub(cnt + px, 1) - 1;
                     key[pos] = p * 4 + t;
-                    wgt[pos] = __fdiv_rn(wt[t], nv);
+                    wgt[pos] = __fdiv_rn(tp.w[t], nv);
                 }
             }
         }
@@ -346,13 +239,12 @@ __global__ void __launch_bounds__(256) k_gdet_multi_taps(const float *__restrict
 }
 
 // d img[b, m, c, y, x] += sum over the pixel's taps in ascending (point, tap) of w * dF[b, p, c]  (one warp per pixel of the
-// B*M maps; the sibling of k_gdet_sum with the frame of map bm = b * M + m)
-__global__ void __launch_bounds__(256) k_gdet_multi_sum(const float *__restrict__ dF, int32_t M, int32_t Ci, int32_t N,
-                                                        int32_t Hf, int32_t Wf, int64_t npx, const int32_t *__restrict__ off,
-                                                        const int32_t *__restrict__ key, const float *__restrict__ wgt,
-                                                        int32_t *__restrict__ key_s, float *__restrict__ wgt_s, int64_t sb,
-                                                        int64_t sm, int64_t sc, int64_t sh, int64_t sw,
-                                                        float *__restrict__ dimg)
+// B*M maps)
+__global__ void __launch_bounds__(256) k_gdet_sum(const float *__restrict__ dF, int32_t M, int32_t Ci, int32_t N, int32_t Hf,
+                                                  int32_t Wf, int64_t npx, const int32_t *__restrict__ off,
+                                                  const int32_t *__restrict__ key, const float *__restrict__ wgt,
+                                                  int32_t *__restrict__ key_s, float *__restrict__ wgt_s, int64_t sb,
+                                                  int64_t sm, int64_t sc, int64_t sh, int64_t sw, float *__restrict__ dimg)
 {
     const int lane = threadIdx.x & 31;
     const int64_t plane = (int64_t)Hf * Wf;
@@ -472,61 +364,66 @@ GdetWs gdet_carve(void *base, int32_t B, int32_t N, int32_t Hf, int32_t Wf)
     w.bytes = o;
     return w;
 }
-}  // namespace
 
-extern "C" size_t cf_point_gather_bwd_det_workspace_bytes(int32_t B, int32_t N, int32_t Hf, int32_t Wf)
-{
-    if (B <= 0 || N <= 0 || Hf <= 0 || Wf <= 0) return 0;
-    return gdet_carve(nullptr, B, N, Hf, Wf).bytes;
-}
 
-// cf_point_gather_bwd with a fixed summation order: CSR of the (point, tap) contributions by pixel, one thread per
-// (pixel, channel) summing its segment in ascending (point, tap) order
-extern "C" int cf_point_gather_bwd_det(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sc, int64_t sh, int64_t sw,
-                                       int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
-                                       const float *d_uv, const float *h_calib, const int64_t *d_num_points, int32_t N,
-                                       float img_w, float img_h, void *d_workspace, void *stream)
+// K-3's fixed-order adjoint for M cameras of one source: CSR of the (point, tap) contributions by pixel of the B*M maps, one
+// thread per (pixel, channel) summing its segment in ascending (point, tap) order; `fn` names the entry point in the error
+// texts
+static int point_gather_bwd_det(const char *fn, const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc,
+                                int64_t sh, int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                const cf::CamSource &src, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
+                                void *d_workspace, void *stream)
 {
     using namespace cf;
+    const char *bm = src.kind == CamSource::kRig ? "B*M" : "B";
     CF_TRY(require_sm100());
-    CF_REQUIRE(d_gfeat && d_gimg && d_points && d_num_points && d_workspace, CF_ERR_ARG, "cf_point_gather_bwd_det: null pointer");
-    CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG,
-               "cf_point_gather_bwd_det: pass exactly one of d_uv / h_calib");
+    CF_REQUIRE(d_gfeat && d_gimg && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points && d_workspace,
+               CF_ERR_ARG, "%s: null pointer", fn);
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
     CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
-               "cf_point_gather_bwd_det: bad extents");
-    CF_REQUIRE((int64_t)4 * B * N < ((int64_t)1 << 31) && (int64_t)B * Hf * Wf < ((int64_t)1 << 31), CF_ERR_ARG,
-               "cf_point_gather_bwd_det: 4*B*N and B*Hf*Wf must stay below 2^31");
+               "%s: bad extents", fn);
+    CF_REQUIRE((int64_t)4 * B * M * N < ((int64_t)1 << 31) && (int64_t)B * M * Hf * Wf < ((int64_t)1 << 31), CF_ERR_ARG,
+               "%s: 4*%s*N and %s*Hf*Wf must stay below 2^31", fn, bm, bm);
     cudaStream_t st = (cudaStream_t)stream;
-    GdetWs w = gdet_carve(d_workspace, B, N, Hf, Wf);
-    GatherArgs a{};
-    a.points = d_points;
-    a.uv = d_uv;
-    if (h_calib)
-        for (int i = 0; i < 12; ++i) a.cal.m[i] = h_calib[i];
-    a.use_calib = h_calib != nullptr;
-    a.num_points = d_num_points;
-    a.N = N;
-    a.Hf = Hf;
-    a.Wf = Wf;
-    a.sx = (float)Wf / img_w;
-    a.sy = (float)Hf / img_h;
-    const int64_t npx = (int64_t)B * Hf * Wf;
-    CF_TRY(cuda_status(cudaMemsetAsync(w.cnt, 0, (size_t)npx * sizeof(int32_t), st), "cf_point_gather_bwd_det memset"));
+    GdetWs w = gdet_carve(d_workspace, B * M, N, Hf, Wf);
+    const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
+    const int64_t npx = (int64_t)B * M * Hf * Wf;
+    char what[64];
+    snprintf(what, sizeof what, "%s memset", fn);
+    CF_TRY(cuda_status(cudaMemsetAsync(w.cnt, 0, (size_t)npx * sizeof(int32_t), st), what));
     const dim3 tg((unsigned)std::min<int64_t>(ceil_div64(N, 256), 148 * 4), (unsigned)B);
-    k_gdet_taps<<<tg, 256, 0, st>>>(a, 0, w.cnt, nullptr, nullptr, nullptr);
+    k_gdet_taps<<<tg, 256, 0, st>>>(src, d_num_points, M, N, Hf, Wf, sx, sy, 0, w.cnt, nullptr, nullptr, nullptr);
     count_launches(1);
     CF_TRY(scan_counts(w.cnt, npx, w.off, w.tiles, st));
-    k_gdet_taps<<<tg, 256, 0, st>>>(a, 1, w.cnt, w.off, w.key, w.wgt);
+    k_gdet_taps<<<tg, 256, 0, st>>>(src, d_num_points, M, N, Hf, Wf, sx, sy, 1, w.cnt, w.off, w.key, w.wgt);
     k_gdet_sum<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div64(npx, 8), 148 * 16)), 256, 0, st>>>(
-        d_gfeat, Ci, N, Hf, Wf, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s, sb, sc, sh, sw, d_gimg);
+        d_gfeat, M, Ci, N, Hf, Wf, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s, sb, sm, sc, sh, sw, d_gimg);
     count_launches(2);
-    return launch_status("cf_point_gather_bwd_det");
+    return launch_status(fn);
 }
+}  // namespace
 
 extern "C" size_t cf_point_gather_multi_bwd_det_workspace_bytes(int32_t B, int32_t M, int32_t N, int32_t Hf, int32_t Wf)
 {
     if (B <= 0 || M <= 0 || N <= 0 || Hf <= 0 || Wf <= 0) return 0;
     return gdet_carve(nullptr, B * M, N, Hf, Wf).bytes;   // B*M maps, up to 4 taps per point in each
+}
+
+extern "C" size_t cf_point_gather_bwd_det_workspace_bytes(int32_t B, int32_t N, int32_t Hf, int32_t Wf)
+{
+    return cf_point_gather_multi_bwd_det_workspace_bytes(B, 1, N, Hf, Wf);
+}
+
+// cf_point_gather_bwd with a fixed summation order: the rig path over B*1 maps
+extern "C" int cf_point_gather_bwd_det(const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sc, int64_t sh, int64_t sw,
+                                       int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
+                                       const float *d_uv, const float *h_calib, const int64_t *d_num_points, int32_t N,
+                                       float img_w, float img_h, void *d_workspace, void *stream)
+{
+    CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG,
+               "cf_point_gather_bwd_det: pass exactly one of d_uv / h_calib");
+    return point_gather_bwd_det("cf_point_gather_bwd_det", d_gfeat, d_gimg, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
+                                cf::camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, d_workspace, stream);
 }
 
 // cf_point_gather_multi_bwd with a fixed summation order: the lists of cf_point_gather_bwd_det over the B*M maps
@@ -535,31 +432,8 @@ extern "C" int cf_point_gather_multi_bwd_det(const float *d_gfeat, float *d_gimg
                                              const float *d_points, const float *d_calib, const int64_t *d_num_points,
                                              int32_t N, float img_w, float img_h, void *d_workspace, void *stream)
 {
-    using namespace cf;
-    CF_TRY(require_sm100());
-    CF_REQUIRE(d_gfeat && d_gimg && d_points && d_calib && d_num_points && d_workspace, CF_ERR_ARG,
-               "cf_point_gather_multi_bwd_det: null pointer");
-    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "cf_point_gather_multi_bwd_det: M=%d cameras, expected 1..%d", M,
-               CF_MAX_CAMERAS);
-    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
-               "cf_point_gather_multi_bwd_det: bad extents");
-    CF_REQUIRE((int64_t)4 * B * M * N < ((int64_t)1 << 31) && (int64_t)B * M * Hf * Wf < ((int64_t)1 << 31), CF_ERR_ARG,
-               "cf_point_gather_multi_bwd_det: 4*B*M*N and B*M*Hf*Wf must stay below 2^31");
     CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN,
                "cf_point_gather_multi_bwd_det: d_calib must be 4-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    GdetWs w = gdet_carve(d_workspace, B * M, N, Hf, Wf);
-    const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
-    const int64_t npx = (int64_t)B * M * Hf * Wf;
-    CF_TRY(cuda_status(cudaMemsetAsync(w.cnt, 0, (size_t)npx * sizeof(int32_t), st), "cf_point_gather_multi_bwd_det memset"));
-    const dim3 tg((unsigned)std::min<int64_t>(ceil_div64(N, 256), 148 * 4), (unsigned)B);
-    k_gdet_multi_taps<<<tg, 256, 0, st>>>(d_points, d_calib, d_num_points, M, N, Hf, Wf, sx, sy, 0, w.cnt, nullptr, nullptr,
-                                          nullptr);
-    count_launches(1);
-    CF_TRY(scan_counts(w.cnt, npx, w.off, w.tiles, st));
-    k_gdet_multi_taps<<<tg, 256, 0, st>>>(d_points, d_calib, d_num_points, M, N, Hf, Wf, sx, sy, 1, w.cnt, w.off, w.key, w.wgt);
-    k_gdet_multi_sum<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div64(npx, 8), 148 * 16)), 256, 0, st>>>(
-        d_gfeat, M, Ci, N, Hf, Wf, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s, sb, sm, sc, sh, sw, d_gimg);
-    count_launches(2);
-    return launch_status("cf_point_gather_multi_bwd_det");
+    return point_gather_bwd_det("cf_point_gather_multi_bwd_det", d_gfeat, d_gimg, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf,
+                                cf::rig_source(d_points, d_calib), d_num_points, N, img_w, img_h, d_workspace, stream);
 }

@@ -10,7 +10,8 @@
 // A bf16 map (cf_point_gather_bf16) stays bf16 in its pixel-major copy; every tap is widened exactly to fp32 and blended
 // with the same fp32 sequence, so the features equal those of the widened fp32 map.
 // A camera rig (cf_point_gather_multi*) projects with device-side (B,M,4,3) calibrations (w > 0 in front) and averages the
-// blends of the cameras that see a point (semantics: include/cf_b200.h).
+// blends of the cameras that see a point (semantics: include/cf_b200.h).  The single-camera entry points run the same
+// kernel with M = 1; only where the map coordinates come from differs (CamSource).
 #include "cf_common.cuh"
 
 namespace cf {
@@ -42,10 +43,6 @@ __global__ void __launch_bounds__(256) k_to_pixel_major(const MT *__restrict__ s
     }
 }
 
-struct Calib {
-    float m[12];  // CRT (4,3) row-major
-};
-
 // four channels of a pixel-major row, widened to fp32 (a bf16 row: one 8-byte load)
 __device__ __forceinline__ float4 ld_px4(const float *row, int32_t c4) { return __ldg(reinterpret_cast<const float4 *>(row) + c4); }
 __device__ __forceinline__ float4 ld_px4(const __nv_bfloat16 *row, int32_t c4)
@@ -55,166 +52,37 @@ __device__ __forceinline__ float4 ld_px4(const __nv_bfloat16 *row, int32_t c4)
                        __uint_as_float(u.y & 0xFFFF0000u));
 }
 
-// one warp per point; lanes stride over float4 channel groups
+// One warp per point.  Lane m < M resolves camera m of the source (M = 1 for the single-camera entry points); a ballot
+// gives the visible set.  Each visible camera's clamped taps and masked weights are shuffled to the warp in ascending
+// camera order, the warp blends its Ci channels (float4 per lane) and sums the blends in registers; one division by n_vis
+// (none for one camera), one store.
 template <typename MT>
-__global__ void __launch_bounds__(256) k_point_gather(const MT *__restrict__ pix,  // (B, Hf*Wf, Ci) pixel-major
-                                                      int64_t pb, int64_t ph, int64_t pw,  // element strides (pc == 1)
-                                                      int32_t Ci, int32_t Hf, int32_t Wf,
-                                                      const float *__restrict__ points, const float *__restrict__ uv,
-                                                      Calib cal, int use_calib, const int64_t *__restrict__ num_points,
-                                                      int32_t N, float sx, float sy, float *__restrict__ feat)
-{
-    const int b = blockIdx.y;
-    const int32_t n = valid_points(num_points, b, N);
-    const int lane = threadIdx.x & 31;
-    const int32_t warps_per_grid = gridDim.x * (blockDim.x >> 5);
-    for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < N; p += warps_per_grid) {
-        if (p >= n) {  // zero padding rows: nothing downstream may ever see uninitialised memory
-            float4 *z = reinterpret_cast<float4 *>(feat + ((size_t)b * N + p) * Ci);
-            for (int32_t c4 = lane; c4 < (Ci >> 2); c4 += 32) z[c4] = make_float4(0.f, 0.f, 0.f, 0.f);
-            continue;
-        }
-        float u, v;
-        if (use_calib) {
-            const float *q = points + ((size_t)b * N + p) * 3;
-            const float x = __ldg(q), y = __ldg(q + 1), z = __ldg(q + 2);
-            float r[3];
-#pragma unroll
-            for (int c = 0; c < 3; ++c)
-                r[c] = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(x, cal.m[c]), __fmul_rn(y, cal.m[3 + c])),
-                                           __fmul_rn(z, cal.m[6 + c])),
-                                 cal.m[9 + c]);
-            u = __fdiv_rn(r[0], r[2]);
-            v = __fdiv_rn(r[1], r[2]);
-        } else {
-            const float2 t = __ldg(reinterpret_cast<const float2 *>(uv) + (size_t)b * N + p);
-            u = t.x;
-            v = t.y;
-        }
-        const float uf = __fsub_rn(__fmul_rn(__fadd_rn(u, 0.5f), sx), 0.5f);
-        const float vf = __fsub_rn(__fmul_rn(__fadd_rn(v, 0.5f), sy), 0.5f);
-        float4 *o = reinterpret_cast<float4 *>(feat + ((size_t)b * N + p) * Ci);
-        const int32_t c4n = Ci >> 2;
-        if (!(uf > -1.0f && uf < (float)Wf && vf > -1.0f && vf < (float)Hf)) {
-            for (int32_t c4 = lane; c4 < c4n; c4 += 32) o[c4] = make_float4(0.f, 0.f, 0.f, 0.f);
-            continue;
-        }
-        const float fx = floorf(uf), fy = floorf(vf);
-        const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
-        const float wx1 = __fsub_rn(uf, fx), wy1 = __fsub_rn(vf, fy);
-        const float wx0 = __fsub_rn(1.0f, wx1), wy0 = __fsub_rn(1.0f, wy1);
-        const bool okx0 = ix >= 0 && ix < Wf, okx1 = ix + 1 >= 0 && ix + 1 < Wf;
-        const bool oky0 = iy >= 0 && iy < Hf, oky1 = iy + 1 >= 0 && iy + 1 < Hf;
-        const float w00 = (okx0 && oky0) ? __fmul_rn(wx0, wy0) : 0.0f;
-        const float w01 = (okx1 && oky0) ? __fmul_rn(wx1, wy0) : 0.0f;
-        const float w10 = (okx0 && oky1) ? __fmul_rn(wx0, wy1) : 0.0f;
-        const float w11 = (okx1 && oky1) ? __fmul_rn(wx1, wy1) : 0.0f;
-        const int32_t x0c = okx0 ? ix : 0, x1c = okx1 ? ix + 1 : 0, y0c = oky0 ? iy : 0, y1c = oky1 ? iy + 1 : 0;
-        const MT *r00 = pix + b * pb + y0c * ph + x0c * pw;
-        const MT *r01 = pix + b * pb + y0c * ph + x1c * pw;
-        const MT *r10 = pix + b * pb + y1c * ph + x0c * pw;
-        const MT *r11 = pix + b * pb + y1c * ph + x1c * pw;
-        for (int32_t c4 = lane; c4 < c4n; c4 += 32) {
-            const float4 a = ld_px4(r00, c4), bq = ld_px4(r01, c4), c = ld_px4(r10, c4), d = ld_px4(r11, c4);
-            float4 r;
-            r.x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.x), __fmul_rn(w01, bq.x)), __fmul_rn(w10, c.x)), __fmul_rn(w11, d.x));
-            r.y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.y), __fmul_rn(w01, bq.y)), __fmul_rn(w10, c.y)), __fmul_rn(w11, d.y));
-            r.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.z), __fmul_rn(w01, bq.z)), __fmul_rn(w10, c.z)), __fmul_rn(w11, d.z));
-            r.w = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.w), __fmul_rn(w01, bq.w)), __fmul_rn(w10, c.w)), __fmul_rn(w11, d.w));
-            o[c4] = r;
-        }
-    }
-}
-
-template <typename MT>
-int point_gather(const MT *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B, int32_t Ci, int32_t Hf,
-                 int32_t Wf, const float *d_points, const float *d_uv, const float *h_calib, const int64_t *d_num_points,
-                 int32_t N, float img_w, float img_h, float *d_feat, void *d_workspace, void *stream)
-{
-    CF_TRY(require_sm100());
-    CF_REQUIRE(d_img_feat && d_points && d_num_points && d_feat, CF_ERR_ARG, "cf_point_gather: null pointer");
-    CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG,
-               "cf_point_gather: pass exactly one of d_uv / h_calib");
-    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0, CF_ERR_ARG, "cf_point_gather: bad extents");
-    CF_REQUIRE(Ci % 4 == 0, CF_ERR_ARG, "cf_point_gather: Ci=%d must be a multiple of 4", Ci);
-    CF_REQUIRE(img_w > 0.0f && img_h > 0.0f, CF_ERR_ARG, "cf_point_gather: bad image size");
-    CF_REQUIRE(aligned16(d_feat), CF_ERR_ALIGN, "cf_point_gather: d_feat must be 16-byte aligned");
-    CF_REQUIRE(d_uv == nullptr || (reinterpret_cast<uintptr_t>(d_uv) & 7u) == 0, CF_ERR_ALIGN,
-               "cf_point_gather: d_uv must be 8-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    const MT *pix = d_img_feat;
-    int64_t pb = sb, ph = sh, pw = sw;
-    if (sc != 1) {
-        CF_REQUIRE(d_workspace != nullptr, CF_ERR_ARG, "cf_point_gather: workspace required for channel-major maps");
-        CF_REQUIRE(aligned16(d_workspace), CF_ERR_ALIGN, "cf_point_gather: workspace must be 16-byte aligned");
-        const int32_t HW = Hf * Wf;
-        dim3 grid((unsigned)((HW + 31) / 32), (unsigned)((Ci + 31) / 32), (unsigned)B);
-        k_to_pixel_major<<<grid, 256, 0, st>>>(d_img_feat, sb, sc, sh, sw, Ci, Hf, Wf, (MT *)d_workspace);
-        count_launches(1);
-        pix = (const MT *)d_workspace;
-        pb = (int64_t)HW * Ci;
-        ph = (int64_t)Wf * Ci;
-        pw = Ci;
-    } else {
-        // four channels per load: 16 bytes of fp32, 8 bytes of bf16
-        CF_REQUIRE((reinterpret_cast<uintptr_t>(d_img_feat) & (4 * sizeof(MT) - 1)) == 0 && sb % 4 == 0 && sh % 4 == 0 &&
-                       sw % 4 == 0,
-                   CF_ERR_ALIGN, "cf_point_gather: channels_last map must be %d-byte aligned per pixel", (int)(4 * sizeof(MT)));
-    }
-    Calib cal{};
-    if (h_calib)
-        for (int i = 0; i < 12; ++i) cal.m[i] = h_calib[i];
-    const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
-    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
-    k_point_gather<<<dim3(blocks, B), 256, 0, st>>>(pix, pb, ph, pw, Ci, Hf, Wf, d_points, d_uv, cal,
-                                                    h_calib != nullptr, d_num_points, N, sx, sy, d_feat);
-    count_launches(1);
-    return launch_status("cf_point_gather");
-}
-
-// Camera rig: one warp per point.  Lane m < M projects the point into camera m (its CRT is read from the device, the same
-// 12 floats for every point of the frame); a ballot gives the visible set.  Each visible camera's taps and weights are
-// shuffled to the warp in ascending camera order, the warp blends its Ci channels (float4 per lane, the sequence of
-// k_point_gather) and sums the blends in registers; one division by n_vis, one store.
-template <typename MT>
-__global__ void __launch_bounds__(256) k_point_gather_multi(const MT *__restrict__ pix,  // (B, M, Hf*Wf, Ci) pixel-major
-                                                            int64_t pb, int64_t pm, int64_t ph, int64_t pw,  // pc == 1
-                                                            int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
-                                                            const float *__restrict__ points, const float *__restrict__ calib,
-                                                            const int64_t *__restrict__ num_points, int32_t N, float sx,
-                                                            float sy, float *__restrict__ feat)
+__global__ void __launch_bounds__(256) k_point_gather(const MT *__restrict__ pix,  // (B, M, Hf*Wf, Ci) pixel-major
+                                                      int64_t pb, int64_t pm, int64_t ph, int64_t pw,  // pc == 1
+                                                      int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const CamSource src,
+                                                      const int64_t *__restrict__ num_points, int32_t N, float sx, float sy,
+                                                      float *__restrict__ feat)
 {
     const int b = blockIdx.y;
     const int32_t n = valid_points(num_points, b, N);
     const int lane = threadIdx.x & 31;
     const int32_t warps_per_grid = gridDim.x * (blockDim.x >> 5);
     const int32_t c4n = Ci >> 2;
-    const float *crt = calib + ((size_t)b * M + (lane < M ? lane : 0)) * 12;
     for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < N; p += warps_per_grid) {
         float4 *o = reinterpret_cast<float4 *>(feat + ((size_t)b * N + p) * Ci);
         unsigned vis = 0;
         float uf = 0.0f, vf = 0.0f;
-        if (p < n) {
-            const float *q = points + ((size_t)b * N + p) * 3;
-            const bool mine = lane < M && rig_project(crt, __ldg(q), __ldg(q + 1), __ldg(q + 2), sx, sy, Hf, Wf, uf, vf);
-            vis = __ballot_sync(0xffffffffu, mine);
-        }
+        if (p < n) vis = __ballot_sync(0xffffffffu, lane < M && cam_project(src, b, N, p, lane, M, sx, sy, Hf, Wf, uf, vf));
         if (vis == 0) {  // padding row, or no camera sees the point
             for (int32_t c4 = lane; c4 < c4n; c4 += 32) o[c4] = make_float4(0.f, 0.f, 0.f, 0.f);
             continue;
         }
-        // this lane's camera: taps and weights exactly as k_point_gather (meaningful on the visible lanes only)
-        const float fx = floorf(uf), fy = floorf(vf);
-        const int32_t ix = (int32_t)fx, iy = (int32_t)fy;
-        const float wx1 = __fsub_rn(uf, fx), wy1 = __fsub_rn(vf, fy);
-        const float wx0 = __fsub_rn(1.0f, wx1), wy0 = __fsub_rn(1.0f, wy1);
-        const bool okx0 = ix >= 0 && ix < Wf, okx1 = ix + 1 >= 0 && ix + 1 < Wf;
-        const bool oky0 = iy >= 0 && iy < Hf, oky1 = iy + 1 >= 0 && iy + 1 < Hf;
-        const float l00 = (okx0 && oky0) ? __fmul_rn(wx0, wy0) : 0.0f;
-        const float l01 = (okx1 && oky0) ? __fmul_rn(wx1, wy0) : 0.0f;
-        const float l10 = (okx0 && oky1) ? __fmul_rn(wx0, wy1) : 0.0f;
-        const float l11 = (okx1 && oky1) ? __fmul_rn(wx1, wy1) : 0.0f;
-        const int32_t lx0 = okx0 ? ix : 0, lx1 = okx1 ? ix + 1 : 0, ly0 = oky0 ? iy : 0, ly1 = oky1 ? iy + 1 : 0;
+        // this lane's camera (meaningful on the visible lanes only): taps outside the map weigh 0 and read corner 0
+        const Taps tp = bilinear_taps(uf, vf, Hf, Wf);
+        const float l00 = tp.in(0) ? tp.w[0] : 0.0f, l01 = tp.in(1) ? tp.w[1] : 0.0f;
+        const float l10 = tp.in(2) ? tp.w[2] : 0.0f, l11 = tp.in(3) ? tp.w[3] : 0.0f;
+        const int32_t lx0 = tp.okx[0] ? tp.x : 0, lx1 = tp.okx[1] ? tp.x + 1 : 0;
+        const int32_t ly0 = tp.oky[0] ? tp.y : 0, ly1 = tp.oky[1] ? tp.y + 1 : 0;
         const int nv = __popc(vis);
         for (int32_t cb = 0; cb < c4n; cb += 32) {  // warp-uniform trip count: every lane takes part in the shuffles
             const int32_t c4 = cb + lane;
@@ -236,7 +104,7 @@ __global__ void __launch_bounds__(256) k_point_gather_multi(const MT *__restrict
                     r.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.z), __fmul_rn(w01, bq.z)), __fmul_rn(w10, c.z)), __fmul_rn(w11, d.z));
                     r.w = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(w00, a.w), __fmul_rn(w01, bq.w)), __fmul_rn(w10, c.w)), __fmul_rn(w11, d.w));
                     if (first) {
-                        acc = r;  // not 0 + r: a -0.0 blend keeps its sign, so one camera gives the bits of k_point_gather
+                        acc = r;  // not 0 + r: a -0.0 blend keeps its sign
                     } else {
                         acc.x = __fadd_rn(acc.x, r.x);
                         acc.y = __fadd_rn(acc.y, r.y);
@@ -257,28 +125,27 @@ __global__ void __launch_bounds__(256) k_point_gather_multi(const MT *__restrict
     }
 }
 
+// K-3 for M cameras of one source; `fn` names the entry point in the error texts
 template <typename MT>
-int point_gather_multi(const MT *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw, int32_t B, int32_t M,
-                       int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_calib,
-                       const int64_t *d_num_points, int32_t N, float img_w, float img_h, float *d_feat, void *d_workspace,
-                       void *stream)
+int point_gather(const char *fn, const MT *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw, int32_t B,
+                 int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const CamSource &src, const int64_t *d_num_points, int32_t N,
+                 float img_w, float img_h, float *d_feat, void *d_workspace, void *stream)
 {
+    const bool rig = src.kind == CamSource::kRig;
     CF_TRY(require_sm100());
-    CF_REQUIRE(d_img_feat && d_points && d_calib && d_num_points && d_feat, CF_ERR_ARG, "cf_point_gather_multi: null pointer");
-    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "cf_point_gather_multi: M=%d cameras, expected 1..%d", M,
-               CF_MAX_CAMERAS);
-    CF_REQUIRE(B > 0 && (int64_t)B * M <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0, CF_ERR_ARG,
-               "cf_point_gather_multi: bad extents");
-    CF_REQUIRE(Ci % 4 == 0, CF_ERR_ARG, "cf_point_gather_multi: Ci=%d must be a multiple of 4", Ci);
-    CF_REQUIRE(img_w > 0.0f && img_h > 0.0f, CF_ERR_ARG, "cf_point_gather_multi: bad image size");
-    CF_REQUIRE(aligned16(d_feat), CF_ERR_ALIGN, "cf_point_gather_multi: d_feat must be 16-byte aligned");
-    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_multi: d_calib must be 4-byte aligned");
+    CF_REQUIRE(d_img_feat && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points && d_feat, CF_ERR_ARG,
+               "%s: null pointer", fn);
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
+    CF_REQUIRE(B > 0 && (int64_t)B * M <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0, CF_ERR_ARG, "%s: bad extents", fn);
+    CF_REQUIRE(Ci % 4 == 0, CF_ERR_ARG, "%s: Ci=%d must be a multiple of 4", fn, Ci);
+    CF_REQUIRE(img_w > 0.0f && img_h > 0.0f, CF_ERR_ARG, "%s: bad image size", fn);
+    CF_REQUIRE(aligned16(d_feat), CF_ERR_ALIGN, "%s: d_feat must be 16-byte aligned", fn);
     cudaStream_t st = (cudaStream_t)stream;
     const MT *pix = d_img_feat;
     int64_t pb = sb, pm = sm, ph = sh, pw = sw;
     if (sc != 1) {
-        CF_REQUIRE(d_workspace != nullptr, CF_ERR_ARG, "cf_point_gather_multi: workspace required for channel-major maps");
-        CF_REQUIRE(aligned16(d_workspace), CF_ERR_ALIGN, "cf_point_gather_multi: workspace must be 16-byte aligned");
+        CF_REQUIRE(d_workspace != nullptr, CF_ERR_ARG, "%s: workspace required for channel-major maps", fn);
+        CF_REQUIRE(aligned16(d_workspace), CF_ERR_ALIGN, "%s: workspace must be 16-byte aligned", fn);
         const int32_t HW = Hf * Wf;
         MT *dst = (MT *)d_workspace;
         const unsigned gx = (unsigned)((HW + 31) / 32), gy = (unsigned)((Ci + 31) / 32);
@@ -297,44 +164,44 @@ int point_gather_multi(const MT *d_img_feat, int64_t sb, int64_t sm, int64_t sc,
         ph = (int64_t)Wf * Ci;
         pw = Ci;
     } else {
+        // four channels per load: 16 bytes of fp32, 8 bytes of bf16
         CF_REQUIRE((reinterpret_cast<uintptr_t>(d_img_feat) & (4 * sizeof(MT) - 1)) == 0 && sb % 4 == 0 && sm % 4 == 0 &&
                        sh % 4 == 0 && sw % 4 == 0,
-                   CF_ERR_ALIGN, "cf_point_gather_multi: channels_last maps must be %d-byte aligned per pixel",
+                   CF_ERR_ALIGN, "%s: channels_last map%s must be %d-byte aligned per pixel", fn, rig ? "s" : "",
                    (int)(4 * sizeof(MT)));
     }
     const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
     const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
-    k_point_gather_multi<<<dim3(blocks, B), 256, 0, st>>>(pix, pb, pm, ph, pw, M, Ci, Hf, Wf, d_points, d_calib, d_num_points,
-                                                          N, sx, sy, d_feat);
+    k_point_gather<<<dim3(blocks, B), 256, 0, st>>>(pix, pb, pm, ph, pw, M, Ci, Hf, Wf, src, d_num_points, N, sx, sy, d_feat);
     count_launches(1);
-    return launch_status("cf_point_gather_multi");
+    return launch_status(fn);
+}
+
+// one camera (logical (B,Ci,Hf,Wf) map): the rig path with M = 1 and the frame stride as camera stride
+template <typename MT>
+int point_gather_one(const MT *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B, int32_t Ci, int32_t Hf,
+                     int32_t Wf, const float *d_points, const float *d_uv, const float *h_calib, const int64_t *d_num_points,
+                     int32_t N, float img_w, float img_h, float *d_feat, void *d_workspace, void *stream)
+{
+    CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG, "cf_point_gather: pass exactly one of d_uv / h_calib");
+    CF_REQUIRE(d_uv == nullptr || (reinterpret_cast<uintptr_t>(d_uv) & 7u) == 0, CF_ERR_ALIGN,
+               "cf_point_gather: d_uv must be 8-byte aligned");
+    return point_gather("cf_point_gather", d_img_feat, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
+                        camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
+}
+
+template <typename MT>
+int point_gather_rig(const MT *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw, int32_t B, int32_t M,
+                     int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_calib,
+                     const int64_t *d_num_points, int32_t N, float img_w, float img_h, float *d_feat, void *d_workspace,
+                     void *stream)
+{
+    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_multi: d_calib must be 4-byte aligned");
+    return point_gather("cf_point_gather_multi", d_img_feat, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, rig_source(d_points, d_calib),
+                        d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
 }
 
 }  // namespace cf
-
-extern "C" size_t cf_gather_workspace_bytes(int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc)
-{
-    if (sc == 1) return 0;
-    return (size_t)B * (size_t)Ci * (size_t)Hf * (size_t)Wf * sizeof(float);
-}
-
-extern "C" int cf_point_gather(const float *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B,
-                               int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_uv,
-                               const float *h_calib, const int64_t *d_num_points, int32_t N, float img_w,
-                               float img_h, float *d_feat, void *d_workspace, void *stream)
-{
-    return cf::point_gather(d_img_feat, sb, sc, sh, sw, B, Ci, Hf, Wf, d_points, d_uv, h_calib, d_num_points, N, img_w, img_h,
-                            d_feat, d_workspace, stream);
-}
-
-extern "C" int cf_point_gather_bf16(const void *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B,
-                                    int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_uv,
-                                    const float *h_calib, const int64_t *d_num_points, int32_t N, float img_w,
-                                    float img_h, float *d_feat, void *d_workspace, void *stream)
-{
-    return cf::point_gather(static_cast<const __nv_bfloat16 *>(d_img_feat), sb, sc, sh, sw, B, Ci, Hf, Wf, d_points, d_uv,
-                            h_calib, d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
-}
 
 extern "C" size_t cf_gather_multi_workspace_bytes(int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc)
 {
@@ -342,13 +209,36 @@ extern "C" size_t cf_gather_multi_workspace_bytes(int32_t B, int32_t M, int32_t 
     return (size_t)B * (size_t)M * (size_t)Ci * (size_t)Hf * (size_t)Wf * sizeof(float);
 }
 
+extern "C" size_t cf_gather_workspace_bytes(int32_t B, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc)
+{
+    return cf_gather_multi_workspace_bytes(B, 1, Ci, Hf, Wf, sc);
+}
+
+extern "C" int cf_point_gather(const float *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B,
+                               int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_uv,
+                               const float *h_calib, const int64_t *d_num_points, int32_t N, float img_w,
+                               float img_h, float *d_feat, void *d_workspace, void *stream)
+{
+    return cf::point_gather_one(d_img_feat, sb, sc, sh, sw, B, Ci, Hf, Wf, d_points, d_uv, h_calib, d_num_points, N, img_w,
+                                img_h, d_feat, d_workspace, stream);
+}
+
+extern "C" int cf_point_gather_bf16(const void *d_img_feat, int64_t sb, int64_t sc, int64_t sh, int64_t sw, int32_t B,
+                                    int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points, const float *d_uv,
+                                    const float *h_calib, const int64_t *d_num_points, int32_t N, float img_w,
+                                    float img_h, float *d_feat, void *d_workspace, void *stream)
+{
+    return cf::point_gather_one(static_cast<const __nv_bfloat16 *>(d_img_feat), sb, sc, sh, sw, B, Ci, Hf, Wf, d_points, d_uv,
+                                h_calib, d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
+}
+
 extern "C" int cf_point_gather_multi(const float *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
                                      int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
                                      const float *d_calib, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
                                      float *d_feat, void *d_workspace, void *stream)
 {
-    return cf::point_gather_multi(d_img_feat, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, d_points, d_calib, d_num_points, N, img_w,
-                                  img_h, d_feat, d_workspace, stream);
+    return cf::point_gather_rig(d_img_feat, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, d_points, d_calib, d_num_points, N, img_w,
+                                img_h, d_feat, d_workspace, stream);
 }
 
 extern "C" int cf_point_gather_multi_bf16(const void *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
@@ -356,6 +246,6 @@ extern "C" int cf_point_gather_multi_bf16(const void *d_img_feat, int64_t sb, in
                                           const float *d_calib, const int64_t *d_num_points, int32_t N, float img_w,
                                           float img_h, float *d_feat, void *d_workspace, void *stream)
 {
-    return cf::point_gather_multi(static_cast<const __nv_bfloat16 *>(d_img_feat), sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, d_points,
-                                  d_calib, d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
+    return cf::point_gather_rig(static_cast<const __nv_bfloat16 *>(d_img_feat), sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, d_points,
+                                d_calib, d_num_points, N, img_w, img_h, d_feat, d_workspace, stream);
 }
