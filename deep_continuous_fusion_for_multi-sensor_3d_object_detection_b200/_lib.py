@@ -13,6 +13,7 @@ CSRC = os.path.join(_PKG, "csrc")
 MODE_FP32, MODE_BF16, MODE_SIMT, MODE_BF16_TABLES = 0, 1, 2, 3
 BWD_DETERMINISTIC = 0x100   # CF_BWD_DETERMINISTIC: OR-ed into the mode of cf_fusion_bwd
 IO_BF16 = 0x200             # CF_IO_BF16: OR-ed into the mode of cf_fusion_fwd / cf_fusion_bwd for bf16 BEV maps
+IO_NHWC = 0x400             # CF_IO_NHWC: OR-ed into the mode of cf_fusion_fwd / cf_fusion_bwd for (B,H,W,C) (channels_last) BEV maps
 # "bf16t" = CF_MODE_BF16_TABLES: bf16 operands AND bf16 layer-1 tables (inference only)
 MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "simt": MODE_SIMT, "bf16t": MODE_BF16_TABLES}
 MAX_K = 16

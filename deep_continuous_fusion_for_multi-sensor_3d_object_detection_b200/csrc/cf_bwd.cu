@@ -276,16 +276,26 @@ __global__ void __launch_bounds__(256) k_bwd_compact(const int32_t *__restrict__
 // G[ci, c] = gout[b, c, cell] for the live cells (32 cells x 32 channels per block through a shared-memory transpose;
 // list neighbours are mostly grid neighbours, so the reads of a warp still fall into few lines).  The only reader of gout:
 // a bf16 gout (CF_IO_BF16) is widened exactly here, and everything downstream is the fp32 path.
-template <typename MT>
+// NHWC (CF_IO_NHWC): gout already holds a cell's channels as one row, so each warp copies 32 channels of a live row
+// straight into G.
+template <typename MT, bool NHWC = false>
 __global__ void __launch_bounds__(256) k_bwd_gather_g(const MT *__restrict__ gout, int32_t C, int64_t cells,
                                                       const int32_t *__restrict__ cell_list,
                                                       const int32_t *__restrict__ counters, float *__restrict__ G)
 {
-    __shared__ float tile[32][33];
     const int32_t n = __ldg(counters);
     const int32_t t0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
     if (t0 >= n) return;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    if constexpr (NHWC) {
+        const int32_t c = c0 + tx;
+        for (int r = ty; r < 32 && t0 + r < n; r += 8) {
+            const int64_t g = __ldg(cell_list + t0 + r);   // b * cells + cell: the row of the cell in a (B,H,W,C) map
+            if (c < C) G[(size_t)(t0 + r) * C + c] = map_ldg(gout + g * C + c);
+        }
+        return;
+    }
+    __shared__ float tile[32][33];
     const int32_t ci = t0 + tx;
     int64_t src = -1;
     if (ci < n) {
@@ -547,6 +557,7 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
     CF_TRY(require_sm100());
     const bool det = (mode & CF_BWD_DETERMINISTIC) != 0;
     const bool io16 = (mode & CF_IO_BF16) != 0;   // d_gout is a bf16 map
+    const bool nhwc = (mode & CF_IO_NHWC) != 0;   // d_gout is a (B,H,W,C) map
     mode = mode_base(mode);
     CF_REQUIRE(d_gout && d_feat && d_points && d_num_points && d_knn_idx && d_W1 && d_b1 && d_W2 && d_b2 && d_W3 &&
                    d_gW1 && d_gb1 && d_gW2 && d_gb2 && d_gW3 && d_gb3 && d_gfeat && d_workspace,
@@ -658,8 +669,13 @@ extern "C" int cf_fusion_bwd(const float *d_gout, const float *d_feat, const flo
 
     // ---- layer 3 ------------------------------------------------------------------------------------------------------
     const dim3 g_grid((unsigned)ceil_div64(ncell, 32), cchunks);
-    if (io16)
-        k_bwd_gather_g<<<g_grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16 *>(d_gout), C, cells, w.cell_list, w.counters, w.G);
+    const __nv_bfloat16 *gout16 = reinterpret_cast<const __nv_bfloat16 *>(d_gout);
+    if (io16 && nhwc)
+        k_bwd_gather_g<__nv_bfloat16, true><<<g_grid, 256, 0, st>>>(gout16, C, cells, w.cell_list, w.counters, w.G);
+    else if (io16)
+        k_bwd_gather_g<<<g_grid, 256, 0, st>>>(gout16, C, cells, w.cell_list, w.counters, w.G);
+    else if (nhwc)
+        k_bwd_gather_g<float, true><<<g_grid, 256, 0, st>>>(d_gout, C, cells, w.cell_list, w.counters, w.G);
     else
         k_bwd_gather_g<<<g_grid, 256, 0, st>>>(d_gout, C, cells, w.cell_list, w.counters, w.G);
     launches += 2;

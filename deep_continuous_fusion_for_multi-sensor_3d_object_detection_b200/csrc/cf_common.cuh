@@ -43,7 +43,7 @@ static inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t
 constexpr int kDetSplits = 128;
 
 // `mode` without its flag bits: the MLP arithmetic (CF_MODE_*) that picks kernels, operand layouts and workspace sizes
-constexpr int32_t kModeFlags = CF_BWD_DETERMINISTIC | CF_IO_BF16;
+constexpr int32_t kModeFlags = CF_BWD_DETERMINISTIC | CF_IO_BF16 | CF_IO_NHWC;
 static inline int32_t mode_base(int32_t mode) { return mode & ~kModeFlags; }
 
 __host__ __device__ static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

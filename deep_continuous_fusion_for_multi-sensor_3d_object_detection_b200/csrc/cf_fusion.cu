@@ -7,7 +7,7 @@ size_t fusion_simt_workspace_bytes(int32_t C);
 int fusion_simt(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_t B, int32_t N, int32_t C,
                 int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy, const float *d_W1,
                 int32_t Ci, const float *d_W2, const float *d_b2, const float *d_W3, const float *d_b3,
-                float *d_out, bool io16, void *d_workspace, cudaStream_t st);
+                float *d_out, bool io16, bool nhwc, void *d_workspace, cudaStream_t st);
 size_t fusion_tc_workspace_bytes(int32_t C, int32_t mode, int32_t B, int32_t H, int32_t W);
 int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_t B, int32_t N, int32_t C,
               int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy, const float *d_W1,
@@ -61,17 +61,18 @@ extern "C" int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t
     CF_REQUIRE((reinterpret_cast<uintptr_t>(d_T) & 31u) == 0 && aligned16(d_workspace), CF_ERR_ALIGN,
                "cf_fusion_fwd: T must be 32-byte aligned, the workspace 16-byte aligned");
     const bool io16 = (mode & CF_IO_BF16) != 0;   // bev / out are bf16 maps
+    const bool nhwc = (mode & CF_IO_NHWC) != 0;   // bev / out are (B,H,W,C) maps
     cudaStream_t st = (cudaStream_t)stream;
-    switch (mode & ~CF_IO_BF16) {
+    switch (mode_base(mode)) {
         case CF_MODE_FP32_SIMT:
             return fusion_simt(d_bev, d_T, d_knn_idx, B, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, d_W2, d_b2, d_W3,
-                               d_b3, d_out, io16, d_workspace, st);
+                               d_b3, d_out, io16, nhwc, d_workspace, st);
         case CF_MODE_FP32:
         case CF_MODE_BF16:
         case CF_MODE_BF16_TABLES:   // d_T holds bf16 rows
             CF_REQUIRE(d_packed == nullptr || aligned16(d_packed), CF_ERR_ALIGN, "cf_fusion_fwd: packed weights must be 16-byte aligned");
             return fusion_tc(d_bev, d_T, d_knn_idx, B, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, d_W2, d_b2, d_W3,
-                             d_b3, d_out, mode, d_packed, d_workspace, st);   // fusion_tc reads CF_IO_BF16 itself
+                             d_b3, d_out, mode, d_packed, d_workspace, st);   // fusion_tc reads CF_IO_BF16 / CF_IO_NHWC itself
         default:
             set_error("cf_fusion_fwd: unknown mode %d", mode);
             return CF_ERR_ARG;

@@ -103,7 +103,8 @@ __global__ void __launch_bounds__(256) k_transpose_sq(const float *__restrict__ 
     Wt[(size_t)i * C + o] = W[idx];
 }
 
-template <typename MT>   // map element: float, or __nv_bfloat16 (CF_IO_BF16: widened on load, rounded once on store)
+// MT: map element, float or __nv_bfloat16 (CF_IO_BF16: widened on load, rounded once on store); NHWC: (B,H,W,C) maps
+template <typename MT, bool NHWC = false>
 __global__ void __launch_bounds__(256) k_fusion_simt(const MT *__restrict__ bev, const float *__restrict__ T,
                                                      const int32_t *__restrict__ knn, int32_t N, int32_t C, int32_t H,
                                                      int32_t W, int32_t K, float x0, float y0, float dx, float dy,
@@ -179,14 +180,15 @@ __global__ void __launch_bounds__(256) k_fusion_simt(const MT *__restrict__ bev,
             __syncthreads();
         }
         for (int idx = tid; idx < 32 * C; idx += 256) {
-            const int c = idx >> 5, r = idx & 31;
+            // consecutive threads on consecutive map elements: cells in NCHW, channels in NHWC
+            const int c = NHWC ? idx % C : idx >> 5, r = NHWC ? idx / C : idx & 31;
             const int64_t cell = cell0 + r;
             if (cell >= cells) continue;
             float s = (float)nval[r] * __ldg(b3 + c);
             const float *pr = pooled + r * ldp;
 #pragma unroll 8
             for (int kk = 0; kk < C; ++kk) s = fmaf(pr[kk], __ldg(Wt3 + (size_t)kk * C + c), s);
-            const size_t o = ((size_t)b * C + c) * cells + cell;
+            const size_t o = NHWC ? ((size_t)b * cells + cell) * C + c : ((size_t)b * C + c) * cells + cell;
             map_st(out + o, map_ldg(bev + o) + s);
         }
     }
@@ -206,7 +208,7 @@ size_t fusion_simt_workspace_bytes(int32_t C) { return (size_t)2 * C * C * sizeo
 int fusion_simt(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_t B, int32_t N, int32_t C,
                 int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy, const float *d_W1,
                 int32_t Ci, const float *d_W2, const float *d_b2, const float *d_W3, const float *d_b3,
-                float *d_out, bool io16, void *d_workspace, cudaStream_t st)
+                float *d_out, bool io16, bool nhwc, void *d_workspace, cudaStream_t st)
 {
     float *Wt2 = (float *)d_workspace, *Wt3 = Wt2 + (size_t)C * C;
     const int tb = (C * C + 255) / 256;
@@ -220,16 +222,27 @@ int fusion_simt(const float *d_bev, const float *d_T, const int32_t *d_knn, int3
                            "k_fusion_simt smem attribute"));
         CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_simt<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024),
                            "k_fusion_simt smem attribute"));
+        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_simt<float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024),
+                           "k_fusion_simt smem attribute"));
+        CF_TRY(cuda_status(cudaFuncSetAttribute(k_fusion_simt<__nv_bfloat16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024),
+                           "k_fusion_simt smem attribute"));
         attr_set = true;
     }
     const int64_t tiles = ceil_div64((int64_t)H * W, 32);
     const int gx = (int)std::min<int64_t>(tiles, (int64_t)sm_count() * 8);
-    if (io16)
-        k_fusion_simt<<<dim3(gx, B), 256, smem, st>>>(reinterpret_cast<const __nv_bfloat16 *>(d_bev), d_T, d_knn, N, C, H, W, K, x0,
-                                                      y0, dx, dy, d_W1, Ci, Wt2, d_b2, Wt3, d_b3, reinterpret_cast<__nv_bfloat16 *>(d_out));
+    const __nv_bfloat16 *bev16 = reinterpret_cast<const __nv_bfloat16 *>(d_bev);
+    __nv_bfloat16 *out16 = reinterpret_cast<__nv_bfloat16 *>(d_out);
+    const dim3 grid(gx, B);
+    if (io16 && nhwc)
+        k_fusion_simt<__nv_bfloat16, true><<<grid, 256, smem, st>>>(bev16, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2,
+                                                                    d_b2, Wt3, d_b3, out16);
+    else if (io16)
+        k_fusion_simt<<<grid, 256, smem, st>>>(bev16, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2, d_b2, Wt3, d_b3, out16);
+    else if (nhwc)
+        k_fusion_simt<float, true><<<grid, 256, smem, st>>>(d_bev, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2, d_b2,
+                                                            Wt3, d_b3, d_out);
     else
-        k_fusion_simt<<<dim3(gx, B), 256, smem, st>>>(d_bev, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2,
-                                                      d_b2, Wt3, d_b3, d_out);
+        k_fusion_simt<<<grid, 256, smem, st>>>(d_bev, d_T, d_knn, N, C, H, W, K, x0, y0, dx, dy, d_W1, Ci, Wt2, d_b2, Wt3, d_b3, d_out);
     count_launches(3);
     return launch_status("cf_fusion_fwd (simt)");
 }

@@ -95,6 +95,56 @@ __host__ __device__ constexpr int tmem_cols_for(int cols)
 
 constexpr int kEW = 16;  // TMEM columns per epilogue step
 constexpr int kCopyBatch = 16;  // channels per copy unit and thread loaded before the first store
+constexpr int kRowBatch = 4;    // NHWC copy units: 16-byte vectors per lane loaded before the first store
+
+// NHWC maps (CF_IO_NHWC): the kEW channels of an epilogue chunk are 16 consecutive elements of the cell's row, moved as
+// 16-byte vectors.  Widening and rounding are those of map_ldcs / map_stcs, so the values equal the NCHW path's bit for bit.
+__device__ __forceinline__ void row_ldcs16(const float *p, float *v)
+{
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const float4 t = __ldcs(reinterpret_cast<const float4 *>(p) + q);
+        v[4 * q] = t.x;
+        v[4 * q + 1] = t.y;
+        v[4 * q + 2] = t.z;
+        v[4 * q + 3] = t.w;
+    }
+}
+__device__ __forceinline__ void row_ldcs16(const __nv_bfloat16 *p, float *v)
+{
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+        const uint4 t = __ldcs(reinterpret_cast<const uint4 *>(p) + q);
+        const uint32_t w[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            v[8 * q + 2 * i] = __uint_as_float(w[i] << 16);
+            v[8 * q + 2 * i + 1] = __uint_as_float(w[i] & 0xFFFF0000u);
+        }
+    }
+}
+__device__ __forceinline__ void row_stcs16(float *p, const float *v)
+{
+#pragma unroll
+    for (int q = 0; q < 4; ++q) __stcs(reinterpret_cast<float4 *>(p) + q, make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]));
+}
+__device__ __forceinline__ void row_stcs16(__nv_bfloat16 *p, const float *v)
+{
+    auto bits = [](float x) { return (uint32_t)__bfloat16_as_ushort(__float2bfloat16_rn(x)); };
+#pragma unroll
+    for (int q = 0; q < 2; ++q) {
+        uint32_t w[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) w[i] = bits(v[8 * q + 2 * i]) | (bits(v[8 * q + 2 * i + 1]) << 16);
+        __stcs(reinterpret_cast<uint4 *>(p) + q, make_uint4(w[0], w[1], w[2], w[3]));
+    }
+}
+// first element of cell `cell` of frame b (channel 0) in an NCHW or NHWC map
+template <bool NHWC>
+__device__ __forceinline__ size_t map_cell(int b, int32_t cell, int C, int64_t cells)
+{
+    return NHWC ? ((size_t)b * cells + cell) * C : (size_t)b * C * cells + cell;
+}
 
 // the "row" a cell without a k-th neighbour gathers: relu(-1e30 - e) = 0, so the operand build needs no select
 #define CF_NEG8 -1e30f, -1e30f, -1e30f, -1e30f, -1e30f, -1e30f, -1e30f, -1e30f
@@ -286,17 +336,39 @@ __device__ __forceinline__ void setup_offsets_and_bias(const TcParams &p, int ti
 }
 
 // the bev values of this thread's first kPre output chunks -> tv (they ride in the registers of the gathered rows)
-template <int C, int G, int kPre, typename MT>
+template <int C, int G, int kPre, bool NHWC, typename MT>
 __device__ __forceinline__ void prefetch_bev(float *tv, const MT *src_bev, int64_t cells, int grp)
 {
 #pragma unroll
     for (int j = 0; j < kPre; ++j) {
         if (grp + j * G < C / kEW) {
+            if constexpr (NHWC) {
+                row_ldcs16(src_bev + (grp + j * G) * kEW, tv + j * kEW);
+            } else {
 #pragma unroll
-            for (int i = 0; i < kEW; ++i) tv[j * kEW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * kEW + i) * cells);
+                for (int i = 0; i < kEW; ++i) tv[j * kEW + i] = map_ldcs(src_bev + (size_t)((grp + j * G) * kEW + i) * cells);
+            }
         }
     }
 }
+
+// the final epilogue of one output chunk cc of an NHWC map: out = bev (+ acc z when R > 0), with the bev values from tv
+// (prefetched chunks, j < kPre) or loaded here.  The sums are those of the NCHW epilogue.
+template <int kPre, typename MT>
+__device__ __forceinline__ void final_chunk_nhwc(float *v, const MT *src_bev, int cc, int j, int R, const float *tv, const float *z)
+{
+    if (j < kPre) {
+#pragma unroll
+        for (int i = 0; i < kEW; ++i) v[i] = tv[(j & 1) * kEW + i];
+    } else {
+        row_ldcs16(src_bev + cc * kEW, v);
+    }
+    if (R > 0) {
+#pragma unroll
+        for (int i = 0; i < kEW; ++i) v[i] = v[i] + z[i];
+    }
+}
+
 
 // ---- layer 3 operand: KC channels of pooled (TMEM, this warp's lanes) -> the A buffer at a_addr; with bias_col, the
 // row's bias column = n_valid (acc = n_valid * b3 + pooled * W3^T) ------------------------------------------------
@@ -438,9 +510,40 @@ struct TileWalk {
 // ---- copy units: cells without a neighbour (back of the list): out = bev ----------------------------------------
 // (thread = cell, the G thread groups split the channels; two units are interleaved after every MLP tile; their list
 // entries were fetched at the start of the tile, so a unit costs one DRAM round trip per channel batch)
-template <int C, int G, typename MT>
+// NHWC: a cell's channels are one row, so the warp copies the rows of its 32 cells (this group's C / G channels of each)
+// with 16-byte accesses, consecutive lanes on consecutive vectors of a row; the cell of row r comes from lane r.
+template <int C, int G, typename MT, bool NHWC>
 __device__ __forceinline__ void copy_units(const TcParams &p, const int32_t (&uframe)[2], const int32_t (&ucell)[2], int grp, int64_t cells)
 {
+    if constexpr (NHWC) {
+        constexpr int V = C / G * (int)sizeof(MT) / 16;   // 16-byte vectors per row and group
+        static_assert(V % kRowBatch == 0, "whole batches per row");
+        const int lane = threadIdx.x & 31;
+#pragma unroll
+        for (int u = 0; u < 2; ++u) {
+            if (uframe[u] >= 0) {   // uniform
+                const size_t o = (size_t)uframe[u] * cells * C + grp * (C / G);
+                const uint4 *src = reinterpret_cast<const uint4 *>(reinterpret_cast<const MT *>(p.bev) + o);
+                uint4 *dst = reinterpret_cast<uint4 *>(reinterpret_cast<MT *>(p.out) + o);
+#pragma unroll 1
+                for (int i0 = lane; i0 < 32 * V; i0 += 32 * kRowBatch) {
+                    uint4 v[kRowBatch];
+                    int64_t e[kRowBatch];
+#pragma unroll
+                    for (int t = 0; t < kRowBatch; ++t) {
+                        const int i = i0 + 32 * t, r = i / V;
+                        const int32_t cell = __shfl_sync(0xffffffffu, ucell[u], r);   // < 0: past the end of the list
+                        e[t] = cell >= 0 ? (int64_t)cell * (C * (int)sizeof(MT) / 16) + (i - r * V) : -1;
+                        if (e[t] >= 0) v[t] = __ldcs(src + e[t]);
+                    }
+#pragma unroll
+                    for (int t = 0; t < kRowBatch; ++t)
+                        if (e[t] >= 0) __stcs(dst + e[t], v[t]);
+                }
+            }
+        }
+        return;
+    }
 #pragma unroll
     for (int u = 0; u < 2; ++u) {
         if (uframe[u] >= 0 && ucell[u] >= 0) {   // uframe is uniform; ucell < 0: a row past the end of the list
@@ -476,7 +579,7 @@ __device__ __forceinline__ void teardown(uint32_t tmem_base, int tmem_cols, int 
     if (warp == 0) tc::tmem_free(tmem_base, tmem_cols);
 }
 
-template <int C, int NS, bool TH = false, typename MT = float>
+template <int C, int NS, bool TH = false, typename MT = float, bool NHWC = false>
 __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks) k_fusion_tc(const TcParams p)
 {
     using TT = typename TableT<TH>::type;   // fp32 tables, or bf16 tables in CF_MODE_BF16_TABLES (NS == 1)
@@ -633,7 +736,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             const uint32_t idx0 = sidx_addr + (uint32_t)((par * K * kTile + rg0 * 8 + r8) * 4);
             const uint32_t ctr0 = sctr_addr + (uint32_t)((par * kTile + rg0 * 8 + r8) * 16);
             const uint32_t dst0 = sA_addr + tc::unit_offset(r8, ku, kc_units) + (uint32_t)(rg0 * kc_units * 128);
-            const MT *src_bev = reinterpret_cast<const MT *>(p.bev) + (size_t)b * C * cells + cell;
+            const MT *src_bev = reinterpret_cast<const MT *>(p.bev) + map_cell<NHWC>(b, cell, C, cells);
             // Pipelined shapes (both layers resident, 4 items per warp and round): tv holds the gathered neighbour rows
             // of the NEXT round while this round's MMA and epilogue run; in the last round the same 32 registers take the
             // bev values of this thread's first two output chunks instead.
@@ -642,7 +745,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             constexpr bool kGatherEarly = kPipe && C <= 32;
             float tv[32];
             auto prefetch_tv = [&]() {
-                if (in_range) prefetch_bev<C, G, kPre>(tv, src_bev, cells, grp);
+                if (in_range) prefetch_bev<C, G, kPre, NHWC>(tv, src_bev, cells, grp);
             };
             if (kPipe && R > 0) {
                 const TT *Tc = Tb + ku * 8, *neg = g_neg + ku * 8;
@@ -799,14 +902,20 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             // ---- final epilogue: out = bev + acc (thread = cell: a warp touches 128 contiguous bytes per channel) ---------
             __syncwarp();
             if (R > 0 || p.out != p.bev) {
-                MT *dst_out = reinterpret_cast<MT *>(p.out) + (size_t)b * C * cells + cell;
+                MT *dst_out = reinterpret_cast<MT *>(p.out) + map_cell<NHWC>(b, cell, C, cells);
 #pragma unroll
                 for (int j = 0; j < (kChunksE + G - 1) / G; ++j) {
                     const int cc = grp + j * G;
                     if (cc < kChunksE) {
                         float z[EW];
                         if (R > 0) tc::tmem_ld<EW>(tmem_acc + lane_off + cc * EW, z);
-                        if (in_range) {
+                        if constexpr (NHWC) {
+                            if (in_range) {
+                                float v[EW];
+                                final_chunk_nhwc<kPre>(v, src_bev, cc, j, R, tv, z);
+                                row_stcs16(dst_out + cc * EW, v);
+                            }
+                        } else if (in_range) {
                             if (j < kPre) {
 #pragma unroll
                                 for (int i = 0; i < EW; ++i)
@@ -834,7 +943,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
         }
         if (!units_ready) walk.fetch_units(db, dq, uframe, ucell);
         units_ready = false;
-        copy_units<C, G, MT>(p, uframe, ucell, grp, cells);
+        copy_units<C, G, MT, NHWC>(p, uframe, ucell, grp, cells);
     }
 
     if (!L::kResident && tid == 0) tc::mbar_wait_a(wbar + (wn & 1) * 8, (wn >> 1) & 1u);   // the weight chunk prefetched for a tile that never came
@@ -871,7 +980,7 @@ struct SkLayout {
     static constexpr int kTmemCols = tmem_cols_for(3 * C);          // two accumulators + the pooled sum
 };
 
-template <int C, int NS, bool TH = false, typename MT = float>
+template <int C, int NS, bool TH = false, typename MT = float, bool NHWC = false>
 __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks) k_fusion_sk(const TcParams p)
 {
     using TT = typename TableT<TH>::type;
@@ -970,7 +1079,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             const uint32_t idx0 = sidx_addr + (uint32_t)((par * K * kTile + rg0 * 8 + r8) * 4);
             const uint32_t ctr0 = sctr_addr + (uint32_t)((par * kTile + rg0 * 8 + r8) * 8);
             const uint32_t dst0 = sA_addr + tc::unit_offset(r8, ku, kc_units) + (uint32_t)(rg0 * kc_units * 128);
-            const MT *src_bev = reinterpret_cast<const MT *>(p.bev) + (size_t)b * C * cells + cell;
+            const MT *src_bev = reinterpret_cast<const MT *>(p.bev) + map_cell<NHWC>(b, cell, C, cells);
             float tv[32];   // neighbour rows of the next round to build; in the last round: bev values of the final epilogue
             auto gather_round = [&](int k) {
 #pragma unroll
@@ -980,7 +1089,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
                 }
             };
             auto prefetch_tv = [&]() {
-                if (in_range) prefetch_bev<C, G, 2>(tv, src_bev, cells, grp);
+                if (in_range) prefetch_bev<C, G, 2, NHWC>(tv, src_bev, cells, grp);
             };
             // A[buf] = relu(T[idx_k] - e) for the rows gathered in tv; bias flag of round k -> Ab[buf]
             auto build_round = [&](int k, uint32_t buf) {
@@ -1091,14 +1200,20 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
             __syncwarp();
             if (R > 0 || p.out != p.bev) {
                 const uint32_t acc_l = tmem_base + (uint32_t)(((R - 1) & 1) * C) + lane_off;
-                MT *dst_out = reinterpret_cast<MT *>(p.out) + (size_t)b * C * cells + cell;
+                MT *dst_out = reinterpret_cast<MT *>(p.out) + map_cell<NHWC>(b, cell, C, cells);
 #pragma unroll
                 for (int j = 0; j < (kChunksE + G - 1) / G; ++j) {
                     const int cc = grp + j * G;
                     if (cc < kChunksE) {
                         float z[EW];
                         if (R > 0) tc::tmem_ld<EW>(acc_l + cc * EW, z);
-                        if (in_range) {
+                        if constexpr (NHWC) {
+                            if (in_range) {
+                                float v[EW];
+                                final_chunk_nhwc<2>(v, src_bev, cc, j, R, tv, z);
+                                row_stcs16(dst_out + cc * EW, v);
+                            }
+                        } else if (in_range) {
                             if (j < 2) {
 #pragma unroll
                                 for (int i = 0; i < EW; ++i)
@@ -1124,7 +1239,7 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
         }
         if (!units_ready) walk.fetch_units(db, dq, uframe, ucell);
         units_ready = false;
-        copy_units<C, G, MT>(p, uframe, ucell, grp, cells);
+        copy_units<C, G, MT, NHWC>(p, uframe, ucell, grp, cells);
     }
 
     teardown(tmem_base, L::kTmemCols, warp);
@@ -1702,12 +1817,12 @@ int resident_ctas(Kern kern, int threads, int smem, int tmem_cols, int *regs_cac
     return CF_OK;
 }
 
-template <bool SK, int C, int NS, bool TH, typename MT>
+template <bool SK, int C, int NS, bool TH, typename MT, bool NHWC>
 int launch_kernel(const TcParams &p, cudaStream_t st)
 {
     using L = std::conditional_t<SK, SkLayout<C, NS>, TcLayout<C, NS>>;
     void (*kern)(TcParams);
-    if constexpr (SK) kern = k_fusion_sk<C, NS, TH, MT>; else kern = k_fusion_tc<C, NS, TH, MT>;
+    if constexpr (SK) kern = k_fusion_sk<C, NS, TH, MT, NHWC>; else kern = k_fusion_tc<C, NS, TH, MT, NHWC>;
     const char *name = SK ? "k_fusion_sk" : "k_fusion_tc";
     constexpr int NT = kTile * TcShape<C>::G;
     const int smem = L::smem_bytes(p.K);
@@ -1729,29 +1844,36 @@ int launch_kernel(const TcParams &p, cudaStream_t st)
 // long (C = 128: 165 -> 148 us), is a wash at C = 64 and loses at C = 32, where the round is all operand build.  At C = 96
 // and 128 it keeps the residency of k_fusion_tc (1 CTA per SM: registers, and its 3C TMEM columns), so it runs wherever its
 // shared memory fits: always, except at C = 128 in fp32 mode (NS = 2) from K = 15 on.
-template <int C, int NS, bool TH, typename MT>
+template <int C, int NS, bool TH, typename MT, bool NHWC>
 int launch_fused(const TcParams &p, cudaStream_t st)
 {
     if constexpr (C == 96 || (C == 128 && NS == 1)) {
         static_assert(SkLayout<C, NS>::smem_bytes(CF_MAX_K) <= 227 * 1024, "k_fusion_sk fits every K at this width");
-        return launch_kernel<true, C, NS, TH, MT>(p, st);
+        return launch_kernel<true, C, NS, TH, MT, NHWC>(p, st);
     } else if constexpr (C == 128) {
-        if (SkLayout<C, NS>::smem_bytes(p.K) <= 227 * 1024) return launch_kernel<true, C, NS, TH, MT>(p, st);
-        return launch_kernel<false, C, NS, TH, MT>(p, st);
+        if (SkLayout<C, NS>::smem_bytes(p.K) <= 227 * 1024) return launch_kernel<true, C, NS, TH, MT, NHWC>(p, st);
+        return launch_kernel<false, C, NS, TH, MT, NHWC>(p, st);
     } else {
-        return launch_kernel<false, C, NS, TH, MT>(p, st);
+        return launch_kernel<false, C, NS, TH, MT, NHWC>(p, st);
     }
 }
 
-// the fused launch of one width for the mode (NS, bf16 tables th) and the map type (io16: bf16 maps)
-template <int C>
-int launch_fused_width(const TcParams &p, int NS, bool th, bool io16, cudaStream_t st)
+// the fused launch of one width for the mode (NS, bf16 tables th) and the map type (io16: bf16 maps) and layout
+template <int C, bool NHWC>
+int launch_fused_layout(const TcParams &p, int NS, bool th, bool io16, cudaStream_t st)
 {
     if (io16)
-        return NS == 2 ? launch_fused<C, 2, false, __nv_bfloat16>(p, st)
-               : th    ? launch_fused<C, 1, true, __nv_bfloat16>(p, st)
-                       : launch_fused<C, 1, false, __nv_bfloat16>(p, st);
-    return NS == 2 ? launch_fused<C, 2, false, float>(p, st) : th ? launch_fused<C, 1, true, float>(p, st) : launch_fused<C, 1, false, float>(p, st);
+        return NS == 2 ? launch_fused<C, 2, false, __nv_bfloat16, NHWC>(p, st)
+               : th    ? launch_fused<C, 1, true, __nv_bfloat16, NHWC>(p, st)
+                       : launch_fused<C, 1, false, __nv_bfloat16, NHWC>(p, st);
+    return NS == 2 ? launch_fused<C, 2, false, float, NHWC>(p, st)
+           : th    ? launch_fused<C, 1, true, float, NHWC>(p, st)
+                   : launch_fused<C, 1, false, float, NHWC>(p, st);
+}
+template <int C>
+int launch_fused_width(const TcParams &p, int NS, bool th, bool io16, bool nhwc, cudaStream_t st)
+{
+    return nhwc ? launch_fused_layout<C, true>(p, NS, th, io16, st) : launch_fused_layout<C, false>(p, NS, th, io16, st);
 }
 
 }  // namespace
@@ -1786,6 +1908,8 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
 {
     CF_REQUIRE(C % 32 == 0, CF_ERR_UNSUPPORTED, "cf_fusion_fwd: tensor-core path needs C %% 32 == 0 (C=%d)", C);
     const bool io16 = (mode & CF_IO_BF16) != 0;   // d_bev / d_out hold bf16 maps
+    const bool nhwc = (mode & CF_IO_NHWC) != 0;   // d_bev / d_out are (B,H,W,C) maps
+    CF_REQUIRE(!nhwc || (aligned16(d_bev) && aligned16(d_out)), CF_ERR_ALIGN, "cf_fusion_fwd: NHWC maps must be 16-byte aligned");
     mode = mode_base(mode);
     const int NS = mode == CF_MODE_FP32 ? 2 : 1;
     // packed W2 | W3 operand images: the caller's cached copy (cf_fusion_pack_weights) or packed here
@@ -1819,12 +1943,12 @@ int fusion_tc(const float *d_bev, const float *d_T, const int32_t *d_knn, int32_
     int rc = CF_ERR_UNSUPPORTED;
     const bool th = mode == CF_MODE_BF16_TABLES;   // d_T holds bf16 rows
     switch (C) {
-        case 32: rc = launch_fused_width<32>(p, NS, th, io16, st); break;
-        case 64: rc = launch_fused_width<64>(p, NS, th, io16, st); break;
-        case 96: rc = launch_fused_width<96>(p, NS, th, io16, st); break;
-        case 128: rc = launch_fused_width<128>(p, NS, th, io16, st); break;
-        case 192: rc = launch_fused_width<192>(p, NS, th, io16, st); break;
-        case 256: rc = launch_fused_width<256>(p, NS, th, io16, st); break;
+        case 32: rc = launch_fused_width<32>(p, NS, th, io16, nhwc, st); break;
+        case 64: rc = launch_fused_width<64>(p, NS, th, io16, nhwc, st); break;
+        case 96: rc = launch_fused_width<96>(p, NS, th, io16, nhwc, st); break;
+        case 128: rc = launch_fused_width<128>(p, NS, th, io16, nhwc, st); break;
+        case 192: rc = launch_fused_width<192>(p, NS, th, io16, nhwc, st); break;
+        case 256: rc = launch_fused_width<256>(p, NS, th, io16, nhwc, st); break;
         default:
             set_error("cf_fusion_fwd: unsupported C=%d on the tensor-core path", C);
             return CF_ERR_UNSUPPORTED;

@@ -213,12 +213,13 @@ class FusionRunner:
     (the same tensors as `.bevs` when `inplace=True`).  Replaying the graph costs one launch on the host instead of the
     ~20 launches and several stream hand-offs of the eager path, which matters when the host is the slow side.
     `dtype=torch.bfloat16`: `.img_feat`, `.bevs` and `.outs` are bf16 maps (half the bytes to copy in and out).
+    `memory_format=torch.channels_last`: `.bevs` and `.outs` are channels_last maps, fused by the NHWC kernels.
     `cameras=M`: a camera rig.  `.img_feat` is (B,M,Ci,Hf,Wf) and `.calib` a static (B,M,4,3) float32 device buffer
     (initialised from `calib`, an (M,4,3) or (B,M,4,3) rig such as geometry.camera_rig, if given): calibrations written into
     it between replays take effect without a new capture."""
 
     def __init__(self, layers, grid, batch, max_points, img_shape, bev_shapes, calib=None, img_size=(640.0, 480.0),
-                 inplace=True, device=None, dtype=torch.float32, cameras=None):
+                 inplace=True, device=None, dtype=torch.float32, cameras=None, memory_format=torch.contiguous_format):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.layers, self.grid, self.calib, self.img_size, self.inplace = list(layers), grid, calib, tuple(img_size), inplace
         self.points = torch.zeros((batch, max_points, 3), dtype=torch.float32, device=dev)
@@ -234,7 +235,8 @@ class FusionRunner:
                 self.calib.copy_(torch.as_tensor(calib, dtype=torch.float32, device=dev).expand(batch, cameras, 4, 3))
             img_shape = (cameras,) + tuple(img_shape)
         self.img_feat = torch.zeros((batch,) + tuple(img_shape), dtype=dtype, device=dev)
-        self.bevs = [torch.zeros((batch,) + tuple(sh), dtype=dtype, device=dev) for sh in bev_shapes]
+        self.bevs = [torch.zeros((batch,) + tuple(sh), dtype=dtype, device=dev).contiguous(memory_format=memory_format)
+                     for sh in bev_shapes]
         self.outs = None
         self.graph = None
         side = torch.cuda.Stream(dev)
@@ -327,7 +329,8 @@ class _FusionFunction(torch.autograd.Function):
         if table is None:
             p1 = packed.w1(w1, mode) if packed is not None else None
             table = ops.point_mlp1(feat, points, num_points, w1, b1, mode=mode, packed=p1)
-        out, _ = ops.fusion_fwd(bev, table, knn_idx, geom, w1, w2, b2, w3, b3, mode=mode, packed=p23, out=out)
+        out, _ = ops.fusion_fwd(bev, table, knn_idx, geom, w1, w2, b2, w3, b3, mode=mode, packed=p23, out=out,
+                                memory_format=ops.map_format(bev))
         # the table is kept for the backward (B*N*C floats: far smaller than the activations autograd keeps for one conv)
         ctx.save_for_backward(feat, points, num_points, knn_idx, w1, b1, w2, b2, w3, b3, table)
         ctx.geom, ctx.mode = geom, mode
@@ -378,7 +381,10 @@ class ContinuousFusion(nn.Module):
     def forward(self, bev, img_feat=None, points=None, num_points=None, calib=None, uv=None, frames: FrameContext = None,
                 geom=None, return_knn: bool = False, out=None):
         """Returns a map of bev's dtype: fp32, or bf16 (under torch.autocast the maps arrive in bf16; autocast does not cast
-        the inputs of this layer, which widens bf16 maps exactly and computes in fp32 with fp32 weights)."""
+        the inputs of this layer, which widens bf16 maps exactly and computes in fp32 with fp32 weights).
+        A channels_last-dense bev (a backbone converted with .to(memory_format=torch.channels_last)) is fused by the NHWC
+        kernels without a layout copy and gives a channels_last map; `out`, if given, must then be channels_last too.
+        Any other bev is fused as an NCHW map."""
         geom = tuple(float(g) for g in geom) if geom is not None else self.geom
         if geom is None:
             raise ValueError("ContinuousFusion: BEV geometry (x0,y0,dx,dy) not set")

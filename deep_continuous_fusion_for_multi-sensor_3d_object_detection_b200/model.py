@@ -320,7 +320,8 @@ class ObjectDetection_DCF(nn.Module):
                 key = f"group{group}"
                 if key not in self.fusion:
                     return x
-                return self.fusion[key](x, frames=frames, out=x if inplace and x.is_contiguous() else None)
+                dense = x.is_contiguous() or x.is_contiguous(memory_format=torch.channels_last)   # NCHW or NHWC kernels
+                return self.fusion[key](x, frames=frames, out=x if inplace and dense else None)
 
         cls, reg = self.lidar_backbone(x_lidar, fuse)
         return torch.cat((cls, reg, self.offset_to_bbox(reg)), dim=1)

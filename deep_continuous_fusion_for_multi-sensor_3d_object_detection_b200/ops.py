@@ -41,6 +41,14 @@ def _map(t: torch.Tensor, name: str, ndim=4):
     return _req(t, name, t.dtype if isinstance(t, torch.Tensor) else torch.float32, ndim)
 
 
+def map_format(t: torch.Tensor):
+    """The layout in which the fused layer reads a BEV map without a copy: torch.channels_last for a channels_last-dense
+    4-D map that is not also NCHW-contiguous, torch.contiguous_format otherwise."""
+    if t.dim() == 4 and not t.is_contiguous() and t.is_contiguous(memory_format=torch.channels_last):
+        return torch.channels_last
+    return torch.contiguous_format
+
+
 def _scratch(nbytes: int, device) -> torch.Tensor:
     """Workspace that the kernels write before they read it.  torch.use_deterministic_algorithms(True) makes torch.empty fill
     new memory (hundreds of MB per backward call here); scratch needs no fill, so it is allocated without one."""
@@ -386,22 +394,36 @@ def point_mlp1_multi(feat, points, num_points, W1s, b1s, packeds, mode="fp32", o
     return outs
 
 
-def fusion_fwd(bev, T, knn_idx, geom, W1, W2, b2, W3, b3, mode="fp32", out=None, workspace=None, packed=None):
+def fusion_fwd(bev, T, knn_idx, geom, W1, W2, b2, W3, b3, mode="fp32", out=None, workspace=None, packed=None,
+               memory_format=torch.contiguous_format):
     """K-4.  out = bev + W3 sum_k relu(W2 relu(T[idx_k] - e_cell) + b2) + n_valid b3.
     `bev` (and `out`, which must have bev's dtype) fp32 or bf16: a bf16 map is widened exactly, the layer computes in fp32 as
-    for an fp32 map and `out` is rounded once to bf16 -- equal to the fp32 result on bev.float(), rounded."""
+    for an fp32 map and `out` is rounded once to bf16 -- equal to the fp32 result on bev.float(), rounded.
+    `memory_format=torch.channels_last`: `bev` (and `out`) are channels_last-dense maps, read and written in place by the NHWC
+    kernels (CF_IO_NHWC); `out=None` allocates a channels_last map.  The values equal those of the NCHW call, bit for bit."""
     lib = load()
     _map(bev, "bev")
+    if memory_format not in (torch.contiguous_format, torch.channels_last):
+        raise ValueError(f"fusion_fwd: memory_format must be torch.contiguous_format or torch.channels_last, got {memory_format}")
+    nhwc = memory_format == torch.channels_last
+    if nhwc and not bev.is_contiguous(memory_format=torch.channels_last):
+        raise ValueError(f"fusion_fwd: memory_format=torch.channels_last needs a channels_last-dense bev, got strides {bev.stride()}")
     if out is not None:
         _map(out, "out")
         if out.dtype != bev.dtype:
             raise ValueError(f"fusion_fwd: out must have bev's dtype {bev.dtype}, got {out.dtype}")
-        if out.shape != bev.shape or out.device != bev.device or not out.is_contiguous():
-            raise ValueError(f"fusion_fwd: out must be a contiguous (dense NCHW) tensor of bev's shape {tuple(bev.shape)} on "
-                             f"{bev.device}, got shape {tuple(out.shape)}, strides {out.stride()}, device {out.device}")
-        if out.data_ptr() == bev.data_ptr() and not bev.is_contiguous():
-            raise ValueError("fusion_fwd: in-place operation (out is bev) needs a contiguous (dense NCHW) map")
-    bev = _contig(bev, "bev", bev.dtype, 4)
+        if nhwc:
+            if out.shape != bev.shape or out.device != bev.device or not out.is_contiguous(memory_format=torch.channels_last):
+                raise ValueError(f"fusion_fwd: out must be a channels_last-dense tensor of bev's shape {tuple(bev.shape)} on "
+                                 f"{bev.device}, got shape {tuple(out.shape)}, strides {out.stride()}, device {out.device}")
+        else:
+            if out.shape != bev.shape or out.device != bev.device or not out.is_contiguous():
+                raise ValueError(f"fusion_fwd: out must be a contiguous (dense NCHW) tensor of bev's shape {tuple(bev.shape)} on "
+                                 f"{bev.device}, got shape {tuple(out.shape)}, strides {out.stride()}, device {out.device}")
+            if out.data_ptr() == bev.data_ptr() and not bev.is_contiguous():
+                raise ValueError("fusion_fwd: in-place operation (out is bev) needs a contiguous (dense NCHW) map")
+    if not nhwc:
+        bev = _contig(bev, "bev", bev.dtype, 4)
     T = _contig(T, "T", table_dtype(mode), 3)
     knn_idx = _contig(knn_idx, "knn_idx", torch.int32, 4)
     B, Cc, H, W = bev.shape
@@ -424,6 +446,8 @@ def fusion_fwd(bev, T, knn_idx, geom, W1, W2, b2, W3, b3, mode="fp32", out=None,
     x0, y0, dx, dy = [float(g) for g in geom]
     if bev.dtype == torch.bfloat16:
         m |= _lib.IO_BF16
+    if nhwc:
+        m |= _lib.IO_NHWC
     check(lib.cf_fusion_fwd(ptr(bev), ptr(T), ptr(knn_idx), B, N, Cc, H, W, K, x0, y0, dx, dy, ptr(W1), Ci, ptr(W2),
                             ptr(b2), ptr(W3), ptr(b3), ptr(out), m, ptr(packed), ptr(workspace), stream_ptr()),
           "cf_fusion_fwd")
@@ -436,10 +460,13 @@ def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2
     `table`: the forward's point_mlp1 output (B,N,C) if it was kept (else it is recomputed); `mode` "simt" keeps every
     GEMM on CUDA cores, any other mode runs them on tcgen05 with fp32-accurate split operands.
     `deterministic`: fixed summation order everywhere (CF_BWD_DETERMINISTIC): identical inputs give bit-identical gradients.
-    `grad_out` fp32 or bf16 (widened exactly; every gradient is fp32)."""
+    `grad_out` fp32 or bf16 (widened exactly; every gradient is fp32).  A channels_last-dense `grad_out` is read in place by
+    the NHWC kernel (CF_IO_NHWC); the gradients do not depend on the layout."""
     lib = load()
     _map(grad_out, "grad_out")
-    grad_out = _contig(grad_out, "grad_out", grad_out.dtype, 4)
+    nhwc = map_format(grad_out) == torch.channels_last
+    if not nhwc:
+        grad_out = _contig(grad_out, "grad_out", grad_out.dtype, 4)
     feat = _contig(feat, "feat", torch.float32, 3)
     points = _contig(points, "points", torch.float32, 3)
     knn_idx = _contig(knn_idx, "knn_idx", torch.int32, 4)
@@ -463,6 +490,8 @@ def fusion_bwd(grad_out, feat, points, num_points, knn_idx, geom, W1, b1, W2, b2
         m |= _lib.BWD_DETERMINISTIC
     if grad_out.dtype == torch.bfloat16:
         m |= _lib.IO_BF16
+    if nhwc:
+        m |= _lib.IO_NHWC
     x0, y0, dx, dy = [float(g) for g in geom]
     check(lib.cf_fusion_bwd(ptr(grad_out), ptr(feat), ptr(points), ptr(num_points), ptr(knn_idx), B, N, Cc, H, W, K, x0, y0,
                             dx, dy, ptr(W1), ptr(b1), Ci, ptr(W2), ptr(b2), ptr(W3), ptr(table), ptr(gW1), ptr(gb1), ptr(gW2),

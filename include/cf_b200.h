@@ -200,10 +200,14 @@ CF_API int cf_fusion_pack_weights(const float *d_W2, const float *d_W3, int32_t 
  *   mode | CF_IO_BF16: d_bev and d_out are bf16 (B,C,H,W) NCHW maps (may alias, as for fp32).  bev is widened exactly to
  *   fp32, everything else is computed as without the flag and out is rounded once to bf16 (nearest even) when stored:
  *   the result equals the fp32 call on the widened map, rounded.  T, weights and the workspace size are unchanged.
- * Every function that takes a `mode` ignores the flag bits (CF_IO_BF16, CF_BWD_DETERMINISTIC) when it picks the
- * arithmetic, the operand layout or a workspace size.
+ *   mode | CF_IO_NHWC: d_bev and d_out are dense (B,H,W,C) maps (PyTorch's channels_last; may alias: in place), 16-byte
+ *   aligned.  Only the addressing of the maps changes: the result is bit-identical to the NCHW call on the same values.
+ *   Combines with CF_IO_BF16.
+ * Every function that takes a `mode` ignores the flag bits (CF_IO_BF16, CF_IO_NHWC, CF_BWD_DETERMINISTIC) when it picks
+ * the arithmetic, the operand layout or a workspace size.
  * ------------------------------------------------------------------------------------------- */
 #define CF_IO_BF16 0x200 /* OR-ed into `mode` of cf_fusion_fwd (bf16 bev / out) and cf_fusion_bwd (bf16 d_gout) */
+#define CF_IO_NHWC 0x400 /* OR-ed into `mode` of cf_fusion_fwd ((B,H,W,C) bev / out) and cf_fusion_bwd ((B,H,W,C) d_gout) */
 CF_API size_t cf_fusion_workspace_bytes(int32_t C, int32_t mode, int32_t B, int32_t H, int32_t W);
 CF_API int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t *d_knn_idx, int32_t B, int32_t N,
                   int32_t C, int32_t H, int32_t W, int32_t K, float x0, float y0, float dx, float dy,
@@ -214,7 +218,9 @@ CF_API int cf_fusion_fwd(const float *d_bev, const float *d_T, const int32_t *d_
 /* ---------------------------------------------------------------------------------------------
  * K-4b backward of cf_point_mlp1 + cf_fusion_fwd for one scale (training only).  d_gout = dL/d out (B,C,H,W);
  * dL/d bev is d_gout itself.  mode | CF_IO_BF16: d_gout is bf16 (widened exactly on load; combines with
- * CF_BWD_DETERMINISTIC, and with it the gradients equal those of the fp32 call on the widened d_gout).  Gradients are ACCUMULATED into d_gW1 (C,Ci+3), d_gb1 (C), d_gW2 (C,C), d_gb2,
+ * CF_BWD_DETERMINISTIC, and with it the gradients equal those of the fp32 call on the widened d_gout).  mode | CF_IO_NHWC:
+ * d_gout is a dense (B,H,W,C) map (combines with CF_IO_BF16 and CF_BWD_DETERMINISTIC; the gradients do not depend on the
+ * layout, and on the deterministic path they are bit-identical to the NCHW call).  Gradients are ACCUMULATED into d_gW1 (C,Ci+3), d_gb1 (C), d_gW2 (C,C), d_gb2,
  * d_gW3, d_gb3 and d_gfeat (B,N,Ci) -- zero them first (d_gfeat collects every scale's contribution).
  * The forward saves only indices, inputs and weights (and, optionally, its table: d_T = the output of
  * cf_point_mlp1, NULL = recompute it); H1/H2/pooled are recomputed into the workspace

@@ -47,6 +47,10 @@ def main(argv=None):
                     "gradients (the fusion layer's fixed-order backward, the trunk's matmul adjoint of the bilinear resizes)")
     ap.add_argument("--amp", action="store_true", help="forward and loss under torch.autocast('cuda', dtype=torch.bfloat16): "
                     "bf16 convolutions, bf16 BEV / camera maps through the fusion layer (fp32 weights and gradients)")
+    ap.add_argument("--channels-last", action="store_true", help="model and inputs converted with "
+                    ".to(memory_format=torch.channels_last): NHWC convolutions, the fusion layer's NHWC kernels")
+    ap.add_argument("--infer", action="store_true", help="time an inference step (forward under torch.no_grad(), the fusion "
+                    "layers fuse in place) instead of a train step")
     a = ap.parse_args(argv)
     if a.deterministic:
         # before CUDA initialises: cuBLAS reads its workspace setting when the first handle is created
@@ -59,13 +63,16 @@ def main(argv=None):
     cfg = dcf.geometry.carla_config(fusion_scales=(1, 2, 3, 4, 5), fusion_k=3)
     torch.manual_seed(rank)
     model = dcf.ObjectDetection_DCF(cfg).to(dev).eval()      # BatchNorm in eval mode, as in the reference (test.py:37)
+    fmt = torch.channels_last if a.channels_last else torch.contiguous_format
+    if a.channels_last:
+        model = model.to(memory_format=fmt)
     if world > 1:
         model = torch.nn.parallel.DistributedDataParallel(model, device_ids=[local], find_unused_parameters=True)
     opt = torch.optim.Adam(model.parameters(), lr=1e-4, betas=(0.9, 0.999), capturable=a.graph)
     wl = dcf.synthetic.make_workload(dict(dcf.synthetic.workload("yaml"), batch=a.batch), seed=200 + rank)
     to = lambda x: torch.from_numpy(np.ascontiguousarray(x)).to(dev)
-    x_lidar = torch.rand(a.batch, 32, 384, 256, device=dev)
-    x_image = torch.randint(0, 255, (a.batch, 3, 480, 640), device=dev, dtype=torch.uint8)
+    x_lidar = torch.rand(a.batch, 32, 384, 256, device=dev).contiguous(memory_format=fmt)
+    x_image = torch.randint(0, 255, (a.batch, 3, 480, 640), device=dev, dtype=torch.uint8).contiguous(memory_format=fmt)
     target = torch.randn(a.batch, 32, 96, 64, device=dev)
     ref_boxes, num_ref = synthetic_labels(a.batch, 300 + rank, dev)
     # every frame of the batch contributes ("sum"); the reference keeps the last frame only (loss.py:71, LossTotal's default)
@@ -83,7 +90,13 @@ def main(argv=None):
     # the autocast weight cache would hold casts made during a graph capture outside the graph's pool: off under --graph
     amp = lambda: torch.autocast("cuda", dtype=torch.bfloat16, enabled=a.amp, cache_enabled=not a.graph)
 
+    def infer():
+        with torch.no_grad(), amp():
+            return model(x_lidar, x_image, **extra)
+
     def step():
+        if a.infer:
+            return infer()
         opt.zero_grad(set_to_none=True)
         with amp():
             pred = model(x_lidar, x_image, **extra)
@@ -105,11 +118,14 @@ def main(argv=None):
         graph = torch.cuda.CUDAGraph()
         opt.zero_grad(set_to_none=True)
         with torch.cuda.graph(graph):
-            with amp():
-                pred = model(x_lidar, x_image, **extra)
-                static_loss = closing_loss(pred)
-            static_loss.backward()
-            opt.step()
+            if a.infer:
+                static_loss = infer()
+            else:
+                with amp():
+                    pred = model(x_lidar, x_image, **extra)
+                    static_loss = closing_loss(pred)
+                static_loss.backward()
+                opt.step()
 
         def step():  # noqa: F811  (gradients are overwritten in place by the replay, nothing to zero)
             graph.replay()
@@ -128,13 +144,14 @@ def main(argv=None):
     dcf.dist_util.barrier()
     torch.cuda.synchronize()
     ms = dcf.dist_util.max_over_ranks([e0.elapsed_time(e1) / a.steps], device=dev)[0]
-    res = {"what": "train step (fwd + bwd + Adam), ObjectDetection_DCF, YAML grid 384x256",
+    what = "inference step (fwd, no_grad)" if a.infer else "train step (fwd + bwd + Adam)"
+    res = {"what": f"{what}, ObjectDetection_DCF, YAML grid 384x256", "memory_format": "channels_last" if a.channels_last else "nchw",
            "fusion": not a.no_fusion, "loss": "mse" if a.mse else "LossTotal (device target assignment)",
            "launch": "cuda_graph_replay" if a.graph else "eager", "deterministic": a.deterministic,
            "amp": "bf16" if a.amp else None,
            "batch_per_gpu": a.batch, "n_gpus": world, "steps": a.steps, "ms_per_step": round(ms, 3),
            "host_enqueue_ms_per_step": round(host_ms, 3),
-           "frames_per_sec": round(a.batch * world / ms * 1e3, 1), "loss_value": float(loss)}
+           "frames_per_sec": round(a.batch * world / ms * 1e3, 1), "loss_value": None if a.infer else float(loss)}
     if rank == 0 and argv is None:
         print(json.dumps(res), flush=True)
     if world > 1:
