@@ -251,14 +251,12 @@ int fusion_simt(const float *d_bev, const float *d_T, const int32_t *d_knn, int3
 
 namespace cf {
 size_t point_mlp1_tc_workspace_bytes(int32_t Ci, int32_t C, int32_t mode);
-int point_mlp1_tc(const float *d_feat, const float *d_points, const int64_t *d_num_points, int32_t B, int32_t N,
-                  int32_t Ci, int32_t C, const float *d_W1, const float *d_b1, float *d_T, int32_t mode,
-                  const void *d_packed, void *d_workspace, cudaStream_t st);
 int point_mlp1_tc_pack(const float *d_W1, int32_t Ci, int32_t C, int32_t mode, void *d_packed, cudaStream_t st);
 int point_mlp1_multi_tc(const float *d_feat, const float *d_points, const int64_t *d_num_points, int32_t B, int32_t N,
                         int32_t Ci, int32_t n_scales, const int32_t *h_C, const float *const *h_W1,
                         const float *const *h_b1, float *const *h_T, int32_t mode, const void *const *h_packed,
                         cudaStream_t st);
+bool point_mlp1_multi_fits(int32_t Ci, int32_t C, int32_t mode);
 }  // namespace cf
 
 extern "C" int cf_point_mlp1_pack_weights(const float *d_W1, int32_t Ci, int32_t C, int32_t mode, void *d_packed, void *stream)
@@ -292,25 +290,24 @@ extern "C" int cf_point_mlp1(const float *d_feat, const float *d_points, const i
     CF_REQUIRE(mode == CF_MODE_FP32 || mode == CF_MODE_BF16 || mode == CF_MODE_FP32_SIMT || mode == CF_MODE_BF16_TABLES, CF_ERR_ARG,
                "cf_point_mlp1: unknown mode %d", mode);
     CF_REQUIRE(aligned16(d_feat) && aligned16(d_T), CF_ERR_ALIGN, "cf_point_mlp1: feat/T must be 16-byte aligned");
-    if (mode == CF_MODE_BF16_TABLES) {   // bf16 rows: the multi-scale kernel with one scale (no FFMA fallback)
+    const bool th = mode == CF_MODE_BF16_TABLES;   // bf16 rows: there is no FFMA kernel to fall back to
+    const bool aligned32 = (reinterpret_cast<uintptr_t>(d_feat) & 31u) == 0 && (reinterpret_cast<uintptr_t>(d_T) & 31u) == 0;
+    if (th) {
         CF_REQUIRE(d_packed != nullptr || d_workspace != nullptr, CF_ERR_ARG, "cf_point_mlp1: CF_MODE_BF16_TABLES needs packed weights or a workspace");
-        CF_REQUIRE(aligned16(d_workspace) && aligned16(d_packed) && (reinterpret_cast<uintptr_t>(d_feat) & 31u) == 0 &&
-                       (reinterpret_cast<uintptr_t>(d_T) & 31u) == 0,
-                   CF_ERR_ALIGN, "cf_point_mlp1: CF_MODE_BF16_TABLES needs 32-byte aligned feat / T and 16-byte aligned weights");
-        const void *img = d_packed;
-        if (!img) {
-            CF_TRY(point_mlp1_tc_pack(d_W1, Ci, C, mode, d_workspace, (cudaStream_t)stream));
-            img = d_workspace;
-        }
-        const int rc = point_mlp1_multi_tc(d_feat, d_points, d_num_points, B, N, Ci, 1, &C, &d_W1, &d_b1, &d_T, mode, &img, (cudaStream_t)stream);
-        if (rc == CF_ERR_UNSUPPORTED) set_error("cf_point_mlp1: CF_MODE_BF16_TABLES does not support Ci=%d, C=%d", Ci, C);
-        return rc;
+        CF_REQUIRE(aligned16(d_workspace) && aligned16(d_packed) && aligned32, CF_ERR_ALIGN,
+                   "cf_point_mlp1: CF_MODE_BF16_TABLES needs 32-byte aligned feat / T and 16-byte aligned weights");
     }
     if (mode != CF_MODE_FP32_SIMT && (d_workspace != nullptr || d_packed != nullptr)) {
         CF_REQUIRE(aligned16(d_workspace) && aligned16(d_packed), CF_ERR_ALIGN, "cf_point_mlp1: workspace / packed weights must be 16-byte aligned");
-        const int rc = point_mlp1_tc(d_feat, d_points, d_num_points, B, N, Ci, C, d_W1, d_b1, d_T, mode, d_packed,
-                                     d_workspace, (cudaStream_t)stream);
-        if (rc != CF_ERR_UNSUPPORTED) return rc;  // shapes without a tensor-core instantiation use the FFMA kernel
+        if (aligned32 && point_mlp1_multi_fits(Ci, C, mode)) {   // the multi-scale kernel with one scale
+            const void *img = d_packed;
+            if (!img) {
+                CF_TRY(point_mlp1_tc_pack(d_W1, Ci, C, mode, d_workspace, (cudaStream_t)stream));
+                img = d_workspace;
+            }
+            return point_mlp1_multi_tc(d_feat, d_points, d_num_points, B, N, Ci, 1, &C, &d_W1, &d_b1, &d_T, mode, &img, (cudaStream_t)stream);
+        }
+        CF_REQUIRE(!th, CF_ERR_UNSUPPORTED, "cf_point_mlp1: CF_MODE_BF16_TABLES does not support Ci=%d, C=%d", Ci, C);
     }
     return point_mlp1_simt(d_feat, d_points, d_num_points, B, N, Ci, C, d_W1, d_b1, d_T, (cudaStream_t)stream);
 }

@@ -1246,164 +1246,13 @@ __global__ void __launch_bounds__(kTile * TcShape<C>::G, TcShape<C>::kMinBlocks)
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// K-4a on tensor cores:  T[b, m, :] = feat[b, m, :] W1[:, :Ci]^T + W1[:, Ci:Ci+3] p_m + b1      (m < num_points[b])
-// Tile = 128 points.  W1's image part stays resident in shared memory; the rank-3 offset term and the bias are
-// added on CUDA cores in the epilogue (Ci+3 = 131 is not an MMA-friendly K).
-// ---------------------------------------------------------------------------------------------------------------
-struct Mlp1Params {
-    const float *feat;
-    const float *points;
-    const int64_t *num_points;
-    const uint8_t *wimg;
-    const float *W1;
-    const float *b1;
-    float *T;
-    int32_t B, N, Ci;
-    int32_t tiles_per_frame;
-};
-
-template <int C>
-struct Mlp1Shape {
-    static constexpr int G = C <= 32 ? 1 : C <= 64 ? 2 : C == 96 || C == 192 ? 3 : 4;  // 128-thread groups per CTA
-};
-
-template <int C, int NS>
-__global__ void __launch_bounds__(kTile * Mlp1Shape<C>::G) k_point_mlp1_tc(const Mlp1Params p)
-{
-    constexpr int G = Mlp1Shape<C>::G, NT = kTile * G, NW = NT / 32;
-    extern __shared__ __align__(1024) uint8_t smem[];
-    __shared__ uint64_t bar;
-    __shared__ uint32_t tmem_slot;
-    const int Ci = p.Ci, kc_units = Ci / 8;
-    const int w_bytes = NS * C * Ci * 2, a_bytes = NS * kTile * Ci * 2;
-    uint8_t *sW = smem;
-    uint8_t *sA = smem + w_bytes;
-    float *sb1 = reinterpret_cast<float *>(smem + w_bytes + a_bytes);
-    float *swx = sb1 + C, *swy = swx + C, *swz = swy + C;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int row = tid & (kTile - 1), grp = tid / kTile;
-    constexpr int kCols = C <= 32 ? 32 : C <= 64 ? 64 : C <= 128 ? 128 : 256;
-
-    if (tid == 0) {
-        tc::mbar_init(&bar, 1);
-        tc::mbar_fence_init();
-    }
-    __syncwarp();
-    if (warp == 0) tc::tmem_alloc(&tmem_slot, kCols);
-    for (int c = tid; c < C; c += NT) {
-        const float *w = p.W1 + (size_t)c * (Ci + 3) + Ci;
-        sb1[c] = __ldg(p.b1 + c);
-        swx[c] = __ldg(w);
-        swy[c] = __ldg(w + 1);
-        swz[c] = __ldg(w + 2);
-    }
-    copy_chunk<NT>(sW, p.wimg, w_bytes);
-    tc::fence_proxy_async();
-    tc::fence_before_sync();
-    __syncthreads();
-    tc::fence_after_sync();
-    const uint32_t tmem_acc = tmem_slot;
-    const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
-    const uint32_t sA_addr = tc::smem_u32(sA), sW_addr = tc::smem_u32(sW);
-    const uint32_t idesc = tc::make_idesc_bf16(kTile, C);
-    const uint32_t sbo = kc_units * 128, lbo = 128;
-    uint32_t phase = 0;
-
-    const int64_t tiles_total = (int64_t)p.tiles_per_frame * p.B;
-    for (int64_t tile = blockIdx.x; tile < tiles_total; tile += gridDim.x) {
-        const int b = (int)(tile / p.tiles_per_frame);
-        const int32_t m0 = (int32_t)(tile - (int64_t)b * p.tiles_per_frame) * kTile;
-        const int32_t n_pts = valid_points(p.num_points, b, p.N);
-        if (m0 >= n_pts) continue;  // uniform across the CTA
-        // A tile: a warp takes one 8-row group x 4 operand units per step, lane (r8 = lane%8, u = lane/8): coalesced
-        // 128-byte row segments in, and each quarter-warp writes 128 contiguous bytes of the operand image (conflict free)
-        const float *fb = p.feat + ((size_t)b * p.N + m0) * Ci;
-        for (int item = warp; item < 16 * (kc_units / 4); item += NW) {
-            const int rg = item / (kc_units / 4), uq = item - rg * (kc_units / 4);
-            const int r = rg * 8 + (lane & 7), ku = uq * 4 + (lane >> 3);
-            float v[8];
-            if (m0 + r < n_pts) {
-                const float4 *src = reinterpret_cast<const float4 *>(fb + (size_t)r * Ci + ku * 8);
-                const float4 t0 = __ldg(src), t1 = __ldg(src + 1);
-                v[0] = t0.x; v[1] = t0.y; v[2] = t0.z; v[3] = t0.w; v[4] = t1.x; v[5] = t1.y; v[6] = t1.z; v[7] = t1.w;
-            } else {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) v[i] = 0.0f;
-            }
-            uint4 hi, lo;
-            tc::split_bf16x8(v, hi, lo, NS == 2);
-            const uint32_t off = tc::unit_offset(r, ku, kc_units);
-            *reinterpret_cast<uint4 *>(sA + off) = hi;
-            if (NS == 2) *reinterpret_cast<uint4 *>(sA + kTile * Ci * 2 + off) = lo;
-        }
-        tc::fence_proxy_async();
-        tc::fence_before_sync();
-        __syncthreads();
-        if (tid == 0) {
-            tc::fence_after_sync();
-            uint32_t acc = 0;
-            for (int kk = 0; kk < Ci / 16; ++kk) {
-                const uint32_t koff = kk * 2 * lbo;
-                const uint64_t a_hi = tc::make_desc(sA_addr + koff, lbo, sbo), w_hi = tc::make_desc(sW_addr + koff, lbo, sbo);
-                tc::mma_bf16(tmem_acc, a_hi, w_hi, idesc, acc);
-                acc = 1;
-                if (NS == 2) {
-                    const uint64_t a_lo = tc::make_desc(sA_addr + kTile * Ci * 2 + koff, lbo, sbo);
-                    const uint64_t w_lo = tc::make_desc(sW_addr + C * Ci * 2 + koff, lbo, sbo);
-                    tc::mma_bf16(tmem_acc, a_hi, w_lo, idesc, 1);
-                    tc::mma_bf16(tmem_acc, a_lo, w_hi, idesc, 1);
-                }
-            }
-            tc::commit(&bar);
-        }
-        tc::mbar_wait(&bar, phase);
-        phase ^= 1u;
-        tc::fence_after_sync();
-        const int32_t m = m0 + row;
-        const bool live = m < n_pts;
-        float px = 0.f, py = 0.f, pz = 0.f;
-        if (live) {
-            const float *q = p.points + ((size_t)b * p.N + m) * 3;
-            px = __ldg(q); py = __ldg(q + 1); pz = __ldg(q + 2);
-        }
-        __syncwarp();
-#pragma unroll 1
-        for (int cc = grp; cc < C / 32; cc += G) {
-            float z[32];
-            tc::tmem_ld32(tmem_acc + lane_off + cc * 32, z);
-            if (live) {
-                float4 *dst = reinterpret_cast<float4 *>(p.T + ((size_t)b * p.N + m) * C + cc * 32);
-#pragma unroll
-                for (int q4 = 0; q4 < 8; ++q4) {
-                    float o[4];
-#pragma unroll
-                    for (int i = 0; i < 2; ++i) {   // the same packed sequence as k_point_mlp1_multi (bit-identical tables)
-                        const int c = cc * 32 + q4 * 4 + 2 * i;
-                        float2 t = tc::fmul2(make_float2(swx[c], swx[c + 1]), make_float2(px, px));
-                        t = tc::ffma2(make_float2(swy[c], swy[c + 1]), make_float2(py, py), t);
-                        t = tc::ffma2(make_float2(swz[c], swz[c + 1]), make_float2(pz, pz), t);
-                        t = tc::fadd2(tc::fadd2(make_float2(z[q4 * 4 + 2 * i], z[q4 * 4 + 2 * i + 1]), t), make_float2(sb1[c], sb1[c + 1]));
-                        o[2 * i] = t.x;
-                        o[2 * i + 1] = t.y;
-                    }
-                    dst[q4] = make_float4(o[0], o[1], o[2], o[3]);
-                }
-            }
-        }
-        tc::fence_before_sync();
-        __syncthreads();
-        tc::fence_after_sync();
-    }
-    __syncthreads();
-    if (warp == 0) tc::tmem_free(tmem_acc, kCols);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// K-4a for SEVERAL scales in one pass.  The camera features of a 128-point tile are split and packed into the UMMA A
-// operand ONCE, then multiplied by every scale's W1 image part: the output channels of all scales form one long N
-// dimension that is walked in chunks of <= 128 columns.  Per chunk: the packed weight rows stream L2 -> shared memory
-// into one of two buffers, one thread issues the K = Ci MMAs into one of two TMEM accumulators, and the epilogue of the
-// previous chunk (rank-3 offset + bias, write T) runs under them.
+// K-4a on tensor cores:  T_s[b, m, :] = feat[b, m, :] W1_s[:, :Ci]^T + W1_s[:, Ci:Ci+3] p_m + b1_s      (m < num_points[b])
+// for one or SEVERAL scales s in one pass (cf_point_mlp1 is the one-scale call).  The camera features of a 128-point
+// tile are split and packed into the UMMA A operand ONCE, then multiplied by every scale's W1 image part: the output
+// channels of all scales form one long N dimension that is walked in chunks of <= 128 columns.  Per chunk: the packed
+// weight rows stream L2 -> shared memory into one of two buffers, one thread issues the K = Ci MMAs into one of two TMEM
+// accumulators, and the epilogue of the previous chunk runs under them.  The rank-3 offset term and the bias are added
+// on CUDA cores in that epilogue (Ci + 3 = 131 is not an MMA-friendly K).
 // ---------------------------------------------------------------------------------------------------------------
 #ifndef CF_L1_PREFETCH
 #define CF_L1_PREFETCH 1
@@ -1566,8 +1415,10 @@ __global__ void __launch_bounds__(kMultiThreads, 1) k_point_mlp1_multi(const Mlp
             }
         }
 #endif
-        // ---- A tile, once for all scales (same lane mapping as k_point_mlp1_tc).  The feature rows stream from DRAM:
-        // the loads of a batch of items are all issued before the first one is split and stored ------------------------
+        // ---- A tile, once for all scales.  An item is one 8-row group x 4 operand units (hence Ci % 32 == 0), lane (r8 = lane % 8, u = lane / 8):
+        // coalesced 128-byte row segments in, and each quarter-warp writes 128 contiguous bytes of the operand image (conflict
+        // free).  The feature rows stream from DRAM: the loads of a batch of items are all issued before the first one is
+        // split and stored -----------------------------------------------------------------------------------------------
         const float *fb = p.feat + ((size_t)b * p.N + m0) * Ci;
         const int n_items = 16 * (kc_units / 4);
         constexpr int kBatch = 4;
@@ -1708,21 +1559,6 @@ __global__ void __launch_bounds__(kMultiThreads, 1) k_point_mlp1_multi(const Mlp
     flush_pending();
     if (tid == 0) tc::bulk_wait0();   // the staged blocks have been written before the shared memory goes away
     if (warp == 0) tc::tmem_free(tmem_base, 2 * kChunkW);
-}
-
-template <int C, int NS>
-int launch_mlp1_tc(const Mlp1Params &p, cudaStream_t st)
-{
-    constexpr int NT = kTile * Mlp1Shape<C>::G;
-    const int smem = NS * (C + kTile) * p.Ci * 2 + 4 * C * 4;
-    CF_TRY(cuda_status(cudaFuncSetAttribute(k_point_mlp1_tc<C, NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem),
-                       "k_point_mlp1_tc smem attribute"));
-    constexpr int kCols = C <= 32 ? 32 : C <= 64 ? 64 : C <= 128 ? 128 : 256;
-    const int per_sm = std::max(1, std::min(std::min((227 * 1024) / (smem + 1024), 512 / kCols), std::min(2048 / NT, 4)));
-    const int64_t tiles = (int64_t)p.tiles_per_frame * p.B;
-    const int64_t grid = std::min<int64_t>(tiles, (int64_t)sm_count() * per_sm);
-    k_point_mlp1_tc<C, NS><<<(unsigned)grid, NT, smem, st>>>(p);
-    return CF_OK;
 }
 
 // a standalone D[128 x N] = A[128 x Kd] * B[N x Kd]^T through exactly the same packing / descriptor / TMEM code,
@@ -1974,34 +1810,6 @@ size_t point_mlp1_tc_workspace_bytes(int32_t Ci, int32_t C, int32_t mode)
     return (size_t)NS * C * Ci * 2 + 256;
 }
 
-// returns CF_ERR_UNSUPPORTED (without setting an error) when the shape has no tensor-core instantiation
-int point_mlp1_tc(const float *d_feat, const float *d_points, const int64_t *d_num_points, int32_t B, int32_t N,
-                  int32_t Ci, int32_t C, const float *d_W1, const float *d_b1, float *d_T, int32_t mode,
-                  const void *d_packed, void *d_workspace, cudaStream_t st)
-{
-    const int NS = mode == CF_MODE_FP32 ? 2 : 1;
-    if (Ci % 16 != 0 || Ci > 256 || C % 32 != 0) return CF_ERR_UNSUPPORTED;
-    if ((size_t)NS * (C + kTile) * Ci * 2 + 4 * C * 4 > 220 * 1024) return CF_ERR_UNSUPPORTED;
-    const uint8_t *img = d_packed ? (const uint8_t *)d_packed : (const uint8_t *)d_workspace;
-    if (!d_packed) CF_TRY(point_mlp1_tc_pack(d_W1, Ci, C, mode, d_workspace, st));
-    Mlp1Params p;
-    p.feat = d_feat; p.points = d_points; p.num_points = d_num_points; p.wimg = img; p.W1 = d_W1; p.b1 = d_b1; p.T = d_T;
-    p.B = B; p.N = N; p.Ci = Ci; p.tiles_per_frame = (N + kTile - 1) / kTile;
-    int rc = CF_ERR_UNSUPPORTED;
-#define CF_M1_CASE(c)                                                              \
-    case c:                                                                        \
-        rc = NS == 2 ? launch_mlp1_tc<c, 2>(p, st) : launch_mlp1_tc<c, 1>(p, st);  \
-        break;
-    switch (C) {
-        CF_M1_CASE(32) CF_M1_CASE(64) CF_M1_CASE(96) CF_M1_CASE(128) CF_M1_CASE(192) CF_M1_CASE(256)
-        default: return CF_ERR_UNSUPPORTED;
-    }
-#undef CF_M1_CASE
-    CF_TRY(rc);
-    count_launches(1);
-    return launch_status("cf_point_mlp1 (tcgen05)");
-}
-
 // 3-D tensor map over a table T (B, N, C) fp32 (or bf16): x = channel (fastest), y = point, z = frame; box 32 (64) x 128 x 1 with the
 // 128-byte swizzle (the layout the epilogue stages).  Rows past N are clipped by the TMA engine.
 static int make_table_map(CUtensorMap *tm, float *base, int32_t C, int32_t N, int32_t B, bool th)
@@ -2028,25 +1836,19 @@ static int make_table_map(CUtensorMap *tm, float *base, int32_t C, int32_t N, in
     return CF_OK;
 }
 
-// returns CF_ERR_UNSUPPORTED (without setting an error) when the shapes do not fit the multi-scale kernel
-int point_mlp1_multi_tc(const float *d_feat, const float *d_points, const int64_t *d_num_points, int32_t B, int32_t N,
-                        int32_t Ci, int32_t n_scales, const int32_t *h_C, const float *const *h_W1,
-                        const float *const *h_b1, float *const *h_T, int32_t mode, const void *const *h_packed,
-                        cudaStream_t st)
+// the chunk table (p.C, p.foff, p.chunk_*, p.n_chunks) and the shared memory of a k_point_mlp1_multi launch; returns
+// CF_ERR_UNSUPPORTED (without setting an error) when the shapes do not fit the kernel
+static int plan_mlp1_multi(Mlp1MultiParams &p, size_t &smem, int32_t Ci, int32_t n_scales, const int32_t *h_C, int32_t mode)
 {
     const int NS = mode == CF_MODE_FP32 ? 2 : 1;
     if (n_scales < 1 || n_scales > kMaxScales || Ci % 32 != 0 || Ci > 256) return CF_ERR_UNSUPPORTED;
-    Mlp1MultiParams p;
-    p.feat = d_feat; p.points = d_points; p.num_points = d_num_points;
-    p.B = B; p.N = N; p.Ci = Ci; p.tiles_per_frame = (N + kTile - 1) / kTile; p.n_scales = n_scales;
     const bool th = mode == CF_MODE_BF16_TABLES;
     const int chunk_w = NS == 2 ? MultiShape<2>::kChunkW : th ? MultiShape<1, true>::kChunkW : MultiShape<1>::kChunkW;
     const int stage_bytes = NS == 2 ? MultiShape<2>::kStageBytes : th ? MultiShape<1, true>::kStageBytes : MultiShape<1>::kStageBytes;
     int chunks = 0, foff = 0;
     for (int s = 0; s < n_scales; ++s) {
         const int C = h_C[s];
-        if (C % 32 != 0 || C < 32 || C > 1024 || !h_packed[s]) return CF_ERR_UNSUPPORTED;
-        p.wimg[s] = (const uint8_t *)h_packed[s]; p.W1[s] = h_W1[s]; p.b1[s] = h_b1[s]; p.T[s] = h_T[s];
+        if (C % 32 != 0 || C < 32 || C > 1024) return CF_ERR_UNSUPPORTED;
         p.C[s] = C; p.foff[s] = foff;
         foff += 4 * C;
         for (int n0 = 0; n0 < C; n0 += chunk_w) {
@@ -2057,16 +1859,42 @@ int point_mlp1_multi_tc(const float *d_feat, const float *d_points, const int64_
     }
     p.n_chunks = chunks;
     const int w_bufs = NS == 2 ? MultiShape<2>::kWBufs : MultiShape<1>::kWBufs;
-    const size_t smem = (size_t)stage_bytes + (size_t)NS * (kTile + w_bufs * chunk_w) * Ci * 2 + (size_t)foff * 4;
-    if (smem > 225 * 1024) return CF_ERR_UNSUPPORTED;
+    smem = (size_t)stage_bytes + (size_t)NS * (kTile + w_bufs * chunk_w) * Ci * 2 + (size_t)foff * 4;
+    return smem > 225 * 1024 ? CF_ERR_UNSUPPORTED : CF_OK;
+}
+
+bool point_mlp1_multi_fits(int32_t Ci, int32_t C, int32_t mode)
+{
+    Mlp1MultiParams p;
+    size_t smem;
+    return plan_mlp1_multi(p, smem, Ci, 1, &C, mode) == CF_OK;
+}
+
+// returns CF_ERR_UNSUPPORTED (without setting an error) when the shapes do not fit the multi-scale kernel
+int point_mlp1_multi_tc(const float *d_feat, const float *d_points, const int64_t *d_num_points, int32_t B, int32_t N,
+                        int32_t Ci, int32_t n_scales, const int32_t *h_C, const float *const *h_W1,
+                        const float *const *h_b1, float *const *h_T, int32_t mode, const void *const *h_packed,
+                        cudaStream_t st)
+{
+    const int NS = mode == CF_MODE_FP32 ? 2 : 1;
+    const bool th = mode == CF_MODE_BF16_TABLES;
+    Mlp1MultiParams p;
+    size_t smem;
+    if (plan_mlp1_multi(p, smem, Ci, n_scales, h_C, mode) != CF_OK) return CF_ERR_UNSUPPORTED;
+    p.feat = d_feat; p.points = d_points; p.num_points = d_num_points;
+    p.B = B; p.N = N; p.Ci = Ci; p.tiles_per_frame = (N + kTile - 1) / kTile; p.n_scales = n_scales;
+    for (int s = 0; s < n_scales; ++s) {
+        if (!h_packed[s]) return CF_ERR_UNSUPPORTED;
+        p.wimg[s] = (const uint8_t *)h_packed[s]; p.W1[s] = h_W1[s]; p.b1[s] = h_b1[s]; p.T[s] = h_T[s];
+    }
     Mlp1Maps maps;
     memset(&maps, 0, sizeof(maps));
-    p.tma_out = stage_bytes > 0 && !tuning().no_tma_store;
+    p.tma_out = (NS == 2 ? MultiShape<2>::kStaged : MultiShape<1>::kStaged) && !tuning().no_tma_store;
     for (int s = 0; s < n_scales; ++s)
         if (((uintptr_t)h_T[s] & 15u) != 0) p.tma_out = 0;
     for (int s = 0; s < n_scales && p.tma_out; ++s)
         if (make_table_map(&maps.m[s], h_T[s], h_C[s], N, B, th) != CF_OK) p.tma_out = 0;   // no tensor maps (old driver): direct stores
-    if (tuning().debug_launch) fprintf(stderr, "k_point_mlp1_multi<%d,%d>: %d chunks, staged TMA stores %d\n", NS, (int)th, chunks, p.tma_out);
+    if (tuning().debug_launch) fprintf(stderr, "k_point_mlp1_multi<%d,%d>: %d chunks, staged TMA stores %d\n", NS, (int)th, p.n_chunks, p.tma_out);
     auto kern = NS == 2 ? k_point_mlp1_multi<2> : th ? k_point_mlp1_multi<1, true> : k_point_mlp1_multi<1>;
     CF_TRY(cuda_status(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem),
                        "k_point_mlp1_multi smem attribute"));

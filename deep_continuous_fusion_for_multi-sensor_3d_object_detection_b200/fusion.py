@@ -120,7 +120,7 @@ class FrameContext:
         streams = self._side_streams(len(layers) + 1)
         dev = self.points.device
         Ci = self.feat.shape[2]
-        multi = (len(layers) > 1 and len(layers) <= 8 and Ci % 32 == 0 and Ci <= 128 and len({l.mode for l in layers}) == 1
+        multi = (len(layers) <= 8 and Ci % 32 == 0 and Ci <= 128 and len({l.mode for l in layers}) == 1
                  and layers[0].mode in ("fp32", "bf16", "bf16t") and all(l.c_bev % 32 == 0 for l in layers)
                  and sum(-(-l.c_bev // 128) for l in layers) <= 16)
         if multi:

@@ -299,7 +299,7 @@ class PackedWeights:
         if m == _lib.MODE_SIMT:
             return None
         C_out, Ci = W1.shape[0], W1.shape[1] - 3
-        if Ci % 16 or Ci > 256 or C_out % 32:
+        if Ci % 32 or Ci > 256 or C_out % 32:
             return None
         key = self._key(W1, mode=m)
         if key != self._key1 or self._repack_in_capture(W1):

@@ -166,8 +166,13 @@ CF_API int cf_point_gather_multi_bwd_det(const float *d_gfeat, float *d_gimg, in
  *   T[b,p,:] = W1[:, :Ci] f_p + W1[:, Ci:Ci+3] (px,py,pz) + b1        so that for BEV cell centre c
  *   relu(W1 [f_p, p - (cx,cy,0)] + b1) = relu(T[b,p,:] - W1[:,Ci]*cx - W1[:,Ci+1]*cy)
  *   d_W1 (C, Ci+3) fp32 row-major (nn.Linear.weight layout), d_b1 (C).  d_T (B,N,C) fp32 out.
- *   mode CF_MODE_FP32 / CF_MODE_BF16: tcgen05 GEMM over the Ci image channels (needs the workspace);
- *   CF_MODE_FP32_SIMT, or shapes without a tensor-core instantiation: FFMA kernel.
+ *   mode CF_MODE_FP32 / CF_MODE_BF16 / CF_MODE_BF16_TABLES: tcgen05 GEMM over the Ci image channels (needs d_packed or
+ *   the workspace), the one-scale call of cf_point_mlp1_multi.  CF_MODE_FP32_SIMT, and CF_MODE_FP32 / CF_MODE_BF16 calls
+ *   that kernel does not take, run the FFMA kernel.  Among them:
+ *     - Ci % 32 == 16 (the tensor-core kernel builds its operand from 32-channel quads);
+ *     - CF_MODE_FP32 with 128 < Ci <= 256 (the split operands do not fit shared memory);
+ *     - feat or T 16-byte but not 32-byte aligned (the kernel moves 32-byte vectors).
+ *   CF_MODE_BF16_TABLES has no FFMA kernel: such calls fail (CF_ERR_UNSUPPORTED, CF_ERR_ALIGN).
  * ------------------------------------------------------------------------------------------- */
 CF_API size_t cf_point_mlp1_workspace_bytes(int32_t Ci, int32_t C, int32_t mode);
 CF_API int cf_point_mlp1(const float *d_feat, const float *d_points, const int64_t *d_num_points, int32_t B,

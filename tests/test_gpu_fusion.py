@@ -94,6 +94,37 @@ def test_point_mlp1_multi_equals_per_scale_calls(dcf, mode):
         assert one[0].abs().max() > 0 and float(tm[1].abs().max()) == 0.0 and float(tm[2, 517:].abs().max()) == 0.0
 
 
+@pytest.mark.parametrize("mode", ["fp32", "bf16"])
+@pytest.mark.parametrize("Ci", [16, 48, 96])
+def test_point_mlp1_camera_widths(dcf, mode, Ci):
+    """cf_point_mlp1 with and without a packed image, incl. ragged frames, at camera widths the other tests do not use.
+    Ci % 32 == 16 has no tensor-core operand layout: the FFMA kernel runs, bit-equal to "simt".  Ci = 96 is a one-scale
+    call of the tensor-core kernel: bit-equal to cf_point_mlp1_multi, and within the mode's tolerance of "simt".  Rows past
+    num_points stay untouched."""
+    torch.manual_seed(43)
+    B, N, C = 3, 1000, 64
+    feat = torch.randn(B, N, Ci, device="cuda")
+    pts = torch.randn(B, N, 3, device="cuda") * 20
+    cnt = torch.tensor([N, 0, 517], dtype=torch.int64, device="cuda")
+    W1 = torch.randn(C, Ci + 3, device="cuda") * 0.1
+    b1 = torch.randn(C, device="cuda")
+    untouched = lambda t: bool((t[1] == 7.0).all()) and bool((t[2, 517:] == 7.0).all())
+    live = lambda t: torch.cat([t[0], t[2, :517]]).cpu().numpy()
+    ref = dcf.ops.point_mlp1(feat, pts, cnt, W1, b1, mode="simt", out=torch.full((B, N, C), 7.0, device="cuda"))
+    pk = dcf.ops.PackedWeights().w1(W1, mode)
+    for packed in (None, pk):
+        got = dcf.ops.point_mlp1(feat, pts, cnt, W1, b1, mode=mode, packed=packed, out=torch.full((B, N, C), 7.0, device="cuda"))
+        torch.cuda.synchronize()
+        assert untouched(ref) and untouched(got)
+        if Ci % 32:
+            assert torch.equal(got, ref), f"packed={packed is not None}"
+        else:
+            multi, = dcf.ops.point_mlp1_multi(feat, pts, cnt, [W1], [b1], [pk], mode=mode,
+                                              outs=[torch.full((B, N, C), 7.0, device="cuda")])
+            assert torch.equal(got, multi), f"packed={packed is not None}"
+            assert rel_err(live(got), live(ref)) <= TOL[mode], f"packed={packed is not None}: {rel_err(live(got), live(ref)):.3e}"
+
+
 def test_bf16_tables_layer1_is_the_rounded_fp32_table(dcf):
     """CF_MODE_BF16_TABLES ("bf16t"): cf_point_mlp1_multi writes exactly round-to-nearest-even bf16 of the CF_MODE_BF16 table
     (full tiles leave through TMA stores, the partial tile of a frame through direct stores), rows past num_points stay
