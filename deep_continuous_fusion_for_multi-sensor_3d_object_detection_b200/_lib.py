@@ -17,10 +17,19 @@ IO_NHWC = 0x400             # CF_IO_NHWC: OR-ed into the mode of cf_fusion_fwd /
 # "bf16t" = CF_MODE_BF16_TABLES: bf16 operands AND bf16 layer-1 tables (inference only)
 MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "simt": MODE_SIMT, "bf16t": MODE_BF16_TABLES}
 MAX_K = 16
-MAX_CAMERAS = 8             # CF_MAX_CAMERAS: cameras of a rig (cf_point_gather_multi)
+MAX_CAMERAS = 8             # CF_MAX_CAMERAS: cameras of a rig (cf_point_gather_multi, cf_point_gather_rig)
 ABI_VERSION = 2
 
 _vp, _i32, _i64, _f32, _sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
+
+
+class CameraMap(C.Structure):
+    """cf_camera_map: one camera of a cf_point_gather_rig* call (its map, ELEMENT strides, extent and image size)."""
+    _fields_ = [("d_map", _vp), ("sb", _i64), ("sc", _i64), ("sh", _i64), ("sw", _i64), ("Hf", _i32), ("Wf", _i32),
+                ("img_w", _f32), ("img_h", _f32)]
+
+
+_cams = C.POINTER(CameraMap)
 
 # name -> (restype, argtypes); mirrors include/cf_b200.h one to one
 SIGNATURES = {
@@ -48,6 +57,12 @@ SIGNATURES = {
     "cf_point_gather_multi_bwd_det_workspace_bytes": (_sz, [_i32, _i32, _i32, _i32, _i32]),
     "cf_point_gather_multi_bwd_det": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _i32, _i32, _i32, _i32, _i32, _vp,
                                                 _vp, _vp, _i32, _f32, _f32, _vp, _vp]),
+    "cf_gather_rig_workspace_bytes": (_sz, [_i32, _i32, _i32, _cams]),
+    "cf_point_gather_rig": (C.c_int, [_cams, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
+    "cf_point_gather_rig_bf16": (C.c_int, [_cams, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
+    "cf_point_gather_rig_bwd": (C.c_int, [_vp, C.POINTER(_vp), _cams, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp]),
+    "cf_point_gather_rig_bwd_det_workspace_bytes": (_sz, [_i32, _i32, _i32, _cams]),
+    "cf_point_gather_rig_bwd_det": (C.c_int, [_vp, C.POINTER(_vp), _cams, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp]),
     "cf_point_mlp1_workspace_bytes": (_sz, [_i32, _i32, _i32]),
     "cf_point_mlp1": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "cf_point_mlp1_pack_weights": (C.c_int, [_vp, _i32, _i32, _i32, _vp, _vp]),

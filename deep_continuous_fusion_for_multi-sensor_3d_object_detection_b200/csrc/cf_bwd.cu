@@ -392,20 +392,30 @@ __global__ void __launch_bounds__(256) k_bwd_scatter(const float *__restrict__ d
     }
 }
 
-// d img[b, m, c, y, x] += (w_mt / n_vis) * dF[b, p, c] for the taps inside the map of every camera m that sees point p
-// (adjoint of k_point_gather; with n_vis == 1 the quotient is w_mt itself).  Lane m < M resolves camera m.
-__global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restrict__ dF, int64_t sb, int64_t sm, int64_t sc,
-                                                          int64_t sh, int64_t sw, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+// *(float *)g += v, g a global-space address.  The gather adjoint's gradient pointers come from the block's camera table as
+// generic pointers, and atomicAdd on a generic pointer compiles to a generic atomic (with a shared-memory fallback) instead
+// of a global reduction.
+__device__ __forceinline__ void red_add_global(size_t g, float v) { asm volatile("red.global.add.f32 [%0], %1;" ::"l"(g), "f"(v) : "memory"); }
+
+// d img_m[b, c, y, x] += (w_mt / n_vis) * dF[b, p, c] for the taps inside the map of every camera m that sees point p
+// (adjoint of k_point_gather; with n_vis == 1 the quotient is w_mt itself).  Lane m < M resolves camera m; cams.map[m] is
+// camera m's gradient, read from the block's camera table.
+__global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restrict__ dF, const RigCams cams, int32_t M, int32_t Ci,
                                                           const CamSource src, const int64_t *__restrict__ num_points,
-                                                          int32_t N, float sx, float sy, float *__restrict__ dimg)
+                                                          int32_t N)
 {
+    __shared__ CamTable ct;
     const int b = blockIdx.y;
-    const int32_t n = valid_points(num_points, b, N);
+    const int32_t n = valid_points(num_points, b, N);  // loaded before the barrier: its latency overlaps the staging
+    stage_cams<float>(ct, cams, M, b);
     const int lane = threadIdx.x & 31;
     const int32_t warps = gridDim.x * (blockDim.x >> 5);
+    const int cl = lane < M ? lane : 0;  // this lane's camera
     for (int32_t p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); p < n; p += warps) {
         float uf = 0.0f, vf = 0.0f;
-        const unsigned vis = __ballot_sync(0xffffffffu, lane < M && cam_project(src, b, N, p, lane, M, sx, sy, Hf, Wf, uf, vf));
+        const int32_t Hf = ct.Hf[cl], Wf = ct.Wf[cl];
+        const unsigned vis =
+            __ballot_sync(0xffffffffu, lane < M && cam_project(src, b, N, p, lane, M, ct.sx[cl], ct.sy[cl], Hf, Wf, uf, vf));
         if (vis == 0) continue;
         const float nv = (float)__popc(vis);
         const Taps tp = bilinear_taps(uf, vf, Hf, Wf);
@@ -420,35 +430,56 @@ __global__ void __launch_bounds__(256) k_point_gather_bwd(const float *__restric
             const float wt[4] = {__shfl_sync(0xffffffffu, l0, m), __shfl_sync(0xffffffffu, l1, m),
                                  __shfl_sync(0xffffffffu, l2, m), __shfl_sync(0xffffffffu, l3, m)};
             const int32_t tx[4] = {ix, ix + 1, ix, ix + 1}, ty[4] = {iy, iy, iy + 1, iy + 1};
-            float *dst = dimg + b * sb + m * sm;
+            const size_t dst = __cvta_generic_to_global(ct.base[m]);
+            const int64_t sc = ct.sc[m], sh = ct.sh[m], sw = ct.sw[m];
             for (int32_t c = lane; c < Ci; c += 32) {
                 const float gval = __ldg(g + c);
                 if (gval == 0.0f) continue;
 #pragma unroll
                 for (int t = 0; t < 4; ++t)
-                    if (in >> t & 1) atomicAdd(dst + c * sc + ty[t] * sh + tx[t] * sw, __fmul_rn(wt[t], gval));
+                    if (in >> t & 1)
+                        red_add_global(dst + sizeof(float) * (c * sc + ty[t] * sh + tx[t] * sw), __fmul_rn(wt[t], gval));
             }
         }
     }
 }
 
-// K-3's atomic adjoint for M cameras of one source; `fn` names the entry point in the error texts
-static int point_gather_bwd(const char *fn, const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc, int64_t sh,
-                            int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const CamSource &src,
-                            const int64_t *d_num_points, int32_t N, float img_w, float img_h, void *stream)
+// K-3's atomic adjoint for the M cameras of h_cams and one source, into the gradients h_gimg[m]; `fn` names the entry point
+// in the error texts
+static int point_gather_bwd(const char *fn, const float *d_gfeat, float *const *h_gimg, const cf_camera_map *h_cams, int32_t B,
+                            int32_t M, int32_t Ci, const CamSource &src, const int64_t *d_num_points, int32_t N, void *stream)
 {
     CF_TRY(require_sm100());
-    CF_REQUIRE(d_gfeat && d_gimg && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points, CF_ERR_ARG,
+    CF_TRY(check_cams(fn, h_cams, M));
+    CF_REQUIRE(d_gfeat && h_gimg && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points, CF_ERR_ARG,
                "%s: null pointer", fn);
-    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
-    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
-               "%s: bad extents", fn);
-    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 16);
-    k_point_gather_bwd<<<dim3(blocks, B), 256, 0, (cudaStream_t)stream>>>(d_gfeat, sb, sm, sc, sh, sw, M, Ci, Hf, Wf, src,
-                                                                          d_num_points, N, (float)Wf / img_w,
-                                                                          (float)Hf / img_h, d_gimg);
+    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0, CF_ERR_ARG, "%s: bad extents", fn);
+    int64_t total;
+    RigCams cams = rig_cams(h_cams, M, &total);
+    for (int m = 0; m < M; ++m) {
+        CF_REQUIRE(h_gimg[m] != nullptr, CF_ERR_ARG, "%s: null pointer (camera %d gradient)", fn, m);
+        cams.map[m] = h_gimg[m];
+    }
+    // at most five blocks per SM and frame: each warp takes a few points, which pays for the block's camera table
+    const int blocks = (int)std::min<int64_t>(ceil_div64(N, 8), 148 * 5);
+    k_point_gather_bwd<<<dim3(blocks, B), 256, 0, (cudaStream_t)stream>>>(d_gfeat, cams, M, Ci, src, d_num_points, N);
     count_launches(1);
     return launch_status(fn);
+}
+
+// the B*M gradients of a (B,M,Ci,Hf,Wf) map with camera stride sm: M equal descriptors
+static int point_gather_bwd_equal(const char *fn, const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc,
+                                  int64_t sh, int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                  const CamSource &src, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
+                                  void *stream)
+{
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
+    CF_REQUIRE(d_gimg != nullptr, CF_ERR_ARG, "%s: null pointer", fn);
+    cf_camera_map cams[CF_MAX_CAMERAS];
+    float *gimg[CF_MAX_CAMERAS];
+    equal_cams(cams, d_gimg, sizeof(float), sb, sm, sc, sh, sw, M, Hf, Wf, img_w, img_h);
+    for (int m = 0; m < M; ++m) gimg[m] = d_gimg + m * sm;
+    return point_gather_bwd(fn, d_gfeat, gimg, cams, B, M, Ci, src, d_num_points, N, stream);
 }
 
 static size_t up256(size_t v) { return (v + 255) / 256 * 256; }
@@ -761,8 +792,8 @@ extern "C" int cf_point_gather_bwd(const float *d_gfeat, float *d_gimg, int64_t 
 {
     using namespace cf;
     CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG, "cf_point_gather_bwd: pass exactly one of d_uv / h_calib");
-    return point_gather_bwd("cf_point_gather_bwd", d_gfeat, d_gimg, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
-                            camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, stream);
+    return point_gather_bwd_equal("cf_point_gather_bwd", d_gfeat, d_gimg, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
+                                  camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, stream);
 }
 
 // adjoint of cf_point_gather_multi: d_gimg (the rig's logical (B,M,Ci,Hf,Wf) shape / strides) += scatter of d_gfeat (B,N,Ci)
@@ -773,6 +804,17 @@ extern "C" int cf_point_gather_multi_bwd(const float *d_gfeat, float *d_gimg, in
 {
     using namespace cf;
     CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_multi_bwd: d_calib must be 4-byte aligned");
-    return point_gather_bwd("cf_point_gather_multi_bwd", d_gfeat, d_gimg, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf,
-                            rig_source(d_points, d_calib), d_num_points, N, img_w, img_h, stream);
+    return point_gather_bwd_equal("cf_point_gather_multi_bwd", d_gfeat, d_gimg, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf,
+                                  rig_source(d_points, d_calib), d_num_points, N, img_w, img_h, stream);
+}
+
+// adjoint of cf_point_gather_rig: h_gimg[m] (camera m's logical (B,Ci,Hf_m,Wf_m) shape, strides of h_cams[m]) += scatter
+extern "C" int cf_point_gather_rig_bwd(const float *d_gfeat, float *const *h_gimg, const cf_camera_map *h_cams, int32_t B,
+                                       int32_t M, int32_t Ci, const float *d_points, const float *d_calib,
+                                       const int64_t *d_num_points, int32_t N, void *stream)
+{
+    using namespace cf;
+    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN, "cf_point_gather_rig_bwd: d_calib must be 4-byte aligned");
+    return point_gather_bwd("cf_point_gather_rig_bwd", d_gfeat, h_gimg, h_cams, B, M, Ci, rig_source(d_points, d_calib),
+                            d_num_points, N, stream);
 }

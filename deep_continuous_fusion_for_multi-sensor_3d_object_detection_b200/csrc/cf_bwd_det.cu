@@ -199,33 +199,36 @@ __global__ void __launch_bounds__(256) k_det_dT(const float *__restrict__ dA, in
     }
 }
 
-// ---- camera-map gradient ---------------------------------------------------------------------------------------------
-// Every (b, m) camera map is one "frame" of the lists (map index bm = b * M + m).  fill == 0: cnt[pixel] += 1 per tap
-// inside its camera's map;  fill == 1: place (key = 4 p + t, weight w_mt / n_vis) into the pixel's segment.  Thread =
-// point of frame blockIdx.y; cameras in ascending order.
-__global__ void __launch_bounds__(256) k_gdet_taps(const CamSource src, const int64_t *__restrict__ num_points, int32_t M,
-                                                   int32_t N, int32_t Hf, int32_t Wf, float sx, float sy, int fill,
+// ---- camera-map gradient ----------------------------------------------------------------------------------------------
+// The pixel space is the concatenation over (b, m) of the camera planes Hf_m * Wf_m: frame b starts at b * total, camera m
+// at cams.plane[m] within it (equal cameras: map index b * M + m).  fill == 0: cnt[pixel] += 1 per tap inside its camera's
+// map;  fill == 1: place (key = 4 p + t, weight w_mt / n_vis) into the pixel's segment.  Thread = point of frame blockIdx.y;
+// cameras in ascending order, the camera loops unrolled so that every camera's constants are read at a fixed index.
+__global__ void __launch_bounds__(256) k_gdet_taps(const CamSource src, const int64_t *__restrict__ num_points,
+                                                   const RigCams cams, int32_t M, int32_t N, int64_t total, int fill,
                                                    int32_t *__restrict__ cnt, const int32_t *__restrict__ off,
                                                    int32_t *__restrict__ key, float *__restrict__ wgt)
 {
     const int b = blockIdx.y;
     const int32_t n = valid_points(num_points, b, N);
-    const int64_t plane = (int64_t)Hf * Wf;
     for (int32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
         // the visible set first (n_vis divides every weight), then the taps of each visible camera, projected again
         unsigned vis = 0;
         float uf, vf;
-        for (int m = 0; m < M; ++m)
-            if (cam_project(src, b, N, p, m, M, sx, sy, Hf, Wf, uf, vf)) vis |= 1u << m;
+#pragma unroll
+        for (int m = 0; m < CF_MAX_CAMERAS; ++m)
+            if (m < M && cam_project(src, b, N, p, m, M, cams.sx[m], cams.sy[m], cams.Hf[m], cams.Wf[m], uf, vf)) vis |= 1u << m;
         const float nv = (float)__popc(vis);
-        for (int m = 0; m < M; ++m) {
+#pragma unroll
+        for (int m = 0; m < CF_MAX_CAMERAS; ++m) {
             if (!(vis >> m & 1u)) continue;
-            cam_project(src, b, N, p, m, M, sx, sy, Hf, Wf, uf, vf);
+            const int32_t Hf = cams.Hf[m], Wf = cams.Wf[m];
+            cam_project(src, b, N, p, m, M, cams.sx[m], cams.sy[m], Hf, Wf, uf, vf);
             const Taps tp = bilinear_taps(uf, vf, Hf, Wf);
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
                 if (!tp.in(t)) continue;
-                const int64_t px = ((int64_t)b * M + m) * plane + (int64_t)(tp.y + (t >> 1)) * Wf + tp.x + (t & 1);
+                const int64_t px = (int64_t)b * total + cams.plane[m] + (int64_t)(tp.y + (t >> 1)) * Wf + tp.x + (t & 1);
                 if (!fill) {
                     atomicAdd(cnt + px, 1);
                 } else {
@@ -238,30 +241,33 @@ __global__ void __launch_bounds__(256) k_gdet_taps(const CamSource src, const in
     }
 }
 
-// d img[b, m, c, y, x] += sum over the pixel's taps in ascending (point, tap) of w * dF[b, p, c]  (one warp per pixel of the
-// B*M maps)
-__global__ void __launch_bounds__(256) k_gdet_sum(const float *__restrict__ dF, int32_t M, int32_t Ci, int32_t N, int32_t Hf,
-                                                  int32_t Wf, int64_t npx, const int32_t *__restrict__ off,
+// d img_m[b, c, y, x] += sum over the pixel's taps in ascending (point, tap) of w * dF[b, p, c]  (one warp per pixel of the
+// pixel space; cams.map[m] is camera m's gradient)
+__global__ void __launch_bounds__(256) k_gdet_sum(const float *__restrict__ dF, const RigCams cams, int32_t Ci, int32_t N,
+                                                  int64_t total, int64_t npx, const int32_t *__restrict__ off,
                                                   const int32_t *__restrict__ key, const float *__restrict__ wgt,
-                                                  int32_t *__restrict__ key_s, float *__restrict__ wgt_s, int64_t sb,
-                                                  int64_t sm, int64_t sc, int64_t sh, int64_t sw, float *__restrict__ dimg)
+                                                  int32_t *__restrict__ key_s, float *__restrict__ wgt_s)
 {
     const int lane = threadIdx.x & 31;
-    const int64_t plane = (int64_t)Hf * Wf;
     const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
     for (int64_t px = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); px < npx; px += warps) {
         const int32_t s0 = __ldg(off + px), L = __ldg(off + px + 1) - s0;
         if (L == 0) continue;
         warp_rank_sort(key, wgt, s0, L, key_s, wgt_s);
-        const int64_t bm = px / plane, yx = px - bm * plane, y = yx / Wf, x = yx - y * Wf;
-        const int64_t b = bm / M, m = bm - b * M;
+        const int64_t b = px / total;
+        const int32_t r = (int32_t)(px - b * total);  // < total <= 2^31 / B
+        int m = 0;
+#pragma unroll
+        for (int k = 1; k < CF_MAX_CAMERAS; ++k) m += r >= cams.plane[k];  // plane[k] = INT32_MAX past the last camera
+        const Cam cm = cam_get(cams, m);
+        const int32_t yx = r - cm.plane, y = yx / cm.Wf, x = yx - y * cm.Wf;
         const float *src = dF + (size_t)b * N * Ci;
-        float *dst = dimg + b * sb + m * sm + y * sh + x * sw;
+        float *dst = (float *)cm.map + b * cm.sb + y * cm.sh + x * cm.sw;
         for (int32_t c = lane; c < Ci; c += 32) {
             float s = 0.0f;
             for (int32_t j = 0; j < L; ++j)
                 s = __fadd_rn(s, __fmul_rn(wgt_s[s0 + j], __ldg(src + (size_t)(key_s[s0 + j] >> 2) * Ci + c)));
-            dst[c * sc] += s;
+            dst[c * cm.sc] += s;
         }
         __syncwarp();
     }
@@ -344,7 +350,7 @@ struct GdetWs {
     size_t bytes;
 };
 
-GdetWs gdet_carve(void *base, int32_t B, int32_t N, int32_t Hf, int32_t Wf)
+GdetWs gdet_carve(void *base, int64_t npx, int64_t taps)
 {
     GdetWs w;
     size_t o = 0;
@@ -353,7 +359,6 @@ GdetWs gdet_carve(void *base, int32_t B, int32_t N, int32_t Hf, int32_t Wf)
         o += (words * 4 + 255) / 256 * 256;
         return p;
     };
-    const size_t npx = (size_t)B * Hf * Wf, taps = (size_t)4 * B * N;
     w.cnt = (int32_t *)take(npx);
     w.off = (int32_t *)take(npx + 1);
     w.key = (int32_t *)take(taps);
@@ -365,53 +370,86 @@ GdetWs gdet_carve(void *base, int32_t B, int32_t N, int32_t Hf, int32_t Wf)
     return w;
 }
 
+// the pixels of the B frames' camera planes
+int64_t gdet_pixels(int32_t B, int32_t M, const cf_camera_map *h_cams)
+{
+    int64_t per = 0;
+    for (int m = 0; m < M; ++m) per += (int64_t)h_cams[m].Hf * h_cams[m].Wf;
+    return (int64_t)B * per;
+}
 
-// K-3's fixed-order adjoint for M cameras of one source: CSR of the (point, tap) contributions by pixel of the B*M maps, one
-// thread per (pixel, channel) summing its segment in ascending (point, tap) order; `fn` names the entry point in the error
-// texts
-static int point_gather_bwd_det(const char *fn, const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc,
-                                int64_t sh, int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
-                                const cf::CamSource &src, const int64_t *d_num_points, int32_t N, float img_w, float img_h,
-                                void *d_workspace, void *stream)
+// K-3's fixed-order adjoint for the M cameras of h_cams and one source, into the gradients h_gimg[m]: CSR of the (point,
+// tap) contributions by pixel of the concatenated camera planes, one thread per (pixel, channel) summing its segment in
+// ascending (point, tap) order; `fn` names the entry point in the error texts
+static int point_gather_bwd_det(const char *fn, const float *d_gfeat, float *const *h_gimg, const cf_camera_map *h_cams,
+                                int32_t B, int32_t M, int32_t Ci, const cf::CamSource &src, const int64_t *d_num_points,
+                                int32_t N, void *d_workspace, void *stream)
 {
     using namespace cf;
     const char *bm = src.kind == CamSource::kRig ? "B*M" : "B";
     CF_TRY(require_sm100());
-    CF_REQUIRE(d_gfeat && d_gimg && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points && d_workspace,
+    CF_TRY(check_cams(fn, h_cams, M));
+    CF_REQUIRE(d_gfeat && h_gimg && src.points && (src.dev || src.kind == CamSource::kHostCrt) && d_num_points && d_workspace,
                CF_ERR_ARG, "%s: null pointer", fn);
-    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
-    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0 && Hf > 0 && Wf > 0 && img_w > 0 && img_h > 0, CF_ERR_ARG,
-               "%s: bad extents", fn);
-    CF_REQUIRE((int64_t)4 * B * M * N < ((int64_t)1 << 31) && (int64_t)B * M * Hf * Wf < ((int64_t)1 << 31), CF_ERR_ARG,
-               "%s: 4*%s*N and %s*Hf*Wf must stay below 2^31", fn, bm, bm);
+    CF_REQUIRE(B > 0 && B <= 65535 && N > 0 && Ci > 0, CF_ERR_ARG, "%s: bad extents", fn);
+    const int64_t npx = gdet_pixels(B, M, h_cams);
+    CF_REQUIRE((int64_t)4 * B * M * N < ((int64_t)1 << 31) && npx < ((int64_t)1 << 31), CF_ERR_ARG,
+               "%s: 4*%s*N and B*Sum_m Hf_m*Wf_m must stay below 2^31", fn, bm);
+    int64_t total;
+    RigCams cams = rig_cams(h_cams, M, &total);
+    for (int m = 0; m < M; ++m) {
+        CF_REQUIRE(h_gimg[m] != nullptr, CF_ERR_ARG, "%s: null pointer (camera %d gradient)", fn, m);
+        cams.map[m] = h_gimg[m];
+    }
     cudaStream_t st = (cudaStream_t)stream;
-    GdetWs w = gdet_carve(d_workspace, B * M, N, Hf, Wf);
-    const float sx = (float)Wf / img_w, sy = (float)Hf / img_h;
-    const int64_t npx = (int64_t)B * M * Hf * Wf;
+    GdetWs w = gdet_carve(d_workspace, npx, (int64_t)4 * B * M * N);
     char what[64];
     snprintf(what, sizeof what, "%s memset", fn);
     CF_TRY(cuda_status(cudaMemsetAsync(w.cnt, 0, (size_t)npx * sizeof(int32_t), st), what));
     const dim3 tg((unsigned)std::min<int64_t>(ceil_div64(N, 256), 148 * 4), (unsigned)B);
-    k_gdet_taps<<<tg, 256, 0, st>>>(src, d_num_points, M, N, Hf, Wf, sx, sy, 0, w.cnt, nullptr, nullptr, nullptr);
+    k_gdet_taps<<<tg, 256, 0, st>>>(src, d_num_points, cams, M, N, total, 0, w.cnt, nullptr, nullptr, nullptr);
     count_launches(1);
     CF_TRY(scan_counts(w.cnt, npx, w.off, w.tiles, st));
-    k_gdet_taps<<<tg, 256, 0, st>>>(src, d_num_points, M, N, Hf, Wf, sx, sy, 1, w.cnt, w.off, w.key, w.wgt);
+    k_gdet_taps<<<tg, 256, 0, st>>>(src, d_num_points, cams, M, N, total, 1, w.cnt, w.off, w.key, w.wgt);
     k_gdet_sum<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>(ceil_div64(npx, 8), 148 * 16)), 256, 0, st>>>(
-        d_gfeat, M, Ci, N, Hf, Wf, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s, sb, sm, sc, sh, sw, d_gimg);
+        d_gfeat, cams, Ci, N, total, npx, w.off, w.key, w.wgt, w.key_s, w.wgt_s);
     count_launches(2);
     return launch_status(fn);
+}
+
+// the B*M gradients of a (B,M,Ci,Hf,Wf) map with camera stride sm: M equal descriptors
+static int point_gather_bwd_det_equal(const char *fn, const float *d_gfeat, float *d_gimg, int64_t sb, int64_t sm, int64_t sc,
+                                      int64_t sh, int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
+                                      const cf::CamSource &src, const int64_t *d_num_points, int32_t N, float img_w,
+                                      float img_h, void *d_workspace, void *stream)
+{
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
+    CF_REQUIRE(d_gimg != nullptr, CF_ERR_ARG, "%s: null pointer", fn);
+    cf_camera_map cams[CF_MAX_CAMERAS];
+    float *gimg[CF_MAX_CAMERAS];
+    cf::equal_cams(cams, d_gimg, sizeof(float), sb, sm, sc, sh, sw, M, Hf, Wf, img_w, img_h);
+    for (int m = 0; m < M; ++m) gimg[m] = d_gimg + m * sm;
+    return point_gather_bwd_det(fn, d_gfeat, gimg, cams, B, M, Ci, src, d_num_points, N, d_workspace, stream);
 }
 }  // namespace
 
 extern "C" size_t cf_point_gather_multi_bwd_det_workspace_bytes(int32_t B, int32_t M, int32_t N, int32_t Hf, int32_t Wf)
 {
     if (B <= 0 || M <= 0 || N <= 0 || Hf <= 0 || Wf <= 0) return 0;
-    return gdet_carve(nullptr, B * M, N, Hf, Wf).bytes;   // B*M maps, up to 4 taps per point in each
+    return gdet_carve(nullptr, (int64_t)B * M * Hf * Wf, (int64_t)4 * B * M * N).bytes;   // B*M maps, up to 4 taps per point in each
 }
 
 extern "C" size_t cf_point_gather_bwd_det_workspace_bytes(int32_t B, int32_t N, int32_t Hf, int32_t Wf)
 {
     return cf_point_gather_multi_bwd_det_workspace_bytes(B, 1, N, Hf, Wf);
+}
+
+extern "C" size_t cf_point_gather_rig_bwd_det_workspace_bytes(int32_t B, int32_t M, int32_t N, const cf_camera_map *h_cams)
+{
+    if (h_cams == nullptr || B <= 0 || M <= 0 || M > CF_MAX_CAMERAS || N <= 0) return 0;
+    for (int m = 0; m < M; ++m)
+        if (h_cams[m].Hf <= 0 || h_cams[m].Wf <= 0) return 0;
+    return gdet_carve(nullptr, gdet_pixels(B, M, h_cams), (int64_t)4 * B * M * N).bytes;
 }
 
 // cf_point_gather_bwd with a fixed summation order: the rig path over B*1 maps
@@ -422,8 +460,9 @@ extern "C" int cf_point_gather_bwd_det(const float *d_gfeat, float *d_gimg, int6
 {
     CF_REQUIRE((d_uv != nullptr) != (h_calib != nullptr), CF_ERR_ARG,
                "cf_point_gather_bwd_det: pass exactly one of d_uv / h_calib");
-    return point_gather_bwd_det("cf_point_gather_bwd_det", d_gfeat, d_gimg, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
-                                cf::camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, d_workspace, stream);
+    return point_gather_bwd_det_equal("cf_point_gather_bwd_det", d_gfeat, d_gimg, sb, sb, sc, sh, sw, B, 1, Ci, Hf, Wf,
+                                      cf::camera_source(d_points, d_uv, h_calib), d_num_points, N, img_w, img_h, d_workspace,
+                                      stream);
 }
 
 // cf_point_gather_multi_bwd with a fixed summation order: the lists of cf_point_gather_bwd_det over the B*M maps
@@ -434,6 +473,17 @@ extern "C" int cf_point_gather_multi_bwd_det(const float *d_gfeat, float *d_gimg
 {
     CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN,
                "cf_point_gather_multi_bwd_det: d_calib must be 4-byte aligned");
-    return point_gather_bwd_det("cf_point_gather_multi_bwd_det", d_gfeat, d_gimg, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf,
-                                cf::rig_source(d_points, d_calib), d_num_points, N, img_w, img_h, d_workspace, stream);
+    return point_gather_bwd_det_equal("cf_point_gather_multi_bwd_det", d_gfeat, d_gimg, sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf,
+                                      cf::rig_source(d_points, d_calib), d_num_points, N, img_w, img_h, d_workspace, stream);
+}
+
+// cf_point_gather_rig_bwd with a fixed summation order: the lists over the concatenated camera planes of the B frames
+extern "C" int cf_point_gather_rig_bwd_det(const float *d_gfeat, float *const *h_gimg, const cf_camera_map *h_cams, int32_t B,
+                                           int32_t M, int32_t Ci, const float *d_points, const float *d_calib,
+                                           const int64_t *d_num_points, int32_t N, void *d_workspace, void *stream)
+{
+    CF_REQUIRE((reinterpret_cast<uintptr_t>(d_calib) & 3u) == 0, CF_ERR_ALIGN,
+               "cf_point_gather_rig_bwd_det: d_calib must be 4-byte aligned");
+    return point_gather_bwd_det("cf_point_gather_rig_bwd_det", d_gfeat, h_gimg, h_cams, B, M, Ci,
+                                cf::rig_source(d_points, d_calib), d_num_points, N, d_workspace, stream);
 }

@@ -109,6 +109,112 @@ static inline CamSource rig_source(const float *d_points, const float *d_calib)
     return s;
 }
 
+// Per-camera constants of the K-3 kernels, passed by value.  Read only at compile-time indices (cam_get, an unrolled select,
+// and stage_cam), which keep the parameter arrays in the constant bank: a dynamically indexed parameter array can be
+// copied to local memory.  `map` is camera m's frame-0 map: the forward's pixel-major rows (sc unused), or the adjoints' fp32 gradient.
+struct RigCams {
+    const void *map[CF_MAX_CAMERAS];
+    int64_t sb[CF_MAX_CAMERAS], sc[CF_MAX_CAMERAS], sh[CF_MAX_CAMERAS], sw[CF_MAX_CAMERAS];  // element strides
+    int32_t Hf[CF_MAX_CAMERAS], Wf[CF_MAX_CAMERAS];
+    float sx[CF_MAX_CAMERAS], sy[CF_MAX_CAMERAS];  // Wf_m / img_w_m, Hf_m / img_h_m
+    int32_t plane[CF_MAX_CAMERAS];  // fixed-order adjoint: first pixel of camera m in a frame's pixel space (prefix of Hf*Wf)
+};
+
+struct Cam {
+    const void *map;
+    int64_t sb, sc, sh, sw;
+    int32_t Hf, Wf, plane;
+    float sx, sy;
+};
+
+// camera m's constants (m need not be known at compile time)
+__device__ __forceinline__ Cam cam_get(const RigCams &r, int m)
+{
+    Cam c{r.map[0], r.sb[0], r.sc[0], r.sh[0], r.sw[0], r.Hf[0], r.Wf[0], r.plane[0], r.sx[0], r.sy[0]};
+#pragma unroll
+    for (int k = 1; k < CF_MAX_CAMERAS; ++k)
+        if (m == k) c = Cam{r.map[k], r.sb[k], r.sc[k], r.sh[k], r.sw[k], r.Hf[k], r.Wf[k], r.plane[k], r.sx[k], r.sy[k]};
+    return c;
+}
+
+// The camera constants of frame b, staged in shared memory by the first M threads of a block: a warp reads camera m's
+// entries at a warp-uniform index (a broadcast), so they take no registers across the loops of the gather kernels.
+struct CamTable {
+    const void *base[CF_MAX_CAMERAS];  // camera m's map of frame b
+    int64_t sc[CF_MAX_CAMERAS], sh[CF_MAX_CAMERAS], sw[CF_MAX_CAMERAS];
+    int32_t Hf[CF_MAX_CAMERAS], Wf[CF_MAX_CAMERAS];
+    float sx[CF_MAX_CAMERAS], sy[CF_MAX_CAMERAS];
+};
+
+template <typename T, int k>
+__device__ __forceinline__ void stage_cam(CamTable &t, const RigCams &r, int b)
+{
+    t.base[k] = static_cast<const T *>(r.map[k]) + b * r.sb[k];
+    t.sc[k] = r.sc[k], t.sh[k] = r.sh[k], t.sw[k] = r.sw[k];
+    t.Hf[k] = r.Hf[k], t.Wf[k] = r.Wf[k];
+    t.sx[k] = r.sx[k], t.sy[k] = r.sy[k];
+}
+
+// thread m < M writes camera m's entries (one branch per camera: a one-camera call runs one short branch), then the block
+// synchronises
+template <typename T>
+__device__ __forceinline__ void stage_cams(CamTable &t, const RigCams &r, int32_t M, int b)
+{
+    static_assert(CF_MAX_CAMERAS == 8, "one case per camera");
+    switch ((int)threadIdx.x < M ? (int)threadIdx.x : -1) {
+    case 0: stage_cam<T, 0>(t, r, b); break;
+    case 1: stage_cam<T, 1>(t, r, b); break;
+    case 2: stage_cam<T, 2>(t, r, b); break;
+    case 3: stage_cam<T, 3>(t, r, b); break;
+    case 4: stage_cam<T, 4>(t, r, b); break;
+    case 5: stage_cam<T, 5>(t, r, b); break;
+    case 6: stage_cam<T, 6>(t, r, b); break;
+    case 7: stage_cam<T, 7>(t, r, b); break;
+    default: break;
+    }
+    __syncthreads();
+}
+
+// host side: the RigCams of M camera descriptors (maps and strides as given; the caller replaces them where it re-lays a
+// map or passes gradients).  `total` receives the pixels of one frame, Sum_m Hf_m * Wf_m.
+static inline RigCams rig_cams(const cf_camera_map *h, int32_t M, int64_t *total)
+{
+    RigCams r{};
+    int64_t acc = 0;
+    for (int m = 0; m < M; ++m) {
+        r.map[m] = h[m].d_map;
+        r.sb[m] = h[m].sb, r.sc[m] = h[m].sc, r.sh[m] = h[m].sh, r.sw[m] = h[m].sw;
+        r.Hf[m] = h[m].Hf, r.Wf[m] = h[m].Wf;
+        r.sx[m] = (float)h[m].Wf / h[m].img_w;
+        r.sy[m] = (float)h[m].Hf / h[m].img_h;
+        r.plane[m] = (int32_t)acc;
+        acc += (int64_t)h[m].Hf * h[m].Wf;
+    }
+    for (int m = M; m < CF_MAX_CAMERAS; ++m) r.plane[m] = INT32_MAX;   // never selected by a pixel of the frame
+    *total = acc;
+    return r;
+}
+
+// host side: the descriptor checks shared by every K-3 entry point -> CF_OK or CF_ERR_ARG (with the text)
+static inline int check_cams(const char *fn, const cf_camera_map *h, int32_t M)
+{
+    CF_REQUIRE(h != nullptr, CF_ERR_ARG, "%s: null camera descriptors", fn);
+    CF_REQUIRE(M >= 1 && M <= CF_MAX_CAMERAS, CF_ERR_ARG, "%s: M=%d cameras, expected 1..%d", fn, M, CF_MAX_CAMERAS);
+    for (int m = 0; m < M; ++m)
+        CF_REQUIRE(h[m].Hf > 0 && h[m].Wf > 0 && h[m].img_w > 0.0f && h[m].img_h > 0.0f, CF_ERR_ARG,
+                   "%s: camera %d: bad extents (Hf=%d, Wf=%d, image %gx%g)", fn, m, h[m].Hf, h[m].Wf, (double)h[m].img_w,
+                   (double)h[m].img_h);
+    return CF_OK;
+}
+
+// M equal descriptors: camera m of a (B,M,Ci,Hf,Wf) map with element strides sb, sm, sc, sh, sw
+static inline void equal_cams(cf_camera_map *h, const void *map, size_t elem, int64_t sb, int64_t sm, int64_t sc, int64_t sh,
+                              int64_t sw, int32_t M, int32_t Hf, int32_t Wf, float img_w, float img_h)
+{
+    for (int m = 0; m < M; ++m)
+        h[m] = cf_camera_map{(const char *)map + m * sm * (int64_t)elem, sb, sc, sh, sw, Hf, Wf, img_w, img_h};
+}
+
 __device__ __forceinline__ float crt_col(float x, float y, float z, float c0, float c3, float c6, float c9)
 {
     return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(x, c0), __fmul_rn(y, c3)), __fmul_rn(z, c6)), c9);

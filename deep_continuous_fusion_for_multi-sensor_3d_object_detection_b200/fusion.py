@@ -21,6 +21,13 @@ MAX_FRAMES_PER_CALL = 64                            # cf_fusion_fwd: frames per 
 _STREAM_POOL = {}   # device index -> side streams, shared by every FrameContext (creating streams per frame is not free)
 
 
+def rig_image_sizes(img_size, M):
+    """M (w, h) image sizes from one pair (every camera) or M pairs."""
+    if np.ndim(img_size) == 1:
+        return [tuple(float(v) for v in img_size)] * M
+    return [tuple(float(v) for v in s) for s in img_size]
+
+
 class FrameContext:
     """Per-batch state shared by every fusion scale: bucketed points and gathered camera features."""
 
@@ -54,7 +61,21 @@ class FrameContext:
     def gather(self, img_feat, calib=None, uv=None, img_size=(640.0, 480.0)):
         """K-3.  A (B,Ci,Hf,Wf) map: one camera, `calib` the reference's (4,3) CRT_tensor or `uv` the projected points.
         A (B,M,Ci,Hf,Wf) map: a rig of M cameras, `calib` a (B,M,4,3) or (M,4,3) CUDA tensor with w > 0 in front
-        (geometry.camera_rig), read on the device; each point gets the mean feature of the cameras that see it."""
+        (geometry.camera_rig), read on the device; each point gets the mean feature of the cameras that see it.
+        A list of M (B,Ci,Hf_m,Wf_m) maps: the same rig with cameras that differ in map and image size; `img_size` is one
+        (w, h) for every camera or M of them."""
+        if isinstance(img_feat, (list, tuple)):
+            if uv is not None:
+                raise ValueError("gather: precomputed uv cannot be used with a camera rig (list of maps); pass the rig's calib")
+            if calib is None:
+                raise ValueError("gather: a camera rig (list of maps) needs calib (B,M,4,3) or (M,4,3)")
+            sizes = rig_image_sizes(img_size, len(img_feat))
+            if torch.is_grad_enabled() and any(isinstance(m, torch.Tensor) and m.requires_grad for m in img_feat):
+                self.feat = _GatherRigFunction.apply(self.points, self.num_points, calib, sizes, *img_feat)
+            else:
+                self.feat, self._gather_ws = ops.point_gather_rig(img_feat, self.points, self.num_points, calib, sizes,
+                                                                  workspace=self._gather_ws)
+            return self.feat
         if isinstance(img_feat, torch.Tensor) and img_feat.dim() == 5:
             if uv is not None:
                 raise ValueError("gather: precomputed uv cannot be used with a camera rig (5-D map); pass the rig's calib")
@@ -216,7 +237,8 @@ class FusionRunner:
     `memory_format=torch.channels_last`: `.bevs` and `.outs` are channels_last maps, fused by the NHWC kernels.
     `cameras=M`: a camera rig.  `.img_feat` is (B,M,Ci,Hf,Wf) and `.calib` a static (B,M,4,3) float32 device buffer
     (initialised from `calib`, an (M,4,3) or (B,M,4,3) rig such as geometry.camera_rig, if given): calibrations written into
-    it between replays take effect without a new capture."""
+    it between replays take effect without a new capture.  With `img_shape` given as M (Ci, Hf_m, Wf_m) tuples (cameras that
+    differ in map size; `img_size` one (w, h) or M of them), `.img_feat` is a list of M static (B,Ci,Hf_m,Wf_m) buffers."""
 
     def __init__(self, layers, grid, batch, max_points, img_shape, bev_shapes, calib=None, img_size=(640.0, 480.0),
                  inplace=True, device=None, dtype=torch.float32, cameras=None, memory_format=torch.contiguous_format):
@@ -226,6 +248,7 @@ class FusionRunner:
         self.num_points = torch.zeros((batch,), dtype=torch.int64, device=dev)
         if dtype not in ops.MAP_DTYPES:
             raise TypeError(f"FusionRunner: dtype must be torch.float32 or torch.bfloat16, got {dtype}")
+        img_feat = None
         if cameras is not None:
             cameras = int(cameras)
             if not 1 <= cameras <= G.MAX_CAMERAS:
@@ -233,8 +256,14 @@ class FusionRunner:
             self.calib = torch.zeros((batch, cameras, 4, 3), dtype=torch.float32, device=dev)
             if calib is not None:
                 self.calib.copy_(torch.as_tensor(calib, dtype=torch.float32, device=dev).expand(batch, cameras, 4, 3))
-            img_shape = (cameras,) + tuple(img_shape)
-        self.img_feat = torch.zeros((batch,) + tuple(img_shape), dtype=dtype, device=dev)
+            if np.ndim(img_shape) == 2:   # one (Ci, Hf_m, Wf_m) per camera
+                if len(img_shape) != cameras:
+                    raise ValueError(f"FusionRunner: {len(img_shape)} image shapes for {cameras} cameras")
+                self.img_size = rig_image_sizes(img_size, cameras)
+                img_feat = [torch.zeros((batch,) + tuple(sh), dtype=dtype, device=dev) for sh in img_shape]
+            else:
+                img_shape = (cameras,) + tuple(img_shape)
+        self.img_feat = torch.zeros((batch,) + tuple(img_shape), dtype=dtype, device=dev) if img_feat is None else img_feat
         self.bevs = [torch.zeros((batch,) + tuple(sh), dtype=dtype, device=dev).contiguous(memory_format=memory_format)
                      for sh in bev_shapes]
         self.outs = None
@@ -317,6 +346,26 @@ class _GatherMultiFunction(torch.autograd.Function):
         gimg = ops.point_gather_multi_bwd(grad_feat, ctx.img_like, points, num_points, calib, img_size=ctx.img_size,
                                           deterministic=det)
         return gimg, None, None, None, None
+
+
+class _GatherRigFunction(torch.autograd.Function):
+    """K-3 of a rig whose cameras differ in map and image size, with its adjoint: one gradient per camera map; the
+    deterministic kernel under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, points, num_points, calib, img_sizes, *maps):
+        feat, _ = ops.point_gather_rig(list(maps), points, num_points, calib, img_sizes)
+        ctx.save_for_backward(points, num_points, calib)
+        ctx.img_sizes, ctx.maps_like = img_sizes, maps
+        return feat
+
+    @staticmethod
+    def backward(ctx, grad_feat):
+        points, num_points, calib = ctx.saved_tensors
+        det = torch.are_deterministic_algorithms_enabled()
+        gimgs = ops.point_gather_rig_bwd(grad_feat, list(ctx.maps_like), points, num_points, calib, ctx.img_sizes,
+                                         deterministic=det)
+        return (None, None, None, None) + tuple(gimgs)
 
 
 class _FusionFunction(torch.autograd.Function):

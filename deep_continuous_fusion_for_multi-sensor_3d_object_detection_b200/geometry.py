@@ -38,6 +38,7 @@ FUSION_DEFAULTS = {
     "fusion_mlp_mode": "fp32",     # "fp32" | "bf16" | "bf16t" (bf16 + bf16 tables, inference only) | "simt" (A12)
     "fusion_bucket_size": 0.5,     # metres, K-1 grid pitch
     "fusion_camera_yaws": None,    # degrees, one per camera of a rig (geometry.camera_rig); None = the single camera
+    "fusion_camera_image_sizes": None,   # [[w, h], ...] one per camera of the rig; None = image_width x image_height each
 }
 
 
@@ -100,8 +101,9 @@ def bucket_grid(config: dict, cell: float | None = None):
     return np.float32(gx0), np.float32(gy0), np.float32(cell), nbx, nby
 
 
-def _projection64(yaw: float = 0.0) -> np.ndarray:
-    """(3,4) float64 projection Cm [R | 0] of the reference camera turned by `yaw` radians about the LiDAR z axis.
+def _projection64(yaw: float = 0.0, width: float = 640.0, height: float = 480.0) -> np.ndarray:
+    """(3,4) float64 projection Cm [R | 0] of the reference camera turned by `yaw` radians about the LiDAR z axis, its
+    intrinsics scaled to a width x height image (fx, cx by width/640, fy, cy by height/480: the same field of view).
 
     The reference builds R with numpy-quaternion's from_euler_angles(v_cam - v_lidar) (:180-188), i.e. the
     Z-Y-Z Euler convention R = Rz(alpha) Ry(beta) Rz(gamma); translation 0; intrinsics from :190-194.  A camera turned by
@@ -119,7 +121,8 @@ def _projection64(yaw: float = 0.0) -> np.ndarray:
     if yaw != 0.0:
         R = R @ rz(-yaw)
     RT = np.concatenate([R, np.zeros((3, 1))], axis=1)
-    Cm = np.array([[268.51188197672957, 0.0, 320.0], [0.0, 268.51188197672957, 240.0], [0.0, 0.0, 1.0]])
+    sx, sy = width / 640.0, height / 480.0
+    Cm = np.array([[268.51188197672957 * sx, 0.0, 320.0 * sx], [0.0, 268.51188197672957 * sy, 240.0 * sy], [0.0, 0.0, 1.0]])
     return Cm @ RT
 
 
@@ -132,13 +135,19 @@ def calibration_crt() -> np.ndarray:
 MAX_CAMERAS = 8   # CF_MAX_CAMERAS of include/cf_b200.h
 
 
-def camera_rig(yaws_deg) -> np.ndarray:
+def camera_rig(yaws_deg, image_sizes=None) -> np.ndarray:
     """(M,4,3) float32 calibrations of a rig of M reference cameras, camera m turned by yaws_deg[m] degrees about the LiDAR
-    z axis (positive toward +y, i.e. to the left), for cf_point_gather_multi: [x y z 1] @ CRT_m = (u*w, v*w, w) with w > 0 in
-    front of the camera.  Computed in float64, rounded once to float32 and negated (exact), so yaw 0 is exactly
-    -calibration_crt() and every camera's (u, v) is the reference camera's (u, v) of the point turned by -yaw."""
+    z axis (positive toward +y, i.e. to the left), for cf_point_gather_multi / cf_point_gather_rig: [x y z 1] @ CRT_m =
+    (u*w, v*w, w) with w > 0 in front of the camera.  Computed in float64, rounded once to float32 and negated (exact), so
+    yaw 0 is exactly -calibration_crt() and every camera's (u, v) is the reference camera's (u, v) of the point turned by
+    -yaw.  `image_sizes`: M (w, h) image sizes; camera m's intrinsics are scaled (in float64) to its image, so it keeps the
+    reference camera's field of view and projects to (u * w/640, v * h/480).  None, or 640 x 480 everywhere, is the
+    reference image."""
     yaws = [float(y) for y in np.asarray(yaws_deg, dtype=np.float64).reshape(-1)]
     if not 1 <= len(yaws) <= MAX_CAMERAS:
         raise ValueError(f"camera_rig: {len(yaws)} cameras, expected 1..{MAX_CAMERAS}")
-    crt = np.stack([_projection64(math.radians(y)).T.astype(np.float32) for y in yaws])
+    sizes = [(640.0, 480.0)] * len(yaws) if image_sizes is None else [tuple(float(v) for v in s) for s in image_sizes]
+    if len(sizes) != len(yaws) or any(len(s) != 2 or not (s[0] > 0 and s[1] > 0) for s in sizes):
+        raise ValueError(f"camera_rig: image_sizes must be {len(yaws)} positive (w, h) pairs, got {image_sizes}")
+    crt = np.stack([_projection64(math.radians(y), w, h).T.astype(np.float32) for y, (w, h) in zip(yaws, sizes)])
     return np.ascontiguousarray(-crt)

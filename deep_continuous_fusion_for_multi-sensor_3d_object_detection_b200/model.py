@@ -277,11 +277,36 @@ class ObjectDetection_DCF(nn.Module):
         yaws = G.fusion_option(config, "fusion_camera_yaws")
         self.cameras = None if yaws is None else len(yaws)
         if yaws is not None:
-            self.register_buffer("rig_calib", torch.from_numpy(G.camera_rig(yaws)), persistent=False)
+            # per-camera image sizes (additive key): each camera's intrinsics are scaled to its own image
+            sizes = G.fusion_option(config, "fusion_camera_image_sizes")
+            if sizes is not None and len(sizes) != len(yaws):
+                raise ValueError(f"fusion_camera_image_sizes: {len(sizes)} sizes for {len(yaws)} cameras")
+            self.camera_sizes = ([(float(config["image_width"]), float(config["image_height"]))] * len(yaws) if sizes is None
+                                 else [(float(w), float(h)) for w, h in sizes])
+            self.register_buffer("rig_calib", torch.from_numpy(G.camera_rig(yaws, sizes)), persistent=False)
+
+    def _camera_stream(self, x_image):
+        """Camera maps of a rig.  (B,M,3,H,W): the one camera stream runs on all B*M images and its channels_last output is
+        viewed as (B,M,Ci,Hf,Wf).  A list of M (B,3,H_m,W_m) images: the stream runs once per distinct image size, on the
+        cameras of that size batched together, and gives the list of M maps (one size: the (B,M,3,H,W) call)."""
+        if isinstance(x_image, torch.Tensor):
+            return self.image_backbone(x_image.flatten(0, 1)).unflatten(0, tuple(x_image.shape[:2]))
+        groups = {}
+        for m, x in enumerate(x_image):
+            groups.setdefault(tuple(x.shape[-2:]), []).append(m)
+        if len(groups) == 1:
+            return self._camera_stream(torch.stack(list(x_image), 1))
+        maps = [None] * len(x_image)
+        for ms in groups.values():
+            f = self.image_backbone(torch.stack([x_image[m] for m in ms], 1).flatten(0, 1)).unflatten(0, (-1, len(ms)))
+            for j, m in enumerate(ms):
+                maps[m] = f[:, j]
+        return maps
 
     def forward(self, x_lidar, x_image, pointcloud_raw=None, num_points_raw=None, projected_loc_uv=None, camera_calib=None):
-        """With `fusion_camera_yaws` in the config, x_image is (B,M,3,H,W) (one image per camera) and `camera_calib`
-        (B,M,4,3) float32, w > 0 in front (geometry.camera_rig), optionally replaces the rig built from the yaws."""
+        """With `fusion_camera_yaws` in the config, x_image is (B,M,3,H,W) (one image per camera) or a list of M (B,3,H_m,W_m)
+        images (cameras of different image sizes, `fusion_camera_image_sizes`), and `camera_calib` (B,M,4,3) float32,
+        w > 0 in front (geometry.camera_rig), optionally replaces the rig built from the yaws."""
         fuse = None
         if self.cameras is None and camera_calib is not None:
             raise ValueError("camera_calib needs a camera rig (config key fusion_camera_yaws)")
@@ -289,7 +314,11 @@ class ObjectDetection_DCF(nn.Module):
             if projected_loc_uv is not None:
                 raise ValueError("projected_loc_uv cannot be used with a camera rig (fusion_camera_yaws): the rig projects "
                                  "every point on the device")
-            if x_image.dim() != 5 or x_image.shape[1] != self.cameras:
+            if isinstance(x_image, (list, tuple)):
+                if len(x_image) != self.cameras or any(not isinstance(x, torch.Tensor) or x.dim() != 4 for x in x_image):
+                    raise ValueError(f"x_image: expected {self.cameras} (B,3,H_m,W_m) images for the {self.cameras}-camera "
+                                     f"rig, got {len(x_image)} entries")
+            elif x_image.dim() != 5 or x_image.shape[1] != self.cameras:
                 raise ValueError(f"x_image: expected (B,{self.cameras},3,H,W) for the {self.cameras}-camera rig, got "
                                  f"{tuple(x_image.shape)}")
         if pointcloud_raw is not None:
@@ -297,13 +326,14 @@ class ObjectDetection_DCF(nn.Module):
                 raise ValueError("num_points_raw is required with pointcloud_raw")
             # K-1 (point bucketing) is launched first, on its side stream: it runs under the camera trunk
             frames = FrameContext(pointcloud_raw.to(x_lidar.device), num_points_raw, self._grid)
-            if self.cameras is None:
-                img_feat = self.image_backbone(x_image)
-            else:   # the one camera stream runs on all B*M images; its channels_last output is viewed as (B,M,Ci,Hf,Wf)
-                img_feat = self.image_backbone(x_image.flatten(0, 1)).unflatten(0, tuple(x_image.shape[:2]))
+            img_feat = self.image_backbone(x_image) if self.cameras is None else self._camera_stream(x_image)
             size = (float(self.config["image_width"]), float(self.config["image_height"]))
             if self.cameras is not None:
-                frames.gather(img_feat, calib=self.rig_calib if camera_calib is None else camera_calib, img_size=size)
+                if isinstance(img_feat, torch.Tensor) and len(set(self.camera_sizes)) > 1:
+                    raise ValueError("x_image: the cameras of fusion_camera_image_sizes differ in size; pass a list of "
+                                     "M (B,3,H_m,W_m) images")
+                frames.gather(img_feat, calib=self.rig_calib if camera_calib is None else camera_calib,
+                              img_size=self.camera_sizes if isinstance(img_feat, list) else self.camera_sizes[0])
             elif projected_loc_uv is not None:
                 frames.gather(img_feat, uv=projected_loc_uv.to(x_lidar.device), img_size=size)
             else:

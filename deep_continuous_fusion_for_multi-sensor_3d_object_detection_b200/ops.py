@@ -227,20 +227,24 @@ def _rig_args(img_feats, points, calib, name):
         raise ValueError(f"{name}: {M} cameras, expected 1..{_lib.MAX_CAMERAS}")
     if Ci % 4:
         raise ValueError(f"{name}: Ci={Ci} must be a multiple of 4")
+    if img_feats.dtype not in MAP_DTYPES:
+        raise TypeError(f"{name}: img_feats: expected dtype torch.float32 or torch.bfloat16, got {img_feats.dtype}")
+    return (B, M, Ci, Hf, Wf, points.shape[1]) + (_rig_calib(points, calib, B, M, name),)
+
+
+def _rig_calib(points, calib, B, M, name):
+    """Checks of a rig's points and (B,M,4,3) / (M,4,3) calibrations -> calib (B,M,4,3), contiguous."""
     if points.dim() != 3 or points.shape[0] != B or points.shape[2] != 3:
         raise ValueError(f"{name}: points must be ({B},N,3), got {tuple(points.shape)}")
     if tuple(calib.shape) not in ((B, M, 4, 3), (M, 4, 3)):
         raise ValueError(f"{name}: calib must be ({B},{M},4,3) or ({M},4,3), got {tuple(calib.shape)}")
     if calib.dtype != torch.float32:
         raise TypeError(f"{name}: calib must be torch.float32, got {calib.dtype}")
-    if img_feats.dtype not in MAP_DTYPES:
-        raise TypeError(f"{name}: img_feats: expected dtype torch.float32 or torch.bfloat16, got {img_feats.dtype}")
     _req(calib, "calib", torch.float32)
     if calib.device != points.device:
         raise ValueError(f"{name}: calib is on {calib.device}, points on {points.device}")
     # (M,4,3): one rig for every frame, broadcast on the device (a copy kernel, no host round trip)
-    calib = calib.expand(B, M, 4, 3).contiguous() if calib.dim() == 3 else calib.contiguous()
-    return B, M, Ci, Hf, Wf, points.shape[1], calib
+    return calib.expand(B, M, 4, 3).contiguous() if calib.dim() == 3 else calib.contiguous()
 
 
 def point_gather_multi(img_feats, points, num_points, calib, img_size=(640.0, 480.0), out=None, workspace=None):
@@ -263,6 +267,91 @@ def point_gather_multi(img_feats, points, num_points, calib, img_size=(640.0, 48
     check(fn(ptr(img_feats), sb, sm, sc, sh, sw, B, M, Ci, Hf, Wf, ptr(points), ptr(calib), ptr(num_points), N,
              float(img_size[0]), float(img_size[1]), ptr(out), ptr(workspace), stream_ptr()), "cf_point_gather_multi")
     return out, workspace
+
+
+def _rig_maps(maps, points, calib, img_sizes, name):
+    """Checks of a rig whose cameras differ in map and image size, made before anything is launched ->
+    (B, M, Ci, N, calib (B,M,4,3), [(w, h)] * M)."""
+    if isinstance(maps, torch.Tensor) or not isinstance(maps, (list, tuple)):
+        raise TypeError(f"{name}: maps must be a list of M (B,Ci,Hf,Wf) tensors, got {type(maps).__name__}")
+    M = len(maps)
+    if not 1 <= M <= _lib.MAX_CAMERAS:
+        raise ValueError(f"{name}: {M} cameras, expected 1..{_lib.MAX_CAMERAS}")
+    for t, what in [(m, f"maps[{i}]") for i, m in enumerate(maps)] + [(points, "points"), (calib, "calib")]:
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"{name}: {what} must be a torch.Tensor, got {type(t).__name__}")
+    for i, m in enumerate(maps):
+        if m.dim() != 4:
+            raise ValueError(f"{name}: maps[{i}] must be (B,Ci,Hf,Wf), got shape {tuple(m.shape)}")
+        if m.dtype not in MAP_DTYPES:
+            raise TypeError(f"{name}: maps[{i}]: expected dtype torch.float32 or torch.bfloat16, got {m.dtype}")
+    B, Ci = maps[0].shape[:2]
+    for i, m in enumerate(maps):
+        if m.shape[0] != B or m.shape[1] != Ci:
+            raise ValueError(f"{name}: maps[{i}] is {tuple(m.shape)}; every camera needs B={B} and Ci={Ci}")
+        if m.dtype != maps[0].dtype:
+            raise TypeError(f"{name}: maps[{i}] is {m.dtype}, maps[0] {maps[0].dtype}: one dtype for every camera")
+        if m.shape[2] < 1 or m.shape[3] < 1:
+            raise ValueError(f"{name}: maps[{i}] has an empty extent {tuple(m.shape)}")
+    if Ci % 4:
+        raise ValueError(f"{name}: Ci={Ci} must be a multiple of 4")
+    sizes = [tuple(float(v) for v in s) for s in img_sizes]
+    if len(sizes) != M or any(len(s) != 2 or not (s[0] > 0 and s[1] > 0) for s in sizes):
+        raise ValueError(f"{name}: img_sizes must be {M} positive (w, h) pairs, got {list(img_sizes)}")
+    calib = _rig_calib(points, calib, B, M, name)
+    return B, M, Ci, points.shape[1], calib, sizes
+
+
+def _camera_maps(tensors, sizes):
+    """The cf_camera_map descriptors of M (B,Ci,Hf,Wf) tensors (host memory, read during the call)."""
+    return (_lib.CameraMap * len(tensors))(*[_lib.CameraMap(t.data_ptr(), *t.stride(), t.shape[2], t.shape[3], w, h)
+                                             for t, (w, h) in zip(tensors, sizes)])
+
+
+def point_gather_rig(maps, points, num_points, calib, img_sizes, out=None, workspace=None):
+    """K-3 for a camera rig whose cameras differ in map and image size (cf_point_gather_rig).  maps: M (B,Ci,Hf_m,Wf_m) maps,
+    one dtype (fp32 or bf16), each NCHW, channels_last (read in place) or any strides; img_sizes: M (w, h) image sizes the
+    calibrations project into; points (B,N,3); calib (B,M,4,3) or (M,4,3) float32 CUDA tensor, w > 0 in front of the camera
+    -> feat (B,N,Ci) fp32: the mean over the cameras that see each point of their bilinear features (zero where none does)."""
+    lib = load()
+    B, M, Ci, N, calib, sizes = _rig_maps(maps, points, calib, img_sizes, "point_gather_rig")
+    _req(num_points, "num_points", torch.int64, 1)
+    for i, m in enumerate(maps):
+        _map(m, f"maps[{i}]")
+    points = _contig(points, "points", torch.float32, 3)
+    cams = _camera_maps(maps, sizes)
+    if out is None:
+        out = torch.empty((B, N, Ci), dtype=torch.float32, device=points.device)
+    need = lib.cf_gather_rig_workspace_bytes(B, M, Ci, cams)
+    if need and (workspace is None or workspace.numel() < need):
+        workspace = torch.empty((need,), dtype=torch.uint8, device=points.device)
+    fn = lib.cf_point_gather_rig_bf16 if maps[0].dtype == torch.bfloat16 else lib.cf_point_gather_rig
+    check(fn(cams, B, M, Ci, ptr(points), ptr(calib), ptr(num_points), N, ptr(out), ptr(workspace), stream_ptr()),
+          "cf_point_gather_rig")
+    return out, workspace
+
+
+def point_gather_rig_bwd(grad_feat, maps_like, points, num_points, calib, img_sizes, deterministic=False):
+    """Adjoint of point_gather_rig: one gradient per camera map (shape, dtype and memory format of maps_like[m]).
+    `deterministic`: each pixel sums its (point, tap) contributions in a fixed order (cf_point_gather_rig_bwd_det).
+    A bf16 map: its taps are summed into an fp32 map, which is rounded to bf16 once at the end."""
+    lib = load()
+    B, M, Ci, N, calib, sizes = _rig_maps(maps_like, points, calib, img_sizes, "point_gather_rig_bwd")
+    _req(num_points, "num_points", torch.int64, 1)
+    grad_feat = _contig(grad_feat, "grad_feat", torch.float32, 3)
+    if tuple(grad_feat.shape) != (B, N, Ci):
+        raise ValueError(f"point_gather_rig_bwd: grad_feat must be {(B, N, Ci)}, got {tuple(grad_feat.shape)}")
+    points = _contig(points, "points", torch.float32, 3)
+    gimgs = [torch.zeros_like(m, dtype=torch.float32) for m in maps_like]
+    cams = _camera_maps(gimgs, sizes)
+    gptrs = (C.c_void_p * M)(*[g.data_ptr() for g in gimgs])
+    args = (ptr(grad_feat), gptrs, cams, B, M, Ci, ptr(points), ptr(calib), ptr(num_points), N)
+    if deterministic:
+        ws = _scratch(lib.cf_point_gather_rig_bwd_det_workspace_bytes(B, M, N, cams), grad_feat.device)
+        check(lib.cf_point_gather_rig_bwd_det(*args, ptr(ws), stream_ptr()), "cf_point_gather_rig_bwd_det")
+    else:
+        check(lib.cf_point_gather_rig_bwd(*args, stream_ptr()), "cf_point_gather_rig_bwd")
+    return [g.to(m.dtype) for g, m in zip(gimgs, maps_like)]
 
 
 class PackedWeights:

@@ -140,8 +140,31 @@ CF_API int cf_point_gather_bf16(const void *d_img_feat, int64_t sb, int64_t sc, 
  *   n_vis == 1 everywhere gives the bits of cf_point_gather_bwd_det.  The order depends on the inputs only (not on the SM
  *   count).  Workspace cf_point_gather_multi_bwd_det_workspace_bytes(B, M, N, Hf, Wf); 4*B*M*N, B*M*Hf*Wf < 2^31.
  * None of these synchronises with the host: all are capturable in a CUDA graph.
+ *
+ * cf_point_gather_rig*: the same rig with cameras that differ in map extent and image size.  Camera m is described by
+ * h_cams[m], a HOST array of M descriptors read during the call (like h_calib: calls stay capturable):
+ *   d_map        logical (B,Ci,Hf,Wf) map of camera m with ELEMENT strides sb, sc, sh, sw (the backward ignores it)
+ *   Hf, Wf       its extent;  img_w, img_h  the image size its calibration projects into
+ * Shared by all cameras: Ci, the map dtype (cf_point_gather_rig: fp32, cf_point_gather_rig_bf16: bf16) and the (B,M,4,3)
+ * device calibrations.  Camera m uses sx_m = Wf_m / img_w_m, sy_m = Hf_m / img_h_m, and its own map for the visibility and
+ * tap tests; the mean over the visible cameras and the adjoint products are those of cf_point_gather_multi*.  M equal
+ * descriptors give the bits of cf_point_gather_multi* (which, like cf_point_gather*, runs this path).
+ *   Forward      sc == 1 cameras (channels_last) are read in place, every pixel 16-byte (bf16: 8-byte) aligned; the
+ *                others are re-laid pixel-major into d_workspace, cf_gather_rig_workspace_bytes(B, M, Ci, h_cams) bytes.
+ *   Backward     h_gimg[m], M DEVICE pointers: camera m's fp32 gradient, logical (B,Ci,Hf_m,Wf_m) with the element
+ *                strides of h_cams[m]; the taps are ACCUMULATED into it.  _bwd: float atomics.  _bwd_det: fixed order; its
+ *                pixel space is the concatenation over (b, m) of the planes Hf_m*Wf_m, each pixel's list in ascending
+ *                (point, tap); workspace cf_point_gather_rig_bwd_det_workspace_bytes(B, M, N, h_cams);
+ *                4*B*M*N < 2^31 and B*Sum_m Hf_m*Wf_m < 2^31.
+ *   1 <= M <= CF_MAX_CAMERAS, B*M <= 65535, Ci % 4 == 0; every check runs before anything is launched.
  * ------------------------------------------------------------------------------------------- */
 #define CF_MAX_CAMERAS 8
+typedef struct cf_camera_map {
+    const void *d_map;          /* logical (B,Ci,Hf,Wf) map of this camera, ELEMENT strides sb, sc, sh, sw */
+    int64_t sb, sc, sh, sw;
+    int32_t Hf, Wf;
+    float img_w, img_h;         /* image size the calibration projects into */
+} cf_camera_map;
 CF_API size_t cf_gather_multi_workspace_bytes(int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, int64_t sc);
 CF_API int cf_point_gather_multi(const float *d_img_feat, int64_t sb, int64_t sm, int64_t sc, int64_t sh, int64_t sw,
                                  int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf, const float *d_points,
@@ -160,6 +183,20 @@ CF_API int cf_point_gather_multi_bwd_det(const float *d_gfeat, float *d_gimg, in
                                          int64_t sw, int32_t B, int32_t M, int32_t Ci, int32_t Hf, int32_t Wf,
                                          const float *d_points, const float *d_calib, const int64_t *d_num_points,
                                          int32_t N, float img_w, float img_h, void *d_workspace, void *stream);
+CF_API size_t cf_gather_rig_workspace_bytes(int32_t B, int32_t M, int32_t Ci, const cf_camera_map *h_cams);
+CF_API int cf_point_gather_rig(const cf_camera_map *h_cams, int32_t B, int32_t M, int32_t Ci, const float *d_points,
+                               const float *d_calib, const int64_t *d_num_points, int32_t N, float *d_feat, void *d_workspace,
+                               void *stream);
+CF_API int cf_point_gather_rig_bf16(const cf_camera_map *h_cams, int32_t B, int32_t M, int32_t Ci, const float *d_points,
+                                    const float *d_calib, const int64_t *d_num_points, int32_t N, float *d_feat,
+                                    void *d_workspace, void *stream);
+CF_API int cf_point_gather_rig_bwd(const float *d_gfeat, float *const *h_gimg, const cf_camera_map *h_cams, int32_t B,
+                                   int32_t M, int32_t Ci, const float *d_points, const float *d_calib,
+                                   const int64_t *d_num_points, int32_t N, void *stream);
+CF_API size_t cf_point_gather_rig_bwd_det_workspace_bytes(int32_t B, int32_t M, int32_t N, const cf_camera_map *h_cams);
+CF_API int cf_point_gather_rig_bwd_det(const float *d_gfeat, float *const *h_gimg, const cf_camera_map *h_cams, int32_t B,
+                                       int32_t M, int32_t Ci, const float *d_points, const float *d_calib,
+                                       const int64_t *d_num_points, int32_t N, void *d_workspace, void *stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K-4a per-point half of MLP layer 1 (exact factorisation of Appendix A8/A9):

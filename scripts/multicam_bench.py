@@ -4,6 +4,7 @@ frame, 128-channel stride-4 camera maps (120 x 160) of 640 x 480 images.
 Reports, as JSON lines (CUDA events; the L2 is overwritten before every timed call, so maps are read from HBM):
   * gather forward, atomic backward and fixed-order backward for M = 1, 3 and 6 cameras (channels_last maps, as the
     model's camera stream emits them) on a LiDAR sweep through the range filter only;
+  * the same for a 5-camera rig whose cameras differ in image and map size (cf_point_gather_rig, Waymo-like sizes);
   * the rig path at M = 1 (calib = -CRT) against cf_point_gather on the standard camera-filtered points, NCHW and
     channels_last (the outputs are checked bit for bit);
   * one fuse_scales step (bucket, gather, tables, KNN, fused layer of the five scales) with 3 cameras against the single
@@ -99,6 +100,21 @@ def main():
         rec["bwd_deterministic"] = timed(lambda: ops.point_gather_multi_bwd(g, img, pts, cnt, rig, img_size=size,
                                                                            deterministic=True))
         emit(rec)
+
+    # a rig whose cameras differ in size (cf_point_gather_rig): Waymo-like, three 1920x1280 front cameras and two 1920x886
+    # side cameras, stride-4 maps (320 x 480 and 222 x 480), channels_last as the camera stream emits them
+    het_yaws, het_sizes = (0.0, 45.0, -45.0, 90.0, -90.0), [(1920.0, 1280.0)] * 3 + [(1920.0, 886.0)] * 2
+    maps = [torch.randn((B, Ci, int(h) // 4 + (int(h) % 4 > 0), int(w) // 4), device="cuda", generator=gen).contiguous(
+        memory_format=torch.channels_last) for w, h in het_sizes]
+    rig = torch.from_numpy(G.camera_rig(het_yaws, het_sizes)).cuda().expand(B, 5, 4, 3).contiguous()
+    feat, ws = ops.point_gather_rig(maps, pts, cnt, rig, het_sizes)
+    g = torch.randn(feat.shape, device="cuda", generator=gen)
+    rec = dict(what="gather_rig_mixed_sizes", cameras=5, yaws=het_yaws, image_sizes=het_sizes,
+               maps=[list(m.shape[2:]) for m in maps], batch=B, points=counts.tolist(), c_img=Ci, layout="channels_last")
+    rec["fwd"] = timed(lambda: ops.point_gather_rig(maps, pts, cnt, rig, het_sizes, out=feat, workspace=ws))
+    rec["bwd_atomic"] = timed(lambda: ops.point_gather_rig_bwd(g, maps, pts, cnt, rig, het_sizes))
+    rec["bwd_deterministic"] = timed(lambda: ops.point_gather_rig_bwd(g, maps, pts, cnt, rig, het_sizes, deterministic=True))
+    emit(rec)
 
     # M = 1 against the single-camera kernel, on the standard (camera-filtered) points
     spts, scnt = torch.from_numpy(wl["points"]).cuda(), torch.from_numpy(wl["num_points"]).cuda()
